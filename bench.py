@@ -6,7 +6,7 @@ Workload (per GPU): 1024 concurrent self-play games, two trees per game as in th
 Boltzmann(1.0) for the first 30 plies then Best), random-init residual policy/value network.
 One "step" = one ply on every game = 1024 positions = 1024 x 800 simulations.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun: one process per GPU, per-GPU game pools, NO data-path collective
 (games are independent units -> weak scaling); only the timing barrier / max-over-ranks uses NCCL.
@@ -173,7 +173,7 @@ def cpu_selfplay_sample(steps: int, warmup: int, trees: int = CPU_SAMPLE_TREES):
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    steps = max(1, args.steps)
+    steps = args.steps
     warm = max(0, args.warmup)  # the same W untimed plies as the repo arm is asked for
     r = cpu_selfplay_sample(steps, warm)
     value = r["sims"] / r["seconds"]
@@ -220,6 +220,26 @@ def workload_config(n_gpus, games=GAMES_PER_GPU):
             "l2": "no flush: each network launch streams a 333 MB fc0 input (>> 126 MB L2) and ~2.9 GB of tree records are resident"}
 
 
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, games):
+    """Writes each [games, ...] array as out_dir/<name>.npy in float32, with game_index.npy naming the games kept. Above
+    DUMP_LIMIT_BYTES in all, a fixed seeded sample of games is kept, so two builds run with the same arguments write
+    the same games."""
+    import numpy as np
+
+    per_game = 8 + sum(4 * (a.size // games) for a in arrays.values())  # float32 rows + the float64 index
+    budget = DUMP_LIMIT_BYTES - 128 * (len(arrays) + 1)  # less one .npy header per file
+    idx = np.arange(games)
+    if games * per_game > budget:
+        idx = np.sort(np.random.default_rng(0).choice(games, budget // per_game, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "game_index.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a[idx], dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -229,7 +249,14 @@ def main():
     ap.add_argument("--games", type=int, default=GAMES_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--gather", action="store_true", help="N > 1: also merge every rank's streamed transitions on rank 0 (BASELINE configs[3]'s host replay buffer) and report the merge time")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the run, write what the last timed ply returned to its caller "
+                    "(rank 0's games) as DIR/<name>.npy in float32: selfplay_* from the device-resident arm, e2e_* from the "
+                    "C-ABI arm; the inputs are seeded, so two builds run with the same arguments can be compared array for array")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; the reference arm has none")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -255,7 +282,7 @@ def main():
 
     games = args.games
     warm = max(3, args.warmup)
-    steps = max(1, args.steps)
+    steps = args.steps
     ctx = omk.Context(device=local_rank, capacity_envs=4, capacity_trees=2 * games, capacity_nodes=CAP_NODES, seed=sharding.rank_seed(1000, rank))
     ctx.net_init_random(0)  # same random-init weights on every rank (no broadcast needed)
     ctx.selfplay_begin(games, COUNT, BATCH, EPS, ALPHA, TEMP, TEMP_THRESHOLD, omk.EVAL_NET)
@@ -330,6 +357,7 @@ def main():
             ctx.pool_new_games(ids=fresh, evaluator=omk.EVAL_NET)
     barrier()
     e2e_s = time.perf_counter() - t0
+    e2e_last = {"e2e_actions": acts, "e2e_policy": pol, "e2e_status": st}  # the last timed ply's results, as the caller got them
     h2d1, d2h1 = ctx.transfer_bytes
     h2d, d2h = h2d1 - h2d0, d2h1 - d2h0
 
@@ -460,6 +488,9 @@ def main():
                 "value": r["sims"] / r["seconds"], "unit": "simulations/s", "cores": r["cores"], "kind": "port",
                 "sample": f"{r['trees']} concurrent trees x 4 plies x {COUNT} sims/move; C oracle (pthreads over trees) + "
                           "PyTorch-CPU fp32 network standing in for TensorFlow-CPU"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"selfplay_boards": t_boards[-1], "selfplay_policy": t_policy[-1],
+                                             "selfplay_status": t_status[-1], "selfplay_actions": t_actions[-1], **e2e_last}, games)
         print(json.dumps(line), flush=True)
     ctx.close()
     if dist:
