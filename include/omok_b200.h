@@ -274,6 +274,36 @@ OMK_API int32_t omk_selfplay_begin(omk_ctx *ctx, const omk_selfplay_config *cfg)
 OMK_API int32_t omk_selfplay_run(omk_ctx *ctx, int32_t plies, int32_t profile, uint8_t *out_boards, float *out_policy,
                          int8_t *out_status, int32_t *out_actions, omk_selfplay_stats *stats);
 
+/* ---------------------------------------------------------------- replay memory
+ * The trainer's replay memory (src/trainer.rs:27,206-352) kept on the device and fed by the self-play driver, so that
+ * the training phase samples, encodes and steps without the host.  It holds the rows trainer.ReplayMemory would hold if
+ * fed by split_episodes one ply at a time: episodes in (ply of the final move, game id) order; per episode the T original
+ * transitions (board before the move, turn from the stone counts, visit policy, z), then the five symmetric copies of each
+ * transition in the order rotate_90, rotate_180, rotate_270, flip_horizontal, flip_vertical; z = 1 (win of the last
+ * mover) or 0 (draw) at the last ply, negated at each earlier one (a draw alternates +0.0 / -0.0).  Beyond the capacity
+ * the oldest rows are dropped after each episode.  Rows are addressed by LOGICAL index: 0 is the oldest row.
+ * Unfinished games are staged on the device across omk_selfplay_run calls; omk_selfplay_begin restarts every game and
+ * drops them.  Storage: 410 bytes per row (246 MB at 600 000 rows) + 32.8 KB of staging per game.                      */
+/* Empty the replay memory and (re)size it to `capacity` rows; 0 frees it and the driver stops feeding it.  The self-play
+ * driver feeds a replay memory that exists at omk_selfplay_begin; creating one (capacity > 0 from 0) while a driver is
+ * active is OMK_ERR_STATE.  Emptying one while a driver is active keeps the games' staged tails.                        */
+OMK_API int32_t omk_replay_reset(omk_ctx *ctx, int64_t capacity);
+/* rows held, rows added since the last reset (dropped ones included), episodes added since the last reset; as of the end
+ * of the last omk_selfplay_run (any may be NULL) */
+OMK_API int32_t omk_replay_info(omk_ctx *ctx, int64_t *out_len, int64_t *out_rows_added, int64_t *out_episodes);
+/* rows[n] = logical indices (OMK_ERR_INVALID outside [0, len)); boards[n*81], turns[n], policy[n*81], z[n] (any may be NULL) */
+OMK_API int32_t omk_replay_get(omk_ctx *ctx, const int64_t *rows, int32_t n, uint8_t *out_boards, uint8_t *out_turns,
+                       float *out_policy, float *out_z);
+/* `steps` gradient steps, each omk_train_step's sequence (forward, loss, backward, all-reduce of an attached communicator,
+ * Adadelta, reporting forward) on a minibatch of m = min(n, len) rows drawn from the replay memory and encoded as
+ * encode_nn_input(board, turn) in Player mode.  Step s draws its rows with Floyd's sample without replacement on the
+ * specified random stream (mix64(seed ^ K), stream = (uint32_t)(first_step + s), counter from 0) (DESIGN.md 4).
+ * out_losses[steps*3] = {p_loss, v_loss, loss} after each update; out_rows[steps*n] (may be NULL) = the logical rows
+ * each step used, in draw order, -1 past m.  No minibatch crosses the host; one synchronisation for the whole call.
+ * An absent or empty replay memory is OMK_ERR_STATE.                                                                     */
+OMK_API int32_t omk_train_replay(omk_ctx *ctx, uint64_t seed, int64_t first_step, int32_t steps, int32_t n, float *out_losses,
+                         int64_t *out_rows);
+
 #ifdef __cplusplus
 }
 #endif

@@ -140,6 +140,10 @@ def load_library():
     L.omk_pool_tree_info.argtypes = [vp, i32, vp, vp]
     L.omk_selfplay_begin.argtypes = [vp, P(SelfPlayConfig)]
     L.omk_selfplay_run.argtypes = [vp, i32, i32, vp, vp, vp, vp, P(SelfPlayStats)]
+    L.omk_replay_reset.argtypes = [vp, i64]
+    L.omk_replay_info.argtypes = [vp, P(i64), P(i64), P(i64)]
+    L.omk_replay_get.argtypes = [vp, vp, i32, vp, vp, vp, vp]
+    L.omk_train_replay.argtypes = [vp, u64, i64, i32, i32, vp, vp]
     for name in declared_symbols():
         fn = getattr(L, name)  # raises AttributeError if the library lacks a declared symbol
         if name not in ("omk_last_error", "omk_ctx_stream", "omk_ctx_launch_count"):
@@ -462,3 +466,36 @@ class Context:
         self._check(self.L.omk_selfplay_run(self.h, plies, int(profile), _ptr(boards), _ptr(policy), _ptr(status),
                                             _ptr(actions), C.byref(stats)))
         return stats, boards, policy, status, actions
+
+    # ---- replay memory on the device ----
+    def replay_reset(self, capacity: int):
+        """Empty the device replay memory and size it to `capacity` rows (0 frees it).  Create it before
+        `selfplay_begin`: the driver feeds the replay memory that exists when it starts."""
+        self._check(self.L.omk_replay_reset(self.h, int(capacity)))
+
+    def replay_info(self):
+        """(rows held, rows added since the last reset, episodes added since the last reset)."""
+        a, b, e = C.c_int64(), C.c_int64(), C.c_int64()
+        self._check(self.L.omk_replay_info(self.h, C.byref(a), C.byref(b), C.byref(e)))
+        return int(a.value), int(b.value), int(e.value)
+
+    def replay_get(self, rows):
+        """Rows by logical index (0 = oldest): (boards [n,81] u8, turns [n] u8, policies [n,81] f32, z [n] f32)."""
+        rows = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+        n = rows.size
+        boards = np.zeros((n, CELLS), dtype=np.uint8)
+        turns = np.zeros(n, dtype=np.uint8)
+        policy = np.zeros((n, CELLS), dtype=np.float32)
+        z = np.zeros(n, dtype=np.float32)
+        self._check(self.L.omk_replay_get(self.h, _ptr(rows), n, _ptr(boards), _ptr(turns), _ptr(policy), _ptr(z)))
+        return boards, turns, policy, z
+
+    def train_replay(self, seed: int, first_step: int, steps: int, n: int, want_rows: bool = False):
+        """`steps` trainer steps on minibatches of min(n, len) rows sampled from the device replay memory (step s on
+        sampler stream first_step + s).  Returns losses [steps, 3] ({p_loss, v_loss, loss} after each update) and, with
+        `want_rows`, the logical rows of each step [steps, n] (-1 past the minibatch size)."""
+        losses = np.zeros((steps, 3), dtype=np.float32)
+        rows = np.zeros((steps, n), dtype=np.int64) if want_rows else None
+        self._check(self.L.omk_train_replay(self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step), int(steps), int(n),
+                                            _ptr(losses), _ptr(rows)))
+        return (losses, rows) if want_rows else losses

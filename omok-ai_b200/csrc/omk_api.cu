@@ -278,6 +278,23 @@ static int32_t check_evaluator(omk_ctx *c, int evaluator) {
     return OMK_OK;
 }
 
+// ------------------------------------------------------------------ replay memory (storage)
+static void replay_free_staging(omk_ctx *c) {
+    Replay &r = c->rp;
+    if (r.stream) cudaStreamSynchronize(r.stream);
+    cudaFree(r.stage_boards); cudaFree(r.stage_pi); cudaFree(r.stage_len);
+    r.stage_boards = nullptr; r.stage_pi = nullptr; r.stage_len = nullptr;
+    r.stage_games = 0;
+}
+static void replay_free(omk_ctx *c) {
+    Replay &r = c->rp;
+    replay_free_staging(c);
+    cudaFree(r.ring.boards); cudaFree(r.ring.turns); cudaFree(r.ring.pi); cudaFree(r.ring.z); cudaFree(r.counters);
+    r.ring = ReplayRing{};
+    r.counters = nullptr;
+    r.added = r.len = r.episodes = 0;
+}
+
 // ------------------------------------------------------------------ context
 extern "C" int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t capacity_trees, int32_t capacity_nodes,
                                   uint64_t seed, omk_ctx **out) {
@@ -383,6 +400,11 @@ extern "C" int32_t omk_ctx_destroy(omk_ctx *c) {
     }
     cudaFree(c->sp_ring_dev);
     if (c->sp_ring_host) cudaFreeHost(c->sp_ring_host);
+    replay_free(c);
+    if (c->rp.stream) {
+        cudaEventDestroy(c->rp.ev_commit);
+        cudaStreamDestroy(c->rp.stream);
+    }
     for (cudaEvent_t e : c->prof_pool) cudaEventDestroy(e);
     cudaEventDestroy(c->ev0);
     cudaEventDestroy(c->ev1);
@@ -1081,6 +1103,22 @@ extern "C" int32_t omk_selfplay_begin(omk_ctx *c, const omk_selfplay_config *cfg
             CK(cudaEventCreateWithFlags(&c->sp_ev_copy[i], cudaEventDisableTiming));
         }
     }
+    // a replay memory that exists now is fed by this driver: staging for every game (the restart below drops the tails
+    // of the previous driver's games, as omk_selfplay_begin restarts every game)
+    replay_free_staging(c);
+    if (c->rp.ring.cap > 0) {
+        Replay &r = c->rp;
+        if (!r.stream) {
+            CK(cudaStreamCreateWithFlags(&r.stream, cudaStreamNonBlocking));
+            CK(cudaEventCreateWithFlags(&r.ev_commit, cudaEventDisableTiming));
+        }
+        const size_t cells = (size_t)n * kCells * kCells;  // 81 plies of 81 cells per game
+        CK(cudaMalloc(&r.stage_boards, cells));
+        CK(cudaMalloc(&r.stage_pi, cells * sizeof(float)));
+        CK(cudaMalloc(&r.stage_len, sizeof(int32_t) * (size_t)n));
+        CK(cudaMemsetAsync(r.stage_len, 0, sizeof(int32_t) * (size_t)n, c->stream));
+        r.stage_games = n;
+    }
     // Agent::new for all 2n trees (stream id = tree id); then cache the root's raw policy for restarts:
     // evaluating the empty board is deterministic, so reusing it is bit-identical to evaluating it again
     launch_reset_requests(c);
@@ -1121,6 +1159,11 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     const size_t tot = (size_t)plies * (size_t)n;
     const SpSlot slot = sp_slot_layout(n);
     const bool want_out = out_boards || out_policy || out_status || out_actions;
+    // Replay feed (when a replay memory existed at omk_selfplay_begin): each lane stages its recorded ply per game; one
+    // commit per ply on the replay stream, behind both lanes' record events, turns the episodes that ended into rows.  A
+    // restarted game stages ply 0 over the finished episode, so each lane waits for the previous ply's commit before its
+    // staging kernel -- one event wait per lane and ply, outside the search rounds.
+    const bool feed = c->rp.stage_games == n && c->rp.ring.cap > 0;
     size_t d2h = 0;
     auto dev_slot = [&](int ply) { return c->sp_ring_dev + (size_t)(ply % kRing) * slot.bytes; };
     auto drain = [&](int ply) -> int32_t {  // pinned slot of `ply` -> the caller's arrays
@@ -1194,6 +1237,10 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
             launch_sample(c, mover + g0, nl, modes + g0, temps + g0, actions + g0, policy_out + (size_t)g0 * kCells, nullptr);
             launch_sp_record(c, nl, mover + g0, actions + g0, policy_out + (size_t)g0 * kCells, d_boards + row * kCells,
                              d_policy + row * kCells, d_actions + row);
+            if (feed) {
+                CK(cudaStreamWaitEvent(c->stream, c->rp.ev_commit, 0));
+                launch_rp_stage(c, g0, nl, d_boards + row * kCells, d_policy + row * kCells);
+            }
             launch_play(c, mover + g0, actions + g0, nl, status + g0);
             launch_reset_requests(c);
             launch_ensure_prepare(c, other + g0, actions + g0, nl);
@@ -1208,7 +1255,12 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
             launch_new_games(c, other + g0, nl, nullptr, status + g0, root_policy);
             launch_sp_advance(c, g0, nl, status, counters);
             span_end(sp);
-            if (want_out) CK(cudaEventRecord(c->sp_ev_rec[ply % kRing][l], c->stream));
+            if (want_out || feed) CK(cudaEventRecord(c->sp_ev_rec[ply % kRing][l], c->stream));
+        }
+        if (feed) {  // this ply's finished episodes -> replay rows, behind both lanes' status of the ply
+            for (int l = 0; l < lanes; ++l) CK(cudaStreamWaitEvent(c->rp.stream, c->sp_ev_rec[ply % kRing][l], 0));
+            launch_rp_commit(c, n, d_status);
+            CK(cudaEventRecord(c->rp.ev_commit, c->rp.stream));
         }
         if (want_out) {  // this ply's slice -> pinned host mirror, behind both lanes' recording kernels
             for (int l = 0; l < lanes; ++l) CK(cudaStreamWaitEvent(c->sp_copy_stream, c->sp_ev_rec[ply % kRing][l], 0));
@@ -1227,6 +1279,7 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     }
     if (lanes == 2) lanes_join(c);
     launch_reset_requests(c);  // folds the last round's request count into the evaluator total
+    if (feed) CK(cudaStreamWaitEvent(c->stream, c->rp.ev_commit, 0));  // every later reader of the replay is behind the last commit
     CK(cudaEventRecord(c->ev1, c->stream));
     if (want_out)
         for (int ply = plies > kRing ? plies - kRing : 0; ply < plies; ++ply) {  // the slots still in flight
@@ -1235,7 +1288,14 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
         }
     CK(copy_d2h(c, h_after, c->dev_sims, sizeof h_after, c->stream));
     CK(copy_d2h(c, &h_fin1, counters, sizeof h_fin1, c->stream));
-    int32_t rc = check_device_error(c);
+    ReplayCounters rp_ctr{};
+    if (feed) CK(copy_d2h(c, &rp_ctr, c->rp.counters, sizeof rp_ctr, c->stream));
+    int32_t rc = check_device_error(c);  // (synchronises the stream)
+    if (feed) {
+        c->rp.added = rp_ctr.added;
+        c->rp.len = rp_ctr.len;
+        c->rp.episodes = rp_ctr.episodes;
+    }
     if (stats) {
         memset(stats, 0, sizeof *stats);
         stats->simulations = (int64_t)(h_after[0] - h_before[0]);
@@ -1259,4 +1319,116 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     c->prof_spans.clear();
     c->prof_level = 0;
     return rc;
+}
+
+// ------------------------------------------------------------------ replay memory (src/trainer.rs:27,206-352 on the device)
+extern "C" int32_t omk_replay_reset(omk_ctx *c, int64_t capacity) {
+    CK(cudaSetDevice(c->device));
+    if (capacity < 0 || capacity > 0x7FFFFFFFLL) return fail(OMK_ERR_INVALID, "capacity must be in [0, 2^31)");
+    Replay &r = c->rp;
+    if (capacity > 0 && r.ring.cap == 0 && c->sp_active)
+        return fail(OMK_ERR_STATE, "a replay memory is fed by the self-play driver only if it exists at omk_selfplay_begin: create it first");
+    CK(cudaStreamSynchronize(c->stream));
+    if (capacity == 0) {
+        replay_free(c);  // the driver stops feeding
+        return OMK_OK;
+    }
+    if (capacity != r.ring.cap) {
+        if (r.stream) CK(cudaStreamSynchronize(r.stream));
+        cudaFree(r.ring.boards); cudaFree(r.ring.turns); cudaFree(r.ring.pi); cudaFree(r.ring.z);
+        r.ring = ReplayRing{};
+        const size_t cap = (size_t)capacity;
+        CK(cudaMalloc(&r.ring.boards, cap * kCells));
+        CK(cudaMalloc(&r.ring.turns, cap));
+        CK(cudaMalloc(&r.ring.pi, cap * kCells * sizeof(float)));
+        CK(cudaMalloc(&r.ring.z, cap * sizeof(float)));
+        r.ring.cap = capacity;
+    }
+    if (!r.counters) CK(cudaMalloc(&r.counters, sizeof(ReplayCounters)));
+    CK(cudaMemsetAsync(r.counters, 0, sizeof(ReplayCounters), c->stream));  // the staged tails of a running driver stay
+    CK(cudaStreamSynchronize(c->stream));
+    r.added = r.len = r.episodes = 0;
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_replay_info(omk_ctx *c, int64_t *out_len, int64_t *out_rows_added, int64_t *out_episodes) {
+    if (out_len) *out_len = c->rp.len;
+    if (out_rows_added) *out_rows_added = c->rp.added;
+    if (out_episodes) *out_episodes = c->rp.episodes;
+    return OMK_OK;
+}
+
+// host row list -> device (validated against the current length)
+static int32_t stage_rows(omk_ctx *c, const int64_t *rows, int32_t n, int64_t **out) {
+    for (int32_t i = 0; i < n; ++i)
+        if (rows[i] < 0 || rows[i] >= c->rp.len)
+            return fail(OMK_ERR_INVALID, "row " + std::to_string(rows[i]) + " outside the replay's " + std::to_string(c->rp.len) + " rows");
+    SCRATCH(0, (size_t)n, *out);
+    CK(copy_h2d(c, *out, rows, sizeof(int64_t) * (size_t)n, c->stream));
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_replay_get(omk_ctx *c, const int64_t *rows, int32_t n, uint8_t *out_boards, uint8_t *out_turns,
+                                  float *out_policy, float *out_z) {
+    CK(cudaSetDevice(c->device));
+    if (n < 0 || (n > 0 && !rows)) return fail(OMK_ERR_INVALID, "bad row list");
+    if (c->rp.ring.cap == 0) return fail(OMK_ERR_STATE, "no replay memory (omk_replay_reset)");
+    if (n == 0) return OMK_OK;
+    int64_t *d_rows = nullptr;
+    int32_t rc = stage_rows(c, rows, n, &d_rows);
+    if (rc) return rc;
+    const size_t nn = (size_t)n;
+    uint8_t *d_bt = nullptr;  // [boards n*81 | turns n]
+    float *d_pz = nullptr;    // [policy n*81 | z n]
+    SCRATCH(1, nn * (kCells + 1), d_bt);
+    SCRATCH(2, nn * (kCells + 1), d_pz);
+    launch_rp_get(c, d_rows, n, d_bt, d_bt + nn * kCells, d_pz, d_pz + nn * kCells);
+    if (out_boards) CK(copy_d2h(c, out_boards, d_bt, nn * kCells, c->stream));
+    if (out_turns) CK(copy_d2h(c, out_turns, d_bt + nn * kCells, nn, c->stream));
+    if (out_policy) CK(copy_d2h(c, out_policy, d_pz, sizeof(float) * nn * kCells, c->stream));
+    if (out_z) CK(copy_d2h(c, out_z, d_pz + nn * kCells, sizeof(float) * nn, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_train_replay(omk_ctx *c, uint64_t seed, int64_t first_step, int32_t steps, int32_t n, float *out_losses,
+                                    int64_t *out_rows) {
+    CK(cudaSetDevice(c->device));
+    if (steps < 1 || n < 1 || !out_losses) return fail(OMK_ERR_INVALID, "need steps >= 1, n >= 1 and out_losses");
+    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
+    const Replay &r = c->rp;
+    if (r.ring.cap == 0) return fail(OMK_ERR_STATE, "no replay memory (omk_replay_reset)");
+    if (r.len == 0) return fail(OMK_ERR_STATE, "the replay memory is empty");
+    const int m = (int)(r.len < n ? r.len : n);  // choose_multiple: min(n, len) rows
+    float *img = nullptr, *pi = nullptr, *z = nullptr;
+    if (const char *e = train_minibatch_buffers(c, m, &img, &pi, &z)) return fail(OMK_ERR_CUDA, std::string("omk_train_replay: ") + e);
+    int64_t *d_rows = nullptr;
+    float *d_losses = nullptr;
+    SCRATCH(0, (size_t)steps * m, d_rows);
+    SCRATCH(1, (size_t)steps * 3, d_losses);
+    c->train_n = 0;
+    launch_rp_sample(c, seed, first_step, steps, r.len, m, d_rows);
+    for (int s = 0; s < steps; ++s) {  // omk_train_step's sequence, the minibatch encoded on the device
+        launch_rp_gather(c, d_rows + (size_t)s * m, m, img, pi, z);
+        if (const char *e = train_backward_resident(c, m)) return fail(OMK_ERR_CUDA, std::string("omk_train_replay: ") + e);
+        if (const char *e = train_apply_step(c)) return fail(OMK_ERR_CUDA, std::string("omk_train_replay: ") + e);
+        c->net_pack_dirty = true;
+        if (const char *e = train_report_losses_device(c, m, d_losses + 3 * (size_t)s))
+            return fail(OMK_ERR_CUDA, std::string("omk_train_replay: ") + e);
+    }
+    CK(copy_d2h(c, out_losses, d_losses, sizeof(float) * 3 * (size_t)steps, c->stream));
+    if (out_rows) {  // [steps][n]: the m rows of each step, then -1
+        CK(cudaMemcpy2DAsync(out_rows, sizeof(int64_t) * (size_t)n, d_rows, sizeof(int64_t) * (size_t)m, sizeof(int64_t) * (size_t)m,
+                             (size_t)steps, cudaMemcpyDeviceToHost, c->stream));
+        c->d2h_bytes += (int64_t)sizeof(int64_t) * steps * m;
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    if (out_rows)
+        for (int s = 0; s < steps; ++s)
+            for (int k = m; k < n; ++k) out_rows[(size_t)s * n + k] = -1;
+    for (int i = 0; i < 3 * steps; ++i)
+        if (!(out_losses[i] == out_losses[i]) || out_losses[i] > 3.0e38f) return fail(OMK_ERR_NUMERIC, "the training loss is not finite");
+    return OMK_OK;
 }

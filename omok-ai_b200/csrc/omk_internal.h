@@ -58,6 +58,32 @@ struct Workspace {  // evaluator request/response buffers [max_rows]; activation
     uint32_t *streams = nullptr;  // [capacity_trees]
 };
 
+// Replay memory on the device (replay_kernels.cu; DESIGN.md 2).  Row a (absolute: rows added since the last reset) lives
+// at a % cap; logical row i (0 = oldest) is absolute row added - len + i.
+struct ReplayRing {
+    uint8_t *boards = nullptr;  // [cap][81]
+    uint8_t *turns = nullptr;   // [cap]
+    float *pi = nullptr;        // [cap][81]
+    float *z = nullptr;         // [cap]
+    long long cap = 0;
+};
+struct ReplayCounters {  // device; advanced by the per-ply commit
+    long long added, len, episodes;
+    uint32_t done, pad;  // arrival counter of the commit's blocks (re-armed)
+};
+struct Replay {
+    ReplayRing ring;
+    ReplayCounters *counters = nullptr;
+    long long added = 0, len = 0, episodes = 0;  // host copy of *counters, refreshed by omk_selfplay_run
+    // staging of the driver's unfinished games: [games][81 plies][81] boards and policies, [games] ply counts
+    int stage_games = 0;  // 0: the driver does not feed the replay
+    uint8_t *stage_boards = nullptr;
+    float *stage_pi = nullptr;
+    int32_t *stage_len = nullptr;
+    cudaStream_t stream = nullptr;      // the per-ply commits
+    cudaEvent_t ev_commit = nullptr;    // the last commit enqueued
+};
+
 }  // namespace omk
 
 struct omk_prof_span {
@@ -126,6 +152,7 @@ struct omk_ctx {
     size_t sp_ring_slot_bytes = 0;
     cudaStream_t sp_copy_stream = nullptr;
     cudaEvent_t sp_ev_rec[kSpRing][2] = {}, sp_ev_copy[kSpRing] = {};
+    omk::Replay rp;                   // device replay memory (omk_replay_reset); fed by the driver when it exists at omk_selfplay_begin
     // pinned host staging
     void *pinned = nullptr;
     size_t pinned_bytes = 0;
@@ -169,6 +196,15 @@ void launch_sp_record(omk_ctx *c, int n, const int32_t *mover, const int32_t *ac
                       uint8_t *boards_out, float *policy_out, int32_t *actions_out);
 void launch_sp_advance(omk_ctx *c, int g0, int n, const int8_t *status, unsigned long long *counters);
 
+// replay_kernels.cu: stage a lane's recorded ply (ring-slot boards / policies of games g0..g0+n-1) on c->stream; commit the
+// ply's finished episodes on the replay stream; sample `steps` minibatches of m logical rows; gather + encode one minibatch;
+// copy rows out for omk_replay_get
+void launch_rp_stage(omk_ctx *c, int g0, int n, const uint8_t *boards, const float *policy);
+void launch_rp_commit(omk_ctx *c, int n, const int8_t *status);
+void launch_rp_sample(omk_ctx *c, uint64_t seed, long long first_step, int steps, long long len, int m, int64_t *rows);
+void launch_rp_gather(omk_ctx *c, const int64_t *rows, int m, float *img, float *pi, float *z);
+void launch_rp_get(omk_ctx *c, const int64_t *rows, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z);
+
 // omk_api.cu: open / close a profiling span of kernel family `kind` (no-op below min_level)
 bool prof_begin(omk_ctx *c, int kind, int min_level);
 void prof_end(omk_ctx *c, bool opened);
@@ -196,6 +232,11 @@ void launch_split16_to_f32(omk_ctx *c, const __half *hi, const __half *lo, float
 const char *train_backward_step(omk_ctx *c, const float *images, const float *pi, const float *z, int n, float **grads_dev);
 const char *train_apply_step(omk_ctx *c);
 const char *train_report_losses(omk_ctx *c, int n, float *out3);
+// the replay path: the minibatch buffers for n positions (filled on the device), then the same forward / losses / backward,
+// and the reporting forward with its losses left in device memory (dst3)
+const char *train_minibatch_buffers(omk_ctx *c, int n, float **img, float **pi, float **z);
+const char *train_backward_resident(omk_ctx *c, int n);
+const char *train_report_losses_device(omk_ctx *c, int n, float *dst3);
 float *train_grad_buffer(omk_ctx *c);
 void train_reset_optimizer(omk_ctx *c);
 void train_free(omk_ctx *c);

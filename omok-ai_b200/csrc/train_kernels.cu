@@ -608,10 +608,26 @@ const char *train_backward_step(omk_ctx *c, const float *images, const float *pi
     TrainState *t = train_state(c);
     if (!train_ensure(c, t, n)) return "training workspace allocation failed";
     if (!train_upload(c, t, images, pi, z, n)) return "copying the minibatch to the device failed";
+    if (grads_dev) *grads_dev = t->grads;
+    return train_backward_resident(c, n);
+}
+
+// the replay path writes the minibatch into these buffers on the device instead of train_upload's copies
+const char *train_minibatch_buffers(omk_ctx *c, int n, float **img, float **pi, float **z) {
+    TrainState *t = train_state(c);
+    if (!train_ensure(c, t, n)) return "training workspace allocation failed";
+    *img = t->img;
+    *pi = t->pi;
+    *z = t->z;
+    return nullptr;
+}
+
+// forward + losses + backward on the minibatch already in the workspace
+const char *train_backward_resident(omk_ctx *c, int n) {
+    TrainState *t = train_state(c);
     train_forward(c, t, n);
     train_losses(c, t, n, true);
     train_backward(c, t, n);
-    if (grads_dev) *grads_dev = t->grads;
     return cudaPeekAtLastError() == cudaSuccess ? nullptr : cudaGetErrorString(cudaGetLastError());
 }
 
@@ -636,8 +652,7 @@ const char *train_apply_step(omk_ctx *c) {
 
 // the reference's second forward: (p_loss, v_loss, loss) of the minibatch uploaded by train_backward_step, with the
 // CURRENT weights; averaged over the ranks when a communicator is attached
-const char *train_report_losses(omk_ctx *c, int n, float *out3) {
-    TrainState *t = train_state(c);
+static const char *report_forward(omk_ctx *c, TrainState *t, int n) {
     if (n > t->cap_n || n <= 0) return "no minibatch on the device";
     train_forward(c, t, n);
     train_losses(c, t, n, false);
@@ -647,6 +662,17 @@ const char *train_report_losses(omk_ctx *c, int n, float *out3) {
         k_scale<<<1, 32, 0, c->stream>>>(t->losses, 3, 1.0f / (float)t->world);
         c->launches++;
     }
+    return nullptr;
+}
+const char *train_report_losses_device(omk_ctx *c, int n, float *dst3) {
+    TrainState *t = train_state(c);
+    if (const char *e = report_forward(c, t, n)) return e;
+    if (cudaMemcpyAsync(dst3, t->losses, sizeof(float) * 3, cudaMemcpyDeviceToDevice, c->stream) != cudaSuccess) return "loss copy failed";
+    return cudaPeekAtLastError() == cudaSuccess ? nullptr : cudaGetErrorString(cudaGetLastError());
+}
+const char *train_report_losses(omk_ctx *c, int n, float *out3) {
+    TrainState *t = train_state(c);
+    if (const char *e = report_forward(c, t, n)) return e;
     c->d2h_bytes += (int64_t)sizeof(float) * 3;
     if (cudaMemcpyAsync(out3, t->losses, sizeof(float) * 3, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return "loss copy failed";
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return "stream synchronisation failed";

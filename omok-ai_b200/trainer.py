@@ -274,6 +274,13 @@ class AbiTrainStep:
         self.steps += 1
         return self.ctx.train_step(images, pi, z)
 
+    def train_replay(self, steps: int, minibatch: int, seed: int):
+        """`steps` steps on minibatches sampled from the context's device replay memory (omk_train_replay): losses
+        [steps, 3].  The sampler streams continue from this object's step count, so consecutive calls draw fresh ones."""
+        losses = self.ctx.train_replay(seed, self.steps, steps, minibatch)
+        self.steps += steps
+        return losses
+
     def numpy_params(self):
         return self.ctx.net_get_params()
 

@@ -111,6 +111,11 @@ extern "C" {
     // device-resident self-play driver (src/trainer.rs:86-204)
     pub fn omk_selfplay_begin(ctx: *mut omk_ctx, cfg: *const omk_selfplay_config) -> i32;
     pub fn omk_selfplay_run(ctx: *mut omk_ctx, plies: i32, profile: i32, out_boards: *mut u8, out_policy: *mut f32, out_status: *mut i8, out_actions: *mut i32, stats: *mut omk_selfplay_stats) -> i32;
+    // device replay memory (src/trainer.rs:27,206-352) and the training phase on it
+    pub fn omk_replay_reset(ctx: *mut omk_ctx, capacity: i64) -> i32;
+    pub fn omk_replay_info(ctx: *mut omk_ctx, out_len: *mut i64, out_rows_added: *mut i64, out_episodes: *mut i64) -> i32;
+    pub fn omk_replay_get(ctx: *mut omk_ctx, rows: *const i64, n: i32, out_boards: *mut u8, out_turns: *mut u8, out_policy: *mut f32, out_z: *mut f32) -> i32;
+    pub fn omk_train_replay(ctx: *mut omk_ctx, seed: u64, first_step: i64, steps: i32, n: i32, out_losses: *mut f32, out_rows: *mut i64) -> i32;
 }
 
 /// The message of the last failing call on this thread.

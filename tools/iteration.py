@@ -6,7 +6,10 @@ the same call.  Single GPU: `python tools/iteration.py`; N GPUs of one node:
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P tools/iteration.py
 Defaults are the reference trainer's: 800 simulations per move here (BASELINE) in rounds of 16, minibatch 128
 (src/config.rs:89-100).  Prints one JSON line (rank 0): self-play throughput, the trainer step time with and without
-the all-reduce (device timed, max over ranks), the all-reduce of the same 22.6 MB timed alone, and the losses."""
+the all-reduce (device timed, max over ranks), the all-reduce of the same 22.6 MB timed alone, and the losses.
+With --device-replay the replay memory lives in the context instead (omk_replay_reset before omk_selfplay_begin): the
+self-play driver feeds it on the device, no transition is streamed, and the whole training phase -- sampling, encoding and
+the steps -- is ONE omk_train_replay call, timed as such (train_phase_s); every rank samples its own replay memory."""
 from __future__ import annotations
 
 import argparse
@@ -25,7 +28,8 @@ sys.path.insert(0, ROOT)
 N_PARAMS = 5_643_250
 
 
-def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False):
+def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
+        device_replay=False, replay_capacity=600_000):
     omk = importlib.import_module("omok-ai_b200")
     trainer = importlib.import_module("omok-ai_b200.trainer")
     sharding = importlib.import_module("omok-ai_b200.sharding")
@@ -37,6 +41,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         import torch.distributed as dist
 
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    if device_replay and (torch_step or gather):
+        raise ValueError("--device-replay trains through omk_train_replay: it excludes --torch-step and --gather")
     my_games = games_per_gpu
     ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games, capacity_nodes=4096, seed=sharding.rank_seed(seed, rank))
     ctx.net_init_random(seed)                       # identical weights on every rank
@@ -51,6 +57,10 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
             dist.broadcast(t, src=0)
             uid = bytes(t.cpu().numpy().tobytes())
         step = trainer.AbiTrainStep(ctx, world=world, rank=rank, unique_id=uid)
+    if device_replay:
+        ctx.replay_reset(replay_capacity)           # before selfplay_begin: the driver feeds the replay that exists then
+        return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
+                                  seed, quiet, replay_capacity)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -139,6 +149,48 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     return out
 
 
+def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity):
+    omk = importlib.import_module("omok-ai_b200")
+    ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
+    ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
+    if dist:
+        dist.barrier()
+    t0 = time.perf_counter()
+    stats = ctx.selfplay_run(plies, profile=0, want_transitions=False)[0]
+    sp_s = time.perf_counter() - t0
+    rows, _, episodes = ctx.replay_info()
+    if rows == 0:
+        raise SystemExit("no game finished during self-play, so the replay memory is empty: raise --plies")
+    per_rank = max(1, minibatch // world)
+    sampler_seed = sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
+    step.train_replay(2, per_rank, sampler_seed)   # warm-up: training workspace, split-K scratch
+    torch.cuda.synchronize()
+    if dist:
+        dist.barrier()
+    t1 = time.perf_counter()
+    losses = step.train_replay(steps, per_rank, sampler_seed)   # the whole training phase: one call, one synchronisation
+    phase_s = time.perf_counter() - t1
+    h2d, _ = ctx.transfer_bytes
+    times, work = sharding.reduce_measurements({"train_phase_s": phase_s, "selfplay_s": sp_s, "selfplay_gpu_ms": float(stats.gpu_ms)},
+                                               {"sims": int(stats.simulations), "positions": int(stats.positions),
+                                                "rows": rows, "episodes": episodes},
+                                               device="cuda" if dist else "cpu")
+    out = {"config": "AlphaZero iteration (BASELINE configs[4]), device replay memory", "n_gpus": world, "games_per_gpu": games,
+           "plies": plies, "sims_per_move": count, "selfplay_sims_per_s": work["sims"] / times["selfplay_s"],
+           "selfplay_positions_per_s": work["positions"] / times["selfplay_s"], "selfplay_wall_s": times["selfplay_s"],
+           "selfplay_gpu_ms": times["selfplay_gpu_ms"], "transitions_streamed_to_host": False,
+           "replay_capacity_per_gpu": capacity, "replay_rows": work["rows"], "replay_episodes": work["episodes"],
+           "train_steps": steps, "global_minibatch": per_rank * world, "train_step": "omk_train_replay (C ABI, fp32 CUDA kernels)",
+           "train_phase_s": times["train_phase_s"], "train_step_ms": times["train_phase_s"] * 1e3 / steps,
+           "first_loss": float(losses[0, 2]), "last_loss": float(losses[-1, 2]), "h2d_bytes_total": h2d}
+    if rank == 0 and not quiet:
+        print(json.dumps(out), flush=True)
+    ctx.close()
+    if dist:
+        dist.destroy_process_group()
+    return out
+
+
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--games-per-gpu", type=int, default=1024)
@@ -148,5 +200,9 @@ if __name__ == "__main__":
     ap.add_argument("--minibatch", type=int, default=128)
     ap.add_argument("--gather", action="store_true", help="merge every rank's transitions on rank 0 (config 4's host replay buffer)")
     ap.add_argument("--torch-step", action="store_true", help="PyTorch-autograd step instead of omk_train_step")
+    ap.add_argument("--device-replay", action="store_true",
+                    help="replay memory on the device, fed by the self-play driver; the training phase is one omk_train_replay call")
+    ap.add_argument("--replay-capacity", type=int, default=600_000, help="rows of the device replay memory per GPU (src/config.rs: 600 000)")
     a = ap.parse_args()
-    run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step)
+    run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
+        device_replay=a.device_replay, replay_capacity=a.replay_capacity)
