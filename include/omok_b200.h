@@ -70,7 +70,8 @@ OMK_API int32_t omk_version(void);
 
 /* ---------------------------------------------------------------- context */
 /* capacity_nodes: node slots per tree (<= 65535).  seed keys the specified
- * counter-based random stream that replaces the reference's thread_rng().     */
+ * counter-based random stream that replaces the reference's thread_rng().
+ * A failed create releases everything it allocated and leaves *out NULL.      */
 OMK_API int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t capacity_trees, int32_t capacity_nodes,
                        uint64_t seed, omk_ctx **out);
 OMK_API int32_t omk_ctx_destroy(omk_ctx *ctx);

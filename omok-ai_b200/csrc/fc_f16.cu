@@ -543,42 +543,19 @@ static bool encode_map_tower_store(CUtensorMap *map, __half *ptr, uint64_t rows)
               CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-struct ActMaps {  // tensor maps over one workspace's activation buffers (each search lane has its own workspace)
-    CUtensorMap map0_a_hi, map0_a_lo, map1_a_hi, map1_a_lo, map2_a_hi, map2_a_lo;
-    CUtensorMap tower_st_hi, tower_st_lo;  // k_tower16's write-out into act0
-    const __half *key[6] = {};  // the six buffers the maps were encoded for (a reallocation may reuse only some addresses)
-    int a_rows = 0;
-    float *splitk_partial = nullptr;  // [splitk_chunks][splitk_rows][512] fp32 partial sums of this workspace's split-K fc0
-    int splitk_rows = 0, splitk_chunks = 0;
-    float4 *bal_partial = nullptr;    // tail-balancing scratch of this workspace's pair fc0: [units][F_BAL_UNIT_F4]
-    int bal_units = 0;
-    uint32_t *bal_flags = nullptr;    // [256]
-};
-struct Fc16State {
+struct Fc16State {  // weight maps, shared by both search lanes (the activation maps live in each lane's Workspace)
     CUtensorMap map0_b_hi, map0_b_lo;  // fc0 (B boxes of 128 rows: the pair kernel loads half tiles)
     CUtensorMap map1_b_hi, map1_b_lo;  // fc1 (B boxes of 256 rows)
     CUtensorMap map2_b_hi, map2_b_lo;  // heads (B = all 128 padded output rows)
-    ActMaps acts[2];
-    int next_victim = 0;
     bool weights_ready = false;
     CUtensorMap map0s_b_hi, map0s_b_lo;  // fc0 weights with 256-row boxes (one-CTA split-K kernel for small batches)
     int pair_slots = 0;                  // CTA pairs of the fc0 pair kernel the device holds at once (0 = not queried yet)
 };
+void Fc16StateFree::operator()(Fc16State *s) const { delete s; }
 
 static Fc16State *state16_of(omk_ctx *c) {
-    if (!c->fc16_state) c->fc16_state = new Fc16State();
-    return reinterpret_cast<Fc16State *>(c->fc16_state);
-}
-
-void fc16_free(omk_ctx *c) {
-    if (c->fc16_state)
-        for (ActMaps &m : reinterpret_cast<Fc16State *>(c->fc16_state)->acts) {
-            cudaFree(m.splitk_partial);
-            cudaFree(m.bal_partial);
-            cudaFree(m.bal_flags);
-        }
-    delete reinterpret_cast<Fc16State *>(c->fc16_state);
-    c->fc16_state = nullptr;
+    if (!c->fc16_state) c->fc16_state.reset(new Fc16State());
+    return c->fc16_state.get();
 }
 
 // (re)build the scaled, split, transposed weights of fc0 and fc1; call after the weights change
@@ -586,14 +563,13 @@ bool fc16_prepare_weights(omk_ctx *c) {
     Fc16State *s = state16_of(c);
     NetWeights &w = c->net;
     if (!w.fc0_wt_h16) {
-        if (cudaMalloc(&w.fc0_wt_h16, sizeof(__half) * (size_t)F_K0 * F_N) != cudaSuccess) return false;
-        if (cudaMalloc(&w.fc0_wt_l16, sizeof(__half) * (size_t)F_K0 * F_N) != cudaSuccess) return false;
-        if (cudaMalloc(&w.fc1_wt_h16, sizeof(__half) * (size_t)F_K1 * F_N) != cudaSuccess) return false;
-        if (cudaMalloc(&w.fc1_wt_l16, sizeof(__half) * (size_t)F_K1 * F_N) != cudaSuccess) return false;
-        if (cudaMalloc(&w.heads_wt_h16, sizeof(__half) * (size_t)F_K1 * 128) != cudaSuccess) return false;
-        if (cudaMalloc(&w.heads_wt_l16, sizeof(__half) * (size_t)F_K1 * 128) != cudaSuccess) return false;
-        if (cudaMalloc(&w.fc_inv_scale, sizeof(float) * 3) != cudaSuccess) return false;
-        if (cudaMalloc(&w.fc_absmax, sizeof(uint32_t) * 3) != cudaSuccess) return false;
+        FcImages f;
+        if (f.fc0_wt_h16.alloc((size_t)F_K0 * F_N) != cudaSuccess || f.fc0_wt_l16.alloc((size_t)F_K0 * F_N) != cudaSuccess ||
+            f.fc1_wt_h16.alloc((size_t)F_K1 * F_N) != cudaSuccess || f.fc1_wt_l16.alloc((size_t)F_K1 * F_N) != cudaSuccess ||
+            f.heads_wt_h16.alloc((size_t)F_K1 * 128) != cudaSuccess || f.heads_wt_l16.alloc((size_t)F_K1 * 128) != cudaSuccess ||
+            f.fc_inv_scale.alloc(3) != cudaSuccess || f.fc_absmax.alloc(3) != cudaSuccess)
+            return false;
+        static_cast<FcImages &>(w) = std::move(f);
     }
     cudaMemsetAsync(w.fc_absmax, 0, sizeof(uint32_t) * 3, c->stream);
     k_absmax_bits<<<592, 256, 0, c->stream>>>(w.t[23], (long long)F_K0 * F_N, w.fc_absmax);
@@ -618,36 +594,13 @@ bool fc16_prepare_weights(omk_ctx *c) {
     return true;
 }
 
-static ActMaps *refresh_maps16(omk_ctx *c, Fc16State *s) {
-    const Workspace &w = c->ws;
-    const __half *key[6] = {w.act0_h16, w.act0_l16, w.act1_h16, w.act1_l16, w.act2_h16, w.act2_l16};
-    for (ActMaps &m : s->acts) {
-        bool same = m.key[0] != nullptr && m.a_rows == w.act_rows;
-        for (int i = 0; i < 6; ++i) same = same && m.key[i] == key[i];
-        if (same) return &m;
-    }
-    ActMaps &m = s->acts[s->next_victim];
-    s->next_victim ^= 1;
-    m.key[0] = nullptr;
-    if (!encode_map16(&m.map0_a_hi, w.act0_h16, (uint64_t)w.act_rows, F_BM, F_K0)) return nullptr;
-    if (!encode_map16(&m.map0_a_lo, w.act0_l16, (uint64_t)w.act_rows, F_BM, F_K0)) return nullptr;
-    if (!encode_map16(&m.map1_a_hi, w.act1_h16, (uint64_t)w.act_rows, F_BM, F_K1)) return nullptr;
-    if (!encode_map16(&m.map1_a_lo, w.act1_l16, (uint64_t)w.act_rows, F_BM, F_K1)) return nullptr;
-    if (!encode_map16(&m.map2_a_hi, w.act2_h16, (uint64_t)w.act_rows, F_BM, F_K1)) return nullptr;
-    if (!encode_map16(&m.map2_a_lo, w.act2_l16, (uint64_t)w.act_rows, F_BM, F_K1)) return nullptr;
-    if (!encode_map_tower_store(&m.tower_st_hi, w.act0_h16, (uint64_t)w.act_rows)) return nullptr;
-    if (!encode_map_tower_store(&m.tower_st_lo, w.act0_l16, (uint64_t)w.act_rows)) return nullptr;
-    for (int i = 0; i < 6; ++i) m.key[i] = key[i];
-    m.a_rows = w.act_rows;
-    return &m;
-}
-
-bool fc16_tower_store_maps(omk_ctx *c, const void **map_hi, const void **map_lo) {
-    ActMaps *am = refresh_maps16(c, state16_of(c));
-    if (!am) return false;
-    *map_hi = &am->tower_st_hi;
-    *map_lo = &am->tower_st_lo;
-    return true;
+bool fc16_encode_act_maps(Activations &a) {
+    ActMaps &m = a.maps;
+    const uint64_t rows = (uint64_t)a.act_rows;
+    return encode_map16(&m.map0_a_hi, a.act0_h16, rows, F_BM, F_K0) && encode_map16(&m.map0_a_lo, a.act0_l16, rows, F_BM, F_K0) &&
+           encode_map16(&m.map1_a_hi, a.act1_h16, rows, F_BM, F_K1) && encode_map16(&m.map1_a_lo, a.act1_l16, rows, F_BM, F_K1) &&
+           encode_map16(&m.map2_a_hi, a.act2_h16, rows, F_BM, F_K1) && encode_map16(&m.map2_a_lo, a.act2_l16, rows, F_BM, F_K1) &&
+           encode_map_tower_store(&m.tower_st_hi, a.act0_h16, rows) && encode_map_tower_store(&m.tower_st_lo, a.act0_l16, rows);
 }
 
 static bool check_launch(const char *what) {
@@ -660,7 +613,7 @@ static bool check_launch(const char *what) {
 // fc0: act0_h16/l16 -> act1_h16/l16 (the A operand of fc1)
 bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
     Fc16State *s = state16_of(c);
-    ActMaps *am = s->weights_ready ? refresh_maps16(c, s) : nullptr;
+    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     const bool fine = c->fc0_chunk == F_CHUNK0_FINE;
     static const int splitk_env = getenv("OMK_FC0_SPLITK_MAX") ? atoi(getenv("OMK_FC0_SPLITK_MAX")) : -1;
@@ -672,14 +625,9 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
         // (128-row tile, N half, chunk) is one CTA and k_fc0_reduce adds the chunks in order.
         const int kChunks = F_K0 / F_BK / (fine ? F_CHUNK0_FINE : F_CHUNK0);
         const int mt = (rows_bound + F_BM - 1) / F_BM, ws_rows = mt * F_BM;
-        if (am->splitk_rows < ws_rows || am->splitk_chunks < kChunks) {  // per workspace: two search lanes may run this path at the same time
-            cudaFree(am->splitk_partial);
-            am->splitk_partial = nullptr;
-            am->splitk_rows = 0;
-            if (cudaMalloc(&am->splitk_partial, sizeof(float) * (size_t)kChunks * ws_rows * F_N) != cudaSuccess) return false;
-            am->splitk_rows = ws_rows;
-            am->splitk_chunks = kChunks;
-        }
+        // per workspace: two search lanes may run this path at the same time
+        if (c->ws.splitk_partial.grow(c->stream, (size_t)kChunks * ws_rows * F_N) != cudaSuccess) return false;
+        float *partial = c->ws.splitk_partial;
         static const int narrow_env = getenv("OMK_FC0_SPLITK_NARROW") ? atoi(getenv("OMK_FC0_SPLITK_NARROW")) : -1;
         if (mt <= (narrow_env >= 0 ? narrow_env : 2)) {
             // one or two row tiles (a single game's rounds of 8, Agent::new): 128-column tiles double the CTAs (72 per row tile
@@ -689,17 +637,17 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
             auto sk = fine ? k_fc16<F_K0, F_CHUNK0_FINE, false, 128, false, true> : k_fc16<F_K0, F_CHUNK0, false, 128, false, true>;
             cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
             sk<<<dim3(F_N / 128, mt, F_K0 / F_BK / F_SPLITK_KB), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-                am->map0_a_hi, am->map0_a_lo, s->map0_b_hi, s->map0_b_lo, c->net.t[24], c->net.fc_inv_scale, am->splitk_partial, nullptr,
+                am->map0_a_hi, am->map0_a_lo, s->map0_b_hi, s->map0_b_lo, c->net.t[24], c->net.fc_inv_scale, partial, nullptr,
                 nullptr, c->ws.n_req, rows_bound, nullptr, nullptr, nullptr, FcBal{});
         } else {
             using Cfg = FcCfg<false, 256>;
             auto sk = fine ? k_fc16<F_K0, F_CHUNK0_FINE, false, 256, false, true> : k_fc16<F_K0, F_CHUNK0, false, 256, false, true>;
             cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
             sk<<<dim3(F_N / F_BN, mt, F_K0 / F_BK / F_SPLITK_KB), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-                am->map0_a_hi, am->map0_a_lo, s->map0s_b_hi, s->map0s_b_lo, c->net.t[24], c->net.fc_inv_scale, am->splitk_partial, nullptr,
+                am->map0_a_hi, am->map0_a_lo, s->map0s_b_hi, s->map0s_b_lo, c->net.t[24], c->net.fc_inv_scale, partial, nullptr,
                 nullptr, c->ws.n_req, rows_bound, nullptr, nullptr, nullptr, FcBal{});
         }
-        k_fc0_reduce<<<(rows_bound * 64 + 255) / 256, 256, 0, c->stream>>>(am->splitk_partial, kChunks, ws_rows, c->net.t[24],
+        k_fc0_reduce<<<(rows_bound * 64 + 255) / 256, 256, 0, c->stream>>>(partial, kChunks, ws_rows, c->net.t[24],
                                                                             c->net.fc_inv_scale, c->ws.act1_h16, c->ws.act1_l16,
                                                                             c->ws.n_req, rows_bound);
         c->launches += 2;
@@ -744,26 +692,17 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
             if (tail > 0) {
                 const int units = R * tail;
                 bool ok = true;
-                if (!am->bal_flags) {
-                    ok = cudaMalloc(&am->bal_flags, sizeof(uint32_t) * 256) == cudaSuccess &&
-                         cudaMemsetAsync(am->bal_flags, 0, sizeof(uint32_t) * 256, c->stream) == cudaSuccess;
-                }
-                if (ok && am->bal_units < units) {
-                    if (cudaStreamSynchronize(c->stream) != cudaSuccess) return false;
-                    cudaFree(am->bal_partial);
-                    am->bal_partial = nullptr;
-                    am->bal_units = 0;
-                    ok = cudaMalloc(&am->bal_partial, sizeof(float4) * F_BAL_UNIT_F4 * (size_t)units) == cudaSuccess;
-                    if (ok) am->bal_units = units;
-                }
-                if (!ok) return false;
+                Workspace &w = c->ws;
+                if (!w.bal_flags)
+                    ok = w.bal_flags.alloc(256) == cudaSuccess && cudaMemsetAsync(w.bal_flags, 0, w.bal_flags.bytes(), c->stream) == cudaSuccess;
+                if (!ok || w.bal_partial.grow(c->stream, F_BAL_UNIT_F4 * (size_t)units) != cudaSuccess) return false;
                 bal.full = T - R;
                 bal.helpers = H;
                 bal.mains = R;
                 bal.tail = tail;
                 bal.m = NC - tail;
-                bal.partial = am->bal_partial;
-                bal.flags = am->bal_flags;
+                bal.partial = w.bal_partial;
+                bal.flags = w.bal_flags;
                 cfg.gridDim = dim3(2 * (T + H), 1);
             }
         }
@@ -778,7 +717,7 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
 // fc1: act1_h16/l16 -> act2_h16/l16 (the A operand of the heads)
 bool launch_fc1_f16(omk_ctx *c, int rows_bound) {
     Fc16State *s = state16_of(c);
-    const ActMaps *am = s->weights_ready ? refresh_maps16(c, s) : nullptr;
+    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     using Cfg = FcCfg<false, 256>;
     auto kern = k_fc16<F_K1, F_CHUNK1, false>;
@@ -794,7 +733,7 @@ bool launch_fc1_f16(omk_ctx *c, int rows_bound) {
 // heads: act2_h16/l16 -> P (softmax of the 81 policy logits) and V (tanh of the value logit)
 bool launch_heads_f16(omk_ctx *c, int rows_bound) {
     Fc16State *s = state16_of(c);
-    const ActMaps *am = s->weights_ready ? refresh_maps16(c, s) : nullptr;
+    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     using Cfg = FcCfg<false, 128>;
     auto kern = k_fc16<F_K1, F_CHUNKH, false, 128, true>;

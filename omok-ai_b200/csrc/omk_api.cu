@@ -55,18 +55,8 @@ extern "C" int32_t omk_version(void) { return 100; }
 // grow-only device scratch slot i of the context (every call that uses it synchronises the stream before it returns)
 template <typename T>
 static int32_t scratch_dev(omk_ctx *c, int i, size_t count, T **out) {
-    omk_ctx::Scratch &s = c->scratch[i];
-    const size_t bytes = count * sizeof(T);
-    if (bytes > s.cap) {
-        CK(cudaStreamSynchronize(c->stream));
-        cudaFree(s.p);
-        s.p = nullptr;
-        s.cap = 0;
-        const size_t want = (bytes + 4095) & ~(size_t)4095;
-        CK(cudaMalloc(&s.p, want));
-        s.cap = want;
-    }
-    *out = reinterpret_cast<T *>(s.p);
+    CK(c->scratch[i].grow(c->stream, count * sizeof(T), 4096));
+    *out = reinterpret_cast<T *>(c->scratch[i].get());
     return OMK_OK;
 }
 #define SCRATCH(i, count, ptr)                          \
@@ -77,18 +67,16 @@ static int32_t scratch_dev(omk_ctx *c, int i, size_t count, T **out) {
 
 static int32_t ensure_workspace(omk_ctx *c, int rows) {
     rows = (rows + 255) / 256 * 256;  // whole 256-row CTA-pair tiles
-    if (rows <= c->ws.max_rows) return OMK_OK;
-    CK(cudaStreamSynchronize(c->stream));
     Workspace &w = c->ws;
-    cudaFree(w.nn_in); cudaFree(w.req_tree); cudaFree(w.req_node); cudaFree(w.P); cudaFree(w.V);
-    w.nn_in = nullptr; w.req_tree = nullptr; w.req_node = nullptr; w.P = nullptr; w.V = nullptr;  // a failed cudaMalloc below must not leave dangling pointers for omk_ctx_destroy
-    w.max_rows = 0;
-    CK(cudaMalloc(&w.nn_in, sizeof(NNIn) * (size_t)rows));
-    CK(cudaMalloc(&w.req_tree, sizeof(uint32_t) * (size_t)rows));
-    CK(cudaMalloc(&w.req_node, sizeof(uint32_t) * (size_t)rows));
-    CK(cudaMalloc(&w.P, sizeof(float) * (size_t)rows * kRow));
-    CK(cudaMalloc(&w.V, sizeof(float) * (size_t)rows));
-    CK(cudaMemsetAsync(w.nn_in, 0, sizeof(NNIn) * (size_t)rows, c->stream));
+    if (rows <= w.max_rows) return OMK_OK;
+    const size_t r = (size_t)rows;
+    w.max_rows = 0;  // until every buffer below holds `rows` rows
+    CK(w.nn_in.grow(c->stream, r));
+    CK(w.req_tree.grow(c->stream, r));
+    CK(w.req_node.grow(c->stream, r));
+    CK(w.P.grow(c->stream, r * kRow));
+    CK(w.V.grow(c->stream, r));
+    CK(cudaMemsetAsync(w.nn_in, 0, w.nn_in.bytes(), c->stream));
     w.max_rows = rows;
     return OMK_OK;
 }
@@ -103,25 +91,21 @@ bool ensure_activations(omk_ctx *c, int rows) {
     if (rows <= w.act_rows && (!want_fp32 || w.act_fp32)) return true;
     if (rows < w.act_rows) rows = w.act_rows;
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return false;
-    void **bufs[] = {(void **)&w.act0_h16, (void **)&w.act0_l16, (void **)&w.act1_h16, (void **)&w.act1_l16, (void **)&w.act2_h16,
-                     (void **)&w.act2_l16, (void **)&w.act2, (void **)&w.logits, (void **)&w.act0, (void **)&w.act1};
-    for (void **b : bufs) {
-        cudaFree(*b);
-        *b = nullptr;
-    }
-    w.act_rows = 0;
-    w.act_fp32 = false;
+    static_cast<Activations &>(w) = Activations{};  // the old buffers go before the new ones are allocated
+    Activations a;
+    auto zeroed = [&](auto &b, size_t count) {  // padded tile rows read zeros, never NaNs
+        return b.alloc(count) == cudaSuccess && cudaMemsetAsync(b, 0, b.bytes(), c->stream) == cudaSuccess;
+    };
     const size_t r = (size_t)rows;
     // (act0: two rows of slack -- k_tower16 stores whole position triples, the last one may reach past `rows`)
-    const size_t sizes[] = {sizeof(__half) * (r + 2) * 10368, sizeof(__half) * (r + 2) * 10368, sizeof(__half) * r * 512, sizeof(__half) * r * 512,
-                            sizeof(__half) * r * 512, sizeof(__half) * r * 512,
-                            sizeof(float) * r * 512, sizeof(float) * r * 128, sizeof(float) * r * 10368, sizeof(float) * r * 512};
-    for (int i = 0; i < (want_fp32 ? 10 : 8); ++i) {
-        if (cudaMalloc(bufs[i], sizes[i]) != cudaSuccess) return false;
-        if (cudaMemsetAsync(*bufs[i], 0, sizes[i], c->stream) != cudaSuccess) return false;  // padded tile rows read zeros, never NaNs
-    }
-    w.act_rows = rows;
-    w.act_fp32 = want_fp32;
+    bool ok = zeroed(a.act0_h16, (r + 2) * 10368) && zeroed(a.act0_l16, (r + 2) * 10368) && zeroed(a.act1_h16, r * 512) &&
+              zeroed(a.act1_l16, r * 512) && zeroed(a.act2_h16, r * 512) && zeroed(a.act2_l16, r * 512) && zeroed(a.act2, r * 512) &&
+              zeroed(a.logits, r * 128);
+    if (ok && want_fp32) ok = zeroed(a.act0, r * 10368) && zeroed(a.act1, r * 512);
+    a.act_rows = rows;
+    a.act_fp32 = want_fp32;
+    if (!ok || !fc16_encode_act_maps(a)) return false;
+    static_cast<Activations &>(w) = std::move(a);
     return true;
 }
 }  // namespace omk
@@ -155,10 +139,8 @@ static int lanes_for(omk_ctx *c, int n) {
         if (cudaStreamCreateWithFlags(&c->lane1_stream, cudaStreamNonBlocking) != cudaSuccess) return 1;
         bool ok = cudaEventCreateWithFlags(&c->lane_fork, cudaEventDisableTiming) == cudaSuccess &&
                   cudaEventCreateWithFlags(&c->lane_join, cudaEventDisableTiming) == cudaSuccess &&
-                  cudaMalloc(&w.n_req, sizeof(uint32_t) * 4) == cudaSuccess &&
-                  cudaMalloc(&w.slot_base, sizeof(uint32_t) * ct) == cudaSuccess &&
-                  cudaMalloc(&w.slot_count, sizeof(uint32_t) * ct) == cudaSuccess &&
-                  cudaMemsetAsync(w.n_req, 0, sizeof(uint32_t) * 4, c->lane1_stream) == cudaSuccess;
+                  w.n_req.alloc(4) == cudaSuccess && w.slot_base.alloc(ct) == cudaSuccess && w.slot_count.alloc(ct) == cudaSuccess &&
+                  cudaMemsetAsync(w.n_req, 0, w.n_req.bytes(), c->lane1_stream) == cudaSuccess;
         if (!ok) {
             cudaGetLastError();
             c->lane_min_trees = 0;  // no second lane on this context
@@ -278,28 +260,27 @@ static int32_t check_evaluator(omk_ctx *c, int evaluator) {
     return OMK_OK;
 }
 
-// ------------------------------------------------------------------ replay memory (storage)
-static void replay_free_staging(omk_ctx *c) {
-    Replay &r = c->rp;
-    if (r.stream) cudaStreamSynchronize(r.stream);
-    cudaFree(r.stage_boards); cudaFree(r.stage_pi); cudaFree(r.stage_len);
-    r.stage_boards = nullptr; r.stage_pi = nullptr; r.stage_len = nullptr;
-    r.stage_games = 0;
-}
-static void replay_free(omk_ctx *c) {
-    Replay &r = c->rp;
-    replay_free_staging(c);
-    cudaFree(r.ring.boards); cudaFree(r.ring.turns); cudaFree(r.ring.pi); cudaFree(r.ring.z); cudaFree(r.counters);
-    r.ring = ReplayRing{};
-    r.counters = nullptr;
-    r.added = r.len = r.episodes = 0;
-}
-
 // ------------------------------------------------------------------ context
-extern "C" int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t capacity_trees, int32_t capacity_nodes,
-                                  uint64_t seed, omk_ctx **out) {
-    if (!out) return fail(OMK_ERR_INVALID, "out is NULL");
-    *out = nullptr;
+omk_ctx::~omk_ctx() {
+    const cudaStream_t streams[] = {stream, lane1_stream, sp_copy_stream, rp.stream};
+    for (cudaStream_t s : streams)
+        if (s) cudaStreamSynchronize(s);
+    for (cudaEvent_t e : prof_pool) cudaEventDestroy(e);
+    for (const omk_prof_span &s : prof_spans) {
+        cudaEventDestroy(s.a);
+        cudaEventDestroy(s.b);
+    }
+    for (int i = 0; i < kSpRing; ++i)
+        for (cudaEvent_t e : {sp_ev_rec[i][0], sp_ev_rec[i][1], sp_ev_copy[i]})
+            if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : {ev0, ev1, lane_fork, lane_join, rp.ev_commit})
+        if (e) cudaEventDestroy(e);
+    for (cudaStream_t s : streams)
+        if (s) cudaStreamDestroy(s);
+}  // the members' destructors release the buffers
+
+static int32_t ctx_create(int32_t device, int32_t capacity_envs, int32_t capacity_trees, int32_t capacity_nodes, uint64_t seed,
+                          std::unique_ptr<omk_ctx> &ctx) {
     if (capacity_envs < 0 || capacity_trees < 0 || capacity_nodes < 2 || capacity_nodes > 65535)
         return fail(OMK_ERR_INVALID, "bad capacity (capacity_nodes must be in [2, 65535])");
     int ndev = 0;
@@ -312,7 +293,8 @@ extern "C" int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t
     CK(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) return fail(OMK_ERR_CUDA, "libomok_b200 is built for sm_100a (B200) only");
 
-    omk_ctx *c = new omk_ctx();
+    ctx.reset(new omk_ctx());
+    omk_ctx *c = ctx.get();
     c->device = device;
     c->n_sms = prop.multiProcessorCount;
     c->cap_envs = capacity_envs;
@@ -330,85 +312,54 @@ extern "C" int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t
     CK(cudaEventCreate(&c->ev0));
     CK(cudaEventCreate(&c->ev1));
     const int ce = capacity_envs > 0 ? capacity_envs : 1, ct = capacity_trees > 0 ? capacity_trees : 1;
-    CK(cudaMalloc(&c->envs, sizeof(EnvRec) * (size_t)ce));
-    CK(cudaMalloc(&c->tree_hdrs, sizeof(TreeHdr) * (size_t)ct));
-    CK(cudaMalloc(&c->tree_nodes, (size_t)ct * (size_t)capacity_nodes * kNodeBytes));
-    CK(cudaMalloc(&c->remap, sizeof(uint16_t) * (size_t)ct * (size_t)capacity_nodes));
-    CK(cudaMalloc(&c->dev_error, sizeof(uint32_t)));
-    CK(cudaMalloc(&c->dev_sims, sizeof(unsigned long long) * 2));
-    CK(cudaMemsetAsync(c->dev_error, 0, sizeof(uint32_t), c->stream));
-    CK(cudaMemsetAsync(c->dev_sims, 0, sizeof(unsigned long long) * 2, c->stream));
-    CK(cudaMemsetAsync(c->tree_hdrs, 0, sizeof(TreeHdr) * (size_t)ct, c->stream));
-    CK(cudaMemsetAsync(c->envs, 0, sizeof(EnvRec) * (size_t)ce, c->stream));
+    CK(c->envs.alloc((size_t)ce));
+    CK(c->tree_hdrs.alloc((size_t)ct));
+    CK(c->tree_nodes.alloc((size_t)ct * (size_t)capacity_nodes * kNodeBytes));
+    CK(c->remap.alloc((size_t)ct * (size_t)capacity_nodes));
+    CK(c->dev_error.alloc(1));
+    CK(c->dev_sims.alloc(2));
+    CK(cudaMemsetAsync(c->dev_error, 0, c->dev_error.bytes(), c->stream));
+    CK(cudaMemsetAsync(c->dev_sims, 0, c->dev_sims.bytes(), c->stream));
+    CK(cudaMemsetAsync(c->tree_hdrs, 0, c->tree_hdrs.bytes(), c->stream));
+    CK(cudaMemsetAsync(c->envs, 0, c->envs.bytes(), c->stream));
     Workspace &w = c->ws;
     const int cm = ce > ct ? ce : ct;
-    CK(cudaMalloc(&w.n_req, sizeof(uint32_t) * 4));
-    CK(cudaMemsetAsync(w.n_req, 0, sizeof(uint32_t) * 4, c->stream));
-    CK(cudaMalloc(&w.slot_base, sizeof(uint32_t) * (size_t)ct));
-    CK(cudaMalloc(&w.slot_count, sizeof(uint32_t) * (size_t)ct));
-    CK(cudaMalloc(&w.ids, sizeof(int32_t) * (size_t)cm));
-    CK(cudaMalloc(&w.actions, sizeof(int32_t) * (size_t)cm));
-    CK(cudaMalloc(&w.modes, (size_t)cm));
-    CK(cudaMalloc(&w.temps, sizeof(float) * (size_t)cm));
-    CK(cudaMalloc(&w.status, (size_t)cm));
-    CK(cudaMalloc(&w.policy_out, sizeof(float) * (size_t)ct * kCells));
-    CK(cudaMalloc(&w.streams, sizeof(uint32_t) * (size_t)ct));
-    for (int i = 0; i < kNetTensors; ++i) CK(cudaMalloc(&c->net.t[i], sizeof(float) * (size_t)kLens[i]));
-    CK(cudaMalloc(&c->net.heads_w, sizeof(float) * 512 * 128));
-    CK(cudaMalloc(&c->net.heads_b, sizeof(float) * 128));
+    CK(w.n_req.alloc(4));
+    CK(cudaMemsetAsync(w.n_req, 0, w.n_req.bytes(), c->stream));
+    CK(w.slot_base.alloc((size_t)ct));
+    CK(w.slot_count.alloc((size_t)ct));
+    CK(w.ids.alloc((size_t)cm));
+    CK(w.actions.alloc((size_t)cm));
+    CK(w.modes.alloc((size_t)cm));
+    CK(w.temps.alloc((size_t)cm));
+    CK(w.status.alloc((size_t)cm));
+    CK(w.policy_out.alloc((size_t)ct * kCells));
+    CK(w.streams.alloc((size_t)ct));
+    for (int i = 0; i < kNetTensors; ++i) CK(c->net.t[i].alloc((size_t)kLens[i]));
+    CK(c->net.heads_w.alloc(512 * 128));
+    CK(c->net.heads_b.alloc(128));
     CK(cudaStreamSynchronize(c->stream));
-    *out = c;
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_ctx_create(int32_t device, int32_t capacity_envs, int32_t capacity_trees, int32_t capacity_nodes,
+                                  uint64_t seed, omk_ctx **out) {
+    if (!out) return fail(OMK_ERR_INVALID, "out is NULL");
+    *out = nullptr;
+    std::unique_ptr<omk_ctx> c;
+    const int32_t rc = ctx_create(device, capacity_envs, capacity_trees, capacity_nodes, seed, c);
+    if (rc != OMK_OK) {
+        c.reset();           // releases whatever was allocated
+        cudaGetLastError();  // the failed call's error must not surface in a later call
+        return rc;
+    }
+    *out = c.release();
     return OMK_OK;
 }
 
 extern "C" int32_t omk_ctx_destroy(omk_ctx *c) {
     if (!c) return OMK_OK;
     cudaSetDevice(c->device);
-    cudaStreamSynchronize(c->stream);
-    Workspace &w = c->ws;
-    void *ptrs[] = {c->envs, c->tree_hdrs, c->tree_nodes, c->remap, c->dev_error, c->dev_sims, w.nn_in, w.req_tree,
-                    w.req_node, w.P, w.V, w.act0, w.act1, w.act2, w.logits, w.n_req, w.slot_base, w.slot_count, w.ids,
-                    w.actions, w.modes, w.temps, w.status, w.policy_out, w.streams, c->net.heads_w, c->net.heads_b,
-                    c->sp_ply, c->sp_buf, w.act0_h16, w.act0_l16, w.act1_h16, w.act1_l16, w.act2_h16, w.act2_l16, c->net.heads_wt_h16, c->net.heads_wt_l16, c->net.fc0_wt_h16, c->net.fc0_wt_l16,
-                    c->net.fc1_wt_h16, c->net.fc1_wt_l16, c->net.fc_inv_scale, c->net.fc_absmax, c->net.tower16_wimg,
-                    c->net.tower16_pimg, c->net.tower16_absmax};
-    fc16_free(c);
-    train_free(c);
-    for (omk_ctx::Scratch &sc : c->scratch) cudaFree(sc.p);
-    free(c->tower16_params_host);
-    if (c->lane1_stream) {
-        cudaStreamSynchronize(c->lane1_stream);
-        Workspace &l = c->lane1_ws;
-        void *lp[] = {l.nn_in, l.req_tree, l.req_node, l.P, l.V, l.act0_h16, l.act0_l16, l.act1_h16, l.act1_l16, l.act2_h16, l.act2_l16,
-                      l.act2, l.logits, l.act0, l.act1, l.n_req, l.slot_base, l.slot_count};
-        for (void *q : lp) cudaFree(q);
-        cudaEventDestroy(c->lane_fork);
-        cudaEventDestroy(c->lane_join);
-        cudaStreamDestroy(c->lane1_stream);
-    }
-    for (void *p : ptrs) cudaFree(p);
-    for (int i = 0; i < kNetTensors; ++i) cudaFree(c->net.t[i]);
-    if (c->pinned) cudaFreeHost(c->pinned);
-    if (c->sp_copy_stream) {
-        cudaStreamSynchronize(c->sp_copy_stream);
-        for (int i = 0; i < omk_ctx::kSpRing; ++i) {
-            cudaEventDestroy(c->sp_ev_rec[i][0]);
-            cudaEventDestroy(c->sp_ev_rec[i][1]);
-            cudaEventDestroy(c->sp_ev_copy[i]);
-        }
-        cudaStreamDestroy(c->sp_copy_stream);
-    }
-    cudaFree(c->sp_ring_dev);
-    if (c->sp_ring_host) cudaFreeHost(c->sp_ring_host);
-    replay_free(c);
-    if (c->rp.stream) {
-        cudaEventDestroy(c->rp.ev_commit);
-        cudaStreamDestroy(c->rp.stream);
-    }
-    for (cudaEvent_t e : c->prof_pool) cudaEventDestroy(e);
-    cudaEventDestroy(c->ev0);
-    cudaEventDestroy(c->ev1);
-    cudaStreamDestroy(c->stream);
     delete c;
     return OMK_OK;
 }
@@ -651,7 +602,7 @@ extern "C" int32_t omk_debug_get_buffer(omk_ctx *c, int32_t which, float *out, i
         CK(cudaStreamSynchronize(c->stream));
         return OMK_OK;
     }
-    const float *src = which == 0 ? c->ws.act0 : which == 1 ? c->ws.act1 : which == 2 ? c->ws.act2 : which == 3 ? c->ws.logits : nullptr;
+    const float *src = which == 0 ? c->ws.act0 : which == 1 ? c->ws.act1 : which == 2 ? c->ws.act2 : which == 3 ? c->ws.logits.get() : nullptr;
     if (!src || !out || count < 0) return fail(OMK_ERR_INVALID, "bad buffer id");
     CK(copy_d2h(c, out, src, sizeof(float) * (size_t)count, c->stream));
     CK(cudaStreamSynchronize(c->stream));
@@ -1028,9 +979,8 @@ static SpSlot sp_slot_layout(int n) {
     s.bytes = s.off_status + up((size_t)n);
     return s;
 }
-static SpLayout sp_layout(omk_ctx *c, int n) {
+static SpLayout sp_layout(uint8_t *base, int n) {
     SpLayout L;
-    uint8_t *base = reinterpret_cast<uint8_t *>(c->sp_buf);
     size_t off = 0;
     auto take = [&](size_t bytes) { uint8_t *p = base + off; off = (off + bytes + 255) & ~(size_t)255; return p; };
     L.mover = reinterpret_cast<int32_t *>(take(sizeof(int32_t) * (size_t)n));
@@ -1052,7 +1002,7 @@ static int32_t sp_refresh_root_policy(omk_ctx *c) {
     if (!c->sp_active || c->sp_cfg.evaluator != OMK_EVAL_NET) return OMK_OK;
     int32_t rc = ensure_workspace(c, 1);
     if (rc) return rc;
-    const SpLayout L = sp_layout(c, c->sp_cfg.n_games);
+    const SpLayout L = sp_layout(c->sp_buf, c->sp_cfg.n_games);
     const uint32_t one = 1;
     CK(cudaMemsetAsync(c->ws.nn_in, 0, sizeof(NNIn), c->stream));  // empty board, Black to move, EnvTurnMode::Player (== k_new_games' request)
     CK(copy_h2d(c, c->ws.n_req, &one, sizeof one, c->stream));
@@ -1073,27 +1023,28 @@ extern "C" int32_t omk_selfplay_begin(omk_ctx *c, const omk_selfplay_config *cfg
     const int rows = n * cfg->batch_size > 2 * n ? n * cfg->batch_size : 2 * n;
     rc = ensure_workspace(c, rows);
     if (rc) return rc;
+    // The driver's buffers are allocated into locals and committed together below: a failed allocation leaves no driver
+    // (sp_active false) rather than half of one.  Each old buffer is released before its successor is allocated.
+    c->sp_active = false;
     c->sp_cfg = *cfg;
-    cudaFree(c->sp_ply);
-    cudaFree(c->sp_buf);
-    c->sp_ply = nullptr;
-    c->sp_buf = nullptr;
-    CK(cudaMalloc(&c->sp_ply, sizeof(int32_t) * (size_t)n));
-    CK(cudaMemsetAsync(c->sp_ply, 0, sizeof(int32_t) * (size_t)n, c->stream));
-    const SpLayout L = sp_layout(c, n);
-    CK(cudaMalloc(&c->sp_buf, L.bytes));
-    CK(cudaMemsetAsync(c->sp_buf, 0, L.bytes, c->stream));
-    const SpLayout M = sp_layout(c, n);
-    // transition ring: device slots + pinned host mirror + copy stream + events
     const SpSlot slot = sp_slot_layout(n);
-    if (slot.bytes != c->sp_ring_slot_bytes) {
-        cudaFree(c->sp_ring_dev);
-        if (c->sp_ring_host) cudaFreeHost(c->sp_ring_host);
-        c->sp_ring_dev = c->sp_ring_host = nullptr;
+    const bool new_ring = slot.bytes != c->sp_ring_slot_bytes;
+    c->sp_ply.reset();
+    c->sp_buf.reset();
+    Buf<int32_t> ply;
+    Buf<uint8_t> buf, ring_dev;
+    PinnedBuf<uint8_t> ring_host;
+    CK(ply.alloc((size_t)n));
+    CK(cudaMemsetAsync(ply, 0, ply.bytes(), c->stream));
+    CK(buf.alloc(sp_layout(nullptr, n).bytes));
+    CK(cudaMemsetAsync(buf, 0, buf.bytes(), c->stream));
+    // transition ring: device slots + pinned host mirror + copy stream + events
+    if (new_ring) {
+        c->sp_ring_dev.reset();
+        c->sp_ring_host.reset();
         c->sp_ring_slot_bytes = 0;
-        CK(cudaMalloc(&c->sp_ring_dev, slot.bytes * omk_ctx::kSpRing));
-        CK(cudaHostAlloc(&c->sp_ring_host, slot.bytes * omk_ctx::kSpRing, cudaHostAllocDefault));
-        c->sp_ring_slot_bytes = slot.bytes;
+        CK(ring_dev.alloc(slot.bytes * omk_ctx::kSpRing));
+        CK(ring_host.alloc(slot.bytes * omk_ctx::kSpRing));
     }
     if (!c->sp_copy_stream) {
         CK(cudaStreamCreateWithFlags(&c->sp_copy_stream, cudaStreamNonBlocking));
@@ -1105,20 +1056,31 @@ extern "C" int32_t omk_selfplay_begin(omk_ctx *c, const omk_selfplay_config *cfg
     }
     // a replay memory that exists now is fed by this driver: staging for every game (the restart below drops the tails
     // of the previous driver's games, as omk_selfplay_begin restarts every game)
-    replay_free_staging(c);
-    if (c->rp.ring.cap > 0) {
-        Replay &r = c->rp;
+    Replay &r = c->rp;
+    if (r.stream) cudaStreamSynchronize(r.stream);  // the last commit reads the old staging
+    r.stage = ReplayStaging{};
+    ReplayStaging stage;
+    if (r.ring.cap > 0) {
         if (!r.stream) {
             CK(cudaStreamCreateWithFlags(&r.stream, cudaStreamNonBlocking));
             CK(cudaEventCreateWithFlags(&r.ev_commit, cudaEventDisableTiming));
         }
         const size_t cells = (size_t)n * kCells * kCells;  // 81 plies of 81 cells per game
-        CK(cudaMalloc(&r.stage_boards, cells));
-        CK(cudaMalloc(&r.stage_pi, cells * sizeof(float)));
-        CK(cudaMalloc(&r.stage_len, sizeof(int32_t) * (size_t)n));
-        CK(cudaMemsetAsync(r.stage_len, 0, sizeof(int32_t) * (size_t)n, c->stream));
-        r.stage_games = n;
+        CK(stage.boards.alloc(cells));
+        CK(stage.pi.alloc(cells));
+        CK(stage.len.alloc((size_t)n));
+        CK(cudaMemsetAsync(stage.len, 0, stage.len.bytes(), c->stream));
+        stage.games = n;
     }
+    c->sp_ply = std::move(ply);
+    c->sp_buf = std::move(buf);
+    if (new_ring) {
+        c->sp_ring_dev = std::move(ring_dev);
+        c->sp_ring_host = std::move(ring_host);
+        c->sp_ring_slot_bytes = slot.bytes;
+    }
+    r.stage = std::move(stage);
+    const SpLayout M = sp_layout(c->sp_buf, n);
     // Agent::new for all 2n trees (stream id = tree id); then cache the root's raw policy for restarts:
     // evaluating the empty board is deterministic, so reusing it is bit-identical to evaluating it again
     launch_reset_requests(c);
@@ -1143,7 +1105,7 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     const int n = cfg.n_games;
     const int rounds = (cfg.count + cfg.batch_size - 1) / cfg.batch_size;
 
-    const SpLayout L = sp_layout(c, n);
+    const SpLayout L = sp_layout(c->sp_buf, n);
     int32_t *mover = L.mover, *other = L.other, *actions = L.actions;
     float *temps = L.temps;
     uint8_t *modes = L.modes;
@@ -1163,7 +1125,7 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     // commit per ply on the replay stream, behind both lanes' record events, turns the episodes that ended into rows.  A
     // restarted game stages ply 0 over the finished episode, so each lane waits for the previous ply's commit before its
     // staging kernel -- one event wait per lane and ply, outside the search rounds.
-    const bool feed = c->rp.stage_games == n && c->rp.ring.cap > 0;
+    const bool feed = c->rp.stage.games == n && c->rp.ring.cap > 0;
     size_t d2h = 0;
     auto dev_slot = [&](int ply) { return c->sp_ring_dev + (size_t)(ply % kRing) * slot.bytes; };
     auto drain = [&](int ply) -> int32_t {  // pinned slot of `ply` -> the caller's arrays
@@ -1329,23 +1291,28 @@ extern "C" int32_t omk_replay_reset(omk_ctx *c, int64_t capacity) {
     if (capacity > 0 && r.ring.cap == 0 && c->sp_active)
         return fail(OMK_ERR_STATE, "a replay memory is fed by the self-play driver only if it exists at omk_selfplay_begin: create it first");
     CK(cudaStreamSynchronize(c->stream));
-    if (capacity == 0) {
-        replay_free(c);  // the driver stops feeding
+    if (capacity == 0) {  // the driver stops feeding
+        if (r.stream) cudaStreamSynchronize(r.stream);
+        r.stage = ReplayStaging{};
+        r.ring = ReplayStore{};
+        r.counters.reset();
+        r.added = r.len = r.episodes = 0;
         return OMK_OK;
     }
     if (capacity != r.ring.cap) {
         if (r.stream) CK(cudaStreamSynchronize(r.stream));
-        cudaFree(r.ring.boards); cudaFree(r.ring.turns); cudaFree(r.ring.pi); cudaFree(r.ring.z);
-        r.ring = ReplayRing{};
+        r.ring = ReplayStore{};
         const size_t cap = (size_t)capacity;
-        CK(cudaMalloc(&r.ring.boards, cap * kCells));
-        CK(cudaMalloc(&r.ring.turns, cap));
-        CK(cudaMalloc(&r.ring.pi, cap * kCells * sizeof(float)));
-        CK(cudaMalloc(&r.ring.z, cap * sizeof(float)));
-        r.ring.cap = capacity;
+        ReplayStore ring;
+        CK(ring.boards.alloc(cap * kCells));
+        CK(ring.turns.alloc(cap));
+        CK(ring.pi.alloc(cap * kCells));
+        CK(ring.z.alloc(cap));
+        ring.cap = capacity;
+        r.ring = std::move(ring);
     }
-    if (!r.counters) CK(cudaMalloc(&r.counters, sizeof(ReplayCounters)));
-    CK(cudaMemsetAsync(r.counters, 0, sizeof(ReplayCounters), c->stream));  // the staged tails of a running driver stay
+    if (!r.counters) CK(r.counters.alloc(1));
+    CK(cudaMemsetAsync(r.counters, 0, r.counters.bytes(), c->stream));  // the staged tails of a running driver stay
     CK(cudaStreamSynchronize(c->stream));
     r.added = r.len = r.episodes = 0;
     return OMK_OK;

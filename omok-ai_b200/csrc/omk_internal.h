@@ -1,7 +1,10 @@
 // omk_internal.h -- host-side context and kernel launcher prototypes (not part of the ABI).
 #pragma once
 #include <cstdint>
+#include <memory>
+#include <utility>
 #include <vector>
+#include <cuda.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
@@ -15,74 +18,165 @@ constexpr int kNetTensors = 31;
 
 enum ApplyMode { kApplySearch = 0, kApplyNewGame = 1, kApplyEnsure = 2 };
 
-struct NetWeights {
-    float *t[kNetTensors] = {};  // device copies in checkpoint order
-    float *heads_w = nullptr;    // [512][128]: cols 0..80 policy, col 81 value, rest 0
-    float *heads_b = nullptr;    // [128]
-    // fp16-split tensor-core path (fc_f16.cu, tower_f16.cu): weights scaled by a power of two, then split hi/lo
-    __half *fc0_wt_h16 = nullptr, *fc0_wt_l16 = nullptr;  // [512][10368] K-major
-    __half *fc1_wt_h16 = nullptr, *fc1_wt_l16 = nullptr;  // [512][512]
-    __half *heads_wt_h16 = nullptr, *heads_wt_l16 = nullptr;  // [128][512]: rows 0..80 policy, 81 value, rest 0
-    float *fc_inv_scale = nullptr;     // [3] 2^-s of fc0, fc1, heads
-    uint32_t *fc_absmax = nullptr;     // [3] max |w| bits
-    uint8_t *tower16_wimg = nullptr;   // 3 x 36 KB pre-swizzled B-operand images
-    float *tower16_pimg = nullptr;     // fp32 stem / bias / depthwise parameters + inverse scales
-    uint32_t *tower16_absmax = nullptr;  // [9]
+// Owner of one allocation of `count` T: device memory (DeviceMem), or pinned host memory (PinnedMem).  Move-only, released on
+// destruction; converts to the raw pointer, so kernels and launchers take T * unchanged.
+struct DeviceMem {
+    static cudaError_t alloc(void **p, size_t bytes) { return cudaMalloc(p, bytes); }
+    static void release(void *p) { cudaFree(p); }
+};
+struct PinnedMem {
+    static cudaError_t alloc(void **p, size_t bytes) { return cudaHostAlloc(p, bytes, cudaHostAllocDefault); }
+    static void release(void *p) { cudaFreeHost(p); }
+};
+template <typename T, typename Mem = DeviceMem>
+class Buf {
+  public:
+    Buf() = default;
+    Buf(const Buf &) = delete;
+    Buf &operator=(const Buf &) = delete;
+    Buf(Buf &&o) noexcept : p_(std::exchange(o.p_, nullptr)), count_(std::exchange(o.count_, 0)) {}
+    Buf &operator=(Buf &&o) noexcept {
+        if (this != &o) {
+            reset();
+            p_ = std::exchange(o.p_, nullptr);
+            count_ = std::exchange(o.count_, 0);
+        }
+        return *this;
+    }
+    ~Buf() { reset(); }
+    operator T *() const { return p_; }
+    T *get() const { return p_; }
+    size_t bytes() const { return sizeof(T) * count_; }
+    void reset() {
+        if (p_) Mem::release(p_);
+        p_ = nullptr;
+        count_ = 0;
+    }
+    // release the current allocation, then allocate `count` elements (on failure the handle is left empty)
+    cudaError_t alloc(size_t count) {
+        reset();
+        void *p = nullptr;
+        const cudaError_t e = Mem::alloc(&p, sizeof(T) * count);
+        if (e != cudaSuccess) return e;
+        p_ = static_cast<T *>(p);
+        count_ = count;
+        return cudaSuccess;
+    }
+    // grow-only: a request beyond the capacity synchronises `s` (work queued there may still use the old allocation), then
+    // allocates `count` rounded up to a multiple of `round` elements
+    cudaError_t grow(cudaStream_t s, size_t count, size_t round = 1) {
+        if (count <= count_) return cudaSuccess;
+        const cudaError_t e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return e;
+        return alloc((count + round - 1) / round * round);
+    }
+
+  private:
+    T *p_ = nullptr;
+    size_t count_ = 0;
+};
+template <typename T>
+using PinnedBuf = Buf<T, PinnedMem>;
+
+// Each group below is allocated into a local instance and moved into its owner only when every allocation succeeded, so no
+// call can find half a group.
+struct FcImages {  // fp16-split tensor-core path (fc_f16.cu): weights scaled by a power of two, then split hi/lo
+    Buf<__half> fc0_wt_h16, fc0_wt_l16;    // [512][10368] K-major
+    Buf<__half> fc1_wt_h16, fc1_wt_l16;    // [512][512]
+    Buf<__half> heads_wt_h16, heads_wt_l16;  // [128][512]: rows 0..80 policy, 81 value, rest 0
+    Buf<float> fc_inv_scale;               // [3] 2^-s of fc0, fc1, heads
+    Buf<uint32_t> fc_absmax;               // [3] max |w| bits
+};
+struct TowerImages {  // tower_f16.cu
+    Buf<uint8_t> tower16_wimg;       // 3 x 36 KB pre-swizzled B-operand images
+    Buf<float> tower16_pimg;         // fp32 stem / bias / depthwise parameters + inverse scales
+    Buf<uint32_t> tower16_absmax;    // [9]
+};
+struct NetWeights : FcImages, TowerImages {
+    Buf<float> t[kNetTensors];  // device copies in checkpoint order
+    Buf<float> heads_w;         // [512][128]: cols 0..80 policy, col 81 value, rest 0
+    Buf<float> heads_b;         // [128]
     bool loaded = false;
 };
 
-struct Workspace {  // evaluator request/response buffers [max_rows]; activation buffers [act_rows], allocated on first use
-    int max_rows = 0;
+struct ActMaps {  // tensor maps (fc_f16.cu) over one workspace's fp16 activation buffers
+    CUtensorMap map0_a_hi, map0_a_lo, map1_a_hi, map1_a_lo, map2_a_hi, map2_a_lo;
+    CUtensorMap tower_st_hi, tower_st_lo;  // k_tower16's write-out into act0
+};
+struct Activations {  // activation buffers [act_rows] of the network, allocated on first use (ensure_activations)
     int act_rows = 0;
-    bool act_fp32 = false;        // the fp32 buffers of the CUDA-core A/B kernels exist (act0, act1)
-    NNIn *nn_in = nullptr;        // [max_rows]
-    uint32_t *req_tree = nullptr; // [max_rows]
-    uint32_t *req_node = nullptr; // [max_rows]
-    float *P = nullptr;           // [max_rows][96]
-    float *V = nullptr;           // [max_rows]
-    __half *act0_h16 = nullptr, *act0_l16 = nullptr;  // [act_rows][10368] fp16 hi/lo split of the tower output == fc0's A operand
-    __half *act1_h16 = nullptr, *act1_l16 = nullptr;  // [act_rows][512] fp16 hi/lo split of fc0's output == fc1's A operand
-    __half *act2_h16 = nullptr, *act2_l16 = nullptr;  // [act_rows][512] fp16 hi/lo split of fc1's output == the heads' A operand
-    float *act2 = nullptr;        // [act_rows][512] fc1 output (fp32: CUDA-core heads, debugging)
-    float *logits = nullptr;      // [act_rows][128]
-    float *act0 = nullptr;        // [act_rows][10368] fp32 tower output (CUDA-core A/B kernels only)
-    float *act1 = nullptr;        // [act_rows][512]   fp32 fc0 output   (CUDA-core A/B kernels only)
-    uint32_t *n_req = nullptr;    // device counter
-    uint32_t *slot_base = nullptr, *slot_count = nullptr;  // [capacity_trees]
-    int32_t *ids = nullptr;       // [capacity_trees] device copy of the call's id list
-    int32_t *actions = nullptr;   // [capacity_trees]
-    uint8_t *modes = nullptr;     // [capacity_trees]
-    float *temps = nullptr;       // [capacity_trees]
-    int8_t *status = nullptr;     // [capacity_trees]
-    float *policy_out = nullptr;  // [capacity_trees][81]
-    uint32_t *streams = nullptr;  // [capacity_trees]
+    bool act_fp32 = false;            // the fp32 buffers of the CUDA-core A/B kernels exist (act0, act1)
+    Buf<__half> act0_h16, act0_l16;   // [act_rows][10368] fp16 hi/lo split of the tower output == fc0's A operand
+    Buf<__half> act1_h16, act1_l16;   // [act_rows][512] fp16 hi/lo split of fc0's output == fc1's A operand
+    Buf<__half> act2_h16, act2_l16;   // [act_rows][512] fp16 hi/lo split of fc1's output == the heads' A operand
+    Buf<float> act2;                  // [act_rows][512] fc1 output (fp32: CUDA-core heads, debugging)
+    Buf<float> logits;                // [act_rows][128]
+    Buf<float> act0;                  // [act_rows][10368] fp32 tower output (CUDA-core A/B kernels only)
+    Buf<float> act1;                  // [act_rows][512]   fp32 fc0 output   (CUDA-core A/B kernels only)
+    ActMaps maps;                     // encoded with the buffers (fc16_encode_act_maps)
+};
+// One search lane's evaluator buffers (LaneScope in omk_api.cu swaps the whole workspace): request/response buffers
+// [max_rows], the activations, and the lane's fc0 scratch
+struct Workspace : Activations {
+    int max_rows = 0;
+    Buf<NNIn> nn_in;            // [max_rows]
+    Buf<uint32_t> req_tree;     // [max_rows]
+    Buf<uint32_t> req_node;     // [max_rows]
+    Buf<float> P;               // [max_rows][96]
+    Buf<float> V;               // [max_rows]
+    Buf<uint32_t> n_req;        // device counter
+    Buf<uint32_t> slot_base, slot_count;  // [capacity_trees]
+    Buf<int32_t> ids;           // [capacity_trees] device copy of the call's id list
+    Buf<int32_t> actions;       // [capacity_trees]
+    Buf<uint8_t> modes;         // [capacity_trees]
+    Buf<float> temps;           // [capacity_trees]
+    Buf<int8_t> status;         // [capacity_trees]
+    Buf<float> policy_out;      // [capacity_trees][81]
+    Buf<uint32_t> streams;      // [capacity_trees]
+    Buf<float> splitk_partial;  // [chunks][rows][512] fp32 partial sums of the split-K fc0 (grow-only)
+    Buf<float4> bal_partial;    // tail-balancing scratch of the pair fc0: [units][F_BAL_UNIT_F4] (grow-only)
+    Buf<uint32_t> bal_flags;    // [256]
 };
 
 // Replay memory on the device (replay_kernels.cu; DESIGN.md 2).  Row a (absolute: rows added since the last reset) lives
 // at a % cap; logical row i (0 = oldest) is absolute row added - len + i.
-struct ReplayRing {
-    uint8_t *boards = nullptr;  // [cap][81]
-    uint8_t *turns = nullptr;   // [cap]
-    float *pi = nullptr;        // [cap][81]
-    float *z = nullptr;         // [cap]
+struct ReplayRing {  // kernel argument: a view of ReplayStore
+    uint8_t *boards;  // [cap][81]
+    uint8_t *turns;   // [cap]
+    float *pi;        // [cap][81]
+    float *z;         // [cap]
+    long long cap;
+};
+struct ReplayStore {
+    Buf<uint8_t> boards, turns;
+    Buf<float> pi, z;
     long long cap = 0;
+    ReplayRing view() const { return {boards, turns, pi, z, cap}; }
 };
 struct ReplayCounters {  // device; advanced by the per-ply commit
     long long added, len, episodes;
     uint32_t done, pad;  // arrival counter of the commit's blocks (re-armed)
 };
+struct ReplayStaging {  // the driver's unfinished games: [games][81 plies][81] boards and policies, [games] ply counts
+    int games = 0;      // 0: the driver does not feed the replay
+    Buf<uint8_t> boards;
+    Buf<float> pi;
+    Buf<int32_t> len;
+};
 struct Replay {
-    ReplayRing ring;
-    ReplayCounters *counters = nullptr;
+    ReplayStore ring;
+    Buf<ReplayCounters> counters;
     long long added = 0, len = 0, episodes = 0;  // host copy of *counters, refreshed by omk_selfplay_run
-    // staging of the driver's unfinished games: [games][81 plies][81] boards and policies, [games] ply counts
-    int stage_games = 0;  // 0: the driver does not feed the replay
-    uint8_t *stage_boards = nullptr;
-    float *stage_pi = nullptr;
-    int32_t *stage_len = nullptr;
+    ReplayStaging stage;
     cudaStream_t stream = nullptr;      // the per-ply commits
     cudaEvent_t ev_commit = nullptr;    // the last commit enqueued
 };
+
+// opaque to this header; their deleters live with them
+struct Fc16State;
+struct TrainState;
+struct Fc16StateFree { void operator()(Fc16State *s) const; };   // fc_f16.cu
+struct TrainStateFree { void operator()(TrainState *t) const; };  // train_kernels.cu
 
 }  // namespace omk
 
@@ -92,6 +186,7 @@ struct omk_prof_span {
 };
 
 struct omk_ctx {
+    ~omk_ctx();  // synchronises every stream of the context before any buffer is released (omk_api.cu)
     int device = 0;
     // profiling spans (CUDA events on the context stream); level 0 none, 1 fc0 only, 2 all families
     int prof_level = 0;
@@ -113,16 +208,16 @@ struct omk_ctx {
     int lane_min_trees = 768;       // searches over fewer trees stay on one lane: each lane should still fill an fc0 wave (env OMK_LANE_MIN_TREES; 0 disables lanes)
     // grow-only device scratch of the granular host-buffer calls (env_step, env_get, net_eval, ...): no cudaMalloc /
     // cudaFree (an implicit device synchronisation each) per call, nothing to leak on an error return
-    struct Scratch { void *p = nullptr; size_t cap = 0; } scratch[3];
+    omk::Buf<uint8_t> scratch[3];
     std::vector<uint8_t> id_seen;   // host scratch of stage_ids: duplicate detection over an id list
     int id_base = 0;                // first tree id of the lane in use when the id list is the identity
 
-    omk::EnvRec *envs = nullptr;
-    omk::TreeHdr *tree_hdrs = nullptr;
-    uint8_t *tree_nodes = nullptr;   // [cap_trees][cap_nodes][kNodeBytes]
-    uint16_t *remap = nullptr;       // [cap_trees][cap_nodes] compaction scratch
-    uint32_t *dev_error = nullptr;   // sticky device error word
-    unsigned long long *dev_sims = nullptr;  // simulations counter
+    omk::Buf<omk::EnvRec> envs;
+    omk::Buf<omk::TreeHdr> tree_hdrs;
+    omk::Buf<uint8_t> tree_nodes;    // [cap_trees][cap_nodes][kNodeBytes]
+    omk::Buf<uint16_t> remap;        // [cap_trees][cap_nodes] compaction scratch
+    omk::Buf<uint32_t> dev_error;    // sticky device error word
+    omk::Buf<unsigned long long> dev_sims;  // simulations counter
 
     omk::NetWeights net;
     omk::Workspace ws;
@@ -130,10 +225,10 @@ struct omk_ctx {
     int fc0_balance = 0;            // fc0 tail balancing of the CTA-pair kernel (fc_f16.cu FcBal): 0 off (default), 1 on
     int fc0_chunk = 9;              // k-blocks of fc0 accumulated in tensor memory per drain: 9 (default) or 3 (finer, more accurate; fc_f16.cu)
     int fc0_mode = 1;               // fc0 + fc1: 1 = tcgen05 3xFP16 k_fc16 (the product path), 0 = fp32 CUDA-core k_gemm (A/B check only)
-    void *fc16_state = nullptr;     // tensor maps of the fp16-split path (fc_f16.cu)
+    std::unique_ptr<omk::Fc16State, omk::Fc16StateFree> fc16_state;  // weight tensor maps of the fp16-split path (fc_f16.cu)
     int tower16_pairs = 0;          // resident CTA pairs of k_tower16 (0 = not queried yet)
-    void *tower16_params_host = nullptr;  // host copy of the tower's fp32 parameter image (kernel argument of k_tower16)
-    void *train_state = nullptr;    // trainer step workspace, Adadelta slots, optional NCCL communicator (train_kernels.cu)
+    std::vector<uint8_t> tower16_params_host;  // host copy of the tower's fp32 parameter image (kernel argument of k_tower16)
+    std::unique_ptr<omk::TrainState, omk::TrainStateFree> train_state;  // trainer step workspace, Adadelta slots, optional NCCL communicator (train_kernels.cu)
     int train_n = 0;                // positions of the minibatch currently on the device (omk_train_backward)
     bool net_pack_dirty = false;    // omk_train_apply changed the fp32 weights: the tensor-core operand images (and a running self-play
                                     // driver's cached root prior) are rebuilt before the next network evaluation (ensure_packed in omk_api.cu)
@@ -142,20 +237,18 @@ struct omk_ctx {
     // self-play driver state
     omk_selfplay_config sp_cfg{};
     bool sp_active = false;
-    int32_t *sp_ply = nullptr;        // [n_games] device ply counters
-    void *sp_buf = nullptr;           // per-game scratch (ids, actions, modes, status, cached root policy)
+    omk::Buf<int32_t> sp_ply;         // [n_games] device ply counters
+    omk::Buf<uint8_t> sp_buf;         // per-game scratch (ids, actions, modes, status, cached root policy)
     // Transition ring of the self-play driver (BASELINE config 4: positions streamed to the host replay buffer): kSpRing
     // ply slots on the device, mirrored in pinned host memory; a ply's slice leaves on `sp_copy_stream` while the next
     // plies search.  Allocated by omk_selfplay_begin for sp_cfg.n_games.
     static constexpr int kSpRing = 4;
-    uint8_t *sp_ring_dev = nullptr, *sp_ring_host = nullptr;  // kSpRing x [boards n*81 | policy n*81 f32 | actions n i32 | status n]
+    omk::Buf<uint8_t> sp_ring_dev;    // kSpRing x [boards n*81 | policy n*81 f32 | actions n i32 | status n]
+    omk::PinnedBuf<uint8_t> sp_ring_host;
     size_t sp_ring_slot_bytes = 0;
     cudaStream_t sp_copy_stream = nullptr;
     cudaEvent_t sp_ev_rec[kSpRing][2] = {}, sp_ev_copy[kSpRing] = {};
     omk::Replay rp;                   // device replay memory (omk_replay_reset); fed by the driver when it exists at omk_selfplay_begin
-    // pinned host staging
-    void *pinned = nullptr;
-    size_t pinned_bytes = 0;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
@@ -222,9 +315,8 @@ bool fc16_prepare_weights(omk_ctx *c);
 bool launch_fc0_f16(omk_ctx *c, int rows_bound);
 bool launch_fc1_f16(omk_ctx *c, int rows_bound);
 bool launch_heads_f16(omk_ctx *c, int rows_bound);
-void fc16_free(omk_ctx *c);
-// tensor maps (CUtensorMap) of k_tower16's TMA write-out over the current workspace's act0_h16 / act0_l16
-bool fc16_tower_store_maps(omk_ctx *c, const void **map_hi, const void **map_lo);
+// encode a.maps over a's fp16 buffers (ensure_activations, whenever it (re)allocates them)
+bool fc16_encode_act_maps(Activations &a);
 void launch_f32_to_split16(omk_ctx *c, const float *x, __half *hi, __half *lo, long long n);
 void launch_split16_to_f32(omk_ctx *c, const __half *hi, const __half *lo, float *x, long long n);
 
@@ -239,7 +331,6 @@ const char *train_backward_resident(omk_ctx *c, int n);
 const char *train_report_losses_device(omk_ctx *c, int n, float *dst3);
 float *train_grad_buffer(omk_ctx *c);
 void train_reset_optimizer(omk_ctx *c);
-void train_free(omk_ctx *c);
 const char *train_comm_unique_id(omk_ctx *c, uint8_t *out128);
 const char *train_comm_init(omk_ctx *c, const uint8_t *id128, int nranks, int rank);
 const char *train_comm_destroy(omk_ctx *c);

@@ -258,13 +258,13 @@ __global__ void k_rp_get(const int64_t *__restrict__ rows, int n, ReplayRing rin
 // ---------------------------------------------------------------------------------------
 void launch_rp_stage(omk_ctx *c, int g0, int n, const uint8_t *boards, const float *policy) {
     if (n <= 0) return;
-    k_rp_stage<<<n, 96, 0, c->stream>>>(g0, n, c->sp_ply, boards, policy, c->rp.stage_boards, c->rp.stage_pi, c->rp.stage_len);
+    k_rp_stage<<<n, 96, 0, c->stream>>>(g0, n, c->sp_ply, boards, policy, c->rp.stage.boards, c->rp.stage.pi, c->rp.stage.len);
     c->launches++;
 }
 void launch_rp_commit(omk_ctx *c, int n, const int8_t *status) {
     const int blocks = n < c->n_sms ? n : c->n_sms;
-    k_rp_commit<<<blocks, kCommitThreads, 0, c->rp.stream>>>(n, status, c->rp.stage_len, c->rp.stage_boards, c->rp.stage_pi,
-                                                             c->rp.ring, c->rp.counters);
+    k_rp_commit<<<blocks, kCommitThreads, 0, c->rp.stream>>>(n, status, c->rp.stage.len, c->rp.stage.boards, c->rp.stage.pi,
+                                                             c->rp.ring.view(), c->rp.counters);
     c->launches++;
 }
 void launch_rp_sample(omk_ctx *c, uint64_t seed, long long first_step, int steps, long long len, int m, int64_t *rows) {
@@ -274,11 +274,11 @@ void launch_rp_sample(omk_ctx *c, uint64_t seed, long long first_step, int steps
     c->launches++;
 }
 void launch_rp_gather(omk_ctx *c, const int64_t *rows, int m, float *img, float *pi, float *z) {
-    k_rp_gather<<<m, 96, 0, c->stream>>>(rows, m, c->rp.ring, c->rp.added - c->rp.len, img, pi, z);
+    k_rp_gather<<<m, 96, 0, c->stream>>>(rows, m, c->rp.ring.view(), c->rp.added - c->rp.len, img, pi, z);
     c->launches++;
 }
 void launch_rp_get(omk_ctx *c, const int64_t *rows, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z) {
-    k_rp_get<<<n, 96, 0, c->stream>>>(rows, n, c->rp.ring, c->rp.added - c->rp.len, boards, turns, pi, z);
+    k_rp_get<<<n, 96, 0, c->stream>>>(rows, n, c->rp.ring.view(), c->rp.added - c->rp.len, boards, turns, pi, z);
     c->launches++;
 }
 

@@ -867,9 +867,11 @@ __global__ void k_tower16_pack(Tower16PackArgs a, const uint32_t *absmax, uint8_
 bool tower16_prepare_weights(omk_ctx *c) {
     NetWeights &w = c->net;
     if (!w.tower16_wimg) {
-        if (cudaMalloc(&w.tower16_wimg, 3 * W16_BYTES) != cudaSuccess) return false;
-        if (cudaMalloc(&w.tower16_pimg, sizeof(float) * P16_FLOATS) != cudaSuccess) return false;
-        if (cudaMalloc(&w.tower16_absmax, sizeof(uint32_t) * 18) != cudaSuccess) return false;
+        TowerImages t;
+        if (t.tower16_wimg.alloc(3 * W16_BYTES) != cudaSuccess || t.tower16_pimg.alloc(P16_FLOATS) != cudaSuccess ||
+            t.tower16_absmax.alloc(18) != cudaSuccess)
+            return false;
+        static_cast<TowerImages &>(w) = std::move(t);
     }
     Tower16PackArgs a;
     a.conv_w = w.t[0];
@@ -885,9 +887,8 @@ bool tower16_prepare_weights(omk_ctx *c) {
     k_tower16_pack<<<16, 256, 0, c->stream>>>(a, w.tower16_absmax, w.tower16_wimg, w.tower16_pimg);
     c->launches += 2;
     // the fp32 parameter image is passed to k_tower16 by value (constant bank): keep a host copy
-    if (!c->tower16_params_host) c->tower16_params_host = malloc(sizeof(Tower16Params));
-    if (!c->tower16_params_host) return false;
-    if (cudaMemcpyAsync(c->tower16_params_host, w.tower16_pimg, sizeof(Tower16Params), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return false;
+    c->tower16_params_host.resize(sizeof(Tower16Params));
+    if (cudaMemcpyAsync(c->tower16_params_host.data(), w.tower16_pimg, sizeof(Tower16Params), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return false;
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return false;
     return true;
 }
@@ -950,15 +951,14 @@ bool launch_tower_f16(omk_ctx *c, const float *images_dev, int rows_bound) {
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     const uint8_t *wimg = c->net.tower16_wimg;
-    if (!c->tower16_params_host) return false;
-    const Tower16Params &params = *reinterpret_cast<const Tower16Params *>(c->tower16_params_host);
+    if (c->tower16_params_host.empty()) return false;
+    const Tower16Params &params = *reinterpret_cast<const Tower16Params *>(c->tower16_params_host.data());
     const NNIn *nn_in = c->ws.nn_in;
     const uint32_t *n_req = c->ws.n_req;
-    const void *mh = nullptr, *ml = nullptr;  // tensor maps of the write-out over this workspace's act0 arrays
-    if (!fc16_tower_store_maps(c, &mh, &ml)) return false;
+    const ActMaps &maps = c->ws.maps;  // the write-out over this workspace's act0 arrays
     const float *pimg = c->net.tower16_pimg;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, wimg, params, nn_in, images_dev, n_req, rows_bound,
-                                             *reinterpret_cast<const CUtensorMap *>(mh), *reinterpret_cast<const CUtensorMap *>(ml), pimg);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, wimg, params, nn_in, images_dev, n_req, rows_bound, maps.tower_st_hi,
+                                             maps.tower_st_lo, pimg);
     if (e != cudaSuccess) fprintf(stderr, "omok_b200: cudaLaunchKernelEx(k_tower16): %s\n", cudaGetErrorString(e));
     c->launches++;
     return e == cudaSuccess;

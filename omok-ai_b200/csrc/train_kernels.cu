@@ -381,23 +381,27 @@ __global__ void k_adadelta(const AdadeltaTensors T, float *__restrict__ accum, f
 // ---------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------
-struct TrainState {
-    int cap_n = 0;  // positions the workspace is sized for
-    float *img = nullptr, *pi = nullptr, *z = nullptr;
-    float *x[4] = {};                      // residual stream after the stem and after each block: [n*81][128]
-    float *h0[3] = {}, *hd[3] = {}, *h1[3] = {};  // per block: conv0 out, depthwise out, pointwise out: [n*81][32]
-    float *a0 = nullptr, *a1 = nullptr;    // fc0 / fc1 outputs [n][512]
-    float *logits = nullptr, *vlogit = nullptr;
-    float *dx = nullptr, *dy = nullptr;    // [n*81][128] gradient of the residual stream / of a block's pre-activation sum
-    float *d32a = nullptr, *d32b = nullptr;  // [n*81][32]
-    float *da0 = nullptr, *da1 = nullptr, *dlogits = nullptr, *dvlogit = nullptr, *row_loss = nullptr;
-    float *losses = nullptr;               // [3] device
-    float *splitk = nullptr;               // split-K partial tiles (grow-only)
-    size_t splitk_cap = 0;
-    float *red_sums = nullptr;             // [kRedSlicesMax][9][32] slice sums of the depthwise weight gradients
-    uint32_t *red_done = nullptr;          // [32] arrival counters of that reduction (self re-arming)
-    float *grads = nullptr;                // flat [kTParams] in checkpoint order
-    float *accum = nullptr, *accum_update = nullptr;  // Adadelta slots, flat
+// The two buffer groups of the training state, each allocated into a local instance and committed whole (train_ensure)
+struct TrainBatch {  // per-minibatch buffers, sized for cap_n positions
+    int cap_n = 0;
+    Buf<float> img, pi, z;
+    Buf<float> x[4];                     // residual stream after the stem and after each block: [n*81][128]
+    Buf<float> h0[3], hd[3], h1[3];      // per block: conv0 out, depthwise out, pointwise out: [n*81][32]
+    Buf<float> a0, a1;                   // fc0 / fc1 outputs [n][512]
+    Buf<float> logits, vlogit;
+    Buf<float> dx, dy;                   // [n*81][128] gradient of the residual stream / of a block's pre-activation sum
+    Buf<float> d32a, d32b;               // [n*81][32]
+    Buf<float> da0, da1, dlogits, dvlogit, row_loss;
+};
+struct TrainOptimizer {
+    Buf<float> grads;                    // flat [kTParams] in checkpoint order
+    Buf<float> accum, accum_update;      // Adadelta slots, flat
+    Buf<float> losses;                   // [3] device
+    Buf<float> red_sums;                 // [kRedSlicesMax][9][32] slice sums of the depthwise weight gradients
+    Buf<uint32_t> red_done;              // [32] arrival counters of that reduction (self re-arming)
+};
+struct TrainState : TrainBatch, TrainOptimizer {
+    Buf<float> splitk;                   // split-K partial tiles (grow-only)
     long long off[kNetTensors + 1] = {};
     long long steps = 0;
     // NCCL (optional, loaded with dlopen)
@@ -407,7 +411,12 @@ struct TrainState {
     int (*p_comm_init_rank)(void **, int, const void * /* ncclUniqueId by value: 128 bytes */, int) = nullptr;
     int (*p_comm_destroy)(void *) = nullptr;
     const char *(*p_err)(int) = nullptr;
+    ~TrainState() {
+        if (comm && p_comm_destroy) p_comm_destroy(comm);
+        if (nccl_lib) dlclose(nccl_lib);
+    }
 };
+void TrainStateFree::operator()(TrainState *t) const { delete t; }
 struct NcclUniqueId { char internal[128]; };
 
 static TrainState *train_state(omk_ctx *c) {
@@ -419,66 +428,43 @@ static TrainState *train_state(omk_ctx *c) {
             o += kTLen[i];
         }
         t->off[kNetTensors] = o;
-        c->train_state = t;
+        c->train_state.reset(t);
     }
-    return reinterpret_cast<TrainState *>(c->train_state);
+    return c->train_state.get();
 }
 
-static TrainState *train_state(omk_ctx *c);
 static float *g_splitk_scratch(omk_ctx *c, size_t floats) {
     TrainState *t = train_state(c);
-    if (floats > t->splitk_cap) {
-        cudaStreamSynchronize(c->stream);
-        cudaFree(t->splitk);
-        t->splitk = nullptr;
-        t->splitk_cap = 0;
-        if (cudaMalloc(&t->splitk, sizeof(float) * floats) != cudaSuccess) return nullptr;
-        t->splitk_cap = floats;
-    }
-    return t->splitk;
-}
-
-static bool talloc(float **p, size_t count) {
-    cudaFree(*p);
-    *p = nullptr;
-    return cudaMalloc(p, sizeof(float) * (count ? count : 1)) == cudaSuccess;
+    return t->splitk.grow(c->stream, floats) == cudaSuccess ? t->splitk.get() : nullptr;
 }
 
 static bool train_ensure(omk_ctx *c, TrainState *t, int n) {
+    auto ok = [](auto &b, size_t count) { return b.alloc(count) == cudaSuccess; };
     if (!t->grads) {
-        if (!talloc(&t->grads, kTParams) || !talloc(&t->accum, kTParams) || !talloc(&t->accum_update, kTParams) || !talloc(&t->losses, 4))
+        TrainOptimizer o;
+        if (!ok(o.grads, kTParams) || !ok(o.accum, kTParams) || !ok(o.accum_update, kTParams) || !ok(o.losses, 4) ||
+            !ok(o.red_sums, (size_t)kRedSlicesMax * kTF) || !ok(o.red_done, 32))
             return false;
-        cudaMemsetAsync(t->accum, 0, sizeof(float) * kTParams, c->stream);
-        cudaMemsetAsync(t->accum_update, 0, sizeof(float) * kTParams, c->stream);
-        if (!talloc(&t->red_sums, (size_t)kRedSlicesMax * kTF) || cudaMalloc(&t->red_done, sizeof(uint32_t) * 32) != cudaSuccess) return false;
-        cudaMemsetAsync(t->red_done, 0, sizeof(uint32_t) * 32, c->stream);
+        cudaMemsetAsync(o.accum, 0, o.accum.bytes(), c->stream);
+        cudaMemsetAsync(o.accum_update, 0, o.accum_update.bytes(), c->stream);
+        cudaMemsetAsync(o.red_done, 0, o.red_done.bytes(), c->stream);
+        static_cast<TrainOptimizer &>(*t) = std::move(o);
     }
     if (n <= t->cap_n) return true;
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return false;
+    static_cast<TrainBatch &>(*t) = TrainBatch{};  // the old buffers go before the new ones are allocated
     const size_t N = (size_t)n, M = N * kCells;
-    bool ok = talloc(&t->img, N * 243) && talloc(&t->pi, N * kCells) && talloc(&t->z, N);
-    for (int i = 0; i < 4; ++i) ok = ok && talloc(&t->x[i], M * kTP);
-    for (int r = 0; r < 3; ++r) ok = ok && talloc(&t->h0[r], M * kTM) && talloc(&t->hd[r], M * kTM) && talloc(&t->h1[r], M * kTM);
-    ok = ok && talloc(&t->a0, N * kTF) && talloc(&t->a1, N * kTF) && talloc(&t->logits, N * kCells) && talloc(&t->vlogit, N) &&
-         talloc(&t->dx, M * kTP) && talloc(&t->dy, M * kTP) && talloc(&t->d32a, M * kTM) && talloc(&t->d32b, M * kTM) &&
-         talloc(&t->da0, N * kTF) && talloc(&t->da1, N * kTF) && talloc(&t->dlogits, N * kCells) && talloc(&t->dvlogit, N) &&
-         talloc(&t->row_loss, 2 * N);
-    t->cap_n = ok ? n : 0;
-    return ok;
-}
-
-void train_free(omk_ctx *c) {
-    if (!c->train_state) return;
-    TrainState *t = reinterpret_cast<TrainState *>(c->train_state);
-    if (t->comm && t->p_comm_destroy) t->p_comm_destroy(t->comm);
-    float *all[] = {t->img, t->pi, t->z, t->x[0], t->x[1], t->x[2], t->x[3], t->h0[0], t->h0[1], t->h0[2], t->hd[0], t->hd[1], t->hd[2],
-                    t->h1[0], t->h1[1], t->h1[2], t->a0, t->a1, t->logits, t->vlogit, t->dx, t->dy, t->d32a, t->d32b, t->da0, t->da1,
-                    t->dlogits, t->dvlogit, t->row_loss, t->losses, t->grads, t->accum, t->accum_update, t->splitk, t->red_sums};
-    for (float *p : all) cudaFree(p);
-    cudaFree(t->red_done);
-    if (t->nccl_lib) dlclose(t->nccl_lib);
-    delete t;
-    c->train_state = nullptr;
+    TrainBatch b;
+    bool all = ok(b.img, N * 243) && ok(b.pi, N * kCells) && ok(b.z, N);
+    for (int i = 0; i < 4; ++i) all = all && ok(b.x[i], M * kTP);
+    for (int r = 0; r < 3; ++r) all = all && ok(b.h0[r], M * kTM) && ok(b.hd[r], M * kTM) && ok(b.h1[r], M * kTM);
+    all = all && ok(b.a0, N * kTF) && ok(b.a1, N * kTF) && ok(b.logits, N * kCells) && ok(b.vlogit, N) && ok(b.dx, M * kTP) &&
+          ok(b.dy, M * kTP) && ok(b.d32a, M * kTM) && ok(b.d32b, M * kTM) && ok(b.da0, N * kTF) && ok(b.da1, N * kTF) &&
+          ok(b.dlogits, N * kCells) && ok(b.dvlogit, N) && ok(b.row_loss, 2 * N);
+    if (!all) return false;
+    b.cap_n = n;
+    static_cast<TrainBatch &>(*t) = std::move(b);
+    return true;
 }
 
 // tensor indices in checkpoint order
@@ -488,14 +474,14 @@ enum { B_W0 = 0, B_B0 = 1, B_DW = 2, B_PW = 3, B_B1 = 4, B_W2 = 5, B_B2 = 6 };
 // the reference network in fp32, keeping every layer the backward pass needs (network.rs:51-262)
 static void train_forward(omk_ctx *c, TrainState *t, int n) {
     cudaStream_t s = c->stream;
-    float *const *W = c->net.t;
+    const Buf<float> *W = c->net.t;
     const int M = n * kCells;
     GemmEpi e;
     e.bias = W[T_CONV_B];
     e.act = 1;
     tgemm<false, false>(c, t->img, W[T_CONV_W], t->x[0], M, kTP, 3, 3, kTP, kTP, e);  // stem: the 243-float slot read as [81][3]
     for (int r = 0; r < 3; ++r) {
-        float *const *B = W + T_BLK0 + 7 * r;
+        const Buf<float> *B = W + T_BLK0 + 7 * r;
         GemmEpi e0;
         e0.bias = B[B_B0];
         e0.act = 1;
@@ -530,8 +516,8 @@ static void train_forward(omk_ctx *c, TrainState *t, int n) {
 }
 
 static void train_losses(omk_ctx *c, TrainState *t, int n, bool with_grads) {
-    k_loss<<<(n + 7) / 8, 256, 0, c->stream>>>(t->logits, t->vlogit, t->pi, t->z, n, with_grads ? t->dlogits : nullptr,
-                                                with_grads ? t->dvlogit : nullptr, t->row_loss);
+    k_loss<<<(n + 7) / 8, 256, 0, c->stream>>>(t->logits, t->vlogit, t->pi, t->z, n, with_grads ? t->dlogits.get() : nullptr,
+                                                with_grads ? t->dvlogit.get() : nullptr, t->row_loss);
     k_loss_reduce<<<1, 32, 0, c->stream>>>(t->row_loss, n, t->losses);
     c->launches += 2;
 }
@@ -539,7 +525,7 @@ static void train_losses(omk_ctx *c, TrainState *t, int n, bool with_grads) {
 // gradients of the mean loss with respect to all 31 tensors, into t->grads (checkpoint order)
 static void train_backward(omk_ctx *c, TrainState *t, int n) {
     cudaStream_t s = c->stream;
-    float *const *W = c->net.t;
+    const Buf<float> *W = c->net.t;
     const int M = n * kCells;
     auto G = [&](int tensor) { return t->grads + t->off[tensor]; };
     GemmEpi none;
@@ -570,7 +556,7 @@ static void train_backward(omk_ctx *c, TrainState *t, int n) {
     c->launches += 9;
     // residual blocks, last to first (network-utils lib.rs:386-461; network.rs:108-111)
     for (int r = 2; r >= 0; --r) {
-        float *const *B = W + T_BLK0 + 7 * r;
+        const Buf<float> *B = W + T_BLK0 + 7 * r;
         const int gb = T_BLK0 + 7 * r;
         const long long tot32 = (long long)M * kTM;
         // (dy = the gradient through the block's last lrelu, written by the GEMM before this block)
