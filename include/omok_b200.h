@@ -305,6 +305,27 @@ OMK_API int32_t omk_replay_get(omk_ctx *ctx, const int64_t *rows, int32_t n, uin
 OMK_API int32_t omk_train_replay(omk_ctx *ctx, uint64_t seed, int64_t first_step, int32_t steps, int32_t n, float *out_losses,
                          int64_t *out_rows);
 
+/* ---------------------------------------------------------------- evaluation against the naive player
+ * The trainer's evaluation phase (src/trainer.rs:487-603) on the device.  The naive player (:506-537) takes the first
+ * empty cell, ascending, where place_stone is terminal (win or draw) for the side to move or, with the turn flipped, for
+ * the opponent; otherwise legal[below(legal_count)] over the ascending empty cells, drawn on the specified random stream
+ * (mix64(seed ^ K_NAIVE), stream id, counter from 0) (DESIGN.md 4); a forced move draws nothing.                      */
+/* the naive player's move for n positions: boards[n*81], turns[n]; streams[n] (NULL: i); out_actions[n] (OMK_NONE on a
+ * full board); out_forced[n] (may be NULL): 1 if the move wins, blocks or fills the last cell, 0 if it was drawn at random */
+OMK_API int32_t omk_naive_move(omk_ctx *ctx, const uint8_t *boards, const uint8_t *turns, int32_t n, uint64_t seed,
+                               const uint32_t *streams, int32_t *out_actions, uint8_t *out_forced);
+/* `episodes` games on the trees first_tree .. first_tree + episodes - 1 (tree stream = tree id; OMK_ERR_STATE if they
+ * overlap an active self-play driver's trees 0 .. 2 * n_games - 1).  The naive player is Black and moves first; game g's
+ * move at ply p (moves already played) uses stream g * 81 + p.  The model answers each move with ensure_action_exists +
+ * play_action, and moves with execute(count, batch_size, epsilon, alpha) + sample_action(Best) + play_action.  One host
+ * round trip per half-move (the live-game count); no host-to-device copy.  out_result[3] = {black (naive) wins, white
+ * (model) wins, draws}; out_moves[episodes*81] (may be NULL) = each game's moves in playing order, -1 past its end;
+ * out_status[episodes] (may be NULL) = final GameStatus; out_stats[4] (may be NULL) = {simulations, positions evaluated,
+ * moves played, host synchronisations}; out_gpu_ms (may be NULL) = CUDA-event time of the call on the context stream. */
+OMK_API int32_t omk_eval_naive(omk_ctx *ctx, int32_t episodes, int32_t first_tree, int32_t count, int32_t batch_size, float epsilon,
+                               float alpha, int32_t evaluator, uint64_t seed, int32_t *out_result, int8_t *out_moves,
+                               int8_t *out_status, int64_t *out_stats, float *out_gpu_ms);
+
 #ifdef __cplusplus
 }
 #endif

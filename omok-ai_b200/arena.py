@@ -6,6 +6,8 @@
   * `play_against_naive_player`  src/trainer.rs:487-603: the naive player takes the first legal move (ascending) that ends
                                  the game for itself, or that would end it for the opponent (a block); else a random
                                  legal move.  The model answers with ParallelMCTSExecutor::execute + Best.
+  * `play_against_naive_player_device`  the same evaluation as ONE call (omk_eval_naive): the naive player's move is a
+                                 kernel, and its random moves follow the specified stream of DESIGN.md 4.
 
 The reference plays its games one after another; games are independent, so all of them run concurrently here (one tree
 per game and model), which changes nothing for any single game.  The naive player's "does this move end the game?" test
@@ -120,3 +122,19 @@ def play_against_naive_player(ctx, episode_count: int = 100, count: int = 800, b
     if moves_out is not None:
         moves_out[:] = log
     return int(result[2]), int(result[3]), int(result[1])
+
+
+def play_against_naive_player_device(ctx, episode_count: int = 100, count: int = 800, batch_size: int = 16, epsilon: float = 0.25,
+                                     alpha: float = 0.03, evaluator: int = B.EVAL_NET, seed: int = 0, first_tree: int = 0,
+                                     moves_out: list | None = None):
+    """Returns (black_win, white_win, draw) like `play_against_naive_player`, from one `omk_eval_naive` call on the trees
+    first_tree .. first_tree + episode_count - 1 (no env slot is used).
+
+    The naive player's random choices do NOT come from numpy: game g's move at ply p (moves already played) draws
+    legal[below(legal_count)] on the specified stream (mix64(seed ^ K_NAIVE), g * 81 + p) (DESIGN.md 4), so any
+    implementation of that stream replays the games.  `moves_out`, if given, receives one list of actions per game."""
+    result, moves, _, _ = ctx.eval_naive(episode_count, count=count, batch_size=batch_size, epsilon=epsilon, alpha=alpha,
+                                         evaluator=evaluator, seed=seed, first_tree=first_tree)
+    if moves_out is not None:
+        moves_out[:] = [[int(a) for a in row if a >= 0] for row in moves]
+    return result

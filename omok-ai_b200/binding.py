@@ -144,6 +144,8 @@ def load_library():
     L.omk_replay_info.argtypes = [vp, P(i64), P(i64), P(i64)]
     L.omk_replay_get.argtypes = [vp, vp, i32, vp, vp, vp, vp]
     L.omk_train_replay.argtypes = [vp, u64, i64, i32, i32, vp, vp]
+    L.omk_naive_move.argtypes = [vp, vp, vp, i32, u64, vp, vp, vp]
+    L.omk_eval_naive.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, u64, vp, vp, vp, vp, P(f32)]
     for name in declared_symbols():
         fn = getattr(L, name)  # raises AttributeError if the library lacks a declared symbol
         if name not in ("omk_last_error", "omk_ctx_stream", "omk_ctx_launch_count"):
@@ -499,3 +501,34 @@ class Context:
         self._check(self.L.omk_train_replay(self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step), int(steps), int(n),
                                             _ptr(losses), _ptr(rows)))
         return (losses, rows) if want_rows else losses
+
+    # ---- evaluation against the naive player ----
+    def naive_move(self, boards, turns, seed: int, streams=None):
+        """The naive player's move for every position (DESIGN.md 4): (actions [n] i32, forced [n] u8: 1 if the move wins,
+        blocks or fills the last cell, 0 if it was drawn on stream streams[i] (default i) of key mix64(seed ^ K_NAIVE))."""
+        boards = np.ascontiguousarray(boards, dtype=np.uint8).reshape(-1, CELLS)
+        turns = np.ascontiguousarray(turns, dtype=np.uint8).reshape(-1)
+        n = boards.shape[0]
+        streams = None if streams is None else np.ascontiguousarray(streams, dtype=np.uint32).reshape(n)
+        actions = np.zeros(n, dtype=np.int32)
+        forced = np.zeros(n, dtype=np.uint8)
+        self._check(self.L.omk_naive_move(self.h, _ptr(boards), _ptr(turns), n, int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(streams),
+                                          _ptr(actions), _ptr(forced)))
+        return actions, forced
+
+    def eval_naive(self, episodes: int, count: int = 800, batch_size: int = 16, epsilon: float = 0.25, alpha: float = 0.03,
+                   evaluator: int = EVAL_NET, seed: int = 0, first_tree: int = 0):
+        """The trainer's evaluation against the naive player in one call, on trees first_tree .. first_tree + episodes - 1.
+        Returns (result (black/naive wins, white/model wins, draws), moves [episodes, 81] i8 (-1 past a game's end),
+        final status [episodes] i8, stats dict: simulations, nn_evals, moves, host_syncs, gpu_ms)."""
+        result = np.zeros(3, dtype=np.int32)
+        moves = np.zeros((episodes, CELLS), dtype=np.int8)
+        status = np.zeros(episodes, dtype=np.int8)
+        stats = np.zeros(4, dtype=np.int64)
+        gpu_ms = C.c_float()
+        self._check(self.L.omk_eval_naive(self.h, episodes, first_tree, count, batch_size, epsilon, alpha, evaluator,
+                                          int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(result), _ptr(moves), _ptr(status), _ptr(stats),
+                                          C.byref(gpu_ms)))
+        info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
+        info["gpu_ms"] = float(gpu_ms.value)
+        return (int(result[0]), int(result[1]), int(result[2])), moves, status, info

@@ -1,0 +1,199 @@
+// eval_kernels.cu -- the trainer's evaluation against the naive player (src/trainer.rs:487-603) on the device: the naive
+// player's move (:506-537) and the bookkeeping omk_eval_naive runs after every half-move.
+#include "omk_internal.h"
+
+namespace omk {
+
+constexpr unsigned kFullMask = 0xffffffffu;
+constexpr int kNaiveWarps = 4;
+constexpr int kAdvanceThreads = 1024;
+
+// The naive player's rule (DESIGN.md 4) for one position, the warp owning it: the first empty cell, ascending, where
+// place_stone is terminal for the mover or, on the same board with the turn flipped, for the opponent; else
+// legal[below(legal_count)] on the stream (key, stream, counter from 0).  A forced move draws nothing.
+__device__ __forceinline__ void naive_pick(const uint32_t *black, const uint32_t *white, uint32_t turn, uint64_t key, uint32_t stream,
+                                           int lane, int32_t *out_action, uint8_t *out_forced) {
+    uint32_t empty[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) empty[k] = ~(black[k] | white[k]);
+    empty[2] &= 0x1FFFFu;
+    const int legal = popc81(empty);
+    const uint32_t *mine = turn == 0 ? black : white, *theirs = turn == 0 ? white : black;
+    uint32_t hit[3];
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        const int a = lane + 32 * j;
+        bool ends = false;
+        if (a < kCells && bit81(empty, a)) {
+            if (legal == 1) {
+                ends = true;  // the last empty cell: Draw (or a win) for either side
+            } else {
+                uint32_t s[3] = {mine[0], mine[1], mine[2]}, o[3] = {theirs[0], theirs[1], theirs[2]};
+                set81(s, a);
+                set81(o, a);
+                ends = makes_five_scalar(s, a) || makes_five_scalar(o, a);
+            }
+        }
+        hit[j] = __ballot_sync(kFullMask, ends);
+    }
+    if (lane != 0) return;
+    int action = OMK_NONE;
+    uint8_t forced = 0;
+    if (hit[0] | hit[1] | hit[2]) {
+        action = hit[0] ? __ffs(hit[0]) - 1 : (hit[1] ? 32 + __ffs(hit[1]) - 1 : 64 + __ffs(hit[2]) - 1);
+        forced = 1;
+    } else if (legal > 0) {
+        uint32_t counter = 0;
+        action = nth_set81(empty, (int)rng_below(key, stream, counter, (uint32_t)legal));
+    }
+    *out_action = action;
+    if (out_forced) *out_forced = forced;
+}
+
+// One warp per position.  Positions come either as cells + turns (omk_naive_move; stream = streams[i] or i) or as the
+// root nodes of trees ids[i] (omk_eval_naive; game g = ids[i] - first_tree, stream = g * 81 + ply[g]).
+struct NaiveArgs {
+    const uint8_t *boards, *turns;  // [n][81], [n]; nullptr: the tree roots below
+    const uint32_t *streams;
+    const int32_t *ids;
+    const uint8_t *nodes;
+    int cap_nodes, first_tree;
+    const int32_t *ply;
+    int n;
+    uint64_t key;
+    int32_t *actions;
+    uint8_t *forced;
+};
+
+__global__ void __launch_bounds__(kNaiveWarps * 32) k_naive_move(NaiveArgs a) {
+    const int i = blockIdx.x * kNaiveWarps + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (i >= a.n) return;
+    uint32_t black[3], white[3], turn, stream;
+    if (a.boards) {
+        const uint8_t *b = a.boards + (size_t)i * kCells;
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            const int c = lane + 32 * j;
+            const uint8_t v = c < kCells ? b[c] : 0;
+            black[j] = __ballot_sync(kFullMask, v == 1);
+            white[j] = __ballot_sync(kFullMask, v == 2);
+        }
+        turn = a.turns[i];
+        stream = a.streams ? a.streams[i] : (uint32_t)i;
+    } else {
+        const int tree = a.ids[i];
+        const NodeHdr h = load_hdr(a.nodes + (size_t)tree * (size_t)a.cap_nodes * kNodeBytes);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            black[k] = h.black[k];
+            white[k] = h.white[k];
+        }
+        turn = h.turn;
+        const int g = tree - a.first_tree;
+        stream = (uint32_t)(g * kCells + a.ply[g]);
+    }
+    naive_pick(black, white, turn, a.key, stream, lane, a.actions + i, a.forced ? a.forced + i : nullptr);
+}
+
+// A fresh evaluation: live list = every game's tree, no move played, nothing tallied.
+__global__ void k_eval_init(int episodes, int first_tree, int32_t *ids, int32_t *ply, int8_t *moves, int8_t *final_status,
+                            int32_t *counters) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < episodes * kCells) moves[t] = -1;
+    if (t < episodes) {
+        ids[t] = first_tree + t;
+        ply[t] = 0;
+        final_status[t] = kInProgress;
+    }
+    if (t < 4) counters[t] = 0;
+}
+
+// After a half-move's k_play on the live trees ids[0..n): append each game's move to its record, tally and record the
+// games that ended, and compact the live list in place, stably (ascending game order is kept).  One block.
+// counters = {BlackWin, WhiteWin, Draw, live count}.
+__global__ void __launch_bounds__(kAdvanceThreads) k_eval_advance(int32_t *ids, int n, const int32_t *actions, const int8_t *status,
+                                                                  int first_tree, int32_t *ply, int8_t *moves, int8_t *final_status,
+                                                                  int32_t *counters, uint32_t *dev_error) {
+    __shared__ int warp_kept[kAdvanceThreads / 32];
+    __shared__ int kept_before;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) kept_before = 0;
+    __syncthreads();
+    for (int c0 = 0; c0 < n; c0 += kAdvanceThreads) {
+        const int i = c0 + threadIdx.x;
+        bool keep = false;
+        int32_t id = 0;
+        if (i < n) {
+            id = ids[i];
+            const int g = id - first_tree;
+            const int st = status[i];
+            moves[(size_t)g * kCells + ply[g]] = (int8_t)actions[i];
+            ply[g] += 1;
+            if (st == kInProgress) {
+                keep = true;
+            } else if (st == kDraw || st == kBlackWin || st == kWhiteWin) {
+                final_status[g] = (int8_t)st;
+                atomicAdd(&counters[st == kBlackWin ? 0 : (st == kWhiteWin ? 1 : 2)], 1);
+            } else {
+                atomicOr(dev_error, 8u);  // Option::None: the move was refused -- the game could never end
+            }
+        }
+        const uint32_t b = __ballot_sync(kFullMask, keep);
+        if (lane == 0) warp_kept[warp] = __popc(b);
+        __syncthreads();  // every id of this chunk has been read before any is overwritten
+        int dst = kept_before + __popc(b & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) dst += warp_kept[w];
+        if (keep) ids[dst] = id;
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < kAdvanceThreads / 32; ++w) kept_before += warp_kept[w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) counters[3] = kept_before;
+}
+
+// ---- launchers ----
+static NaiveArgs naive_args(int n, uint64_t key, int32_t *actions, uint8_t *forced) {
+    NaiveArgs a{};
+    a.n = n;
+    a.key = key;
+    a.actions = actions;
+    a.forced = forced;
+    return a;
+}
+void launch_naive_move_boards(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, const uint32_t *streams, int n, uint64_t key,
+                              int32_t *actions, uint8_t *forced) {
+    if (n <= 0) return;
+    NaiveArgs a = naive_args(n, key, actions, forced);
+    a.boards = boards;
+    a.turns = turns;
+    a.streams = streams;
+    k_naive_move<<<(n + kNaiveWarps - 1) / kNaiveWarps, kNaiveWarps * 32, 0, c->stream>>>(a);
+    c->launches++;
+}
+void launch_naive_move_trees(omk_ctx *c, const int32_t *ids, int n, int first_tree, const int32_t *ply, uint64_t key, int32_t *actions) {
+    if (n <= 0) return;
+    NaiveArgs a = naive_args(n, key, actions, nullptr);
+    a.ids = ids;
+    a.nodes = c->tree_nodes;
+    a.cap_nodes = c->cap_nodes;
+    a.first_tree = first_tree;
+    a.ply = ply;
+    k_naive_move<<<(n + kNaiveWarps - 1) / kNaiveWarps, kNaiveWarps * 32, 0, c->stream>>>(a);
+    c->launches++;
+}
+void launch_eval_init(omk_ctx *c, int episodes, int first_tree, int32_t *ids, int32_t *ply, int8_t *moves, int8_t *final_status,
+                      int32_t *counters) {
+    const int total = episodes * kCells;
+    k_eval_init<<<(total + 255) / 256, 256, 0, c->stream>>>(episodes, first_tree, ids, ply, moves, final_status, counters);
+    c->launches++;
+}
+void launch_eval_advance(omk_ctx *c, int32_t *ids, int n, const int32_t *actions, const int8_t *status, int first_tree, int32_t *ply,
+                         int8_t *moves, int8_t *final_status, int32_t *counters) {
+    k_eval_advance<<<1, kAdvanceThreads, 0, c->stream>>>(ids, n, actions, status, first_tree, ply, moves, final_status, counters,
+                                                          c->dev_error);
+    c->launches++;
+}
+
+}  // namespace omk

@@ -170,6 +170,7 @@ static int32_t check_device_error(omk_ctx *c) {
     if (e & 1u) return fail(OMK_ERR_CAPACITY, "a tree ran out of node slots (capacity_nodes=" + std::to_string(c->cap_nodes) + ")");
     if (e & 4u)
         return fail(OMK_ERR_STATE, "the self-play driver sampled a move its tree refused (play_action returned None): the transition stream of this call is not usable");
+    if (e & 8u) return fail(OMK_ERR_STATE, "the evaluation played a move its tree refused (play_action returned None): its result is not usable");
     if (e & 2u)
         return fail(OMK_ERR_NUMERIC, "the network produced a non-finite policy or value (activation beyond the fp16 operand range "
                                      "of the tensor-core path, |x| >= 65504, or non-finite weights)");
@@ -743,17 +744,10 @@ extern "C" int32_t omk_pool_new_games(omk_ctx *c, const int32_t *ids, int32_t n,
     return check_device_error(c);
 }
 
-extern "C" int32_t omk_pool_search(omk_ctx *c, const int32_t *ids, int32_t n, int32_t count, int32_t batch_size, float epsilon,
-                                   float alpha, int32_t evaluator) {
-    CK(cudaSetDevice(c->device));
-    int32_t rc = check_evaluator(c, evaluator);
-    if (rc) return rc;
-    if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
-    if (count < 0) return fail(OMK_ERR_INVALID, "count < 0");
-    const int32_t *d_ids;
-    rc = stage_ids(c, ids, n, &d_ids, c->cap_trees);
-    if (rc) return rc;
-    if (n == 0 || count == 0) return OMK_OK;
+// execute(count, batch_size, epsilon, alpha) on the n >= 1 trees of d_ids (nullptr: 0..n-1), queued on the context stream;
+// the caller checks the device error word
+static int32_t search_rounds(omk_ctx *c, const int32_t *d_ids, int n, int count, int batch_size, float epsilon, float alpha,
+                             int evaluator) {
     const int rounds = (count + batch_size - 1) / batch_size;  // parallel_mcts_executor.rs:39-42,207
     // large searches run as two lanes (halves of the id list) on two streams: per-tree results do not depend on the split
     const int lanes = lanes_for(c, n);
@@ -761,7 +755,7 @@ extern "C" int32_t omk_pool_search(omk_ctx *c, const int32_t *ids, int32_t n, in
     const int lane_first[2] = {0, lane_n[0]};
     for (int l = 0; l < lanes; ++l) {
         LaneScope scope(c, l, 0);
-        rc = ensure_workspace(c, lane_n[l] * batch_size);
+        int32_t rc = ensure_workspace(c, lane_n[l] * batch_size);
         if (rc) return rc;
     }
     if (lanes == 2) lanes_fork(c);
@@ -777,6 +771,22 @@ extern "C" int32_t omk_pool_search(omk_ctx *c, const int32_t *ids, int32_t n, in
         }
     }
     if (lanes == 2) lanes_join(c);
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_pool_search(omk_ctx *c, const int32_t *ids, int32_t n, int32_t count, int32_t batch_size, float epsilon,
+                                   float alpha, int32_t evaluator) {
+    CK(cudaSetDevice(c->device));
+    int32_t rc = check_evaluator(c, evaluator);
+    if (rc) return rc;
+    if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
+    if (count < 0) return fail(OMK_ERR_INVALID, "count < 0");
+    const int32_t *d_ids;
+    rc = stage_ids(c, ids, n, &d_ids, c->cap_trees);
+    if (rc) return rc;
+    if (n == 0 || count == 0) return OMK_OK;
+    rc = search_rounds(c, d_ids, n, count, batch_size, epsilon, alpha, evaluator);
+    if (rc) return rc;
     return check_device_error(c);
 }
 
@@ -1397,5 +1407,132 @@ extern "C" int32_t omk_train_replay(omk_ctx *c, uint64_t seed, int64_t first_ste
             for (int k = m; k < n; ++k) out_rows[(size_t)s * n + k] = -1;
     for (int i = 0; i < 3 * steps; ++i)
         if (!(out_losses[i] == out_losses[i]) || out_losses[i] > 3.0e38f) return fail(OMK_ERR_NUMERIC, "the training loss is not finite");
+    return OMK_OK;
+}
+
+// ------------------------------------------------------------------ evaluation against the naive player (src/trainer.rs:487-603)
+extern "C" int32_t omk_naive_move(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, uint64_t seed,
+                                  const uint32_t *streams, int32_t *out_actions, uint8_t *out_forced) {
+    CK(cudaSetDevice(c->device));
+    if (n < 0 || (n > 0 && (!boards || !turns || !out_actions))) return fail(OMK_ERR_INVALID, "bad arguments");
+    for (size_t i = 0; i < (size_t)n * kCells; ++i)
+        if (boards[i] > 2) return fail(OMK_ERR_INVALID, "a cell is not 0 (Empty), 1 (Black) or 2 (White)");
+    for (int32_t i = 0; i < n; ++i)
+        if (turns[i] > 1) return fail(OMK_ERR_INVALID, "a turn is not 0 (Black) or 1 (White)");
+    if (n == 0) return OMK_OK;
+    const size_t nn = (size_t)n;
+    uint8_t *d_pos = nullptr, *d_forced = nullptr;  // [boards n*81 | turns n]
+    uint32_t *d_sa = nullptr;                       // [streams n | actions n]
+    SCRATCH(0, nn * (kCells + 1), d_pos);
+    SCRATCH(1, 2 * nn, d_sa);
+    SCRATCH(2, nn, d_forced);
+    int32_t *d_actions = reinterpret_cast<int32_t *>(d_sa + nn);
+    CK(copy_h2d(c, d_pos, boards, nn * kCells, c->stream));
+    CK(copy_h2d(c, d_pos + nn * kCells, turns, nn, c->stream));
+    if (streams) CK(copy_h2d(c, d_sa, streams, sizeof(uint32_t) * nn, c->stream));
+    launch_naive_move_boards(c, d_pos, d_pos + nn * kCells, streams ? d_sa : nullptr, n, mix64(seed ^ kNaiveKey), d_actions,
+                             out_forced ? d_forced : nullptr);
+    CK(copy_d2h(c, out_actions, d_actions, sizeof(int32_t) * nn, c->stream));
+    if (out_forced) CK(copy_d2h(c, out_forced, d_forced, nn, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    return OMK_OK;
+}
+
+// fold every lane's pending request count into the evaluated-positions total (dev_sims[1])
+static void fold_requests(omk_ctx *c) {
+    if (c->lane1_stream) {
+        lanes_fork(c);
+        {
+            LaneScope scope(c, 1, 0);
+            launch_reset_requests(c);
+        }
+        lanes_join(c);
+    }
+    launch_reset_requests(c);
+}
+
+extern "C" int32_t omk_eval_naive(omk_ctx *c, int32_t episodes, int32_t first_tree, int32_t count, int32_t batch_size, float epsilon,
+                                  float alpha, int32_t evaluator, uint64_t seed, int32_t *out_result, int8_t *out_moves,
+                                  int8_t *out_status, int64_t *out_stats, float *out_gpu_ms) {
+    CK(cudaSetDevice(c->device));
+    if (!out_result) return fail(OMK_ERR_INVALID, "out_result is NULL");
+    if (episodes < 1 || first_tree < 0 || first_tree > c->cap_trees - episodes)
+        return fail(OMK_ERR_INVALID, "need episodes >= 1 and the trees first_tree .. first_tree + episodes - 1 inside capacity_trees");
+    if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
+    if (count < 1) return fail(OMK_ERR_INVALID, "count < 1");
+    if (c->sp_active && first_tree < 2 * c->sp_cfg.n_games)
+        return fail(OMK_ERR_STATE, "the trees overlap the active self-play driver's trees 0 .. 2 * n_games - 1");
+    int32_t rc = check_evaluator(c, evaluator);  // with the network: weights a training step changed are packed first
+    if (rc) return rc;
+    const int E = episodes;
+    const size_t e = (size_t)E;
+    // [simulations and evaluations before / after (4 u64) | counters (4 i32) | final status E | moves E*81] leave in one copy;
+    // then the live tree ids, the half-move's actions, each game's ply and the half-move's statuses
+    const size_t off_cnt = 32, off_fin = 48, off_moves = off_fin + e, out_bytes = off_moves + e * kCells;
+    const size_t off_ids = (out_bytes + 255) & ~(size_t)255, off_act = off_ids + 4 * e, off_ply = off_act + 4 * e, off_st = off_ply + 4 * e;
+    CK(c->eval_buf.grow(c->stream, off_st + e, 4096));
+    rc = ensure_workspace(c, E);
+    if (rc) return rc;
+    uint8_t *base = c->eval_buf;
+    unsigned long long *sims = reinterpret_cast<unsigned long long *>(base);
+    int32_t *counters = reinterpret_cast<int32_t *>(base + off_cnt);
+    int8_t *fin = reinterpret_cast<int8_t *>(base + off_fin), *moves = reinterpret_cast<int8_t *>(base + off_moves);
+    int32_t *ids = reinterpret_cast<int32_t *>(base + off_ids), *actions = reinterpret_cast<int32_t *>(base + off_act);
+    int32_t *ply = reinterpret_cast<int32_t *>(base + off_ply);
+    int8_t *status = reinterpret_cast<int8_t *>(base + off_st);
+    const uint64_t key = mix64(seed ^ kNaiveKey);
+
+    fold_requests(c);  // counts earlier calls left pending are not this call's
+    CK(cudaMemcpyAsync(sims, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev0, c->stream));
+    launch_eval_init(c, E, first_tree, ids, ply, moves, fin, counters);
+    // Agent::new for every game's tree (stream id = tree id)
+    launch_reset_requests(c);
+    launch_new_games(c, ids, E, nullptr, nullptr, nullptr);
+    RUN_EVAL(c, evaluator, E);
+    launch_apply(c, ids, E, kApplyNewGame);
+    int64_t n_moves = 0, syncs = 0;
+    int32_t n = E;
+    for (int half = 0; n > 0 && half < kCells; ++half) {  // a game ends after at most 81 moves
+        if (half % 2 == 0) {  // the naive player (Black), then ensure_action_exists + play_action in the model's tree
+            launch_naive_move_trees(c, ids, n, first_tree, ply, key, actions);
+            launch_reset_requests(c);
+            launch_ensure_prepare(c, ids, actions, n);
+            RUN_EVAL(c, evaluator, n);
+            launch_apply(c, ids, n, kApplyEnsure);
+        } else {  // the model (White): execute(count, batch_size, epsilon, alpha) + sample_action(Best)
+            rc = search_rounds(c, ids, n, count, batch_size, epsilon, alpha, evaluator);
+            if (rc) return rc;
+            launch_sample(c, ids, n, nullptr, nullptr, actions, nullptr, nullptr);
+        }
+        launch_play(c, ids, actions, n, status);
+        launch_eval_advance(c, ids, n, actions, status, first_tree, ply, moves, fin, counters);
+        n_moves += n;
+        // the half-move's one host round trip: the live count sizes the next launches
+        CK(copy_d2h(c, &n, counters + 3, sizeof n, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        ++syncs;
+    }
+    fold_requests(c);
+    CK(cudaMemcpyAsync(sims + 2, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev1, c->stream));
+    std::vector<uint8_t> host(out_bytes);
+    CK(copy_d2h(c, host.data(), base, out_bytes, c->stream));
+    rc = check_device_error(c);  // (synchronises the stream)
+    ++syncs;
+    if (rc) return rc;
+    const unsigned long long *h_sims = reinterpret_cast<const unsigned long long *>(host.data());
+    const int32_t *h_cnt = reinterpret_cast<const int32_t *>(host.data() + off_cnt);
+    for (int k = 0; k < 3; ++k) out_result[k] = h_cnt[k];
+    if (out_status) memcpy(out_status, host.data() + off_fin, e);
+    if (out_moves) memcpy(out_moves, host.data() + off_moves, e * kCells);
+    if (out_stats) {
+        out_stats[0] = (int64_t)(h_sims[2] - h_sims[0]);
+        out_stats[1] = (int64_t)(h_sims[3] - h_sims[1]);
+        out_stats[2] = n_moves;
+        out_stats[3] = syncs;
+    }
+    if (out_gpu_ms) CK(cudaEventElapsedTime(out_gpu_ms, c->ev0, c->ev1));
     return OMK_OK;
 }

@@ -132,6 +132,8 @@ __host__ __device__ __forceinline__ uint32_t rng_u32(uint64_t seed, uint32_t str
     const uint64_t k = mix64(seed + kGolden * ((uint64_t)stream + 1));
     return (uint32_t)(mix64(k + kGolden * ((uint64_t)counter + 1)) >> 32);
 }
+// the naive player's random moves run on the key mix64(seed ^ kNaiveKey) (eval_kernels.cu)
+constexpr uint64_t kNaiveKey = 0xA0761D6478BD642Full;
 // rand 0.8.5 UniformInt::<u32>::sample_single (widening multiply + conservative zone)
 __device__ __forceinline__ uint32_t rng_below(uint64_t seed, uint32_t stream, uint32_t &counter, uint32_t bound) {
     const uint32_t zone = (bound << __clz(bound)) - 1u;

@@ -249,6 +249,7 @@ struct omk_ctx {
     cudaStream_t sp_copy_stream = nullptr;
     cudaEvent_t sp_ev_rec[kSpRing][2] = {}, sp_ev_copy[kSpRing] = {};
     omk::Replay rp;                   // device replay memory (omk_replay_reset); fed by the driver when it exists at omk_selfplay_begin
+    omk::Buf<uint8_t> eval_buf;       // omk_eval_naive's per-call state (grow-only)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
@@ -297,6 +298,17 @@ void launch_rp_commit(omk_ctx *c, int n, const int8_t *status);
 void launch_rp_sample(omk_ctx *c, uint64_t seed, long long first_step, int steps, long long len, int m, int64_t *rows);
 void launch_rp_gather(omk_ctx *c, const int64_t *rows, int m, float *img, float *pi, float *z);
 void launch_rp_get(omk_ctx *c, const int64_t *rows, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z);
+
+// eval_kernels.cu: the naive player's move (trainer.rs:506-537) for positions given as cells + turns, or for the roots of
+// the live trees of omk_eval_naive; that driver's set-up and its bookkeeping after each half-move (move records, tallies,
+// stable compaction of the live list; counters = {BlackWin, WhiteWin, Draw, live})
+void launch_naive_move_boards(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, const uint32_t *streams, int n, uint64_t key,
+                              int32_t *actions, uint8_t *forced);
+void launch_naive_move_trees(omk_ctx *c, const int32_t *ids, int n, int first_tree, const int32_t *ply, uint64_t key, int32_t *actions);
+void launch_eval_init(omk_ctx *c, int episodes, int first_tree, int32_t *ids, int32_t *ply, int8_t *moves, int8_t *final_status,
+                      int32_t *counters);
+void launch_eval_advance(omk_ctx *c, int32_t *ids, int n, const int32_t *actions, const int8_t *status, int first_tree, int32_t *ply,
+                         int8_t *moves, int8_t *final_status, int32_t *counters);
 
 // omk_api.cu: open / close a profiling span of kernel family `kind` (no-op below min_level)
 bool prof_begin(omk_ctx *c, int kind, int min_level);

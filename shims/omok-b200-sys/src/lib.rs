@@ -116,6 +116,9 @@ extern "C" {
     pub fn omk_replay_info(ctx: *mut omk_ctx, out_len: *mut i64, out_rows_added: *mut i64, out_episodes: *mut i64) -> i32;
     pub fn omk_replay_get(ctx: *mut omk_ctx, rows: *const i64, n: i32, out_boards: *mut u8, out_turns: *mut u8, out_policy: *mut f32, out_z: *mut f32) -> i32;
     pub fn omk_train_replay(ctx: *mut omk_ctx, seed: u64, first_step: i64, steps: i32, n: i32, out_losses: *mut f32, out_rows: *mut i64) -> i32;
+    // evaluation against the naive player (src/trainer.rs:487-603)
+    pub fn omk_naive_move(ctx: *mut omk_ctx, boards: *const u8, turns: *const u8, n: i32, seed: u64, streams: *const u32, out_actions: *mut i32, out_forced: *mut u8) -> i32;
+    pub fn omk_eval_naive(ctx: *mut omk_ctx, episodes: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, seed: u64, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
 }
 
 /// The message of the last failing call on this thread.

@@ -9,7 +9,10 @@ Defaults are the reference trainer's: 800 simulations per move here (BASELINE) i
 the all-reduce (device timed, max over ranks), the all-reduce of the same 22.6 MB timed alone, and the losses.
 With --device-replay the replay memory lives in the context instead (omk_replay_reset before omk_selfplay_begin): the
 self-play driver feeds it on the device, no transition is streamed, and the whole training phase -- sampling, encoding and
-the steps -- is ONE omk_train_replay call, timed as such (train_phase_s); every rank samples its own replay memory."""
+the steps -- is ONE omk_train_replay call, timed as such (train_phase_s); every rank samples its own replay memory.
+With --evaluate EPISODES the trained weights then play the trainer's evaluation against the naive player
+(src/trainer.rs:487-603) as ONE omk_eval_naive call on trees past the self-play driver's 2 * games, so the driver stays
+active for the next iteration; it reports eval_phase_s and the naive player's wins, the model's wins and the draws."""
 from __future__ import annotations
 
 import argparse
@@ -29,7 +32,7 @@ N_PARAMS = 5_643_250
 
 
 def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
-        device_replay=False, replay_capacity=600_000):
+        device_replay=False, replay_capacity=600_000, evaluate=0):
     omk = importlib.import_module("omok-ai_b200")
     trainer = importlib.import_module("omok-ai_b200.trainer")
     sharding = importlib.import_module("omok-ai_b200.sharding")
@@ -44,7 +47,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     if device_replay and (torch_step or gather):
         raise ValueError("--device-replay trains through omk_train_replay: it excludes --torch-step and --gather")
     my_games = games_per_gpu
-    ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games, capacity_nodes=4096, seed=sharding.rank_seed(seed, rank))
+    ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games + evaluate, capacity_nodes=4096,
+                      seed=sharding.rank_seed(seed, rank))
     ctx.net_init_random(seed)                       # identical weights on every rank
     if torch_step:
         step = trainer.TrainStep(ctx.net_get_params(), device=f"cuda:{local}")
@@ -60,7 +64,7 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     if device_replay:
         ctx.replay_reset(replay_capacity)           # before selfplay_begin: the driver feeds the replay that exists then
         return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
-                                  seed, quiet, replay_capacity)
+                                  seed, quiet, replay_capacity, evaluate)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -141,6 +145,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
            "train_step_ms": times["step_ms"], "train_step_ms_without_allreduce": times["local_ms"],
            "allreduce_22.6MB_alone_ms": times["allreduce_ms"], "allreduce_bytes_per_step": N_PARAMS * 4 if world > 1 else 0,
            "first_loss": losses[0][2], "last_loss": losses[-1][2], "policy_sums_to_one": bool(abs(float(p[0].sum()) - 1) < 1e-3)}
+    if evaluate:
+        out.update(_evaluate(ctx, evaluate, 2 * my_games, count, batch, seed))
     if rank == 0 and not quiet:
         print(json.dumps(out), flush=True)
     ctx.close()
@@ -149,7 +155,19 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     return out
 
 
-def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity):
+def _evaluate(ctx, episodes, first_tree, count, batch, seed):
+    """The evaluation phase: the current weights against the naive player, one omk_eval_naive call."""
+    omk = importlib.import_module("omok-ai_b200")
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    (black, white, draw), _, _, stats = ctx.eval_naive(episodes, count=count, batch_size=batch, epsilon=0.25, alpha=0.03,
+                                                       evaluator=omk.EVAL_NET, seed=seed, first_tree=first_tree)
+    return {"eval_episodes": episodes, "eval_phase_s": time.perf_counter() - t0, "eval_naive_wins": black, "eval_model_wins": white,
+            "eval_draws": draw, "eval_moves": stats["moves"], "eval_host_syncs": stats["host_syncs"], "eval_gpu_ms": stats["gpu_ms"]}
+
+
+def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity,
+                       evaluate=0):
     omk = importlib.import_module("omok-ai_b200")
     ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
     ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
@@ -183,6 +201,8 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
            "train_steps": steps, "global_minibatch": per_rank * world, "train_step": "omk_train_replay (C ABI, fp32 CUDA kernels)",
            "train_phase_s": times["train_phase_s"], "train_step_ms": times["train_phase_s"] * 1e3 / steps,
            "first_loss": float(losses[0, 2]), "last_loss": float(losses[-1, 2]), "h2d_bytes_total": h2d}
+    if evaluate:
+        out.update(_evaluate(ctx, evaluate, 2 * games, count, batch, seed))
     if rank == 0 and not quiet:
         print(json.dumps(out), flush=True)
     ctx.close()
@@ -203,6 +223,8 @@ if __name__ == "__main__":
     ap.add_argument("--device-replay", action="store_true",
                     help="replay memory on the device, fed by the self-play driver; the training phase is one omk_train_replay call")
     ap.add_argument("--replay-capacity", type=int, default=600_000, help="rows of the device replay memory per GPU (src/config.rs: 600 000)")
+    ap.add_argument("--evaluate", type=int, default=0, metavar="EPISODES",
+                    help="after training, play EPISODES games against the naive player on the device (omk_eval_naive)")
     a = ap.parse_args()
     run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
-        device_replay=a.device_replay, replay_capacity=a.replay_capacity)
+        device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate)
