@@ -326,6 +326,29 @@ OMK_API int32_t omk_eval_naive(omk_ctx *ctx, int32_t episodes, int32_t first_tre
                                float alpha, int32_t evaluator, uint64_t seed, int32_t *out_result, int8_t *out_moves,
                                int8_t *out_status, int64_t *out_stats, float *out_gpu_ms);
 
+/* ---------------------------------------------------------------- the opponent network and the arena
+ * The opponent network: a second set of weights in the context, read only by omk_opponent_eval and omk_match.  Training,
+ * self-play, the searches and omk_net_* never read or change it; loading it changes nothing they produce.             */
+OMK_API int32_t omk_opponent_load_params(omk_ctx *ctx, const float *const *tensors, const int64_t *lens); /* as omk_net_load_params */
+/* device-to-device copy of the network's current fp32 weights (e.g. before a training phase), images rebuilt from them;
+ * OMK_ERR_STATE if no network is loaded */
+OMK_API int32_t omk_opponent_from_net(omk_ctx *ctx);
+OMK_API int32_t omk_opponent_eval(omk_ctx *ctx, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+                                  float *out_p, float *out_v); /* omk_net_eval with the opponent's weights */
+/* benchmark/src/main.rs:14-108 on the device: 2 * pairs games; games 0 .. pairs-1 the network opens (Black), games
+ * pairs .. 2*pairs-1 the opponent opens.  Every move = execute(count, batch_size, epsilon, alpha) + sample_action(Best) +
+ * play_action in the mover's tree, then ensure_action_exists + play_action in the other model's tree.
+ * Trees: the network's tree of game j is first_tree + j, the opponent's is first_tree + 2*pairs + j; both have random
+ * stream j % pairs (so arena.play_match on two contexts with this context's seed replays it game by game).  OMK_ERR_STATE
+ * if they overlap an active self-play driver's trees 0 .. 2 * n_games - 1.
+ * evaluator OMK_EVAL_NET: network vs opponent (both must be loaded); OMK_EVAL_HASH: the hash evaluator on both sides.
+ * out_result[3] = {network wins, opponent wins, draws}; out_moves[2*pairs*81] (may be NULL) each game's moves, -1 past its
+ * end; out_status[2*pairs] (may be NULL) final GameStatus; out_stats[4] (may be NULL) = {simulations, positions evaluated,
+ * moves, host synchronisations}; out_gpu_ms (may be NULL).  One host round trip per half-move; no host-to-device copy. */
+OMK_API int32_t omk_match(omk_ctx *ctx, int32_t pairs, int32_t first_tree, int32_t count, int32_t batch_size, float epsilon,
+                          float alpha, int32_t evaluator, int32_t *out_result, int8_t *out_moves, int8_t *out_status,
+                          int64_t *out_stats, float *out_gpu_ms);
+
 #ifdef __cplusplus
 }
 #endif

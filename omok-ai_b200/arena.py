@@ -3,6 +3,8 @@
   * `play_match`                 benchmark/src/main.rs:14-108 + benchmark/src/agent.rs:14-47: two models, GAME_COUNT games,
                                  half with each side moving first; every move = MCTSExecutor::run(800, 8, eps 0, alpha 1)
                                  then `sample_action(Best)`; the opponent follows with ensure_action_exists + play_action.
+  * `play_match_device`          the same match as ONE call (omk_match) between the context's network (left) and its
+                                 opponent network (right): both legs run at once, each model's half-move on its own lane.
   * `play_against_naive_player`  src/trainer.rs:487-603: the naive player takes the first legal move (ascending) that ends
                                  the game for itself, or that would end it for the opponent (a block); else a random
                                  legal move.  The model answers with ParallelMCTSExecutor::execute + Best.
@@ -60,6 +62,19 @@ def play_match(ctx_left, ctx_right, game_count: int = 100, count: int = 800, bat
     if moves_out is not None:
         moves_out[:] = log
     return wins["left"], wins["right"], wins["draw"]
+
+
+def play_match_device(ctx, game_count: int = 100, count: int = 800, batch_size: int = 8, epsilon: float = 0.0, alpha: float = 1.0,
+                      evaluator: int = B.EVAL_NET, first_tree: int = 0, moves_out: list | None = None):
+    """Returns (network wins, opponent wins, draws) like `play_match` with left = the network and right = the opponent
+    (`Context.opponent_load_params` / `opponent_from_net`), from one `omk_match` call of `game_count // 2` pairs on the trees
+    first_tree .. first_tree + 2 * game_count - 1.  `play_match` on two contexts with this context's seed replays it game
+    by game.  `moves_out`, if given, receives one move list per game in `play_match`'s order."""
+    result, moves, _, _ = ctx.match(game_count // 2, first_tree=first_tree, count=count, batch_size=batch_size, epsilon=epsilon,
+                                    alpha=alpha, evaluator=evaluator)
+    if moves_out is not None:
+        moves_out[:] = [[int(a) for a in row if a >= 0] for row in moves]
+    return result
 
 
 def naive_moves(ctx, boards: np.ndarray, turns: np.ndarray, rng: np.random.Generator) -> np.ndarray:

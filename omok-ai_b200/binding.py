@@ -146,6 +146,10 @@ def load_library():
     L.omk_train_replay.argtypes = [vp, u64, i64, i32, i32, vp, vp]
     L.omk_naive_move.argtypes = [vp, vp, vp, i32, u64, vp, vp, vp]
     L.omk_eval_naive.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, u64, vp, vp, vp, vp, P(f32)]
+    L.omk_opponent_load_params.argtypes = [vp, P(vp), P(i64)]
+    L.omk_opponent_from_net.argtypes = [vp]
+    L.omk_opponent_eval.argtypes = [vp, vp, vp, i32, i32, vp, vp]
+    L.omk_match.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
     for name in declared_symbols():
         fn = getattr(L, name)  # raises AttributeError if the library lacks a declared symbol
         if name not in ("omk_last_error", "omk_ctx_stream", "omk_ctx_launch_count"):
@@ -529,6 +533,46 @@ class Context:
         self._check(self.L.omk_eval_naive(self.h, episodes, first_tree, count, batch_size, epsilon, alpha, evaluator,
                                           int(seed) & 0xFFFFFFFFFFFFFFFF, _ptr(result), _ptr(moves), _ptr(status), _ptr(stats),
                                           C.byref(gpu_ms)))
+        info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
+        info["gpu_ms"] = float(gpu_ms.value)
+        return (int(result[0]), int(result[1]), int(result[2])), moves, status, info
+
+    # ---- the opponent network and the arena ----
+    def opponent_load_params(self, params):
+        """A second set of weights, read only by opponent_eval and match (training, self-play and the searches never see it)."""
+        arrs = [np.ascontiguousarray(p, dtype=np.float32).reshape(-1) for p in params]
+        ptrs = (C.c_void_p * 31)(*[a.ctypes.data for a in arrs])
+        lens = (C.c_int64 * 31)(*[a.size for a in arrs])
+        self._check(self.L.omk_opponent_load_params(self.h, ptrs, lens))
+
+    def opponent_from_net(self):
+        """The opponent becomes a device-side copy of the network's current weights (e.g. the snapshot before training)."""
+        self._check(self.L.omk_opponent_from_net(self.h))
+
+    def opponent_eval(self, boards, turns, mode: int = 0, want_v: bool = True):
+        """net_eval with the opponent's weights."""
+        boards = np.ascontiguousarray(boards, dtype=np.uint8).reshape(-1, CELLS)
+        turns = np.ascontiguousarray(turns, dtype=np.uint8).reshape(-1)
+        n = boards.shape[0]
+        p = np.zeros((n, CELLS), dtype=np.float32)
+        v = np.zeros(n, dtype=np.float32) if want_v else None
+        self._check(self.L.omk_opponent_eval(self.h, _ptr(boards), _ptr(turns), n, mode, _ptr(p), _ptr(v)))
+        return p, v
+
+    def match(self, pairs: int, first_tree: int = 0, count: int = 800, batch_size: int = 8, epsilon: float = 0.0, alpha: float = 1.0,
+              evaluator: int = EVAL_NET):
+        """The benchmark's arena between the network and the opponent in one call: 2 * pairs games, the network opens games
+        0 .. pairs - 1, the opponent the rest; trees first_tree .. first_tree + 4 * pairs - 1.  Returns (result (network wins,
+        opponent wins, draws), moves [2 * pairs, 81] i8 (-1 past a game's end), final status [2 * pairs] i8, stats dict:
+        simulations, nn_evals, moves, host_syncs, gpu_ms)."""
+        games = 2 * pairs
+        result = np.zeros(3, dtype=np.int32)
+        moves = np.zeros((max(games, 0), CELLS), dtype=np.int8)
+        status = np.zeros(max(games, 0), dtype=np.int8)
+        stats = np.zeros(4, dtype=np.int64)
+        gpu_ms = C.c_float()
+        self._check(self.L.omk_match(self.h, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, _ptr(result), _ptr(moves),
+                                     _ptr(status), _ptr(stats), C.byref(gpu_ms)))
         info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
         info["gpu_ms"] = float(gpu_ms.value)
         return (int(result[0]), int(result[1]), int(result[2])), moves, status, info

@@ -1,5 +1,6 @@
 // eval_kernels.cu -- the trainer's evaluation against the naive player (src/trainer.rs:487-603) on the device: the naive
-// player's move (:506-537) and the bookkeeping omk_eval_naive runs after every half-move.
+// player's move (:506-537) and the bookkeeping omk_eval_naive runs after every half-move; the same bookkeeping for the
+// arena between the network and the opponent (omk_match, benchmark/src/main.rs:14-108).
 #include "omk_internal.h"
 
 namespace omk {
@@ -153,6 +154,81 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_eval_advance(int32_t *ids, 
     if (threadIdx.x == 0) counters[3] = kept_before;
 }
 
+// A fresh match: tree k of the 4 * pairs is first_tree + k, laid out [model][leg][pairs] (network 0, opponent 1), so game j
+// (leg j / pairs) has the network's tree first_tree + j and the opponent's first_tree + 2 * pairs + j; both use stream j % pairs.
+__global__ void k_match_init(int pairs, int first_tree, int32_t *ids, uint32_t *streams, int8_t *moves, int8_t *final_status,
+                             int32_t *counters) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    const int games = 2 * pairs;
+    if (t < games * kCells) moves[t] = -1;
+    if (t < 2 * games) ids[t] = first_tree + t;
+    if (t < games) {
+        streams[t] = (uint32_t)(t % pairs);
+        final_status[t] = kInProgress;
+    }
+    if (t < 8) counters[t] = 0;
+}
+
+// After a half-move of both legs, one block per leg: append each live game's move at ply `half`, check that the other
+// model's tree took the previous move (other_status, from the second half-move on), tally and record the games that ended
+// (BlackWin for the side that opened: the network in leg 0), and compact the leg's live list stably -- both models' tree ids
+// and the moves, which the other model's trees take next -- so a game's two trees stay in step.  Block 0 also copies the device
+// error word next to the live counts.
+__global__ void __launch_bounds__(kAdvanceThreads) k_match_advance(int pairs, int first_tree, int half, int live0, int live1, int32_t *ids,
+                                                                   int32_t *actions, const int8_t *status, const int8_t *other_status,
+                                                                   int8_t *moves, int8_t *final_status, int32_t *counters,
+                                                                   uint32_t *dev_error) {
+    __shared__ int warp_kept[kAdvanceThreads / 32];
+    __shared__ int kept_before;
+    const int leg = blockIdx.x, n = leg ? live1 : live0;
+    int32_t *ids_net = ids + leg * pairs, *ids_opp = ids + (2 + leg) * pairs, *act = actions + leg * pairs;
+    const int8_t *st_leg = status + leg * pairs, *ost_leg = other_status + leg * pairs;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) kept_before = 0;
+    __syncthreads();
+    for (int c0 = 0; c0 < n; c0 += kAdvanceThreads) {
+        const int i = c0 + threadIdx.x;
+        bool keep = false;
+        int32_t tn = 0, to = 0, a = 0;
+        if (i < n) {
+            tn = ids_net[i];
+            to = ids_opp[i];
+            a = act[i];
+            const int g = tn - first_tree;
+            const int st = st_leg[i];
+            moves[(size_t)g * kCells + half] = (int8_t)a;
+            if (half > 0 && ost_leg[i] != kInProgress) atomicOr(dev_error, 16u);
+            if (st == kInProgress) {
+                keep = true;
+            } else if (st == kDraw || st == kBlackWin || st == kWhiteWin) {
+                final_status[g] = (int8_t)st;
+                const int opener = g < pairs ? 0 : 1;
+                atomicAdd(&counters[st == kDraw ? 2 : (st == kBlackWin ? opener : 1 - opener)], 1);
+            } else {
+                atomicOr(dev_error, 16u);  // Option::None: the move was refused -- the game could never end
+            }
+        }
+        const uint32_t b = __ballot_sync(kFullMask, keep);
+        if (lane == 0) warp_kept[warp] = __popc(b);
+        __syncthreads();  // every entry of this chunk has been read before any is overwritten
+        int dst = kept_before + __popc(b & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) dst += warp_kept[w];
+        if (keep) {
+            ids_net[dst] = tn;
+            ids_opp[dst] = to;
+            act[dst] = a;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < kAdvanceThreads / 32; ++w) kept_before += warp_kept[w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        counters[4 + leg] = kept_before;
+        if (leg == 0) counters[3] = (int32_t)atomicOr(dev_error, 0u);  // read back with the live counts
+    }
+}
+
 // ---- launchers ----
 static NaiveArgs naive_args(int n, uint64_t key, int32_t *actions, uint8_t *forced) {
     NaiveArgs a{};
@@ -193,6 +269,18 @@ void launch_eval_advance(omk_ctx *c, int32_t *ids, int n, const int32_t *actions
                          int8_t *moves, int8_t *final_status, int32_t *counters) {
     k_eval_advance<<<1, kAdvanceThreads, 0, c->stream>>>(ids, n, actions, status, first_tree, ply, moves, final_status, counters,
                                                           c->dev_error);
+    c->launches++;
+}
+void launch_match_init(omk_ctx *c, int pairs, int first_tree, int32_t *ids, uint32_t *streams, int8_t *moves, int8_t *final_status,
+                       int32_t *counters) {
+    const int total = 2 * pairs * kCells;
+    k_match_init<<<(total + 255) / 256, 256, 0, c->stream>>>(pairs, first_tree, ids, streams, moves, final_status, counters);
+    c->launches++;
+}
+void launch_match_advance(omk_ctx *c, int pairs, int first_tree, int half, const int *live, int32_t *ids, int32_t *actions,
+                          const int8_t *status, const int8_t *other_status, int8_t *moves, int8_t *final_status, int32_t *counters) {
+    k_match_advance<<<2, kAdvanceThreads, 0, c->stream>>>(pairs, first_tree, half, live[0], live[1], ids, actions, status, other_status,
+                                                           moves, final_status, counters, c->dev_error);
     c->launches++;
 }
 

@@ -543,13 +543,8 @@ static bool encode_map_tower_store(CUtensorMap *map, __half *ptr, uint64_t rows)
               CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-struct Fc16State {  // weight maps, shared by both search lanes (the activation maps live in each lane's Workspace)
-    CUtensorMap map0_b_hi, map0_b_lo;  // fc0 (B boxes of 128 rows: the pair kernel loads half tiles)
-    CUtensorMap map1_b_hi, map1_b_lo;  // fc1 (B boxes of 256 rows)
-    CUtensorMap map2_b_hi, map2_b_lo;  // heads (B = all 128 padded output rows)
-    bool weights_ready = false;
-    CUtensorMap map0s_b_hi, map0s_b_lo;  // fc0 weights with 256-row boxes (one-CTA split-K kernel for small batches)
-    int pair_slots = 0;                  // CTA pairs of the fc0 pair kernel the device holds at once (0 = not queried yet)
+struct Fc16State {  // what belongs to the device, shared by both models and both search lanes
+    int pair_slots = 0;  // CTA pairs of the fc0 pair kernel the device holds at once (0 = not queried yet)
 };
 void Fc16StateFree::operator()(Fc16State *s) const { delete s; }
 
@@ -560,8 +555,7 @@ static Fc16State *state16_of(omk_ctx *c) {
 
 // (re)build the scaled, split, transposed weights of fc0 and fc1; call after the weights change
 bool fc16_prepare_weights(omk_ctx *c) {
-    Fc16State *s = state16_of(c);
-    NetWeights &w = c->net;
+    NetWeights &w = *c->model;
     if (!w.fc0_wt_h16) {
         FcImages f;
         if (f.fc0_wt_h16.alloc((size_t)F_K0 * F_N) != cudaSuccess || f.fc0_wt_l16.alloc((size_t)F_K0 * F_N) != cudaSuccess ||
@@ -582,15 +576,15 @@ bool fc16_prepare_weights(omk_ctx *c) {
     k_fc16_split_weights<<<dim3(F_K1 / 32, 128 / 32), 256, 0, c->stream>>>(w.heads_w, w.fc_absmax + 2, w.heads_wt_h16, w.heads_wt_l16,
                                                                          w.fc_inv_scale + 2, F_K1, 128);
     c->launches += 6;
-    if (!encode_map16(&s->map0_b_hi, w.fc0_wt_h16, F_N, 128, F_K0)) return false;
-    if (!encode_map16(&s->map0_b_lo, w.fc0_wt_l16, F_N, 128, F_K0)) return false;
-    if (!encode_map16(&s->map0s_b_hi, w.fc0_wt_h16, F_N, F_BN, F_K0)) return false;
-    if (!encode_map16(&s->map0s_b_lo, w.fc0_wt_l16, F_N, F_BN, F_K0)) return false;
-    if (!encode_map16(&s->map1_b_hi, w.fc1_wt_h16, F_N, F_BN, F_K1)) return false;
-    if (!encode_map16(&s->map1_b_lo, w.fc1_wt_l16, F_N, F_BN, F_K1)) return false;
-    if (!encode_map16(&s->map2_b_hi, w.heads_wt_h16, 128, 128, F_K1)) return false;
-    if (!encode_map16(&s->map2_b_lo, w.heads_wt_l16, 128, 128, F_K1)) return false;
-    s->weights_ready = true;
+    if (!encode_map16(&w.map0_b_hi, w.fc0_wt_h16, F_N, 128, F_K0)) return false;
+    if (!encode_map16(&w.map0_b_lo, w.fc0_wt_l16, F_N, 128, F_K0)) return false;
+    if (!encode_map16(&w.map0s_b_hi, w.fc0_wt_h16, F_N, F_BN, F_K0)) return false;
+    if (!encode_map16(&w.map0s_b_lo, w.fc0_wt_l16, F_N, F_BN, F_K0)) return false;
+    if (!encode_map16(&w.map1_b_hi, w.fc1_wt_h16, F_N, F_BN, F_K1)) return false;
+    if (!encode_map16(&w.map1_b_lo, w.fc1_wt_l16, F_N, F_BN, F_K1)) return false;
+    if (!encode_map16(&w.map2_b_hi, w.heads_wt_h16, 128, 128, F_K1)) return false;
+    if (!encode_map16(&w.map2_b_lo, w.heads_wt_l16, 128, 128, F_K1)) return false;
+    w.weights_ready = true;
     return true;
 }
 
@@ -612,8 +606,8 @@ static bool check_launch(const char *what) {
 
 // fc0: act0_h16/l16 -> act1_h16/l16 (the A operand of fc1)
 bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
-    Fc16State *s = state16_of(c);
-    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
+    const NetWeights &m = *c->model;
+    const ActMaps *am = m.weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     const bool fine = c->fc0_chunk == F_CHUNK0_FINE;
     static const int splitk_env = getenv("OMK_FC0_SPLITK_MAX") ? atoi(getenv("OMK_FC0_SPLITK_MAX")) : -1;
@@ -637,18 +631,18 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
             auto sk = fine ? k_fc16<F_K0, F_CHUNK0_FINE, false, 128, false, true> : k_fc16<F_K0, F_CHUNK0, false, 128, false, true>;
             cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
             sk<<<dim3(F_N / 128, mt, F_K0 / F_BK / F_SPLITK_KB), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-                am->map0_a_hi, am->map0_a_lo, s->map0_b_hi, s->map0_b_lo, c->net.t[24], c->net.fc_inv_scale, partial, nullptr,
+                am->map0_a_hi, am->map0_a_lo, m.map0_b_hi, m.map0_b_lo, m.t[24], m.fc_inv_scale, partial, nullptr,
                 nullptr, c->ws.n_req, rows_bound, nullptr, nullptr, nullptr, FcBal{});
         } else {
             using Cfg = FcCfg<false, 256>;
             auto sk = fine ? k_fc16<F_K0, F_CHUNK0_FINE, false, 256, false, true> : k_fc16<F_K0, F_CHUNK0, false, 256, false, true>;
             cudaFuncSetAttribute(sk, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
             sk<<<dim3(F_N / F_BN, mt, F_K0 / F_BK / F_SPLITK_KB), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-                am->map0_a_hi, am->map0_a_lo, s->map0s_b_hi, s->map0s_b_lo, c->net.t[24], c->net.fc_inv_scale, partial, nullptr,
+                am->map0_a_hi, am->map0_a_lo, m.map0s_b_hi, m.map0s_b_lo, m.t[24], m.fc_inv_scale, partial, nullptr,
                 nullptr, c->ws.n_req, rows_bound, nullptr, nullptr, nullptr, FcBal{});
         }
-        k_fc0_reduce<<<(rows_bound * 64 + 255) / 256, 256, 0, c->stream>>>(partial, kChunks, ws_rows, c->net.t[24],
-                                                                            c->net.fc_inv_scale, c->ws.act1_h16, c->ws.act1_l16,
+        k_fc0_reduce<<<(rows_bound * 64 + 255) / 256, 256, 0, c->stream>>>(partial, kChunks, ws_rows, m.t[24],
+                                                                            m.fc_inv_scale, c->ws.act1_h16, c->ws.act1_l16,
                                                                             c->ws.n_req, rows_bound);
         c->launches += 2;
         return check_launch("fc0 (fp16 split, split-K)");
@@ -668,8 +662,8 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const float *bias_p = c->net.t[24];
-    const float *inv_p = c->net.fc_inv_scale;
+    const float *bias_p = m.t[24];
+    const float *inv_p = m.fc_inv_scale;
     float *c_f32 = nullptr;
     __half *c_hi = c->ws.act1_h16, *c_lo = c->ws.act1_l16;
     const uint32_t *nreq_p = c->ws.n_req;
@@ -678,12 +672,13 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
     // tail balancing (see FcBal): the last, partial wave of tiles shares its K range with the otherwise idle pairs
     FcBal bal{};
     if (!fine && c->fc0_balance) {
-        if (s->pair_slots == 0) {
+        Fc16State *st = state16_of(c);
+        if (st->pair_slots == 0) {
             int n = 0;
             if (cudaOccupancyMaxActiveClusters(&n, kern, &cfg) != cudaSuccess) { cudaGetLastError(); n = 0; }
-            s->pair_slots = n > 0 ? n : -1;
+            st->pair_slots = n > 0 ? n : -1;
         }
-        const int P = s->pair_slots, T = (F_N / F_BN) * pairs, NC = F_K0 / F_BK / F_CHUNK0;
+        const int P = st->pair_slots, T = (F_N / F_BN) * pairs, NC = F_K0 / F_BK / F_CHUNK0;
         const int R = P > 0 ? T % P : 0, H = P - R;
         if (R > 0 && R <= 128 && H > 0) {
             int tail = 0;
@@ -707,7 +702,7 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
             }
         }
     }
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, am->map0_a_hi, am->map0_a_lo, s->map0_b_hi, s->map0_b_lo, bias_p, inv_p, c_f32,
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, am->map0_a_hi, am->map0_a_lo, m.map0_b_hi, m.map0_b_lo, bias_p, inv_p, c_f32,
                                              c_hi, c_lo, nreq_p, rows_bound, no_p, no_v, no_err, bal);
     if (e != cudaSuccess) fprintf(stderr, "omok_b200: cudaLaunchKernelEx(k_fc16 pair): %s\n", cudaGetErrorString(e));
     c->launches++;
@@ -716,15 +711,15 @@ bool launch_fc0_f16(omk_ctx *c, int rows_bound) {
 
 // fc1: act1_h16/l16 -> act2_h16/l16 (the A operand of the heads)
 bool launch_fc1_f16(omk_ctx *c, int rows_bound) {
-    Fc16State *s = state16_of(c);
-    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
+    const NetWeights &m = *c->model;
+    const ActMaps *am = m.weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     using Cfg = FcCfg<false, 256>;
     auto kern = k_fc16<F_K1, F_CHUNK1, false>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
     const int mt = (rows_bound + F_BM - 1) / F_BM;
     kern<<<dim3(F_N / F_BN, mt), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-        am->map1_a_hi, am->map1_a_lo, s->map1_b_hi, s->map1_b_lo, c->net.t[26], c->net.fc_inv_scale + 1, nullptr, c->ws.act2_h16,
+        am->map1_a_hi, am->map1_a_lo, m.map1_b_hi, m.map1_b_lo, m.t[26], m.fc_inv_scale + 1, nullptr, c->ws.act2_h16,
         c->ws.act2_l16, c->ws.n_req, rows_bound, nullptr, nullptr, nullptr, FcBal{});
     c->launches++;
     return check_launch("fc1 (fp16 split)");
@@ -732,15 +727,15 @@ bool launch_fc1_f16(omk_ctx *c, int rows_bound) {
 
 // heads: act2_h16/l16 -> P (softmax of the 81 policy logits) and V (tanh of the value logit)
 bool launch_heads_f16(omk_ctx *c, int rows_bound) {
-    Fc16State *s = state16_of(c);
-    const ActMaps *am = s->weights_ready ? &c->ws.maps : nullptr;
+    const NetWeights &m = *c->model;
+    const ActMaps *am = m.weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     using Cfg = FcCfg<false, 128>;
     auto kern = k_fc16<F_K1, F_CHUNKH, false, 128, true>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
     const int mt = (rows_bound + F_BM - 1) / F_BM;
     kern<<<dim3(1, mt), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-        am->map2_a_hi, am->map2_a_lo, s->map2_b_hi, s->map2_b_lo, c->net.heads_b, c->net.fc_inv_scale + 2, nullptr, nullptr, nullptr,
+        am->map2_a_hi, am->map2_a_lo, m.map2_b_hi, m.map2_b_lo, m.heads_b, m.fc_inv_scale + 2, nullptr, nullptr, nullptr,
         c->ws.n_req, rows_bound, c->ws.P, c->ws.V, c->dev_error, FcBal{});
     c->launches++;
     return check_launch("heads (fp16 split)");

@@ -379,8 +379,8 @@ __global__ void k_init_normal(float *w, long long n, float scale, uint64_t seed,
 }
 
 void net_pack_heads(omk_ctx *c) {
-    k_pack_heads<<<(kFc * 128 + 255) / 256, 256, 0, c->stream>>>(c->net.t[29], c->net.t[30], c->net.t[27], c->net.t[28],
-                                                                  c->net.heads_w, c->net.heads_b);
+    k_pack_heads<<<(kFc * 128 + 255) / 256, 256, 0, c->stream>>>(c->model->t[29], c->model->t[30], c->model->t[27], c->model->t[28],
+                                                                  c->model->heads_w, c->model->heads_b);
     c->launches++;
 }
 
@@ -417,12 +417,12 @@ bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
     if (max_rows <= 0) return true;
     bool ok = true;
     TowerWeights tw;
-    tw.conv_w = c->net.t[0];
-    tw.conv_b = c->net.t[1];
+    tw.conv_w = c->model->t[0];
+    tw.conv_b = c->model->t[1];
     for (int r = 0; r < 3; ++r) {
         const int b = 2 + 7 * r;
-        tw.w0[r] = c->net.t[b + 0]; tw.b0[r] = c->net.t[b + 1]; tw.dw[r] = c->net.t[b + 2]; tw.pw[r] = c->net.t[b + 3];
-        tw.b1[r] = c->net.t[b + 4]; tw.w2[r] = c->net.t[b + 5]; tw.b2[r] = c->net.t[b + 6];
+        tw.w0[r] = c->model->t[b + 0]; tw.b0[r] = c->model->t[b + 1]; tw.dw[r] = c->model->t[b + 2]; tw.pw[r] = c->model->t[b + 3];
+        tw.b1[r] = c->model->t[b + 4]; tw.w2[r] = c->model->t[b + 5]; tw.b2[r] = c->model->t[b + 6];
     }
     if (!ensure_activations(c, max_rows)) {
         fprintf(stderr, "omok_b200: activation workspace allocation failed (%d rows)\n", max_rows);
@@ -449,7 +449,7 @@ bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
         ok = launch_fc0_f16(c, max_rows) && ok;
         c->launches--;
     } else {
-        k_gemm<<<dim3(kFc / GN, mt), 256, 0, c->stream>>>(c->ws.act0, c->net.t[23], c->net.t[24], c->ws.act1, c->ws.n_req,
+        k_gemm<<<dim3(kFc / GN, mt), 256, 0, c->stream>>>(c->ws.act0, c->model->t[23], c->model->t[24], c->ws.act1, c->ws.n_req,
                                                           max_rows, kFc, kFlat, 1);
         launch_f32_to_split16(c, c->ws.act1, c->ws.act1_h16, c->ws.act1_l16, n1);  // keeps debug buffer 9 meaningful
     }
@@ -459,7 +459,7 @@ bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
         ok = launch_fc1_f16(c, max_rows) && ok;
         c->launches--;
     } else {
-        k_gemm<<<dim3(kFc / GN, mt), 256, 0, c->stream>>>(c->ws.act1, c->net.t[25], c->net.t[26], c->ws.act2, c->ws.n_req,
+        k_gemm<<<dim3(kFc / GN, mt), 256, 0, c->stream>>>(c->ws.act1, c->model->t[25], c->model->t[26], c->ws.act2, c->ws.n_req,
                                                           max_rows, kFc, kFc, 1);
     }
     prof_end(c, sp);
@@ -467,7 +467,7 @@ bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
     if (c->fc0_mode == 1) {  // heads GEMM + tanh / softmax in one tensor-core kernel
         ok = launch_heads_f16(c, max_rows) && ok;
     } else {
-        k_gemm<<<dim3(1, mt), 256, 0, c->stream>>>(c->ws.act2, c->net.heads_w, c->net.heads_b, c->ws.logits, c->ws.n_req, max_rows,
+        k_gemm<<<dim3(1, mt), 256, 0, c->stream>>>(c->ws.act2, c->model->heads_w, c->model->heads_b, c->ws.logits, c->ws.n_req, max_rows,
                                                    128, kFc, 0);
         k_heads<<<(max_rows + 7) / 8, 256, 0, c->stream>>>(c->ws.logits, c->ws.n_req, max_rows, c->ws.P, c->ws.V);
         c->launches++;

@@ -130,13 +130,21 @@ struct LaneScope {
         c->id_base = 0;
     }
 };
-// how many lanes a search over n trees uses; creates lane 1 on first use
-static int lanes_for(omk_ctx *c, int n) {
-    if (c->lane_min_trees <= 0 || n < c->lane_min_trees || n < 2) return 1;
+// RAII: the evaluator launches in scope read the opponent's weights (either lane may evaluate either model)
+struct ModelScope {
+    omk_ctx *c;
+    NetWeights *saved;
+    ModelScope(omk_ctx *ctx, bool opponent) : c(ctx), saved(ctx->model) {
+        if (opponent) c->model = &c->opp;
+    }
+    ~ModelScope() { c->model = saved; }
+};
+// creates lane 1 on first use; false: this context has no second lane
+static bool lane1_ready(omk_ctx *c) {
     if (!c->lane1_stream) {
         Workspace &w = c->lane1_ws;
         const size_t ct = (size_t)(c->cap_trees > 0 ? c->cap_trees : 1);
-        if (cudaStreamCreateWithFlags(&c->lane1_stream, cudaStreamNonBlocking) != cudaSuccess) return 1;
+        if (cudaStreamCreateWithFlags(&c->lane1_stream, cudaStreamNonBlocking) != cudaSuccess) return false;
         bool ok = cudaEventCreateWithFlags(&c->lane_fork, cudaEventDisableTiming) == cudaSuccess &&
                   cudaEventCreateWithFlags(&c->lane_join, cudaEventDisableTiming) == cudaSuccess &&
                   w.n_req.alloc(4) == cudaSuccess && w.slot_base.alloc(ct) == cudaSuccess && w.slot_count.alloc(ct) == cudaSuccess &&
@@ -144,10 +152,15 @@ static int lanes_for(omk_ctx *c, int n) {
         if (!ok) {
             cudaGetLastError();
             c->lane_min_trees = 0;  // no second lane on this context
-            return 1;
+            return false;
         }
     }
-    return 2;
+    return true;
+}
+// how many lanes a search over n trees uses
+static int lanes_for(omk_ctx *c, int n) {
+    if (c->lane_min_trees <= 0 || n < c->lane_min_trees || n < 2) return 1;
+    return lane1_ready(c) ? 2 : 1;
 }
 static void lanes_fork(omk_ctx *c) {  // lane 1 starts after everything already queued on the main stream
     cudaEventRecord(c->lane_fork, c->stream);
@@ -171,6 +184,9 @@ static int32_t check_device_error(omk_ctx *c) {
     if (e & 4u)
         return fail(OMK_ERR_STATE, "the self-play driver sampled a move its tree refused (play_action returned None): the transition stream of this call is not usable");
     if (e & 8u) return fail(OMK_ERR_STATE, "the evaluation played a move its tree refused (play_action returned None): its result is not usable");
+    if (e & 16u)
+        return fail(OMK_ERR_STATE, "the match played a move a tree refused (play_action returned None), or a game's two trees fell out of step: "
+                                   "its result is not usable");
     if (e & 2u)
         return fail(OMK_ERR_NUMERIC, "the network produced a non-finite policy or value (activation beyond the fp16 operand range "
                                      "of the tensor-core path, |x| >= 65504, or non-finite weights)");
@@ -419,9 +435,13 @@ extern "C" int32_t omk_net_init_random(omk_ctx *c, uint64_t seed) {
     return sp_refresh_root_policy(c);
 }
 
-static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float *out_p, float *out_v) {
-    int32_t rc_p = ensure_packed(c);
-    if (rc_p) return rc_p;
+// opponent: the opponent's weights (omk_opponent_eval), which no training step changes
+static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float *out_p, float *out_v, bool opponent = false) {
+    if (!opponent) {
+        int32_t rc_p = ensure_packed(c);
+        if (rc_p) return rc_p;
+    }
+    ModelScope scope(c, opponent);
     if (!net_forward(c, images_dev, n)) return fail(OMK_ERR_CUDA, "the network forward failed to launch (see stderr)");
     // P rows are padded to 96 floats on the device; compact on the way out
     CK(cudaMemcpy2DAsync(out_p, sizeof(float) * kCells, c->ws.P, sizeof(float) * kRow, sizeof(float) * kCells, (size_t)n,
@@ -433,10 +453,10 @@ static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float
     return check_device_error(c);  // OMK_ERR_NUMERIC when the network produced a non-finite output
 }
 
-extern "C" int32_t omk_net_eval(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
-                                float *out_p, float *out_v) {
+static int32_t eval_boards(omk_ctx *c, bool opponent, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+                           float *out_p, float *out_v) {
     CK(cudaSetDevice(c->device));
-    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
+    if (!(opponent ? c->opp : c->net).loaded) return fail(OMK_ERR_STATE, opponent ? "opponent weights not loaded" : "network weights not loaded");
     if (n < 0 || !boards || !turns || !out_p) return fail(OMK_ERR_INVALID, "bad arguments");
     if (n == 0) return OMK_OK;
     int32_t rc = ensure_workspace(c, n);
@@ -447,7 +467,11 @@ extern "C" int32_t omk_net_eval(omk_ctx *c, const uint8_t *boards, const uint8_t
     CK(copy_h2d(c, d_boards, boards, (size_t)n * kCells, c->stream));
     CK(copy_h2d(c, d_turns, turns, (size_t)n, c->stream));
     launch_pack_boards(c, d_boards, d_turns, n, mode);
-    return net_eval_common(c, n, nullptr, out_p, out_v);
+    return net_eval_common(c, n, nullptr, out_p, out_v, opponent);
+}
+extern "C" int32_t omk_net_eval(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+                                float *out_p, float *out_v) {
+    return eval_boards(c, false, boards, turns, n, mode, out_p, out_v);
 }
 
 extern "C" int32_t omk_net_eval_images(omk_ctx *c, const float *images, int32_t n, float *out_p, float *out_v) {
@@ -744,6 +768,16 @@ extern "C" int32_t omk_pool_new_games(omk_ctx *c, const int32_t *ids, int32_t n,
     return check_device_error(c);
 }
 
+// round r of execute(count, batch_size, epsilon, alpha) on the n trees of ids (nullptr: the lane's slice), on the lane in use
+static int32_t search_round(omk_ctx *c, const int32_t *ids, int n, int r, int batch_size, float epsilon, float alpha, int evaluator) {
+    if (r == 0) launch_root_noise(c, ids, n, epsilon, alpha);
+    launch_reset_requests(c);
+    launch_select_expand(c, ids, n, batch_size);
+    RUN_EVAL(c, evaluator, n * batch_size);
+    launch_apply(c, ids, n, kApplySearch);
+    return OMK_OK;
+}
+
 // execute(count, batch_size, epsilon, alpha) on the n >= 1 trees of d_ids (nullptr: 0..n-1), queued on the context stream;
 // the caller checks the device error word
 static int32_t search_rounds(omk_ctx *c, const int32_t *d_ids, int n, int count, int batch_size, float epsilon, float alpha,
@@ -763,11 +797,8 @@ static int32_t search_rounds(omk_ctx *c, const int32_t *d_ids, int n, int count,
         for (int l = 0; l < lanes; ++l) {
             LaneScope scope(c, l, lane_first[l]);
             const int32_t *ids_l = d_ids ? d_ids + lane_first[l] : nullptr;
-            if (r == 0) launch_root_noise(c, ids_l, lane_n[l], epsilon, alpha);
-            launch_reset_requests(c);
-            launch_select_expand(c, ids_l, lane_n[l], batch_size);
-            RUN_EVAL(c, evaluator, lane_n[l] * batch_size);
-            launch_apply(c, ids_l, lane_n[l], kApplySearch);
+            const int32_t rc = search_round(c, ids_l, lane_n[l], r, batch_size, epsilon, alpha, evaluator);
+            if (rc) return rc;
         }
     }
     if (lanes == 2) lanes_join(c);
@@ -1527,6 +1558,189 @@ extern "C" int32_t omk_eval_naive(omk_ctx *c, int32_t episodes, int32_t first_tr
     for (int k = 0; k < 3; ++k) out_result[k] = h_cnt[k];
     if (out_status) memcpy(out_status, host.data() + off_fin, e);
     if (out_moves) memcpy(out_moves, host.data() + off_moves, e * kCells);
+    if (out_stats) {
+        out_stats[0] = (int64_t)(h_sims[2] - h_sims[0]);
+        out_stats[1] = (int64_t)(h_sims[3] - h_sims[1]);
+        out_stats[2] = n_moves;
+        out_stats[3] = syncs;
+    }
+    if (out_gpu_ms) CK(cudaEventElapsedTime(out_gpu_ms, c->ev0, c->ev1));
+    return OMK_OK;
+}
+
+// ------------------------------------------------------------------ the opponent network and the arena (benchmark/src/main.rs:14-108)
+// the opponent's fp32 tensors, allocated on first use (all or nothing)
+static int32_t opponent_alloc(omk_ctx *c) {
+    if (c->opp.t[0]) return OMK_OK;
+    NetWeights w;
+    for (int i = 0; i < kNetTensors; ++i) CK(w.t[i].alloc((size_t)kLens[i]));
+    CK(w.heads_w.alloc(512 * 128));
+    CK(w.heads_b.alloc(128));
+    c->opp = std::move(w);
+    return OMK_OK;
+}
+// after the opponent's fp32 tensors changed: its packed heads and operand images (what omk_net_load_params does for the network)
+static int32_t opponent_prepare(omk_ctx *c) {
+    ModelScope scope(c, true);
+    net_pack_heads(c);
+    if (!fc16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split fc weight preparation failed (opponent)");
+    if (!tower16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split tower weight preparation failed (opponent)");
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    c->opp.loaded = true;
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_opponent_load_params(omk_ctx *c, const float *const *tensors, const int64_t *lens) {
+    CK(cudaSetDevice(c->device));
+    for (int i = 0; i < kNetTensors; ++i)
+        if (!tensors[i] || lens[i] != kLens[i])
+            return fail(OMK_ERR_INVALID, "tensor " + std::to_string(i) + ": expected " + std::to_string(kLens[i]) + " elements");
+    int32_t rc = opponent_alloc(c);
+    if (rc) return rc;
+    c->opp.loaded = false;  // until the images below are built
+    for (int i = 0; i < kNetTensors; ++i)
+        CK(copy_h2d(c, c->opp.t[i], tensors[i], sizeof(float) * (size_t)kLens[i], c->stream));
+    return opponent_prepare(c);
+}
+
+extern "C" int32_t omk_opponent_from_net(omk_ctx *c) {
+    CK(cudaSetDevice(c->device));
+    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
+    int32_t rc = opponent_alloc(c);
+    if (rc) return rc;
+    c->opp.loaded = false;
+    for (int i = 0; i < kNetTensors; ++i)
+        CK(cudaMemcpyAsync(c->opp.t[i], c->net.t[i], sizeof(float) * (size_t)kLens[i], cudaMemcpyDeviceToDevice, c->stream));
+    return opponent_prepare(c);
+}
+
+extern "C" int32_t omk_opponent_eval(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode, float *out_p,
+                                     float *out_v) {
+    return eval_boards(c, true, boards, turns, n, mode, out_p, out_v);
+}
+
+// stage s of one mover's half-move in omk_match, on the lane and with the model in use: 0 = ensure_action_exists + play_action of
+// the other model's previous move in the mover's trees (none before the first half-move); 1 .. rounds = the search rounds;
+// rounds + 1 = sample_action(Best) + play_action
+static int32_t match_stage(omk_ctx *c, int stage, int rounds, int half, const int32_t *trees, int n, int32_t *act, int8_t *status,
+                           int8_t *other_status, int batch_size, float epsilon, float alpha, int evaluator) {
+    if (stage == 0) {
+        if (half == 0) return OMK_OK;
+        launch_reset_requests(c);
+        launch_ensure_prepare(c, trees, act, n);
+        RUN_EVAL(c, evaluator, n);
+        launch_apply(c, trees, n, kApplyEnsure);
+        launch_play(c, trees, act, n, other_status);
+        return OMK_OK;
+    }
+    if (stage <= rounds) return search_round(c, trees, n, stage - 1, batch_size, epsilon, alpha, evaluator);
+    launch_sample(c, trees, n, nullptr, nullptr, act, nullptr, nullptr);
+    launch_play(c, trees, act, n, status);
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_match(omk_ctx *c, int32_t pairs, int32_t first_tree, int32_t count, int32_t batch_size, float epsilon,
+                             float alpha, int32_t evaluator, int32_t *out_result, int8_t *out_moves, int8_t *out_status,
+                             int64_t *out_stats, float *out_gpu_ms) {
+    CK(cudaSetDevice(c->device));
+    if (!out_result) return fail(OMK_ERR_INVALID, "out_result is NULL");
+    if (pairs < 1 || first_tree < 0 || (int64_t)first_tree + 4 * (int64_t)pairs > c->cap_trees)
+        return fail(OMK_ERR_INVALID, "need pairs >= 1 and the trees first_tree .. first_tree + 4 * pairs - 1 inside capacity_trees");
+    if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
+    if (count < 1) return fail(OMK_ERR_INVALID, "count < 1");
+    if (evaluator != OMK_EVAL_NET && evaluator != OMK_EVAL_HASH) return fail(OMK_ERR_INVALID, "unknown evaluator");
+    if (c->sp_active && first_tree < 2 * c->sp_cfg.n_games)
+        return fail(OMK_ERR_STATE, "the trees overlap the active self-play driver's trees 0 .. 2 * n_games - 1");
+    int32_t rc = check_evaluator(c, evaluator);  // with the network: weights a training step changed are packed first
+    if (rc) return rc;
+    if (evaluator == OMK_EVAL_NET && !c->opp.loaded)
+        return fail(OMK_ERR_STATE, "opponent weights not loaded (omk_opponent_load_params / omk_opponent_from_net)");
+    const int P = pairs;
+    const size_t g = 2 * (size_t)P;  // games
+    // [simulations and evaluations before / after (4 u64) | counters (8 i32) | final status g | moves g*81] leave in one copy;
+    // then the tree ids [model][leg][P] (network 0, opponent 1), the games' random streams [g], and per leg [leg][P] the moves
+    // of the half-move, the mover's statuses and the statuses of the other model's play_action
+    const size_t off_cnt = 32, off_fin = 64, off_moves = off_fin + g, out_bytes = off_moves + g * kCells;
+    const size_t off_ids = (out_bytes + 255) & ~(size_t)255, off_str = off_ids + 8 * g, off_act = off_str + 4 * g, off_st = off_act + 4 * g,
+                 off_ost = off_st + g;
+    CK(c->eval_buf.grow(c->stream, off_ost + g, 4096));
+    // both legs run at once, the network's half-move on lane 0 and the opponent's on lane 1
+    const bool two_lanes = c->lane_min_trees > 0 && lane1_ready(c);
+    const int rows = P * batch_size > 2 * P ? P * batch_size : 2 * P;
+    for (int l = 0; l < (two_lanes ? 2 : 1); ++l) {
+        LaneScope scope(c, l, 0);
+        rc = ensure_workspace(c, rows);
+        if (rc) return rc;
+    }
+    uint8_t *base = c->eval_buf;
+    unsigned long long *sims = reinterpret_cast<unsigned long long *>(base);
+    int32_t *counters = reinterpret_cast<int32_t *>(base + off_cnt);
+    int8_t *fin = reinterpret_cast<int8_t *>(base + off_fin), *moves = reinterpret_cast<int8_t *>(base + off_moves);
+    int32_t *ids = reinterpret_cast<int32_t *>(base + off_ids), *actions = reinterpret_cast<int32_t *>(base + off_act);
+    uint32_t *streams = reinterpret_cast<uint32_t *>(base + off_str);
+    int8_t *status = reinterpret_cast<int8_t *>(base + off_st), *other_status = reinterpret_cast<int8_t *>(base + off_ost);
+
+    fold_requests(c);  // counts earlier calls left pending are not this call's
+    CK(cudaMemcpyAsync(sims, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev0, c->stream));
+    launch_match_init(c, P, first_tree, ids, streams, moves, fin, counters);
+    for (int m = 0; m < 2; ++m) {  // Agent::new for every game's tree of model m, under model m's weights
+        ModelScope scope(c, m == 1);
+        launch_reset_requests(c);
+        launch_new_games(c, ids + m * g, (int)g, streams, nullptr, nullptr);
+        RUN_EVAL(c, evaluator, (int)g);
+        launch_apply(c, ids + m * g, (int)g, kApplyNewGame);
+    }
+    const int rounds = (count + batch_size - 1) / batch_size;  // parallel_mcts_executor.rs:39-42,207
+    int32_t back[3] = {0, P, P};  // {device error word, live games in leg 0, in leg 1}
+    int *live = back + 1;
+    int64_t n_moves = 0, syncs = 0;
+    // a game ends after at most 81 moves; a device error (out of node slots, a non-finite network output, a refused move)
+    // ends the match at the half-move that raised it
+    for (int half = 0; (live[0] > 0 || live[1] > 0) && back[0] == 0 && half < kCells; ++half) {
+        // the movers of this half-move: the network in leg half % 2, the opponent in the other leg
+        struct Part {
+            int leg;
+            bool opponent;
+        } part[2];
+        int parts = 0;
+        for (int m = 0; m < 2; ++m) {
+            const int leg = (half + m) % 2;
+            if (live[leg] > 0) part[parts++] = {leg, m == 1};
+        }
+        const int lanes = two_lanes && parts == 2 ? 2 : 1;
+        if (lanes == 2) lanes_fork(c);
+        for (int stage = 0; stage < rounds + 2 && rc == OMK_OK; ++stage)
+            for (int p = 0; p < parts && rc == OMK_OK; ++p) {
+                LaneScope lane(c, lanes == 2 ? p : 0, 0);
+                ModelScope model(c, part[p].opponent);
+                const int leg = part[p].leg;
+                rc = match_stage(c, stage, rounds, half, ids + ((part[p].opponent ? 2 : 0) + leg) * P, live[leg], actions + leg * P,
+                                 status + leg * P, other_status + leg * P, batch_size, epsilon, alpha, evaluator);
+            }
+        if (lanes == 2) lanes_join(c);  // on an error too: nothing queued on lane 1 is left unordered with the main stream
+        if (rc) return rc;
+        launch_match_advance(c, P, first_tree, half, live, ids, actions, status, other_status, moves, fin, counters);
+        n_moves += live[0] + live[1];
+        // the half-move's one host round trip: both legs' live counts size the next launches
+        CK(copy_d2h(c, back, counters + 3, sizeof back, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        ++syncs;
+    }
+    fold_requests(c);
+    CK(cudaMemcpyAsync(sims + 2, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev1, c->stream));
+    std::vector<uint8_t> host(out_bytes);
+    CK(copy_d2h(c, host.data(), base, out_bytes, c->stream));
+    rc = check_device_error(c);  // (synchronises the stream)
+    ++syncs;
+    if (rc) return rc;
+    const unsigned long long *h_sims = reinterpret_cast<const unsigned long long *>(host.data());
+    const int32_t *h_cnt = reinterpret_cast<const int32_t *>(host.data() + off_cnt);
+    for (int k = 0; k < 3; ++k) out_result[k] = h_cnt[k];
+    if (out_status) memcpy(out_status, host.data() + off_fin, g);
+    if (out_moves) memcpy(out_moves, host.data() + off_moves, g * kCells);
     if (out_stats) {
         out_stats[0] = (int64_t)(h_sims[2] - h_sims[0]);
         out_stats[1] = (int64_t)(h_sims[3] - h_sims[1]);

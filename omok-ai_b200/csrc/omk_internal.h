@@ -92,10 +92,20 @@ struct TowerImages {  // tower_f16.cu
     Buf<float> tower16_pimg;         // fp32 stem / bias / depthwise parameters + inverse scales
     Buf<uint32_t> tower16_absmax;    // [9]
 };
-struct NetWeights : FcImages, TowerImages {
+struct WeightMaps {  // tensor maps (fc_f16.cu) over one model's fp16 weight images
+    CUtensorMap map0_b_hi, map0_b_lo;    // fc0 (B boxes of 128 rows: the pair kernel loads half tiles)
+    CUtensorMap map0s_b_hi, map0s_b_lo;  // fc0 weights with 256-row boxes (one-CTA split-K kernel for small batches)
+    CUtensorMap map1_b_hi, map1_b_lo;    // fc1 (B boxes of 256 rows)
+    CUtensorMap map2_b_hi, map2_b_lo;    // heads (B = all 128 padded output rows)
+    bool weights_ready = false;
+};
+// Everything derived from one set of weights.  The context holds two: the network (`net`: every entry point, the trainer)
+// and the opponent (`opp`: omk_opponent_eval, omk_match).  The evaluator reads the active one, omk_ctx::model.
+struct NetWeights : FcImages, TowerImages, WeightMaps {
     Buf<float> t[kNetTensors];  // device copies in checkpoint order
     Buf<float> heads_w;         // [512][128]: cols 0..80 policy, col 81 value, rest 0
     Buf<float> heads_b;         // [128]
+    std::vector<uint8_t> tower16_params_host;  // host copy of the tower's fp32 parameter image (kernel argument of k_tower16)
     bool loaded = false;
 };
 
@@ -219,15 +229,16 @@ struct omk_ctx {
     omk::Buf<uint32_t> dev_error;    // sticky device error word
     omk::Buf<unsigned long long> dev_sims;  // simulations counter
 
-    omk::NetWeights net;
+    omk::NetWeights net;            // the network
+    omk::NetWeights opp;            // the opponent (omk_opponent_load_params / omk_opponent_from_net); buffers allocated on first load
+    omk::NetWeights *model = &net;  // the weights the evaluator reads: `net`, or `opp` inside a ModelScope (omk_api.cu)
     omk::Workspace ws;
     int virtual_loss = 0;           // opt-in, non-reference search mode (omk_search_set_virtual_loss); refused with the parity evaluator
     int fc0_balance = 0;            // fc0 tail balancing of the CTA-pair kernel (fc_f16.cu FcBal): 0 off (default), 1 on
     int fc0_chunk = 9;              // k-blocks of fc0 accumulated in tensor memory per drain: 9 (default) or 3 (finer, more accurate; fc_f16.cu)
     int fc0_mode = 1;               // fc0 + fc1: 1 = tcgen05 3xFP16 k_fc16 (the product path), 0 = fp32 CUDA-core k_gemm (A/B check only)
-    std::unique_ptr<omk::Fc16State, omk::Fc16StateFree> fc16_state;  // weight tensor maps of the fp16-split path (fc_f16.cu)
+    std::unique_ptr<omk::Fc16State, omk::Fc16StateFree> fc16_state;  // the device's occupancy answers for the fp16-split path (fc_f16.cu)
     int tower16_pairs = 0;          // resident CTA pairs of k_tower16 (0 = not queried yet)
-    std::vector<uint8_t> tower16_params_host;  // host copy of the tower's fp32 parameter image (kernel argument of k_tower16)
     std::unique_ptr<omk::TrainState, omk::TrainStateFree> train_state;  // trainer step workspace, Adadelta slots, optional NCCL communicator (train_kernels.cu)
     int train_n = 0;                // positions of the minibatch currently on the device (omk_train_backward)
     bool net_pack_dirty = false;    // omk_train_apply changed the fp32 weights: the tensor-core operand images (and a running self-play
@@ -249,7 +260,7 @@ struct omk_ctx {
     cudaStream_t sp_copy_stream = nullptr;
     cudaEvent_t sp_ev_rec[kSpRing][2] = {}, sp_ev_copy[kSpRing] = {};
     omk::Replay rp;                   // device replay memory (omk_replay_reset); fed by the driver when it exists at omk_selfplay_begin
-    omk::Buf<uint8_t> eval_buf;       // omk_eval_naive's per-call state (grow-only)
+    omk::Buf<uint8_t> eval_buf;       // omk_eval_naive's and omk_match's per-call state (grow-only)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
@@ -309,6 +320,13 @@ void launch_eval_init(omk_ctx *c, int episodes, int first_tree, int32_t *ids, in
                       int32_t *counters);
 void launch_eval_advance(omk_ctx *c, int32_t *ids, int n, const int32_t *actions, const int8_t *status, int first_tree, int32_t *ply,
                          int8_t *moves, int8_t *final_status, int32_t *counters);
+// omk_match (DESIGN.md 4): its set-up, and its bookkeeping after each half-move of both legs.  ids = [model][leg][pairs] tree
+// ids of the live games (network 0, opponent 1), actions / status / other_status = [leg][pairs], counters = {network wins,
+// opponent wins, draws, device error word, live in leg 0, live in leg 1}
+void launch_match_init(omk_ctx *c, int pairs, int first_tree, int32_t *ids, uint32_t *streams, int8_t *moves, int8_t *final_status,
+                       int32_t *counters);
+void launch_match_advance(omk_ctx *c, int pairs, int first_tree, int half, const int *live, int32_t *ids, int32_t *actions,
+                          const int8_t *status, const int8_t *other_status, int8_t *moves, int8_t *final_status, int32_t *counters);
 
 // omk_api.cu: open / close a profiling span of kernel family `kind` (no-op below min_level)
 bool prof_begin(omk_ctx *c, int kind, int min_level);

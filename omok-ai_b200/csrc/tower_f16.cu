@@ -865,7 +865,7 @@ __global__ void k_tower16_pack(Tower16PackArgs a, const uint32_t *absmax, uint8_
 }
 
 bool tower16_prepare_weights(omk_ctx *c) {
-    NetWeights &w = c->net;
+    NetWeights &w = *c->model;
     if (!w.tower16_wimg) {
         TowerImages t;
         if (t.tower16_wimg.alloc(3 * W16_BYTES) != cudaSuccess || t.tower16_pimg.alloc(P16_FLOATS) != cudaSuccess ||
@@ -887,8 +887,8 @@ bool tower16_prepare_weights(omk_ctx *c) {
     k_tower16_pack<<<16, 256, 0, c->stream>>>(a, w.tower16_absmax, w.tower16_wimg, w.tower16_pimg);
     c->launches += 2;
     // the fp32 parameter image is passed to k_tower16 by value (constant bank): keep a host copy
-    c->tower16_params_host.resize(sizeof(Tower16Params));
-    if (cudaMemcpyAsync(c->tower16_params_host.data(), w.tower16_pimg, sizeof(Tower16Params), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return false;
+    w.tower16_params_host.resize(sizeof(Tower16Params));
+    if (cudaMemcpyAsync(w.tower16_params_host.data(), w.tower16_pimg, sizeof(Tower16Params), cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return false;
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return false;
     return true;
 }
@@ -950,13 +950,14 @@ bool launch_tower_f16(omk_ctx *c, const float *images_dev, int rows_bound) {
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    const uint8_t *wimg = c->net.tower16_wimg;
-    if (c->tower16_params_host.empty()) return false;
-    const Tower16Params &params = *reinterpret_cast<const Tower16Params *>(c->tower16_params_host.data());
+    const NetWeights &m = *c->model;
+    const uint8_t *wimg = m.tower16_wimg;
+    if (m.tower16_params_host.empty()) return false;
+    const Tower16Params &params = *reinterpret_cast<const Tower16Params *>(m.tower16_params_host.data());
     const NNIn *nn_in = c->ws.nn_in;
     const uint32_t *n_req = c->ws.n_req;
     const ActMaps &maps = c->ws.maps;  // the write-out over this workspace's act0 arrays
-    const float *pimg = c->net.tower16_pimg;
+    const float *pimg = m.tower16_pimg;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, wimg, params, nn_in, images_dev, n_req, rows_bound, maps.tower_st_hi,
                                              maps.tower_st_lo, pimg);
     if (e != cudaSuccess) fprintf(stderr, "omok_b200: cudaLaunchKernelEx(k_tower16): %s\n", cudaGetErrorString(e));

@@ -119,6 +119,11 @@ extern "C" {
     // evaluation against the naive player (src/trainer.rs:487-603)
     pub fn omk_naive_move(ctx: *mut omk_ctx, boards: *const u8, turns: *const u8, n: i32, seed: u64, streams: *const u32, out_actions: *mut i32, out_forced: *mut u8) -> i32;
     pub fn omk_eval_naive(ctx: *mut omk_ctx, episodes: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, seed: u64, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
+    // the opponent network and the arena (benchmark/src/main.rs:14-108)
+    pub fn omk_opponent_load_params(ctx: *mut omk_ctx, tensors: *const *const f32, lens: *const i64) -> i32;
+    pub fn omk_opponent_from_net(ctx: *mut omk_ctx) -> i32;
+    pub fn omk_opponent_eval(ctx: *mut omk_ctx, boards: *const u8, turns: *const u8, n: i32, mode: i32, out_p: *mut f32, out_v: *mut f32) -> i32;
+    pub fn omk_match(ctx: *mut omk_ctx, pairs: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
 }
 
 /// The message of the last failing call on this thread.

@@ -12,7 +12,11 @@ self-play driver feeds it on the device, no transition is streamed, and the whol
 the steps -- is ONE omk_train_replay call, timed as such (train_phase_s); every rank samples its own replay memory.
 With --evaluate EPISODES the trained weights then play the trainer's evaluation against the naive player
 (src/trainer.rs:487-603) as ONE omk_eval_naive call on trees past the self-play driver's 2 * games, so the driver stays
-active for the next iteration; it reports eval_phase_s and the naive player's wins, the model's wins and the draws."""
+active for the next iteration; it reports eval_phase_s and the naive player's wins, the model's wins and the draws.
+With --gate GAMES the network is copied into the context's opponent before the training phase (omk_opponent_from_net), and
+after training the trained network plays GAMES games against that snapshot at the benchmark's constants (800 simulations,
+batch 8, epsilon 0, alpha 1; benchmark/src/main.rs) as ONE omk_match call on trees past the driver's and the evaluation's:
+AlphaZero's gating question, whether this iteration's network beats the last one."""
 from __future__ import annotations
 
 import argparse
@@ -32,7 +36,7 @@ N_PARAMS = 5_643_250
 
 
 def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
-        device_replay=False, replay_capacity=600_000, evaluate=0):
+        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0):
     omk = importlib.import_module("omok-ai_b200")
     trainer = importlib.import_module("omok-ai_b200.trainer")
     sharding = importlib.import_module("omok-ai_b200.sharding")
@@ -46,8 +50,11 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     if device_replay and (torch_step or gather):
         raise ValueError("--device-replay trains through omk_train_replay: it excludes --torch-step and --gather")
+    if gate and gate < 2:
+        raise ValueError("--gate GAMES needs at least 2 games: one opened by each side")
     my_games = games_per_gpu
-    ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games + evaluate, capacity_nodes=4096,
+    ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games + evaluate + 4 * (gate // 2),
+                      capacity_nodes=4096,
                       seed=sharding.rank_seed(seed, rank))
     ctx.net_init_random(seed)                       # identical weights on every rank
     if torch_step:
@@ -64,7 +71,7 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     if device_replay:
         ctx.replay_reset(replay_capacity)           # before selfplay_begin: the driver feeds the replay that exists then
         return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
-                                  seed, quiet, replay_capacity, evaluate)
+                                  seed, quiet, replay_capacity, evaluate, gate)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -90,6 +97,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         mem.add_episode(flat_b[: 4 * minibatch], flat_p[: 4 * minibatch], 0.0)
 
     # ---- training phase: data parallel over the minibatch, one gradient all-reduce per step ----
+    if gate:
+        ctx.opponent_from_net()                     # the snapshot the trained network has to beat
     per_rank = max(1, minibatch // world)
     batches = [mem.sample(per_rank) for _ in range(steps + 2)]
     enc = [(trainer.encode_nn_input(b, t), pi, z) for b, t, pi, z in batches]
@@ -147,6 +156,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
            "first_loss": losses[0][2], "last_loss": losses[-1][2], "policy_sums_to_one": bool(abs(float(p[0].sum()) - 1) < 1e-3)}
     if evaluate:
         out.update(_evaluate(ctx, evaluate, 2 * my_games, count, batch, seed))
+    if gate:
+        out.update(_gate(ctx, gate, 2 * my_games + evaluate))
     if rank == 0 and not quiet:
         print(json.dumps(out), flush=True)
     ctx.close()
@@ -166,8 +177,20 @@ def _evaluate(ctx, episodes, first_tree, count, batch, seed):
             "eval_draws": draw, "eval_moves": stats["moves"], "eval_host_syncs": stats["host_syncs"], "eval_gpu_ms": stats["gpu_ms"]}
 
 
+def _gate(ctx, games, first_tree):
+    """The gating match: the trained network against the snapshot taken before training, one omk_match call at the
+    benchmark's constants."""
+    omk = importlib.import_module("omok-ai_b200")
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    (net, snap, draw), _, _, stats = ctx.match(games // 2, first_tree=first_tree, count=800, batch_size=8, epsilon=0.0, alpha=1.0,
+                                               evaluator=omk.EVAL_NET)
+    return {"gate_games": 2 * (games // 2), "gate_phase_s": time.perf_counter() - t0, "gate_trained_wins": net, "gate_snapshot_wins": snap,
+            "gate_draws": draw, "gate_moves": stats["moves"], "gate_host_syncs": stats["host_syncs"], "gate_gpu_ms": stats["gpu_ms"]}
+
+
 def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity,
-                       evaluate=0):
+                       evaluate=0, gate=0):
     omk = importlib.import_module("omok-ai_b200")
     ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
     ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
@@ -181,6 +204,8 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
         raise SystemExit("no game finished during self-play, so the replay memory is empty: raise --plies")
     per_rank = max(1, minibatch // world)
     sampler_seed = sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
+    if gate:
+        ctx.opponent_from_net()                     # the snapshot the trained network has to beat
     step.train_replay(2, per_rank, sampler_seed)   # warm-up: training workspace, split-K scratch
     torch.cuda.synchronize()
     if dist:
@@ -203,6 +228,8 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
            "first_loss": float(losses[0, 2]), "last_loss": float(losses[-1, 2]), "h2d_bytes_total": h2d}
     if evaluate:
         out.update(_evaluate(ctx, evaluate, 2 * games, count, batch, seed))
+    if gate:
+        out.update(_gate(ctx, gate, 2 * games + evaluate))
     if rank == 0 and not quiet:
         print(json.dumps(out), flush=True)
     ctx.close()
@@ -225,6 +252,9 @@ if __name__ == "__main__":
     ap.add_argument("--replay-capacity", type=int, default=600_000, help="rows of the device replay memory per GPU (src/config.rs: 600 000)")
     ap.add_argument("--evaluate", type=int, default=0, metavar="EPISODES",
                     help="after training, play EPISODES games against the naive player on the device (omk_eval_naive)")
+    ap.add_argument("--gate", type=int, default=0, metavar="GAMES",
+                    help="after training, play GAMES games of the trained network against its pre-training snapshot (omk_match)")
     a = ap.parse_args()
     run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
-        device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate)
+        device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate,
+        gate=a.gate)
