@@ -349,6 +349,33 @@ OMK_API int32_t omk_match(omk_ctx *ctx, int32_t pairs, int32_t first_tree, int32
                           float alpha, int32_t evaluator, int32_t *out_result, int8_t *out_moves, int8_t *out_status,
                           int64_t *out_stats, float *out_gpu_ms);
 
+/* ---------------------------------------------------------------- model slots and the tournament
+ * A context holds 16 weight sets ("model slots").  Slot 0 is the network, slot 1 the opponent (omk_opponent_* are the calls
+ * below with slot 1); slots 2 .. 15 are further weight sets, read only by omk_model_eval and omk_tournament.  A slot's device
+ * buffers (about 45 MB) are allocated on its first load.  Slot 0 is OMK_ERR_INVALID in omk_model_load_params and
+ * omk_model_from_net: omk_net_load_params and the trainer own it. */
+OMK_API int32_t omk_model_load_params(omk_ctx *ctx, int32_t slot, const float *const *tensors, const int64_t *lens); /* as omk_net_load_params */
+/* device-to-device copy of the network's current fp32 weights (a snapshot); OMK_ERR_STATE if no network is loaded */
+OMK_API int32_t omk_model_from_net(omk_ctx *ctx, int32_t slot);
+OMK_API int32_t omk_model_eval(omk_ctx *ctx, int32_t slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+                               float *out_p, float *out_v); /* omk_net_eval with slot `slot`'s weights; slot 0 == omk_net_eval */
+/* A round-robin of omk_match over n_models (2 .. 16) distinct slots[]: P = n(n-1)/2 pairings (i, j), i < j, in lexicographic
+ * order.  Pairing p is exactly omk_match(pairs, ...) with slots[i] as the network ("left") and slots[j] as the opponent
+ * ("right"), on the trees first_tree + 4*pairs*p .. laid out as omk_match lays out its trees at that first tree; game g of
+ * pairing p has random stream g % pairs.  Every game equals its game in that omk_match call.  At each half-move a model
+ * searches all its pairings' movers as one group under its weights; the groups alternate over the two search lanes.
+ * evaluator OMK_EVAL_NET: every listed slot must be loaded (OMK_ERR_STATE otherwise) and the network too, as in omk_match;
+ * OMK_EVAL_HASH: the hash evaluator for every model (refused with virtual loss on).  OMK_ERR_STATE if the trees overlap an
+ * active self-play driver's trees 0 .. 2 * n_games - 1.  A device error (out of node slots, a non-finite network output, a
+ * refused move) ends the call at that half-move: OMK_ERR_CAPACITY, OMK_ERR_NUMERIC or OMK_ERR_STATE.
+ * out_result[3*P]: per pairing {left wins, right wins, draws}; out_moves[P*2*pairs*81] and out_status[P*2*pairs] (may be
+ * NULL): row p*2*pairs + g is pairing p's game g, as in omk_match; out_stats[4] (may be NULL) = {simulations, positions
+ * evaluated, moves, host synchronisations}; out_gpu_ms (may be NULL).  One host round trip of 4*(n_models+1) bytes per
+ * half-move; no host-to-device copy. */
+OMK_API int32_t omk_tournament(omk_ctx *ctx, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
+                               int32_t batch_size, float epsilon, float alpha, int32_t evaluator, int32_t *out_result, int8_t *out_moves,
+                               int8_t *out_status, int64_t *out_stats, float *out_gpu_ms);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,6 +5,9 @@
                                  then `sample_action(Best)`; the opponent follows with ensure_action_exists + play_action.
   * `play_match_device`          the same match as ONE call (omk_match) between the context's network (left) and its
                                  opponent network (right): both legs run at once, each model's half-move on its own lane.
+  * `play_tournament_device`     a round-robin of that match over up to 16 model slots of one context as ONE call
+                                 (omk_tournament); each model searches all its pairings' movers as one batch per half-move.
+  * `ratings`                    a Bradley-Terry fit, in Elo units, of a tournament's pairwise results.
   * `play_against_naive_player`  src/trainer.rs:487-603: the naive player takes the first legal move (ascending) that ends
                                  the game for itself, or that would end it for the opponent (a block); else a random
                                  legal move.  The model answers with ParallelMCTSExecutor::execute + Best.
@@ -75,6 +78,53 @@ def play_match_device(ctx, game_count: int = 100, count: int = 800, batch_size: 
     if moves_out is not None:
         moves_out[:] = [[int(a) for a in row if a >= 0] for row in moves]
     return result
+
+
+def play_tournament_device(ctx, slots, game_count: int = 100, count: int = 800, batch_size: int = 8, epsilon: float = 0.0,
+                           alpha: float = 1.0, evaluator: int = B.EVAL_NET, first_tree: int = 0, moves_out: list | None = None):
+    """A round-robin of `play_match_device` over the model slots `slots` (`Context.model_load_params` / `model_from_net`; slot 0
+    is the network, slot 1 the opponent) from one `omk_tournament` call of `game_count // 2` pairs per pairing, on the trees
+    first_tree .. first_tree + 2 * game_count * P - 1.  Pairing p = (i, j), i < j in lexicographic order, is
+    `play_match_device` with slots[i] left and slots[j] right.  Returns the [P, 3] table of (left wins, right wins, draws).
+    `moves_out`, if given, receives per pairing one move list per game in `play_match`'s order."""
+    result, moves, _, _ = ctx.tournament(slots, game_count // 2, first_tree=first_tree, count=count, batch_size=batch_size,
+                                         epsilon=epsilon, alpha=alpha, evaluator=evaluator)
+    if moves_out is not None:
+        moves_out[:] = [[[int(a) for a in row if a >= 0] for row in pairing] for pairing in moves]
+    return result
+
+
+def ratings(result, n_models: int, iterations: int = 100000, tol: float = 1e-12) -> np.ndarray:
+    """Elo ratings of the n_models models of a tournament from its [P, 3] table of (left wins, right wins, draws), pairings
+    (i, j), i < j, in lexicographic order: the maximum-likelihood Bradley-Terry strengths (Hunter's MM iteration), each
+    reported as 400 * log10(strength / strength of model 0), so model 0 (slots[0]) is rated 0.  A draw counts as half a win
+    to each side, and every pairing gets one virtual draw, which keeps a clean sweep finite.  Deterministic; with two models
+    the rating difference is 400 * log10((w + d/2 + 0.5) / (l + d/2 + 0.5))."""
+    r = np.asarray(result, dtype=np.float64).reshape(-1, 3)
+    n = int(n_models)
+    if n < 2 or r.shape[0] != n * (n - 1) // 2:
+        raise ValueError(f"need n_models >= 2 and n(n-1)/2 = {n * (n - 1) // 2} pairings, got {r.shape[0]}")
+    if (r < 0).any():
+        raise ValueError("negative game counts")
+    games = np.zeros((n, n))   # games[i, j]: games between i and j, the virtual draw included
+    score = np.zeros(n)        # each model's wins + draws / 2, virtual draws included
+    p = 0
+    for i in range(n):
+        for j in range(i + 1, n):
+            w, l, d = r[p]
+            games[i, j] = games[j, i] = w + l + d + 1.0
+            score[i] += w + 0.5 * d + 0.5
+            score[j] += l + 0.5 * d + 0.5
+            p += 1
+    gamma = np.ones(n)
+    for _ in range(iterations):
+        nxt = score / (games / (gamma[:, None] + gamma[None, :])).sum(axis=1)
+        nxt /= nxt[0]
+        done = np.max(np.abs(np.log(nxt) - np.log(gamma))) < tol
+        gamma = nxt
+        if done:
+            break
+    return 400.0 * np.log10(gamma)
 
 
 def naive_moves(ctx, boards: np.ndarray, turns: np.ndarray, rng: np.random.Generator) -> np.ndarray:

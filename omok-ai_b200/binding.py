@@ -150,6 +150,10 @@ def load_library():
     L.omk_opponent_from_net.argtypes = [vp]
     L.omk_opponent_eval.argtypes = [vp, vp, vp, i32, i32, vp, vp]
     L.omk_match.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
+    L.omk_model_load_params.argtypes = [vp, i32, P(vp), P(i64)]
+    L.omk_model_from_net.argtypes = [vp, i32]
+    L.omk_model_eval.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
+    L.omk_tournament.argtypes = [vp, i32, vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
     for name in declared_symbols():
         fn = getattr(L, name)  # raises AttributeError if the library lacks a declared symbol
         if name not in ("omk_last_error", "omk_ctx_stream", "omk_ctx_launch_count"):
@@ -576,3 +580,45 @@ class Context:
         info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
         info["gpu_ms"] = float(gpu_ms.value)
         return (int(result[0]), int(result[1]), int(result[2])), moves, status, info
+
+    # ---- model slots and the tournament ----
+    def model_load_params(self, slot: int, params):
+        """Weights into model slot `slot` (1 .. 15; 1 is the opponent), read only by model_eval, match (slot 1) and tournament."""
+        arrs = [np.ascontiguousarray(p, dtype=np.float32).reshape(-1) for p in params]
+        ptrs = (C.c_void_p * 31)(*[a.ctypes.data for a in arrs])
+        lens = (C.c_int64 * 31)(*[a.size for a in arrs])
+        self._check(self.L.omk_model_load_params(self.h, slot, ptrs, lens))
+
+    def model_from_net(self, slot: int):
+        """Model slot `slot` becomes a device-side copy of the network's current weights (a snapshot)."""
+        self._check(self.L.omk_model_from_net(self.h, slot))
+
+    def model_eval(self, slot: int, boards, turns, mode: int = 0, want_v: bool = True):
+        """net_eval with model slot `slot`'s weights (slot 0 is the network)."""
+        boards = np.ascontiguousarray(boards, dtype=np.uint8).reshape(-1, CELLS)
+        turns = np.ascontiguousarray(turns, dtype=np.uint8).reshape(-1)
+        n = boards.shape[0]
+        p = np.zeros((n, CELLS), dtype=np.float32)
+        v = np.zeros(n, dtype=np.float32) if want_v else None
+        self._check(self.L.omk_model_eval(self.h, slot, _ptr(boards), _ptr(turns), n, mode, _ptr(p), _ptr(v)))
+        return p, v
+
+    def tournament(self, slots, pairs: int, first_tree: int = 0, count: int = 800, batch_size: int = 8, epsilon: float = 0.0,
+                   alpha: float = 1.0, evaluator: int = EVAL_NET):
+        """A round-robin of `match` over the model slots `slots` in one call: pairing p = (i, j), i < j in lexicographic order,
+        is match(pairs) with slots[i] as the network (left) and slots[j] as the opponent (right), on the trees
+        first_tree + 4 * pairs * p ..  Returns (result [P, 3] i32 (left wins, right wins, draws), moves [P, 2 * pairs, 81] i8
+        (-1 past a game's end), final status [P, 2 * pairs] i8, stats dict: simulations, nn_evals, moves, host_syncs, gpu_ms)."""
+        s = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
+        n_pairings = max(s.size * (s.size - 1) // 2, 0)
+        games = max(2 * pairs, 0)
+        result = np.zeros((n_pairings, 3), dtype=np.int32)
+        moves = np.zeros((n_pairings, games, CELLS), dtype=np.int8)
+        status = np.zeros((n_pairings, games), dtype=np.int8)
+        stats = np.zeros(4, dtype=np.int64)
+        gpu_ms = C.c_float()
+        self._check(self.L.omk_tournament(self.h, s.size, _ptr(s), pairs, first_tree, count, batch_size, epsilon, alpha, evaluator,
+                                          _ptr(result), _ptr(moves), _ptr(status), _ptr(stats), C.byref(gpu_ms)))
+        info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
+        info["gpu_ms"] = float(gpu_ms.value)
+        return result, moves, status, info

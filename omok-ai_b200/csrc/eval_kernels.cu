@@ -1,6 +1,7 @@
 // eval_kernels.cu -- the trainer's evaluation against the naive player (src/trainer.rs:487-603) on the device: the naive
 // player's move (:506-537) and the bookkeeping omk_eval_naive runs after every half-move; the same bookkeeping for the
-// arena between the network and the opponent (omk_match, benchmark/src/main.rs:14-108).
+// arena between the network and the opponent (omk_match, benchmark/src/main.rs:14-108), and for a round-robin of that arena
+// over up to kModelSlots models (omk_tournament).
 #include "omk_internal.h"
 
 namespace omk {
@@ -229,6 +230,130 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_match_advance(int pairs, in
     }
 }
 
+// ---- the tournament (omk_tournament): omk_match's bookkeeping over n models and their n(n-1)/2 pairings ----
+// pairing p = (a, b), a < b, in lexicographic order
+__device__ __forceinline__ void tourney_pairing(int p, int n, int &a, int &b) {
+    a = 0;
+    while (p >= n - 1 - a) p -= n - 1 - a++;
+    b = a + 1 + p;
+}
+// the r-th pairing (in pairing order) of model m, and m's side in it (0 left, 1 right)
+__device__ __forceinline__ void tourney_model_pairing(int m, int r, int n, int &p, int &side) {
+    const int a = r < m ? r : m, b = r < m ? m : r + 1;
+    p = a * n - a * (a + 1) / 2 + (b - a - 1);
+    side = r < m ? 1 : 0;
+}
+
+// A fresh tournament: pairing p's trees are first_tree + 4 * pairs * p + omk_match's layout, every game live, nothing tallied.
+// Model m's list gids[m] holds every tree of m (both legs of each of its pairings, in pairing order) with the tree's stream in
+// gstr[m], for Agent::new under m's weights.
+__global__ void k_tourney_init(TourneyState t) {
+    const int Q = t.pairs, P = t.n * (t.n - 1) / 2, per_model = (t.n - 1) * 2 * Q;
+    const long long total = (long long)P * 2 * Q * kCells;
+    for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < total; k += (long long)gridDim.x * blockDim.x) {
+        t.moves[k] = -1;
+        if (k < 4LL * Q * P) t.ids[k] = t.first_tree + (int)k;
+        if (k < 2LL * Q * P) {
+            t.actions[k] = -1;
+            t.final_status[k] = kInProgress;
+        }
+        if (k < 2 * P) t.live[k] = Q;
+        if (k < 3 * P) t.counters[k] = 0;
+        if (k < (long long)t.n * per_model) {
+            const int m = (int)(k / per_model), i = (int)(k % per_model), w = i % (2 * Q);
+            int p, side;
+            tourney_model_pairing(m, i / (2 * Q), t.n, p, side);
+            t.gids[(size_t)m * t.gcap + i] = t.first_tree + 4 * Q * p + side * 2 * Q + w;
+            t.gstr[(size_t)m * t.gcap + i] = (uint32_t)(w % Q);
+        }
+    }
+}
+
+// After half-move `half`, one block per (pairing, leg): k_match_advance for that leg, with the movers' actions and statuses
+// read out of their model's group segment.  The left model moves in leg half % 2, the right one in the other leg.
+__global__ void __launch_bounds__(kAdvanceThreads) k_tourney_advance(TourneyState t, int half, uint32_t *dev_error) {
+    __shared__ int warp_kept[kAdvanceThreads / 32];
+    __shared__ int kept_before;
+    const int p = blockIdx.x >> 1, leg = blockIdx.x & 1, Q = t.pairs;
+    int a_model, b_model;
+    tourney_pairing(p, t.n, a_model, b_model);
+    const int mover = leg == half % 2 ? a_model : b_model;
+    const int n = t.live[2 * p + leg];
+    const size_t seg = (size_t)mover * t.gcap + t.off[2 * p + leg];
+    const int32_t *g_act = t.gact + seg;
+    const int8_t *g_st = t.gst + seg, *g_ost = t.gost + seg;
+    int32_t *ids_l = t.ids + (size_t)(4 * p + leg) * Q, *ids_r = t.ids + (size_t)(4 * p + 2 + leg) * Q;
+    int32_t *act = t.actions + (size_t)(2 * p + leg) * Q;
+    const int base = t.first_tree + 4 * Q * p;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (threadIdx.x == 0) kept_before = 0;
+    __syncthreads();
+    for (int c0 = 0; c0 < n; c0 += kAdvanceThreads) {
+        const int i = c0 + threadIdx.x;
+        bool keep = false;
+        int32_t tl = 0, tr = 0, a = 0;
+        if (i < n) {
+            tl = ids_l[i];
+            tr = ids_r[i];
+            a = g_act[i];
+            const int g = tl - base;
+            const int st = g_st[i];
+            const size_t row = (size_t)p * 2 * Q + g;
+            t.moves[row * kCells + half] = (int8_t)a;
+            if (half > 0 && g_ost[i] != kInProgress) atomicOr(dev_error, 16u);
+            if (st == kInProgress) {
+                keep = true;
+            } else if (st == kDraw || st == kBlackWin || st == kWhiteWin) {
+                t.final_status[row] = (int8_t)st;
+                const int opener = g < Q ? 0 : 1;
+                atomicAdd(&t.counters[3 * p + (st == kDraw ? 2 : (st == kBlackWin ? opener : 1 - opener))], 1);
+            } else {
+                atomicOr(dev_error, 16u);  // Option::None: the move was refused -- the game could never end
+            }
+        }
+        const uint32_t b = __ballot_sync(kFullMask, keep);
+        if (lane == 0) warp_kept[warp] = __popc(b);
+        __syncthreads();  // every entry of this chunk has been read before any is overwritten
+        int dst = kept_before + __popc(b & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) dst += warp_kept[w];
+        if (keep) {
+            ids_l[dst] = tl;
+            ids_r[dst] = tr;
+            act[dst] = a;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0)
+            for (int w = 0; w < kAdvanceThreads / 32; ++w) kept_before += warp_kept[w];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) t.live[2 * p + leg] = kept_before;
+}
+
+// The groups of half-move `half`, one block per model m: the concatenation, in pairing order, of the live lists of the legs
+// m moves in (its trees, and the moves they take first: the other side's previous ones), each segment's offset, and the
+// group's size.  Block 0 also copies the device error word next to the sizes.
+__global__ void k_tourney_gather(TourneyState t, int half, uint32_t *dev_error) {
+    const int m = blockIdx.x, Q = t.pairs;
+    int32_t *g_ids = t.gids + (size_t)m * t.gcap, *g_act = t.gact + (size_t)m * t.gcap;
+    int o = 0;
+    for (int r = 0; r < t.n - 1; ++r) {
+        int p, side;
+        tourney_model_pairing(m, r, t.n, p, side);
+        const int leg = (half + side) % 2, cnt = t.live[2 * p + leg];
+        const int32_t *src_ids = t.ids + (size_t)(4 * p + 2 * side + leg) * Q, *src_act = t.actions + (size_t)(2 * p + leg) * Q;
+        for (int j = threadIdx.x; j < cnt; j += blockDim.x) {
+            g_ids[o + j] = src_ids[j];
+            g_act[o + j] = src_act[j];
+        }
+        if (threadIdx.x == 0) t.off[2 * p + leg] = o;
+        o += cnt;
+    }
+    if (threadIdx.x == 0) {
+        t.back[1 + m] = o;
+        if (m == 0) t.back[0] = (int32_t)atomicOr(dev_error, 0u);  // read back with the sizes
+    }
+}
+
 // ---- launchers ----
 static NaiveArgs naive_args(int n, uint64_t key, int32_t *actions, uint8_t *forced) {
     NaiveArgs a{};
@@ -281,6 +406,20 @@ void launch_match_advance(omk_ctx *c, int pairs, int first_tree, int half, const
                           const int8_t *status, const int8_t *other_status, int8_t *moves, int8_t *final_status, int32_t *counters) {
     k_match_advance<<<2, kAdvanceThreads, 0, c->stream>>>(pairs, first_tree, half, live[0], live[1], ids, actions, status, other_status,
                                                            moves, final_status, counters, c->dev_error);
+    c->launches++;
+}
+void launch_tourney_init(omk_ctx *c, const TourneyState &t) {
+    const long long total = (long long)t.n * (t.n - 1) / 2 * 2 * t.pairs * kCells;
+    const int blocks = (int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
+    k_tourney_init<<<blocks, 256, 0, c->stream>>>(t);
+    c->launches++;
+}
+void launch_tourney_advance(omk_ctx *c, const TourneyState &t, int half) {
+    k_tourney_advance<<<t.n * (t.n - 1), kAdvanceThreads, 0, c->stream>>>(t, half, c->dev_error);
+    c->launches++;
+}
+void launch_tourney_gather(omk_ctx *c, const TourneyState &t, int half) {
+    k_tourney_gather<<<t.n, 256, 0, c->stream>>>(t, half, c->dev_error);
     c->launches++;
 }
 

@@ -130,13 +130,11 @@ struct LaneScope {
         c->id_base = 0;
     }
 };
-// RAII: the evaluator launches in scope read the opponent's weights (either lane may evaluate either model)
+// RAII: the evaluator launches in scope read the weights of model slot `slot` (either lane may evaluate any model)
 struct ModelScope {
     omk_ctx *c;
     NetWeights *saved;
-    ModelScope(omk_ctx *ctx, bool opponent) : c(ctx), saved(ctx->model) {
-        if (opponent) c->model = &c->opp;
-    }
+    ModelScope(omk_ctx *ctx, int slot) : c(ctx), saved(ctx->model) { c->model = &c->slot(slot); }
     ~ModelScope() { c->model = saved; }
 };
 // creates lane 1 on first use; false: this context has no second lane
@@ -435,13 +433,13 @@ extern "C" int32_t omk_net_init_random(omk_ctx *c, uint64_t seed) {
     return sp_refresh_root_policy(c);
 }
 
-// opponent: the opponent's weights (omk_opponent_eval), which no training step changes
-static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float *out_p, float *out_v, bool opponent = false) {
-    if (!opponent) {
+// slot: the model whose weights evaluate (omk_model_eval); only the network's (slot 0) are changed by training steps
+static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float *out_p, float *out_v, int slot = 0) {
+    if (slot == 0) {
         int32_t rc_p = ensure_packed(c);
         if (rc_p) return rc_p;
     }
-    ModelScope scope(c, opponent);
+    ModelScope scope(c, slot);
     if (!net_forward(c, images_dev, n)) return fail(OMK_ERR_CUDA, "the network forward failed to launch (see stderr)");
     // P rows are padded to 96 floats on the device; compact on the way out
     CK(cudaMemcpy2DAsync(out_p, sizeof(float) * kCells, c->ws.P, sizeof(float) * kRow, sizeof(float) * kCells, (size_t)n,
@@ -453,10 +451,13 @@ static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float
     return check_device_error(c);  // OMK_ERR_NUMERIC when the network produced a non-finite output
 }
 
-static int32_t eval_boards(omk_ctx *c, bool opponent, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+static std::string slot_name(int slot) {
+    return slot == 0 ? "network" : (slot == 1 ? "opponent" : "model slot " + std::to_string(slot));
+}
+static int32_t eval_boards(omk_ctx *c, int slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
                            float *out_p, float *out_v) {
     CK(cudaSetDevice(c->device));
-    if (!(opponent ? c->opp : c->net).loaded) return fail(OMK_ERR_STATE, opponent ? "opponent weights not loaded" : "network weights not loaded");
+    if (!c->slot(slot).loaded) return fail(OMK_ERR_STATE, slot_name(slot) + " weights not loaded");
     if (n < 0 || !boards || !turns || !out_p) return fail(OMK_ERR_INVALID, "bad arguments");
     if (n == 0) return OMK_OK;
     int32_t rc = ensure_workspace(c, n);
@@ -467,11 +468,11 @@ static int32_t eval_boards(omk_ctx *c, bool opponent, const uint8_t *boards, con
     CK(copy_h2d(c, d_boards, boards, (size_t)n * kCells, c->stream));
     CK(copy_h2d(c, d_turns, turns, (size_t)n, c->stream));
     launch_pack_boards(c, d_boards, d_turns, n, mode);
-    return net_eval_common(c, n, nullptr, out_p, out_v, opponent);
+    return net_eval_common(c, n, nullptr, out_p, out_v, slot);
 }
 extern "C" int32_t omk_net_eval(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
                                 float *out_p, float *out_v) {
-    return eval_boards(c, false, boards, turns, n, mode, out_p, out_v);
+    return eval_boards(c, 0, boards, turns, n, mode, out_p, out_v);
 }
 
 extern "C" int32_t omk_net_eval_images(omk_ctx *c, const float *images, int32_t n, float *out_p, float *out_v) {
@@ -1568,56 +1569,79 @@ extern "C" int32_t omk_eval_naive(omk_ctx *c, int32_t episodes, int32_t first_tr
     return OMK_OK;
 }
 
-// ------------------------------------------------------------------ the opponent network and the arena (benchmark/src/main.rs:14-108)
-// the opponent's fp32 tensors, allocated on first use (all or nothing)
-static int32_t opponent_alloc(omk_ctx *c) {
-    if (c->opp.t[0]) return OMK_OK;
+// ------------------------------------------------------------------ model slots, the opponent network and the arena (benchmark/src/main.rs:14-108)
+// slot s's fp32 tensors, allocated on first use (all or nothing)
+static int32_t model_alloc(omk_ctx *c, int slot) {
+    NetWeights &m = c->slot(slot);
+    if (m.t[0]) return OMK_OK;
     NetWeights w;
     for (int i = 0; i < kNetTensors; ++i) CK(w.t[i].alloc((size_t)kLens[i]));
     CK(w.heads_w.alloc(512 * 128));
     CK(w.heads_b.alloc(128));
-    c->opp = std::move(w);
+    m = std::move(w);
     return OMK_OK;
 }
-// after the opponent's fp32 tensors changed: its packed heads and operand images (what omk_net_load_params does for the network)
-static int32_t opponent_prepare(omk_ctx *c) {
-    ModelScope scope(c, true);
+// after slot s's fp32 tensors changed: its packed heads and operand images (what omk_net_load_params does for the network)
+static int32_t model_prepare(omk_ctx *c, int slot) {
+    ModelScope scope(c, slot);
+    const std::string who = slot == 1 ? std::string(" (opponent)") : " (model slot " + std::to_string(slot) + ")";
     net_pack_heads(c);
-    if (!fc16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split fc weight preparation failed (opponent)");
-    if (!tower16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split tower weight preparation failed (opponent)");
+    if (!fc16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split fc weight preparation failed" + who);
+    if (!tower16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split tower weight preparation failed" + who);
     CK(cudaStreamSynchronize(c->stream));
     CK(cudaGetLastError());
-    c->opp.loaded = true;
+    c->slot(slot).loaded = true;
+    return OMK_OK;
+}
+static int32_t check_model_slot(int slot) {
+    if (slot == 0) return fail(OMK_ERR_INVALID, "slot 0 is the network: omk_net_load_params and the trainer own it");
+    if (slot < 1 || slot >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [1, " + std::to_string(kModelSlots - 1) + "]");
     return OMK_OK;
 }
 
-extern "C" int32_t omk_opponent_load_params(omk_ctx *c, const float *const *tensors, const int64_t *lens) {
+extern "C" int32_t omk_model_load_params(omk_ctx *c, int32_t slot, const float *const *tensors, const int64_t *lens) {
     CK(cudaSetDevice(c->device));
+    int32_t rc = check_model_slot(slot);
+    if (rc) return rc;
     for (int i = 0; i < kNetTensors; ++i)
         if (!tensors[i] || lens[i] != kLens[i])
             return fail(OMK_ERR_INVALID, "tensor " + std::to_string(i) + ": expected " + std::to_string(kLens[i]) + " elements");
-    int32_t rc = opponent_alloc(c);
+    rc = model_alloc(c, slot);
     if (rc) return rc;
-    c->opp.loaded = false;  // until the images below are built
+    NetWeights &m = c->slot(slot);
+    m.loaded = false;  // until the images below are built
     for (int i = 0; i < kNetTensors; ++i)
-        CK(copy_h2d(c, c->opp.t[i], tensors[i], sizeof(float) * (size_t)kLens[i], c->stream));
-    return opponent_prepare(c);
+        CK(copy_h2d(c, m.t[i], tensors[i], sizeof(float) * (size_t)kLens[i], c->stream));
+    return model_prepare(c, slot);
 }
 
-extern "C" int32_t omk_opponent_from_net(omk_ctx *c) {
+extern "C" int32_t omk_model_from_net(omk_ctx *c, int32_t slot) {
     CK(cudaSetDevice(c->device));
-    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
-    int32_t rc = opponent_alloc(c);
+    int32_t rc = check_model_slot(slot);
     if (rc) return rc;
-    c->opp.loaded = false;
+    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
+    rc = model_alloc(c, slot);
+    if (rc) return rc;
+    NetWeights &m = c->slot(slot);
+    m.loaded = false;
     for (int i = 0; i < kNetTensors; ++i)
-        CK(cudaMemcpyAsync(c->opp.t[i], c->net.t[i], sizeof(float) * (size_t)kLens[i], cudaMemcpyDeviceToDevice, c->stream));
-    return opponent_prepare(c);
+        CK(cudaMemcpyAsync(m.t[i], c->net.t[i], sizeof(float) * (size_t)kLens[i], cudaMemcpyDeviceToDevice, c->stream));
+    return model_prepare(c, slot);
 }
 
+extern "C" int32_t omk_model_eval(omk_ctx *c, int32_t slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
+                                  float *out_p, float *out_v) {
+    if (slot < 0 || slot >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
+    return eval_boards(c, slot, boards, turns, n, mode, out_p, out_v);
+}
+
+extern "C" int32_t omk_opponent_load_params(omk_ctx *c, const float *const *tensors, const int64_t *lens) {
+    return omk_model_load_params(c, 1, tensors, lens);
+}
+extern "C" int32_t omk_opponent_from_net(omk_ctx *c) { return omk_model_from_net(c, 1); }
 extern "C" int32_t omk_opponent_eval(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode, float *out_p,
                                      float *out_v) {
-    return eval_boards(c, true, boards, turns, n, mode, out_p, out_v);
+    return omk_model_eval(c, 1, boards, turns, n, mode, out_p, out_v);
 }
 
 // stage s of one mover's half-move in omk_match, on the lane and with the model in use: 0 = ensure_action_exists + play_action of
@@ -1741,6 +1765,147 @@ extern "C" int32_t omk_match(omk_ctx *c, int32_t pairs, int32_t first_tree, int3
     for (int k = 0; k < 3; ++k) out_result[k] = h_cnt[k];
     if (out_status) memcpy(out_status, host.data() + off_fin, g);
     if (out_moves) memcpy(out_moves, host.data() + off_moves, g * kCells);
+    if (out_stats) {
+        out_stats[0] = (int64_t)(h_sims[2] - h_sims[0]);
+        out_stats[1] = (int64_t)(h_sims[3] - h_sims[1]);
+        out_stats[2] = n_moves;
+        out_stats[3] = syncs;
+    }
+    if (out_gpu_ms) CK(cudaEventElapsedTime(out_gpu_ms, c->ev0, c->ev1));
+    return OMK_OK;
+}
+
+// ------------------------------------------------------------------ the tournament: omk_match over every pairing of up to 16 models
+extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
+                                  int32_t batch_size, float epsilon, float alpha, int32_t evaluator, int32_t *out_result,
+                                  int8_t *out_moves, int8_t *out_status, int64_t *out_stats, float *out_gpu_ms) {
+    CK(cudaSetDevice(c->device));
+    if (!out_result) return fail(OMK_ERR_INVALID, "out_result is NULL");
+    if (n_models < 2 || n_models > kModelSlots || !slots)
+        return fail(OMK_ERR_INVALID, "need 2 <= n_models <= " + std::to_string(kModelSlots) + " and a slot list");
+    bool listed[kModelSlots] = {};
+    for (int m = 0; m < n_models; ++m) {
+        if (slots[m] < 0 || slots[m] >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
+        if (listed[slots[m]]) return fail(OMK_ERR_INVALID, "duplicate model slot in the tournament");
+        listed[slots[m]] = true;
+    }
+    const int n = n_models, P = n * (n - 1) / 2;
+    if (pairs < 1 || first_tree < 0 || (int64_t)first_tree + 4 * (int64_t)pairs * P > c->cap_trees)
+        return fail(OMK_ERR_INVALID, "need pairs >= 1 and the trees first_tree .. first_tree + 4 * pairs * n(n-1)/2 - 1 inside capacity_trees");
+    if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
+    if (count < 1) return fail(OMK_ERR_INVALID, "count < 1");
+    if (evaluator != OMK_EVAL_NET && evaluator != OMK_EVAL_HASH) return fail(OMK_ERR_INVALID, "unknown evaluator");
+    if (c->sp_active && first_tree < 2 * c->sp_cfg.n_games)
+        return fail(OMK_ERR_STATE, "the trees overlap the active self-play driver's trees 0 .. 2 * n_games - 1");
+    int32_t rc = check_evaluator(c, evaluator);  // with the network: weights a training step changed are packed first
+    if (rc) return rc;
+    if (evaluator == OMK_EVAL_NET)
+        for (int m = 0; m < n; ++m)
+            if (!c->slot(slots[m]).loaded) return fail(OMK_ERR_STATE, slot_name(slots[m]) + " weights not loaded");
+    const int Q = pairs;
+    const size_t G = 2 * (size_t)Q * P;  // games
+    const int gcap = (n - 1) * 2 * Q;     // a model's trees: its init list, and twice its largest group
+    // [simulations and evaluations before / after (4 u64) | counters [P][3] i32 | final status G | moves G*81] leave in one copy;
+    // then the per-pairing lists and the per-model groups (TourneyState)
+    const size_t off_cnt = 32, off_fin = off_cnt + 12 * (size_t)P, off_moves = off_fin + G, out_bytes = off_moves + G * kCells;
+    size_t end = (out_bytes + 255) & ~(size_t)255;
+    auto take = [&](size_t bytes) {
+        const size_t o = end;
+        end = (end + bytes + 15) & ~(size_t)15;
+        return o;
+    };
+    const size_t mg = (size_t)n * gcap;
+    const size_t off_ids = take(8 * G), off_act = take(4 * G), off_live = take(8 * (size_t)P), off_off = take(8 * (size_t)P),
+                 off_back = take(4 * (size_t)(n + 1)), off_gids = take(4 * mg), off_gact = take(4 * mg), off_gstr = take(4 * mg),
+                 off_gst = take(mg), off_gost = take(mg);
+    CK(c->eval_buf.grow(c->stream, end, 4096));
+    // the groups run interleaved over both lanes, group k on lane k % 2
+    const bool two_lanes = c->lane_min_trees > 0 && lane1_ready(c);
+    const int rows = (n - 1) * Q * batch_size > gcap ? (n - 1) * Q * batch_size : gcap;
+    for (int l = 0; l < (two_lanes ? 2 : 1); ++l) {
+        LaneScope scope(c, l, 0);
+        rc = ensure_workspace(c, rows);
+        if (rc) return rc;
+    }
+    uint8_t *base = c->eval_buf;
+    unsigned long long *sims = reinterpret_cast<unsigned long long *>(base);
+    TourneyState t;
+    t.n = n;
+    t.pairs = Q;
+    t.first_tree = first_tree;
+    t.gcap = gcap;
+    t.counters = reinterpret_cast<int32_t *>(base + off_cnt);
+    t.final_status = reinterpret_cast<int8_t *>(base + off_fin);
+    t.moves = reinterpret_cast<int8_t *>(base + off_moves);
+    t.ids = reinterpret_cast<int32_t *>(base + off_ids);
+    t.actions = reinterpret_cast<int32_t *>(base + off_act);
+    t.live = reinterpret_cast<int32_t *>(base + off_live);
+    t.off = reinterpret_cast<int32_t *>(base + off_off);
+    t.back = reinterpret_cast<int32_t *>(base + off_back);
+    t.gids = reinterpret_cast<int32_t *>(base + off_gids);
+    t.gact = reinterpret_cast<int32_t *>(base + off_gact);
+    t.gstr = reinterpret_cast<uint32_t *>(base + off_gstr);
+    t.gst = reinterpret_cast<int8_t *>(base + off_gst);
+    t.gost = reinterpret_cast<int8_t *>(base + off_gost);
+
+    fold_requests(c);  // counts earlier calls left pending are not this call's
+    CK(cudaMemcpyAsync(sims, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev0, c->stream));
+    launch_tourney_init(c, t);
+    for (int m = 0; m < n; ++m) {  // Agent::new for every tree of model m, under model m's weights
+        ModelScope scope(c, slots[m]);
+        launch_reset_requests(c);
+        launch_new_games(c, t.gids + (size_t)m * gcap, gcap, t.gstr + (size_t)m * gcap, nullptr, nullptr);
+        RUN_EVAL(c, evaluator, gcap);
+        launch_apply(c, t.gids + (size_t)m * gcap, gcap, kApplyNewGame);
+    }
+    launch_tourney_gather(c, t, 0);
+    const int rounds = (count + batch_size - 1) / batch_size;  // parallel_mcts_executor.rs:39-42,207
+    std::vector<int32_t> back((size_t)n + 1, (n - 1) * Q);     // {device error word, each model's group size}
+    back[0] = 0;
+    const int32_t *size = back.data() + 1;
+    std::vector<int> movers;
+    int64_t n_moves = 0, syncs = 0;
+    // a game ends after at most 81 moves; a device error (out of node slots, a non-finite network output, a refused move)
+    // ends the tournament at the half-move that raised it
+    for (int half = 0; back[0] == 0 && half < kCells; ++half) {
+        movers.clear();
+        for (int m = 0; m < n; ++m)
+            if (size[m] > 0) movers.push_back(m);
+        if (movers.empty()) break;
+        const int lanes = two_lanes && movers.size() >= 2 ? 2 : 1;
+        if (lanes == 2) lanes_fork(c);
+        for (int stage = 0; stage < rounds + 2 && rc == OMK_OK; ++stage)
+            for (size_t k = 0; k < movers.size() && rc == OMK_OK; ++k) {
+                const int m = movers[k];
+                const size_t g0 = (size_t)m * gcap;
+                LaneScope lane(c, lanes == 2 ? (int)(k % 2) : 0, 0);
+                ModelScope model(c, slots[m]);
+                rc = match_stage(c, stage, rounds, half, t.gids + g0, size[m], t.gact + g0, t.gst + g0, t.gost + g0, batch_size, epsilon,
+                                 alpha, evaluator);
+            }
+        if (lanes == 2) lanes_join(c);  // on an error too: nothing queued on lane 1 is left unordered with the main stream
+        if (rc) return rc;
+        launch_tourney_advance(c, t, half);
+        launch_tourney_gather(c, t, half + 1);
+        for (int m : movers) n_moves += size[m];
+        // the half-move's one host round trip: the group sizes size the next launches
+        CK(copy_d2h(c, back.data(), t.back, sizeof(int32_t) * back.size(), c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        ++syncs;
+    }
+    fold_requests(c);
+    CK(cudaMemcpyAsync(sims + 2, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
+    CK(cudaEventRecord(c->ev1, c->stream));
+    std::vector<uint8_t> host(out_bytes);
+    CK(copy_d2h(c, host.data(), base, out_bytes, c->stream));
+    rc = check_device_error(c);  // (synchronises the stream)
+    ++syncs;
+    if (rc) return rc;
+    const unsigned long long *h_sims = reinterpret_cast<const unsigned long long *>(host.data());
+    memcpy(out_result, host.data() + off_cnt, 12 * (size_t)P);
+    if (out_status) memcpy(out_status, host.data() + off_fin, G);
+    if (out_moves) memcpy(out_moves, host.data() + off_moves, G * kCells);
     if (out_stats) {
         out_stats[0] = (int64_t)(h_sims[2] - h_sims[0]);
         out_stats[1] = (int64_t)(h_sims[3] - h_sims[1]);

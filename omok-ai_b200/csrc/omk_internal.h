@@ -15,6 +15,7 @@ namespace omk {
 
 constexpr int kMaxBatchPerTree = 64;  // per-tree requests per round (evaluate_batch_size)
 constexpr int kNetTensors = 31;
+constexpr int kModelSlots = 16;  // weight sets per context: 0 the network, 1 the opponent, 2 .. 15 further models (omk_model_*)
 
 enum ApplyMode { kApplySearch = 0, kApplyNewGame = 1, kApplyEnsure = 2 };
 
@@ -99,8 +100,9 @@ struct WeightMaps {  // tensor maps (fc_f16.cu) over one model's fp16 weight ima
     CUtensorMap map2_b_hi, map2_b_lo;    // heads (B = all 128 padded output rows)
     bool weights_ready = false;
 };
-// Everything derived from one set of weights.  The context holds two: the network (`net`: every entry point, the trainer)
-// and the opponent (`opp`: omk_opponent_eval, omk_match).  The evaluator reads the active one, omk_ctx::model.
+// Everything derived from one set of weights.  The context holds kModelSlots: the network (slot 0, `net`: every entry point,
+// the trainer), the opponent (slot 1, `opp`: omk_opponent_eval, omk_match) and further models (slots 2 .., `more`:
+// omk_model_eval, omk_tournament).  The evaluator reads the active one, omk_ctx::model.
 struct NetWeights : FcImages, TowerImages, WeightMaps {
     Buf<float> t[kNetTensors];  // device copies in checkpoint order
     Buf<float> heads_w;         // [512][128]: cols 0..80 policy, col 81 value, rest 0
@@ -230,8 +232,10 @@ struct omk_ctx {
     omk::Buf<unsigned long long> dev_sims;  // simulations counter
 
     omk::NetWeights net;            // the network
-    omk::NetWeights opp;            // the opponent (omk_opponent_load_params / omk_opponent_from_net); buffers allocated on first load
-    omk::NetWeights *model = &net;  // the weights the evaluator reads: `net`, or `opp` inside a ModelScope (omk_api.cu)
+    omk::NetWeights opp;            // the opponent, slot 1 (omk_opponent_load_params / omk_opponent_from_net); buffers allocated on first load
+    omk::NetWeights more[omk::kModelSlots - 2];  // slots 2 .. (omk_model_load_params / omk_model_from_net); buffers allocated on first load
+    omk::NetWeights *model = &net;  // the weights the evaluator reads: `net`, or another slot inside a ModelScope (omk_api.cu)
+    omk::NetWeights &slot(int s) { return s == 0 ? net : (s == 1 ? opp : more[s - 2]); }
     omk::Workspace ws;
     int virtual_loss = 0;           // opt-in, non-reference search mode (omk_search_set_virtual_loss); refused with the parity evaluator
     int fc0_balance = 0;            // fc0 tail balancing of the CTA-pair kernel (fc_f16.cu FcBal): 0 off (default), 1 on
@@ -260,7 +264,7 @@ struct omk_ctx {
     cudaStream_t sp_copy_stream = nullptr;
     cudaEvent_t sp_ev_rec[kSpRing][2] = {}, sp_ev_copy[kSpRing] = {};
     omk::Replay rp;                   // device replay memory (omk_replay_reset); fed by the driver when it exists at omk_selfplay_begin
-    omk::Buf<uint8_t> eval_buf;       // omk_eval_naive's and omk_match's per-call state (grow-only)
+    omk::Buf<uint8_t> eval_buf;       // omk_eval_naive's, omk_match's and omk_tournament's per-call state (grow-only)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
@@ -327,6 +331,25 @@ void launch_match_init(omk_ctx *c, int pairs, int first_tree, int32_t *ids, uint
                        int32_t *counters);
 void launch_match_advance(omk_ctx *c, int pairs, int first_tree, int half, const int *live, int32_t *ids, int32_t *actions,
                           const int8_t *status, const int8_t *other_status, int8_t *moves, int8_t *final_status, int32_t *counters);
+// omk_tournament (DESIGN.md 4): n models, P = n(n-1)/2 pairings (i < j, lexicographic), `pairs` games per leg of each.  The
+// per-pairing state is omk_match's: ids [P][side][leg][pairs] (left 0, right 1), actions [P][leg][pairs], live [P][leg],
+// counters [P][3] = {left wins, right wins, draws}, moves [P][2 * pairs][81], final status [P][2 * pairs].  Model m's group
+// (its movers of one half-move, over all its pairings in order) is [m][gcap] in gids / gact / gst / gost, and off [P][leg] is
+// where a (pairing, leg)'s movers sit in their model's group.  back = {device error word, group size of each model}.
+struct TourneyState {
+    int n, pairs, first_tree, gcap;
+    int32_t *ids, *actions, *live, *off, *counters, *back;
+    int32_t *gids, *gact;  // [n][gcap]
+    int8_t *gst, *gost;    // [n][gcap]: the movers' play_action statuses, and their trees' statuses taking the other side's move
+    uint32_t *gstr;        // [n][gcap]: random streams of k_tourney_init's per-model lists of all the model's trees
+    int8_t *moves, *final_status;
+};
+// set-up: every pairing's trees, all games live, nothing tallied; gids / gstr = every tree of each model with its stream
+void launch_tourney_init(omk_ctx *c, const TourneyState &t);
+// after half-move `half`: record, check, tally and compact each (pairing, leg) from its movers' group segment
+void launch_tourney_advance(omk_ctx *c, const TourneyState &t, int half);
+// the groups of half-move `half` from the compacted lists: gids, gact (the move each tree takes in stage 0), off, back
+void launch_tourney_gather(omk_ctx *c, const TourneyState &t, int half);
 
 // omk_api.cu: open / close a profiling span of kernel family `kind` (no-op below min_level)
 bool prof_begin(omk_ctx *c, int kind, int min_level);
