@@ -375,6 +375,22 @@ OMK_API int32_t omk_model_eval(omk_ctx *ctx, int32_t slot, const uint8_t *boards
 OMK_API int32_t omk_tournament(omk_ctx *ctx, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
                                int32_t batch_size, float epsilon, float alpha, int32_t evaluator, int32_t *out_result, int8_t *out_moves,
                                int8_t *out_status, int64_t *out_stats, float *out_gpu_ms);
+/* omk_tournament with the naive player (omk_naive_move's rule, key mix64(seed ^ K_NAIVE)) as participant 0 and slots[k] as
+ * participant k + 1, for n_models (1 .. 16) distinct slots: N = n_models + 1 participants, P = N(N-1)/2 pairings (a, b),
+ * a < b, in lexicographic order over participants, so the first n_models are (naive, slots[k]), the naive player "left" and
+ * opening games 0 .. pairs - 1.  Pairing p uses the trees first_tree + 4*pairs*p .. in omk_match's layout; in a naive
+ * pairing the naive side's 2*pairs trees are reserved and never touched, and the model's tree of game g has random stream
+ * g % pairs.  The naive player's move at half-move h of game g reads the board from the root of the model's tree of that
+ * game and draws on stream g*81 + h; the model takes it at its next half-move (ensure_action_exists + play_action), unless
+ * it ended the game.  So model-model pairing (i+1, j+1) equals pairing (i, j) of omk_tournament(slots, ...) game by game,
+ * and games 0 .. pairs - 1 of (naive, slots[k]) equal omk_eval_naive(pairs, first_tree = 0, ..., seed) with slots[k] as the
+ * network.  evaluator OMK_EVAL_NET: every listed slot must be loaded, and the network too (OMK_ERR_STATE otherwise).
+ * Errors, outputs and accounting are omk_tournament's with N participants: one host round trip of 4*(N+1) bytes per
+ * half-move, no host-to-device copy.  arena.ratings(out_result, N) then rates the naive player at 0 Elo. */
+OMK_API int32_t omk_tournament_naive(omk_ctx *ctx, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree,
+                                     int32_t count, int32_t batch_size, float epsilon, float alpha, int32_t evaluator, uint64_t seed,
+                                     int32_t *out_result, int8_t *out_moves, int8_t *out_status, int64_t *out_stats,
+                                     float *out_gpu_ms);
 
 #ifdef __cplusplus
 }

@@ -7,6 +7,8 @@
                                  opponent network (right): both legs run at once, each model's half-move on its own lane.
   * `play_tournament_device`     a round-robin of that match over up to 16 model slots of one context as ONE call
                                  (omk_tournament); each model searches all its pairings' movers as one batch per half-move.
+  * `play_tournament_naive_device`  the same round-robin with the naive player below as participant 0 (omk_tournament_naive),
+                                 so `ratings` puts every model on one scale, with the naive player at 0 Elo.
   * `ratings`                    a Bradley-Terry fit, in Elo units, of a tournament's pairwise results.
   * `play_against_naive_player`  src/trainer.rs:487-603: the naive player takes the first legal move (ascending) that ends
                                  the game for itself, or that would end it for the opponent (a block); else a random
@@ -89,6 +91,23 @@ def play_tournament_device(ctx, slots, game_count: int = 100, count: int = 800, 
     `moves_out`, if given, receives per pairing one move list per game in `play_match`'s order."""
     result, moves, _, _ = ctx.tournament(slots, game_count // 2, first_tree=first_tree, count=count, batch_size=batch_size,
                                          epsilon=epsilon, alpha=alpha, evaluator=evaluator)
+    if moves_out is not None:
+        moves_out[:] = [[[int(a) for a in row if a >= 0] for row in pairing] for pairing in moves]
+    return result
+
+
+def play_tournament_naive_device(ctx, slots, seed: int = 0, game_count: int = 100, count: int = 800, batch_size: int = 8,
+                                 epsilon: float = 0.0, alpha: float = 1.0, evaluator: int = B.EVAL_NET, first_tree: int = 0,
+                                 moves_out: list | None = None):
+    """`play_tournament_device` with the naive player as participant 0 and slots[k] as participant k + 1, from one
+    `omk_tournament_naive` call of `game_count // 2` pairs per pairing on the trees first_tree .. first_tree + 2 * game_count * P - 1,
+    P = N(N-1)/2 over the N = len(slots) + 1 participants.  The first len(slots) pairings are (naive, slots[k]), the naive
+    player left and opening the first half of the games; its random moves draw on stream g * 81 + h of key
+    mix64(seed ^ K_NAIVE) (DESIGN.md 4).  Returns the [P, 3] table of (left wins, right wins, draws), so
+    `ratings(table, len(slots) + 1)` rates the naive player at 0 Elo and slots[k] at entry k + 1: every tournament against the
+    naive player shares that zero.  `moves_out` as in `play_tournament_device`."""
+    result, moves, _, _ = ctx.tournament_naive(slots, game_count // 2, seed=seed, first_tree=first_tree, count=count,
+                                               batch_size=batch_size, epsilon=epsilon, alpha=alpha, evaluator=evaluator)
     if moves_out is not None:
         moves_out[:] = [[[int(a) for a in row if a >= 0] for row in pairing] for pairing in moves]
     return result

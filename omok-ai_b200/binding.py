@@ -154,6 +154,7 @@ def load_library():
     L.omk_model_from_net.argtypes = [vp, i32]
     L.omk_model_eval.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
     L.omk_tournament.argtypes = [vp, i32, vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
+    L.omk_tournament_naive.argtypes = [vp, i32, vp, i32, i32, i32, i32, f32, f32, i32, u64, vp, vp, vp, vp, P(f32)]
     for name in declared_symbols():
         fn = getattr(L, name)  # raises AttributeError if the library lacks a declared symbol
         if name not in ("omk_last_error", "omk_ctx_stream", "omk_ctx_launch_count"):
@@ -609,16 +610,31 @@ class Context:
         is match(pairs) with slots[i] as the network (left) and slots[j] as the opponent (right), on the trees
         first_tree + 4 * pairs * p ..  Returns (result [P, 3] i32 (left wins, right wins, draws), moves [P, 2 * pairs, 81] i8
         (-1 past a game's end), final status [P, 2 * pairs] i8, stats dict: simulations, nn_evals, moves, host_syncs, gpu_ms)."""
+        return self._tournament(slots, 0, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, None)
+
+    def tournament_naive(self, slots, pairs: int, seed: int = 0, first_tree: int = 0, count: int = 800, batch_size: int = 8,
+                         epsilon: float = 0.0, alpha: float = 1.0, evaluator: int = EVAL_NET):
+        """`tournament` with the naive player (naive_move's rule on seed `seed`) as participant 0 and slots[k] as participant
+        k + 1: N = len(slots) + 1 participants, P = N(N-1)/2 pairings over participants, the first len(slots) of them
+        (naive, slots[k]) with the naive player left, opening games 0 .. pairs - 1.  Returns `tournament`'s tuple."""
+        return self._tournament(slots, 1, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, seed)
+
+    def _tournament(self, slots, extra, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, seed):
         s = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
-        n_pairings = max(s.size * (s.size - 1) // 2, 0)
+        n = s.size + extra  # participants
+        n_pairings = max(n * (n - 1) // 2, 0)
         games = max(2 * pairs, 0)
         result = np.zeros((n_pairings, 3), dtype=np.int32)
         moves = np.zeros((n_pairings, games, CELLS), dtype=np.int8)
         status = np.zeros((n_pairings, games), dtype=np.int8)
         stats = np.zeros(4, dtype=np.int64)
         gpu_ms = C.c_float()
-        self._check(self.L.omk_tournament(self.h, s.size, _ptr(s), pairs, first_tree, count, batch_size, epsilon, alpha, evaluator,
-                                          _ptr(result), _ptr(moves), _ptr(status), _ptr(stats), C.byref(gpu_ms)))
+        outs = (_ptr(result), _ptr(moves), _ptr(status), _ptr(stats), C.byref(gpu_ms))
+        args = (self.h, s.size, _ptr(s), pairs, first_tree, count, batch_size, epsilon, alpha, evaluator)
+        if seed is None:
+            self._check(self.L.omk_tournament(*args, *outs))
+        else:
+            self._check(self.L.omk_tournament_naive(*args, int(seed) & 0xFFFFFFFFFFFFFFFF, *outs))
         info = dict(zip(("simulations", "nn_evals", "moves", "host_syncs"), (int(x) for x in stats)))
         info["gpu_ms"] = float(gpu_ms.value)
         return result, moves, status, info

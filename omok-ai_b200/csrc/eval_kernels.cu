@@ -1,7 +1,7 @@
 // eval_kernels.cu -- the trainer's evaluation against the naive player (src/trainer.rs:487-603) on the device: the naive
 // player's move (:506-537) and the bookkeeping omk_eval_naive runs after every half-move; the same bookkeeping for the
 // arena between the network and the opponent (omk_match, benchmark/src/main.rs:14-108), and for a round-robin of that arena
-// over up to kModelSlots models (omk_tournament).
+// over up to kModelSlots models, optionally with the naive player as participant 0 (omk_tournament, omk_tournament_naive).
 #include "omk_internal.h"
 
 namespace omk {
@@ -12,9 +12,10 @@ constexpr int kAdvanceThreads = 1024;
 
 // The naive player's rule (DESIGN.md 4) for one position, the warp owning it: the first empty cell, ascending, where
 // place_stone is terminal for the mover or, on the same board with the turn flipped, for the opponent; else
-// legal[below(legal_count)] on the stream (key, stream, counter from 0).  A forced move draws nothing.
+// legal[below(legal_count)] on the stream (key, stream, counter from 0).  A forced move draws nothing.  out_status (may be
+// null): place_stone's result for the move on this board (OMK_NONE when there is none).
 __device__ __forceinline__ void naive_pick(const uint32_t *black, const uint32_t *white, uint32_t turn, uint64_t key, uint32_t stream,
-                                           int lane, int32_t *out_action, uint8_t *out_forced) {
+                                           int lane, int32_t *out_action, uint8_t *out_forced, int8_t *out_status) {
     uint32_t empty[3];
 #pragma unroll
     for (int k = 0; k < 3; ++k) empty[k] = ~(black[k] | white[k]);
@@ -50,10 +51,21 @@ __device__ __forceinline__ void naive_pick(const uint32_t *black, const uint32_t
     }
     *out_action = action;
     if (out_forced) *out_forced = forced;
+    if (out_status) {
+        int status = OMK_NONE;
+        if (action != OMK_NONE) {
+            uint32_t s[3] = {mine[0], mine[1], mine[2]};
+            set81(s, action);
+            status = makes_five_scalar(s, action) ? (turn == 0 ? kBlackWin : kWhiteWin) : (legal == 1 ? kDraw : kInProgress);
+        }
+        *out_status = (int8_t)status;
+    }
 }
 
 // One warp per position.  Positions come either as cells + turns (omk_naive_move; stream = streams[i] or i) or as the
-// root nodes of trees ids[i] (omk_eval_naive; game g = ids[i] - first_tree, stream = g * 81 + ply[g]).
+// root nodes of trees ids[i]: omk_eval_naive's (game g = ids[i] - first_tree, stream = g * 81 + ply[g]), or, with ply null,
+// the opponents' trees of omk_tournament_naive (tree first_tree + 4 * pairs * p + 2 * pairs + g of pairing p holds game g,
+// stream = g * 81 + half; every live game of a pairing has played `half` moves).
 struct NaiveArgs {
     const uint8_t *boards, *turns;  // [n][81], [n]; nullptr: the tree roots below
     const uint32_t *streams;
@@ -61,10 +73,12 @@ struct NaiveArgs {
     const uint8_t *nodes;
     int cap_nodes, first_tree;
     const int32_t *ply;
+    int pairs, half;
     int n;
     uint64_t key;
     int32_t *actions;
     uint8_t *forced;
+    int8_t *status;  // [n] place_stone's result of each move (may be null)
 };
 
 __global__ void __launch_bounds__(kNaiveWarps * 32) k_naive_move(NaiveArgs a) {
@@ -92,10 +106,16 @@ __global__ void __launch_bounds__(kNaiveWarps * 32) k_naive_move(NaiveArgs a) {
             white[k] = h.white[k];
         }
         turn = h.turn;
-        const int g = tree - a.first_tree;
-        stream = (uint32_t)(g * kCells + a.ply[g]);
+        if (a.ply) {
+            const int g = tree - a.first_tree;
+            stream = (uint32_t)(g * kCells + a.ply[g]);
+        } else {
+            const int g = (tree - a.first_tree) % (4 * a.pairs) - 2 * a.pairs;
+            stream = (uint32_t)(g * kCells + a.half);
+        }
     }
-    naive_pick(black, white, turn, a.key, stream, lane, a.actions + i, a.forced ? a.forced + i : nullptr);
+    naive_pick(black, white, turn, a.key, stream, lane, a.actions + i, a.forced ? a.forced + i : nullptr,
+               a.status ? a.status + i : nullptr);
 }
 
 // A fresh evaluation: live list = every game's tree, no move played, nothing tallied.
@@ -230,7 +250,9 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_match_advance(int pairs, in
     }
 }
 
-// ---- the tournament (omk_tournament): omk_match's bookkeeping over n models and their n(n-1)/2 pairings ----
+// ---- the tournament (omk_tournament): omk_match's bookkeeping over n participants and their n(n-1)/2 pairings ----
+// With t.naive, participant 0 is the naive player: it has no trees (its side of its pairings is reserved and never touched),
+// and it moves by k_naive_move on the roots of its opponents' trees, which hold the current positions.
 // pairing p = (a, b), a < b, in lexicographic order
 __device__ __forceinline__ void tourney_pairing(int p, int n, int &a, int &b) {
     a = 0;
@@ -270,7 +292,9 @@ __global__ void k_tourney_init(TourneyState t) {
 }
 
 // After half-move `half`, one block per (pairing, leg): k_match_advance for that leg, with the movers' actions and statuses
-// read out of their model's group segment.  The left model moves in leg half % 2, the right one in the other leg.
+// read out of their model's group segment.  The left model moves in leg half % 2, the right one in the other leg.  The naive
+// player's statuses are those of its moves on the board (k_naive_move); it has no tree to take the other side's move, so
+// there is no other_status to check.
 __global__ void __launch_bounds__(kAdvanceThreads) k_tourney_advance(TourneyState t, int half, uint32_t *dev_error) {
     __shared__ int warp_kept[kAdvanceThreads / 32];
     __shared__ int kept_before;
@@ -278,6 +302,7 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_tourney_advance(TourneyStat
     int a_model, b_model;
     tourney_pairing(p, t.n, a_model, b_model);
     const int mover = leg == half % 2 ? a_model : b_model;
+    const bool check_other = half > 0 && !(t.naive && mover == 0);
     const int n = t.live[2 * p + leg];
     const size_t seg = (size_t)mover * t.gcap + t.off[2 * p + leg];
     const int32_t *g_act = t.gact + seg;
@@ -300,7 +325,7 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_tourney_advance(TourneyStat
             const int st = g_st[i];
             const size_t row = (size_t)p * 2 * Q + g;
             t.moves[row * kCells + half] = (int8_t)a;
-            if (half > 0 && g_ost[i] != kInProgress) atomicOr(dev_error, 16u);
+            if (check_other && g_ost[i] != kInProgress) atomicOr(dev_error, 16u);
             if (st == kInProgress) {
                 keep = true;
             } else if (st == kDraw || st == kBlackWin || st == kWhiteWin) {
@@ -331,7 +356,8 @@ __global__ void __launch_bounds__(kAdvanceThreads) k_tourney_advance(TourneyStat
 
 // The groups of half-move `half`, one block per model m: the concatenation, in pairing order, of the live lists of the legs
 // m moves in (its trees, and the moves they take first: the other side's previous ones), each segment's offset, and the
-// group's size.  Block 0 also copies the device error word next to the sizes.
+// group's size.  The naive player's group lists its opponents' trees of those legs: the boards it reads.  Block 0 also
+// copies the device error word next to the sizes.
 __global__ void k_tourney_gather(TourneyState t, int half, uint32_t *dev_error) {
     const int m = blockIdx.x, Q = t.pairs;
     int32_t *g_ids = t.gids + (size_t)m * t.gcap, *g_act = t.gact + (size_t)m * t.gcap;
@@ -339,8 +365,8 @@ __global__ void k_tourney_gather(TourneyState t, int half, uint32_t *dev_error) 
     for (int r = 0; r < t.n - 1; ++r) {
         int p, side;
         tourney_model_pairing(m, r, t.n, p, side);
-        const int leg = (half + side) % 2, cnt = t.live[2 * p + leg];
-        const int32_t *src_ids = t.ids + (size_t)(4 * p + 2 * side + leg) * Q, *src_act = t.actions + (size_t)(2 * p + leg) * Q;
+        const int leg = (half + side) % 2, cnt = t.live[2 * p + leg], trees = t.naive && m == 0 ? 1 - side : side;
+        const int32_t *src_ids = t.ids + (size_t)(4 * p + 2 * trees + leg) * Q, *src_act = t.actions + (size_t)(2 * p + leg) * Q;
         for (int j = threadIdx.x; j < cnt; j += blockDim.x) {
             g_ids[o + j] = src_ids[j];
             g_act[o + j] = src_act[j];
@@ -381,6 +407,19 @@ void launch_naive_move_trees(omk_ctx *c, const int32_t *ids, int n, int first_tr
     a.cap_nodes = c->cap_nodes;
     a.first_tree = first_tree;
     a.ply = ply;
+    k_naive_move<<<(n + kNaiveWarps - 1) / kNaiveWarps, kNaiveWarps * 32, 0, c->stream>>>(a);
+    c->launches++;
+}
+void launch_tourney_naive_move(omk_ctx *c, const TourneyState &t, int half, int n, uint64_t key) {
+    if (n <= 0) return;
+    NaiveArgs a = naive_args(n, key, t.gact, nullptr);
+    a.ids = t.gids;
+    a.nodes = c->tree_nodes;
+    a.cap_nodes = c->cap_nodes;
+    a.first_tree = t.first_tree;
+    a.pairs = t.pairs;
+    a.half = half;
+    a.status = t.gst;
     k_naive_move<<<(n + kNaiveWarps - 1) / kNaiveWarps, kNaiveWarps * 32, 0, c->stream>>>(a);
     c->launches++;
 }

@@ -1776,20 +1776,25 @@ extern "C" int32_t omk_match(omk_ctx *c, int32_t pairs, int32_t first_tree, int3
 }
 
 // ------------------------------------------------------------------ the tournament: omk_match over every pairing of up to 16 models
-extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
-                                  int32_t batch_size, float epsilon, float alpha, int32_t evaluator, int32_t *out_result,
-                                  int8_t *out_moves, int8_t *out_status, int64_t *out_stats, float *out_gpu_ms) {
+// naive: participant 0 is the naive player (seeded by `seed`, DESIGN.md 4) and participant k + 1 is slots[k]; otherwise
+// participant k is slots[k] and `seed` is unused
+static int32_t tournament(omk_ctx *c, bool naive, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
+                          int32_t batch_size, float epsilon, float alpha, int32_t evaluator, uint64_t seed, int32_t *out_result,
+                          int8_t *out_moves, int8_t *out_status, int64_t *out_stats, float *out_gpu_ms) {
     CK(cudaSetDevice(c->device));
     if (!out_result) return fail(OMK_ERR_INVALID, "out_result is NULL");
-    if (n_models < 2 || n_models > kModelSlots || !slots)
-        return fail(OMK_ERR_INVALID, "need 2 <= n_models <= " + std::to_string(kModelSlots) + " and a slot list");
+    const int min_models = naive ? 1 : 2;
+    if (n_models < min_models || n_models > kModelSlots || !slots)
+        return fail(OMK_ERR_INVALID, "need " + std::to_string(min_models) + " <= n_models <= " + std::to_string(kModelSlots) + " and a slot list");
     bool listed[kModelSlots] = {};
     for (int m = 0; m < n_models; ++m) {
         if (slots[m] < 0 || slots[m] >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
         if (listed[slots[m]]) return fail(OMK_ERR_INVALID, "duplicate model slot in the tournament");
         listed[slots[m]] = true;
     }
-    const int n = n_models, P = n * (n - 1) / 2;
+    const int n = n_models + (naive ? 1 : 0), P = n * (n - 1) / 2;  // participants, pairings
+    const int first_model = naive ? 1 : 0;
+    auto slot_of = [&](int m) { return slots[m - first_model]; };  // participant m >= first_model
     if (pairs < 1 || first_tree < 0 || (int64_t)first_tree + 4 * (int64_t)pairs * P > c->cap_trees)
         return fail(OMK_ERR_INVALID, "need pairs >= 1 and the trees first_tree .. first_tree + 4 * pairs * n(n-1)/2 - 1 inside capacity_trees");
     if (batch_size < 1 || batch_size > kMaxBatchPerTree) return fail(OMK_ERR_INVALID, "batch_size must be in [1, 64]");
@@ -1800,11 +1805,11 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
     int32_t rc = check_evaluator(c, evaluator);  // with the network: weights a training step changed are packed first
     if (rc) return rc;
     if (evaluator == OMK_EVAL_NET)
-        for (int m = 0; m < n; ++m)
+        for (int m = 0; m < n_models; ++m)
             if (!c->slot(slots[m]).loaded) return fail(OMK_ERR_STATE, slot_name(slots[m]) + " weights not loaded");
     const int Q = pairs;
     const size_t G = 2 * (size_t)Q * P;  // games
-    const int gcap = (n - 1) * 2 * Q;     // a model's trees: its init list, and twice its largest group
+    const int gcap = (n - 1) * 2 * Q;     // a participant's trees: its init list, and twice its largest group
     // [simulations and evaluations before / after (4 u64) | counters [P][3] i32 | final status G | moves G*81] leave in one copy;
     // then the per-pairing lists and the per-model groups (TourneyState)
     const size_t off_cnt = 32, off_fin = off_cnt + 12 * (size_t)P, off_moves = off_fin + G, out_bytes = off_moves + G * kCells;
@@ -1834,6 +1839,7 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
     t.pairs = Q;
     t.first_tree = first_tree;
     t.gcap = gcap;
+    t.naive = naive ? 1 : 0;
     t.counters = reinterpret_cast<int32_t *>(base + off_cnt);
     t.final_status = reinterpret_cast<int8_t *>(base + off_fin);
     t.moves = reinterpret_cast<int8_t *>(base + off_moves);
@@ -1852,8 +1858,8 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
     CK(cudaMemcpyAsync(sims, c->dev_sims, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToDevice, c->stream));
     CK(cudaEventRecord(c->ev0, c->stream));
     launch_tourney_init(c, t);
-    for (int m = 0; m < n; ++m) {  // Agent::new for every tree of model m, under model m's weights
-        ModelScope scope(c, slots[m]);
+    for (int m = first_model; m < n; ++m) {  // Agent::new for every tree of model m, under model m's weights
+        ModelScope scope(c, slot_of(m));
         launch_reset_requests(c);
         launch_new_games(c, t.gids + (size_t)m * gcap, gcap, t.gstr + (size_t)m * gcap, nullptr, nullptr);
         RUN_EVAL(c, evaluator, gcap);
@@ -1861,8 +1867,9 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
     }
     launch_tourney_gather(c, t, 0);
     const int rounds = (count + batch_size - 1) / batch_size;  // parallel_mcts_executor.rs:39-42,207
-    std::vector<int32_t> back((size_t)n + 1, (n - 1) * Q);     // {device error word, each model's group size}
+    std::vector<int32_t> back((size_t)n + 1, (n - 1) * Q);     // {device error word, each participant's group size}
     back[0] = 0;
+    const uint64_t naive_key = mix64(seed ^ kNaiveKey);
     const int32_t *size = back.data() + 1;
     std::vector<int> movers;
     int64_t n_moves = 0, syncs = 0;
@@ -1873,14 +1880,21 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
         for (int m = 0; m < n; ++m)
             if (size[m] > 0) movers.push_back(m);
         if (movers.empty()) break;
-        const int lanes = two_lanes && movers.size() >= 2 ? 2 : 1;
+        // the naive player searches nothing: its half-move is one launch on lane 0 in the last stage, and the models' groups
+        // alternate over the lanes as they would without it
+        const int naive_moves = naive && size[0] > 0 ? 1 : 0;
+        const int lanes = two_lanes && movers.size() - naive_moves >= 2 ? 2 : 1;
         if (lanes == 2) lanes_fork(c);
         for (int stage = 0; stage < rounds + 2 && rc == OMK_OK; ++stage)
             for (size_t k = 0; k < movers.size() && rc == OMK_OK; ++k) {
                 const int m = movers[k];
+                if (naive && m == 0) {
+                    if (stage == rounds + 1) launch_tourney_naive_move(c, t, half, size[0], naive_key);
+                    continue;
+                }
                 const size_t g0 = (size_t)m * gcap;
-                LaneScope lane(c, lanes == 2 ? (int)(k % 2) : 0, 0);
-                ModelScope model(c, slots[m]);
+                LaneScope lane(c, lanes == 2 ? (int)((k - naive_moves) % 2) : 0, 0);
+                ModelScope model(c, slot_of(m));
                 rc = match_stage(c, stage, rounds, half, t.gids + g0, size[m], t.gact + g0, t.gst + g0, t.gost + g0, batch_size, epsilon,
                                  alpha, evaluator);
             }
@@ -1914,4 +1928,19 @@ extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *s
     }
     if (out_gpu_ms) CK(cudaEventElapsedTime(out_gpu_ms, c->ev0, c->ev1));
     return OMK_OK;
+}
+
+extern "C" int32_t omk_tournament(omk_ctx *c, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree, int32_t count,
+                                  int32_t batch_size, float epsilon, float alpha, int32_t evaluator, int32_t *out_result,
+                                  int8_t *out_moves, int8_t *out_status, int64_t *out_stats, float *out_gpu_ms) {
+    return tournament(c, false, n_models, slots, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, 0, out_result,
+                      out_moves, out_status, out_stats, out_gpu_ms);
+}
+
+extern "C" int32_t omk_tournament_naive(omk_ctx *c, int32_t n_models, const int32_t *slots, int32_t pairs, int32_t first_tree,
+                                        int32_t count, int32_t batch_size, float epsilon, float alpha, int32_t evaluator, uint64_t seed,
+                                        int32_t *out_result, int8_t *out_moves, int8_t *out_status, int64_t *out_stats,
+                                        float *out_gpu_ms) {
+    return tournament(c, true, n_models, slots, pairs, first_tree, count, batch_size, epsilon, alpha, evaluator, seed, out_result,
+                      out_moves, out_status, out_stats, out_gpu_ms);
 }

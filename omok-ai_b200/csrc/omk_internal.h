@@ -331,13 +331,14 @@ void launch_match_init(omk_ctx *c, int pairs, int first_tree, int32_t *ids, uint
                        int32_t *counters);
 void launch_match_advance(omk_ctx *c, int pairs, int first_tree, int half, const int *live, int32_t *ids, int32_t *actions,
                           const int8_t *status, const int8_t *other_status, int8_t *moves, int8_t *final_status, int32_t *counters);
-// omk_tournament (DESIGN.md 4): n models, P = n(n-1)/2 pairings (i < j, lexicographic), `pairs` games per leg of each.  The
+// omk_tournament (DESIGN.md 4): n participants, P = n(n-1)/2 pairings (i < j, lexicographic), `pairs` games per leg of each.
+// naive: participant 0 is the naive player (omk_tournament_naive), the others are models; otherwise all n are models.  The
 // per-pairing state is omk_match's: ids [P][side][leg][pairs] (left 0, right 1), actions [P][leg][pairs], live [P][leg],
 // counters [P][3] = {left wins, right wins, draws}, moves [P][2 * pairs][81], final status [P][2 * pairs].  Model m's group
 // (its movers of one half-move, over all its pairings in order) is [m][gcap] in gids / gact / gst / gost, and off [P][leg] is
 // where a (pairing, leg)'s movers sit in their model's group.  back = {device error word, group size of each model}.
 struct TourneyState {
-    int n, pairs, first_tree, gcap;
+    int n, pairs, first_tree, gcap, naive;
     int32_t *ids, *actions, *live, *off, *counters, *back;
     int32_t *gids, *gact;  // [n][gcap]
     int8_t *gst, *gost;    // [n][gcap]: the movers' play_action statuses, and their trees' statuses taking the other side's move
@@ -350,6 +351,9 @@ void launch_tourney_init(omk_ctx *c, const TourneyState &t);
 void launch_tourney_advance(omk_ctx *c, const TourneyState &t, int half);
 // the groups of half-move `half` from the compacted lists: gids, gact (the move each tree takes in stage 0), off, back
 void launch_tourney_gather(omk_ctx *c, const TourneyState &t, int half);
+// the naive player's half-move `half`: its n moves, and their statuses on the board, from the roots of the trees of its group
+// (participant 0's gids) into its gact / gst; key = mix64(seed ^ kNaiveKey)
+void launch_tourney_naive_move(omk_ctx *c, const TourneyState &t, int half, int n, uint64_t key);
 
 // omk_api.cu: open / close a profiling span of kernel family `kind` (no-op below min_level)
 bool prof_begin(omk_ctx *c, int kind, int min_level);

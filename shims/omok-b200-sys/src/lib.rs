@@ -129,6 +129,7 @@ extern "C" {
     pub fn omk_model_from_net(ctx: *mut omk_ctx, slot: i32) -> i32;
     pub fn omk_model_eval(ctx: *mut omk_ctx, slot: i32, boards: *const u8, turns: *const u8, n: i32, mode: i32, out_p: *mut f32, out_v: *mut f32) -> i32;
     pub fn omk_tournament(ctx: *mut omk_ctx, n_models: i32, slots: *const i32, pairs: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
+    pub fn omk_tournament_naive(ctx: *mut omk_ctx, n_models: i32, slots: *const i32, pairs: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, seed: u64, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
 }
 
 /// The message of the last failing call on this thread.
