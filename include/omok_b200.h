@@ -304,6 +304,26 @@ OMK_API int32_t omk_replay_get(omk_ctx *ctx, const int64_t *rows, int32_t n, uin
  * An absent or empty replay memory is OMK_ERR_STATE.                                                                     */
 OMK_API int32_t omk_train_replay(omk_ctx *ctx, uint64_t seed, int64_t first_step, int32_t steps, int32_t n, float *out_losses,
                          int64_t *out_rows);
+/* The trainer's loss terms of model slot `slot` (0 .. 15, 0 = the network) on replay rows, changing nothing: rows[n] logical
+ * indices, or rows == NULL for the logical range [first, first + n).  Per row, from the policy logits l[81] and the value
+ * logit of the tensor-core forward on encode_nn_input(board, turn) in Player mode (the evaluator's network, with the logits
+ * kept instead of turned into probabilities; omk_debug_set_fc0_mode(ctx, 0) selects the CUDA-core heads GEMM):
+ *   p_loss = -sum_a pi[a] * (l[a] - logsumexp(l))      (softmax_cross_entropy_with_logits over all 81 cells, as the trainer)
+ *   v_loss = (z - tanh(value logit))^2
+ *   top1   = 1 if the first maximum of l (ascending cell order) is the first maximum of pi, else 0
+ * with the trainer's own loss kernel.  out_means points to a double[4] = {mean p_loss, mean v_loss, mean p_loss + mean v_loss,
+ * mean top1} in fp64, in a specified order: the rows [1024 b, 1024 b + 1024) of the call are added in row order from 0.0, then
+ * these block sums in ascending b, each sum divided by n; so the means depend on the rows only.  (It is declared void * because
+ * the ABI's declarations stay within the scalar types the Rust bindings mirror, which have no double: pass a double[4], from
+ * Rust a [f64; 4] as *mut c_void.)  out_row_p_loss[n], out_row_v_loss[n]
+ * and out_row_top1[n] (each may be NULL) are the per-row terms.  Rows are read as of the end of the last omk_selfplay_run, as
+ * omk_replay_info reports them; no tree, env slot, replay row, self-play or optimizer state is touched, so an active
+ * self-play driver's next omk_selfplay_run is unchanged.  A network changed by training is re-packed first, as by every
+ * evaluating call.  OMK_ERR_STATE: no or an empty replay memory, slot not loaded; OMK_ERR_INVALID: slot outside 0 .. 15, a row
+ * outside [0, len), n < 1, out_means NULL; OMK_ERR_NUMERIC: a non-finite logit or loss.  The rows are evaluated in chunks of
+ * 16 384; no host-to-device copy with rows == NULL; one synchronisation (after the first call's allocations). */
+OMK_API int32_t omk_replay_score(omk_ctx *ctx, int32_t slot, const int64_t *rows, int64_t first, int32_t n, void *out_means,
+                                 float *out_row_p_loss, float *out_row_v_loss, uint8_t *out_row_top1);
 
 /* ---------------------------------------------------------------- evaluation against the naive player
  * The trainer's evaluation phase (src/trainer.rs:487-603) on the device.  The naive player (:506-537) takes the first

@@ -144,6 +144,7 @@ def load_library():
     L.omk_replay_info.argtypes = [vp, P(i64), P(i64), P(i64)]
     L.omk_replay_get.argtypes = [vp, vp, i32, vp, vp, vp, vp]
     L.omk_train_replay.argtypes = [vp, u64, i64, i32, i32, vp, vp]
+    L.omk_replay_score.argtypes = [vp, i32, vp, i64, i32, vp, vp, vp, vp]
     L.omk_naive_move.argtypes = [vp, vp, vp, i32, u64, vp, vp, vp]
     L.omk_eval_naive.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, u64, vp, vp, vp, vp, P(f32)]
     L.omk_opponent_load_params.argtypes = [vp, P(vp), P(i64)]
@@ -510,6 +511,25 @@ class Context:
         self._check(self.L.omk_train_replay(self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(first_step), int(steps), int(n),
                                             _ptr(losses), _ptr(rows)))
         return (losses, rows) if want_rows else losses
+
+    def replay_score(self, slot: int = 0, rows=None, first: int = 0, n=None, per_row: bool = False):
+        """The trainer's loss terms of model slot `slot` (0 = the network) on replay rows, changing nothing: the logical rows
+        `rows`, or the range [first, first + n) (n defaults to the rest of the memory).  Returns the means (p_loss, v_loss,
+        p_loss + v_loss, top-1 agreement of the policy logits with pi) in fp64, summed in a specified order; with `per_row`,
+        (means, p_loss [n] f32, v_loss [n] f32, top1 [n] u8)."""
+        if rows is not None:
+            rows = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+            n = rows.size
+        elif n is None:
+            n = self.replay_info()[0] - int(first)
+        n = int(n)
+        means = np.zeros(4, dtype=np.float64)
+        p = np.zeros(max(n, 0), dtype=np.float32) if per_row else None
+        v = np.zeros(max(n, 0), dtype=np.float32) if per_row else None
+        top1 = np.zeros(max(n, 0), dtype=np.uint8) if per_row else None
+        self._check(self.L.omk_replay_score(self.h, int(slot), _ptr(rows), int(first), n, _ptr(means), _ptr(p), _ptr(v), _ptr(top1)))
+        out = tuple(float(x) for x in means)
+        return (out, p, v, top1) if per_row else out
 
     # ---- evaluation against the naive player ----
     def naive_move(self, boards, turns, seed: int, streams=None):

@@ -93,11 +93,13 @@ struct FcCfg {
 };
 
 // BN = 256: fc0 / fc1 tiles.  BN = 128 with HEADS: the policy/value heads (512 -> 81 | 1, padded to 128 columns): a drain
-// thread owns a whole row of logits, so tanh (value, network.rs:188-202) and softmax (policy, :227-247) finish in registers.
+// thread owns a whole row of logits, so tanh (value, network.rs:188-202) and softmax (policy, :227-247) finish in registers;
+// with LOGITS it stores the row's 82 logits to C [rows][128] instead (policy 0..80, value 81: the layout the CUDA-core heads
+// GEMM writes to ws.logits), for the replay score's losses.
 // SPLITK (small batches): blockIdx.z selects F_SPLITK_KB k-blocks; the CTA writes the raw fp32 partial sums of each of their chunks
 // to C[z][gridDim.y * 128 rows][512] and k_fc0_reduce adds the chunks in order -- the same partial sums in the same order as the
 // unsplit kernel, so a row's result stays bit-identical whatever the batch size (recorded-mode parity).
-template <int K, int CHUNK, bool PAIR, int BN = 256, bool HEADS = false, bool SPLITK = false>
+template <int K, int CHUNK, bool PAIR, int BN = 256, bool HEADS = false, bool SPLITK = false, bool LOGITS = false>
 __global__ void __launch_bounds__((FcCfg<PAIR, BN>::kThreads), 1)
     k_fc16(const __grid_constant__ CUtensorMap map_a_hi, const __grid_constant__ CUtensorMap map_a_lo,
            const __grid_constant__ CUtensorMap map_b_hi, const __grid_constant__ CUtensorMap map_b_lo,
@@ -110,6 +112,7 @@ __global__ void __launch_bounds__((FcCfg<PAIR, BN>::kThreads), 1)
     constexpr int CG = PAIR ? 2 : 1;
     static_assert(K % F_BK == 0 && (K / F_BK) % CHUNK == 0, "chunking must tile K");
     static_assert(!SPLITK || (!PAIR && !HEADS), "split-K is the one-CTA fc0 variant");
+    static_assert(!LOGITS || HEADS, "LOGITS is an epilogue of the heads");
     // split-K: one CTA walks F_SPLITK_KB k-blocks = several chunks, and stores every chunk's partial sums separately
     constexpr int NKB = SPLITK ? F_SPLITK_KB : K / F_BK;      // k-blocks this CTA walks
     static_assert(!SPLITK || (F_SPLITK_KB % CHUNK == 0 && (K / F_BK) % F_SPLITK_KB == 0), "split-K groups must tile K");
@@ -344,6 +347,23 @@ __global__ void __launch_bounds__((FcCfg<PAIR, BN>::kThreads), 1)
         const float inv_scale = *inv_scale_p;  // undo the power-of-two weight scaling (exact)
         if constexpr (SPLITK) {
             // (the chunks' partial sums were stored in the drain loop)
+        } else if constexpr (LOGITS) {
+            if (row < rows) {
+                // the logits exactly as the branch below forms them before softmax / tanh
+                float *lrow = C + (size_t)row * 128;
+                bool finite = true;
+#pragma unroll
+                for (int j = 0; j < 80; j += 4) {
+                    const float4 o = make_float4(fmaf(acc[j], inv_scale, brow[j]), fmaf(acc[j + 1], inv_scale, brow[j + 1]),
+                                                 fmaf(acc[j + 2], inv_scale, brow[j + 2]), fmaf(acc[j + 3], inv_scale, brow[j + 3]));
+                    finite = finite && fabsf(o.x) < INFINITY && fabsf(o.y) < INFINITY && fabsf(o.z) < INFINITY && fabsf(o.w) < INFINITY;
+                    *reinterpret_cast<float4 *>(lrow + j) = o;
+                }
+                const float l80 = fmaf(acc[80], inv_scale, brow[80]), vlogit = fmaf(acc[kCells], inv_scale, brow[kCells]);
+                if (!finite || !(fabsf(l80) < INFINITY) || !(fabsf(vlogit) < INFINITY)) atomicOr(dev_error, 2u);
+                lrow[80] = l80;
+                lrow[kCells] = vlogit;
+            }
         } else if constexpr (HEADS) {
             if (row < rows) {
                 // logits: columns 0..80 policy, 81 value (k_pack_heads); same softmax / tanh arithmetic as k_heads
@@ -725,18 +745,20 @@ bool launch_fc1_f16(omk_ctx *c, int rows_bound) {
     return check_launch("fc1 (fp16 split)");
 }
 
-// heads: act2_h16/l16 -> P (softmax of the 81 policy logits) and V (tanh of the value logit)
-bool launch_heads_f16(omk_ctx *c, int rows_bound) {
+// heads: act2_h16/l16 -> P (softmax of the 81 policy logits) and V (tanh of the value logit), or with `logits` the 82
+// logits into ws.logits
+bool launch_heads_f16(omk_ctx *c, int rows_bound, bool logits) {
     const NetWeights &m = *c->model;
     const ActMaps *am = m.weights_ready ? &c->ws.maps : nullptr;
     if (!am) return false;
     using Cfg = FcCfg<false, 128>;
-    auto kern = k_fc16<F_K1, F_CHUNKH, false, 128, true>;
+    auto kern = logits ? k_fc16<F_K1, F_CHUNKH, false, 128, true, false, true> : k_fc16<F_K1, F_CHUNKH, false, 128, true>;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
     const int mt = (rows_bound + F_BM - 1) / F_BM;
     kern<<<dim3(1, mt), Cfg::kThreads, Cfg::kSmemBytes, c->stream>>>(
-        am->map2_a_hi, am->map2_a_lo, m.map2_b_hi, m.map2_b_lo, m.heads_b, m.fc_inv_scale + 2, nullptr, nullptr, nullptr,
-        c->ws.n_req, rows_bound, c->ws.P, c->ws.V, c->dev_error, FcBal{});
+        am->map2_a_hi, am->map2_a_lo, m.map2_b_hi, m.map2_b_lo, m.heads_b, m.fc_inv_scale + 2, logits ? c->ws.logits.get() : nullptr,
+        nullptr, nullptr, c->ws.n_req, rows_bound, logits ? nullptr : c->ws.P.get(), logits ? nullptr : c->ws.V.get(), c->dev_error,
+        FcBal{});
     c->launches++;
     return check_launch("heads (fp16 split)");
 }

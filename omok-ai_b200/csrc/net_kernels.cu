@@ -411,7 +411,8 @@ void launch_net_init_random(omk_ctx *c, uint64_t seed) {
 
 // false: a launch, a tensor-map encode or an activation-buffer allocation failed -- ws.P / ws.V hold nothing the caller may
 // use (the message went to stderr); callers must not run k_apply on them and return OMK_ERR_CUDA.
-bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
+// logits: the heads leave each row's 82 logits in ws.logits [rows][128] (policy 0..80, value 81) and write no P / V.
+bool net_forward(omk_ctx *c, const float *images_dev, int max_rows, bool logits) {
     cudaFuncSetAttribute(k_tower, cudaFuncAttributeMaxDynamicSharedMemorySize, kTowerSmemBytes);
     if (max_rows > c->ws.max_rows) max_rows = c->ws.max_rows;
     if (max_rows <= 0) return true;
@@ -464,13 +465,15 @@ bool net_forward(omk_ctx *c, const float *images_dev, int max_rows) {
     }
     prof_end(c, sp);
     sp = prof_begin(c, OMK_K_HEADS, 2);
-    if (c->fc0_mode == 1) {  // heads GEMM + tanh / softmax in one tensor-core kernel
-        ok = launch_heads_f16(c, max_rows) && ok;
+    if (c->fc0_mode == 1) {  // heads GEMM + tanh / softmax (or the logits) in one tensor-core kernel
+        ok = launch_heads_f16(c, max_rows, logits) && ok;
     } else {
         k_gemm<<<dim3(1, mt), 256, 0, c->stream>>>(c->ws.act2, c->model->heads_w, c->model->heads_b, c->ws.logits, c->ws.n_req, max_rows,
                                                    128, kFc, 0);
-        k_heads<<<(max_rows + 7) / 8, 256, 0, c->stream>>>(c->ws.logits, c->ws.n_req, max_rows, c->ws.P, c->ws.V);
-        c->launches++;
+        if (!logits) {
+            k_heads<<<(max_rows + 7) / 8, 256, 0, c->stream>>>(c->ws.logits, c->ws.n_req, max_rows, c->ws.P, c->ws.V);
+            c->launches++;
+        }
     }
     prof_end(c, sp);
     c->launches += 3;  // tower, fc0, fc1 (launch_heads_f16 / the CUDA-core heads counted above)

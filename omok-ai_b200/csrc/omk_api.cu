@@ -1,6 +1,7 @@
 // omk_api.cu -- extern "C" boundary of libomok_b200.so (see include/omok_b200.h).
 // Host-side orchestration only: pool allocation, argument staging, kernel sequencing.
 // There is no CPU compute path: every operation is a CUDA kernel on the context's stream.
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -1391,7 +1392,7 @@ extern "C" int32_t omk_replay_get(omk_ctx *c, const int64_t *rows, int32_t n, ui
     float *d_pz = nullptr;    // [policy n*81 | z n]
     SCRATCH(1, nn * (kCells + 1), d_bt);
     SCRATCH(2, nn * (kCells + 1), d_pz);
-    launch_rp_get(c, d_rows, n, d_bt, d_bt + nn * kCells, d_pz, d_pz + nn * kCells);
+    launch_rp_get(c, d_rows, 0, n, d_bt, d_bt + nn * kCells, d_pz, d_pz + nn * kCells);
     if (out_boards) CK(copy_d2h(c, out_boards, d_bt, nn * kCells, c->stream));
     if (out_turns) CK(copy_d2h(c, out_turns, d_bt + nn * kCells, nn, c->stream));
     if (out_policy) CK(copy_d2h(c, out_policy, d_pz, sizeof(float) * nn * kCells, c->stream));
@@ -1439,6 +1440,62 @@ extern "C" int32_t omk_train_replay(omk_ctx *c, uint64_t seed, int64_t first_ste
             for (int k = m; k < n; ++k) out_rows[(size_t)s * n + k] = -1;
     for (int i = 0; i < 3 * steps; ++i)
         if (!(out_losses[i] == out_losses[i]) || out_losses[i] > 3.0e38f) return fail(OMK_ERR_NUMERIC, "the training loss is not finite");
+    return OMK_OK;
+}
+
+// ------------------------------------------------------------------ the trainer's losses of a model on replay rows
+// Rows per network forward: a whole 600 000-row memory at once would need tens of GB of activations.
+constexpr int kScoreChunk = 16384;
+
+extern "C" int32_t omk_replay_score(omk_ctx *c, int32_t slot, const int64_t *rows, int64_t first, int32_t n, void *out_means,
+                                    float *out_row_p_loss, float *out_row_v_loss, uint8_t *out_row_top1) {
+    CK(cudaSetDevice(c->device));
+    if (slot < 0 || slot >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
+    if (n < 1 || !out_means) return fail(OMK_ERR_INVALID, "need n >= 1 and out_means");
+    const Replay &r = c->rp;
+    if (r.ring.cap == 0) return fail(OMK_ERR_STATE, "no replay memory (omk_replay_reset)");
+    if (r.len == 0) return fail(OMK_ERR_STATE, "the replay memory is empty");
+    if (!c->slot(slot).loaded) return fail(OMK_ERR_STATE, slot_name(slot) + " weights not loaded");
+    if (!rows && (first < 0 || first > r.len - n))
+        return fail(OMK_ERR_INVALID, "rows [first, first + n) outside the replay's " + std::to_string(r.len) + " rows");
+    int32_t rc = OMK_OK;
+    if (slot == 0 && (rc = ensure_packed(c)) != OMK_OK) return rc;
+    int64_t *d_rows = nullptr;
+    if (rows && (rc = stage_rows(c, rows, n, &d_rows)) != OMK_OK) return rc;
+    // per-row buffers of all n rows (the reduction runs once, over all of them), and one chunk's gathered rows:
+    //   floats [row_loss 2n | p_loss n | v_loss n | pi chunk*81 | z chunk]
+    //   bytes  [means 4 f64 | block sums 3 f64 per 1024 rows | top1 n | boards chunk*81 | turns chunk]
+    const size_t nn = (size_t)n, chunk = nn < (size_t)kScoreChunk ? nn : (size_t)kScoreChunk, blocks = (nn + 1023) / 1024;
+    float *fbuf = nullptr;
+    uint8_t *bbuf = nullptr;
+    SCRATCH(1, 4 * nn + chunk * (kCells + 1), fbuf);
+    SCRATCH(2, 32 + 24 * blocks + nn + chunk * (kCells + 1), bbuf);
+    float *row_loss = fbuf, *p_loss = fbuf + 2 * nn, *v_loss = fbuf + 3 * nn, *pi = fbuf + 4 * nn, *z = pi + chunk * kCells;
+    double *means = reinterpret_cast<double *>(bbuf), *block_sums = means + 4;
+    uint8_t *top1 = bbuf + 32 + 24 * blocks, *boards = top1 + nn, *turns = boards + chunk * kCells;
+    if ((rc = ensure_workspace(c, (int)chunk)) != OMK_OK) return rc;
+    {
+        ModelScope scope(c, slot);
+        for (size_t off = 0; off < nn; off += chunk) {
+            const int m = (int)(nn - off < chunk ? nn - off : chunk);
+            launch_rp_get(c, d_rows ? d_rows + off : nullptr, first + (long long)off, m, boards, turns, pi, z);
+            launch_pack_boards(c, boards, turns, m, OMK_TURN_MODE_PLAYER);
+            if (!net_forward(c, nullptr, m, true)) return fail(OMK_ERR_CUDA, "the network forward failed to launch (see stderr)");
+            launch_loss_rows(c, c->ws.logits, 128, c->ws.logits + kCells, 128, pi, z, m, row_loss + 2 * off, top1 + off);
+        }
+    }
+    CK(cudaMemsetAsync(c->ws.n_req, 0, sizeof(uint32_t), c->stream));  // the rows are no search's evaluations (dev_sims)
+    launch_score_reduce(c, row_loss, top1, (long long)nn, p_loss, v_loss, block_sums, means);
+    double h_means[4];  // staged here: out_means is written only when the call succeeds
+    CK(copy_d2h(c, h_means, means, sizeof h_means, c->stream));
+    if (out_row_p_loss) CK(copy_d2h(c, out_row_p_loss, p_loss, sizeof(float) * nn, c->stream));
+    if (out_row_v_loss) CK(copy_d2h(c, out_row_v_loss, v_loss, sizeof(float) * nn, c->stream));
+    if (out_row_top1) CK(copy_d2h(c, out_row_top1, top1, nn, c->stream));
+    if ((rc = check_device_error(c)) != OMK_OK) return rc;  // (the call's one synchronisation) a non-finite logit: OMK_ERR_NUMERIC
+    for (int k = 0; k < 4; ++k)
+        if (!std::isfinite(h_means[k]))
+            return fail(OMK_ERR_NUMERIC, "a loss of the replay rows is not finite (non-finite weights or logits)");
+    memcpy(out_means, h_means, sizeof h_means);
     return OMK_OK;
 }
 

@@ -307,12 +307,12 @@ void launch_sp_advance(omk_ctx *c, int g0, int n, const int8_t *status, unsigned
 
 // replay_kernels.cu: stage a lane's recorded ply (ring-slot boards / policies of games g0..g0+n-1) on c->stream; commit the
 // ply's finished episodes on the replay stream; sample `steps` minibatches of m logical rows; gather + encode one minibatch;
-// copy rows out for omk_replay_get
+// copy rows out for omk_replay_get / omk_replay_score (rows == nullptr: the logical rows first .. first + n - 1)
 void launch_rp_stage(omk_ctx *c, int g0, int n, const uint8_t *boards, const float *policy);
 void launch_rp_commit(omk_ctx *c, int n, const int8_t *status);
 void launch_rp_sample(omk_ctx *c, uint64_t seed, long long first_step, int steps, long long len, int m, int64_t *rows);
 void launch_rp_gather(omk_ctx *c, const int64_t *rows, int m, float *img, float *pi, float *z);
-void launch_rp_get(omk_ctx *c, const int64_t *rows, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z);
+void launch_rp_get(omk_ctx *c, const int64_t *rows, long long first, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z);
 
 // eval_kernels.cu: the naive player's move (trainer.rs:506-537) for positions given as cells + turns, or for the roots of
 // the live trees of omk_eval_naive; that driver's set-up and its bookkeeping after each half-move (move records, tallies,
@@ -360,7 +360,8 @@ bool prof_begin(omk_ctx *c, int kind, int min_level);
 void prof_end(omk_ctx *c, bool opened);
 
 // net_kernels.cu
-bool net_forward(omk_ctx *c, const float *images_dev /* or nullptr: use ws.nn_in */, int max_rows);  // false: nothing usable in ws.P / ws.V
+// false: nothing usable in ws.P / ws.V; logits: the heads' logits into ws.logits [rows][128] instead of P / V (omk_replay_score)
+bool net_forward(omk_ctx *c, const float *images_dev /* or nullptr: use ws.nn_in */, int max_rows, bool logits = false);
 void net_pack_heads(omk_ctx *c);
 void launch_net_init_random(omk_ctx *c, uint64_t seed);
 
@@ -371,7 +372,7 @@ bool ensure_activations(omk_ctx *c, int rows);
 bool fc16_prepare_weights(omk_ctx *c);
 bool launch_fc0_f16(omk_ctx *c, int rows_bound);
 bool launch_fc1_f16(omk_ctx *c, int rows_bound);
-bool launch_heads_f16(omk_ctx *c, int rows_bound);
+bool launch_heads_f16(omk_ctx *c, int rows_bound, bool logits);
 // encode a.maps over a's fp16 buffers (ensure_activations, whenever it (re)allocates them)
 bool fc16_encode_act_maps(Activations &a);
 void launch_f32_to_split16(omk_ctx *c, const float *x, __half *hi, __half *lo, long long n);
@@ -387,6 +388,16 @@ const char *train_minibatch_buffers(omk_ctx *c, int n, float **img, float **pi, 
 const char *train_backward_resident(omk_ctx *c, int n);
 const char *train_report_losses_device(omk_ctx *c, int n, float *dst3);
 float *train_grad_buffer(omk_ctx *c);
+// the trainer's per-row loss terms (k_loss, no gradients) of n rows whose logits sit in rows of `lstride` floats and whose value
+// logits are vlogit[i * vstride] -> row_loss[2n] = {p_loss, v_loss} per row, top1[n] (may be nullptr: the first maximum of the
+// logits is the first maximum of pi)
+void launch_loss_rows(omk_ctx *c, const float *logits, int lstride, const float *vlogit, int vstride, const float *pi, const float *z,
+                      int n, float *row_loss, uint8_t *top1);
+// omk_replay_score's means of n rows' row_loss / top1: block b adds rows [1024 b, 1024 b + 1024) in row order in fp64 from 0.0, the
+// block sums are added in ascending b -> means4 = {mean p_loss, mean v_loss, their sum, mean top1}; also de-interleaves row_loss
+// into p_out[n], v_out[n].  block_sums: [ceil(n / 1024)][3]
+void launch_score_reduce(omk_ctx *c, const float *row_loss, const uint8_t *top1, long long n, float *p_out, float *v_out,
+                         double *block_sums, double *means4);
 void train_reset_optimizer(omk_ctx *c);
 const char *train_comm_unique_id(omk_ctx *c, uint8_t *out128);
 const char *train_comm_init(omk_ctx *c, const uint8_t *id128, int nranks, int rank);

@@ -237,12 +237,12 @@ __global__ void k_rp_gather(const int64_t *__restrict__ rows, int m, ReplayRing 
     if (threadIdx.x == 0) z[i] = ring.z[phys];
 }
 
-// ---- omk_replay_get: logical rows -> host layout ----
-__global__ void k_rp_get(const int64_t *__restrict__ rows, int n, ReplayRing ring, long long base, uint8_t *__restrict__ boards,
-                         uint8_t *__restrict__ turns, float *__restrict__ pi, float *__restrict__ z) {
+// ---- omk_replay_get / omk_replay_score: logical rows rows[i] (or first + i without a list) -> host layout ----
+__global__ void k_rp_get(const int64_t *__restrict__ rows, long long first, int n, ReplayRing ring, long long base,
+                         uint8_t *__restrict__ boards, uint8_t *__restrict__ turns, float *__restrict__ pi, float *__restrict__ z) {
     const int i = blockIdx.x;
     if (i >= n) return;
-    const size_t phys = (size_t)((base + rows[i]) % ring.cap);
+    const size_t phys = (size_t)((base + (rows ? rows[i] : first + i)) % ring.cap);
     for (int c = threadIdx.x; c < kCells; c += blockDim.x) {
         boards[(size_t)i * kCells + c] = ring.boards[phys * kCells + c];
         pi[(size_t)i * kCells + c] = ring.pi[phys * kCells + c];
@@ -277,8 +277,8 @@ void launch_rp_gather(omk_ctx *c, const int64_t *rows, int m, float *img, float 
     k_rp_gather<<<m, 96, 0, c->stream>>>(rows, m, c->rp.ring.view(), c->rp.added - c->rp.len, img, pi, z);
     c->launches++;
 }
-void launch_rp_get(omk_ctx *c, const int64_t *rows, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z) {
-    k_rp_get<<<n, 96, 0, c->stream>>>(rows, n, c->rp.ring.view(), c->rp.added - c->rp.len, boards, turns, pi, z);
+void launch_rp_get(omk_ctx *c, const int64_t *rows, long long first, int n, uint8_t *boards, uint8_t *turns, float *pi, float *z) {
+    k_rp_get<<<n, 96, 0, c->stream>>>(rows, first, n, c->rp.ring.view(), c->rp.added - c->rp.len, boards, turns, pi, z);
     c->launches++;
 }
 

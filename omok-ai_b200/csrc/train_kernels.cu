@@ -286,14 +286,30 @@ __global__ void k_dw_wgrad(const float *__restrict__ in, const float *__restrict
     if (threadIdx.x == 0) done[tap] = 0u;
 }
 
+// the first maximum (lowest index among equal values) of a warp's (value, index) candidates
+__device__ __forceinline__ int warp_first_argmax(float v, int idx) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, v, off);
+        const int oi = __shfl_xor_sync(0xffffffffu, idx, off);
+        if (ov > v || (ov == v && oi < idx)) {
+            v = ov;
+            idx = oi;
+        }
+    }
+    return idx;
+}
+
 // per position: softmax cross entropy with the visit policy, squared value error, and their logit gradients for the
-// MEAN losses (1/n folded in).  row_loss[2*i] = policy term, [2*i+1] = value term.
-__global__ void k_loss(const float *__restrict__ logits /*[n][81]*/, const float *__restrict__ vlogit /*[n]*/, const float *__restrict__ pi,
-                       const float *__restrict__ z, int n, float *__restrict__ dlogits, float *__restrict__ dvlogit,
-                       float *__restrict__ row_loss) {
+// MEAN losses (1/n folded in).  row_loss[2*i] = policy term, [2*i+1] = value term.  Row i's logits are logits[i * lstride ..],
+// its value logit vlogit[i * vstride] (the trainer: 81 and 1; omk_replay_score reads the evaluator's [rows][128] in place).
+// top1 (may be nullptr): 1 if the first maximum of the logits (ascending cell order) is the first maximum of pi, else 0.
+__global__ void k_loss(const float *__restrict__ logits, int lstride, const float *__restrict__ vlogit, int vstride,
+                       const float *__restrict__ pi, const float *__restrict__ z, int n, float *__restrict__ dlogits,
+                       float *__restrict__ dvlogit, float *__restrict__ row_loss, uint8_t *__restrict__ top1) {
     const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
     if (row >= n) return;
-    const float *l = logits + (size_t)row * kCells, *t = pi + (size_t)row * kCells;
+    const float *l = logits + (size_t)row * lstride, *t = pi + (size_t)row * kCells;
     float v[3], tv[3], mx = -INFINITY, tsum = 0.0f;
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
@@ -328,15 +344,28 @@ __global__ void k_loss(const float *__restrict__ logits /*[n][81]*/, const float
     }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) pl += __shfl_xor_sync(0xffffffffu, pl, off);
+    bool agree = false;
+    if (top1) {  // each lane's candidates are in ascending cell order, so a strict > keeps the first maximum
+        float bl = v[0], bt = tv[0];
+        int il = lane, it = lane;
+#pragma unroll
+        for (int j = 1; j < 3; ++j) {
+            const int c = lane + 32 * j;
+            if (c < kCells && v[j] > bl) { bl = v[j]; il = c; }
+            if (c < kCells && tv[j] > bt) { bt = tv[j]; it = c; }
+        }
+        agree = warp_first_argmax(bl, il) == warp_first_argmax(bt, it);
+    }
     if (lane == 0) {
         // tanh and its derivative from one exponential: 1 - tanh^2 = 4e / (1 + e)^2 with e = exp(-2|x|) keeps its relative
         // accuracy where tanh saturates (value logits have a scale of ~20; 1 - v*v would cancel to a few bits there)
-        const float xl = vlogit[row], ex2 = expf(-2.0f * fabsf(xl)), den = 1.0f + ex2;
+        const float xl = vlogit[(size_t)row * vstride], ex2 = expf(-2.0f * fabsf(xl)), den = 1.0f + ex2;
         const float val = copysignf((1.0f - ex2) / den, xl), sech2 = 4.0f * ex2 / (den * den);
         const float d = val - z[row];
         row_loss[2 * row] = pl;
         row_loss[2 * row + 1] = d * d;
         if (dvlogit) dvlogit[row] = 2.0f * d * sech2 * invn;
+        if (top1) top1[row] = agree ? 1 : 0;
     }
 }
 // (p_loss, v_loss, loss) = means over the rows, summed in row order by one thread per term (n is a minibatch)
@@ -348,6 +377,50 @@ __global__ void k_loss_reduce(const float *__restrict__ row_loss, int n, float *
     }
     __syncthreads();
     if (threadIdx.x == 0) out3[2] = out3[0] + out3[1];
+}
+
+// omk_replay_score's means (DESIGN.md 2): block b's three sums over rows [1024 b, 1024 b + 1024), each in row order in fp64 from
+// 0.0 by one thread, so they depend on nothing but the rows; row_loss is de-interleaved into p_out / v_out on the way
+constexpr int kScoreBlock = 1024;
+__global__ void __launch_bounds__(kScoreBlock) k_score_reduce(const float *__restrict__ row_loss, const uint8_t *__restrict__ top1,
+                                                              long long n, float *__restrict__ p_out, float *__restrict__ v_out,
+                                                              double *__restrict__ block_sums) {
+    __shared__ float sp[kScoreBlock], sv[kScoreBlock];
+    __shared__ uint8_t st[kScoreBlock];
+    const long long r0 = (long long)blockIdx.x * kScoreBlock, i = r0 + threadIdx.x;
+    const int m = (int)min((long long)kScoreBlock, n - r0);
+    if (threadIdx.x < m) {
+        const float2 pv = reinterpret_cast<const float2 *>(row_loss)[i];
+        sp[threadIdx.x] = pv.x;
+        sv[threadIdx.x] = pv.y;
+        st[threadIdx.x] = top1[i];
+        p_out[i] = pv.x;
+        v_out[i] = pv.y;
+    }
+    __syncthreads();
+    if (threadIdx.x < 3) {
+        double s = 0.0;
+        if (threadIdx.x == 0) for (int k = 0; k < m; ++k) s += (double)sp[k];
+        else if (threadIdx.x == 1) for (int k = 0; k < m; ++k) s += (double)sv[k];
+        else for (int k = 0; k < m; ++k) s += (double)st[k];
+        block_sums[3 * (size_t)blockIdx.x + threadIdx.x] = s;
+    }
+}
+// the block sums in ascending block order -> {mean p_loss, mean v_loss, mean p_loss + mean v_loss, mean top1}
+__global__ void k_score_means(const double *__restrict__ block_sums, int blocks, long long n, double *__restrict__ means4) {
+    __shared__ double mean[3];
+    if (threadIdx.x < 3) {
+        double s = 0.0;
+        for (int b = 0; b < blocks; ++b) s += block_sums[3 * (size_t)b + threadIdx.x];
+        mean[threadIdx.x] = s / (double)n;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        means4[0] = mean[0];
+        means4[1] = mean[1];
+        means4[2] = mean[0] + mean[1];
+        means4[3] = mean[2];
+    }
 }
 
 __global__ void k_scale(float *x, long long n, float f) {
@@ -516,8 +589,8 @@ static void train_forward(omk_ctx *c, TrainState *t, int n) {
 }
 
 static void train_losses(omk_ctx *c, TrainState *t, int n, bool with_grads) {
-    k_loss<<<(n + 7) / 8, 256, 0, c->stream>>>(t->logits, t->vlogit, t->pi, t->z, n, with_grads ? t->dlogits.get() : nullptr,
-                                                with_grads ? t->dvlogit.get() : nullptr, t->row_loss);
+    k_loss<<<(n + 7) / 8, 256, 0, c->stream>>>(t->logits, kCells, t->vlogit, 1, t->pi, t->z, n, with_grads ? t->dlogits.get() : nullptr,
+                                                with_grads ? t->dvlogit.get() : nullptr, t->row_loss, nullptr);
     k_loss_reduce<<<1, 32, 0, c->stream>>>(t->row_loss, n, t->losses);
     c->launches += 2;
 }
@@ -663,6 +736,19 @@ const char *train_report_losses(omk_ctx *c, int n, float *out3) {
     if (cudaMemcpyAsync(out3, t->losses, sizeof(float) * 3, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess) return "loss copy failed";
     if (cudaStreamSynchronize(c->stream) != cudaSuccess) return "stream synchronisation failed";
     return cudaPeekAtLastError() == cudaSuccess ? nullptr : cudaGetErrorString(cudaGetLastError());
+}
+
+void launch_loss_rows(omk_ctx *c, const float *logits, int lstride, const float *vlogit, int vstride, const float *pi, const float *z,
+                      int n, float *row_loss, uint8_t *top1) {
+    k_loss<<<(n + 7) / 8, 256, 0, c->stream>>>(logits, lstride, vlogit, vstride, pi, z, n, nullptr, nullptr, row_loss, top1);
+    c->launches++;
+}
+void launch_score_reduce(omk_ctx *c, const float *row_loss, const uint8_t *top1, long long n, float *p_out, float *v_out,
+                         double *block_sums, double *means4) {
+    const int blocks = (int)((n + kScoreBlock - 1) / kScoreBlock);
+    k_score_reduce<<<blocks, kScoreBlock, 0, c->stream>>>(row_loss, top1, n, p_out, v_out, block_sums);
+    k_score_means<<<1, 32, 0, c->stream>>>(block_sums, blocks, n, means4);
+    c->launches += 2;
 }
 
 float *train_grad_buffer(omk_ctx *c) { return train_state(c)->grads; }

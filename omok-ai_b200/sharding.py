@@ -21,7 +21,8 @@ def rank_seed(base_seed: int, rank: int) -> int:
 
 
 def reduce_measurements(times: dict[str, float], work: dict[str, int], device: str = "cpu"):
-    """max-over-ranks of every time, sum-over-ranks of every work counter.  No-op without a process group."""
+    """max-over-ranks of every time, sum-over-ranks of every work counter (an int counter stays an int, a float one -- e.g. a
+    mean weighted by its rows -- a float).  No-op without a process group."""
     dist = torch.distributed
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
         return dict(times), dict(work)
@@ -30,7 +31,8 @@ def reduce_measurements(times: dict[str, float], work: dict[str, int], device: s
     w = torch.tensor([float(work[k]) for k in wk], dtype=torch.float64, device=device)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dist.all_reduce(w, op=dist.ReduceOp.SUM)
-    return {k: float(v) for k, v in zip(tk, t.tolist())}, {k: int(round(v)) for k, v in zip(wk, w.tolist())}
+    return ({k: float(v) for k, v in zip(tk, t.tolist())},
+            {k: float(v) if isinstance(work[k], float) else int(round(v)) for k, v in zip(wk, w.tolist())})
 
 
 def gather_replay(boards: torch.Tensor, policy: torch.Tensor, status: torch.Tensor, dst: int = 0):

@@ -16,7 +16,12 @@ active for the next iteration; it reports eval_phase_s and the naive player's wi
 With --gate GAMES the network is copied into the context's opponent before the training phase (omk_opponent_from_net), and
 after training the trained network plays GAMES games against that snapshot at the benchmark's constants (800 simulations,
 batch 8, epsilon 0, alpha 1; benchmark/src/main.rs) as ONE omk_match call on trees past the driver's and the evaluation's:
-AlphaZero's gating question, whether this iteration's network beats the last one."""
+AlphaZero's gating question, whether this iteration's network beats the last one.
+With --device-replay --score the rows this phase's self-play committed, which no step has trained on yet, are a held-out
+set: the network's loss terms on them (policy cross-entropy, value MSE, their sum, and top-1 agreement of the policy with
+the visit distribution) are measured by ONE omk_replay_score call before the training phase and one after it, and with
+--gate also for the snapshot; no game is played.  Under torchrun every rank scores its own memory and the means are
+combined weighted by rows."""
 from __future__ import annotations
 
 import argparse
@@ -36,7 +41,7 @@ N_PARAMS = 5_643_250
 
 
 def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
-        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0):
+        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0, score=False):
     omk = importlib.import_module("omok-ai_b200")
     trainer = importlib.import_module("omok-ai_b200.trainer")
     sharding = importlib.import_module("omok-ai_b200.sharding")
@@ -50,6 +55,8 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     if device_replay and (torch_step or gather):
         raise ValueError("--device-replay trains through omk_train_replay: it excludes --torch-step and --gather")
+    if score and not device_replay:
+        raise ValueError("--score reads the device replay memory: it needs --device-replay")
     if gate and gate < 2:
         raise ValueError("--gate GAMES needs at least 2 games: one opened by each side")
     my_games = games_per_gpu
@@ -71,7 +78,7 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
     if device_replay:
         ctx.replay_reset(replay_capacity)           # before selfplay_begin: the driver feeds the replay that exists then
         return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
-                                  seed, quiet, replay_capacity, evaluate, gate)
+                                  seed, quiet, replay_capacity, evaluate, gate, score)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -189,19 +196,38 @@ def _gate(ctx, games, first_tree):
             "gate_draws": draw, "gate_moves": stats["moves"], "gate_host_syncs": stats["host_syncs"], "gate_gpu_ms": stats["gpu_ms"]}
 
 
+SCORE_TERMS = ("p_loss", "v_loss", "loss", "top1")
+
+
+def _score(ctx, slot, first, n):
+    """Model slot `slot`'s loss terms on the logical replay rows [first, first + n): one omk_replay_score call, and its wall
+    time."""
+    if n == 0:
+        return (0.0,) * 4, 0.0
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    means = ctx.replay_score(slot, first=first, n=n)
+    return means, time.perf_counter() - t0
+
+
 def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity,
-                       evaluate=0, gate=0):
+                       evaluate=0, gate=0, score=False):
     omk = importlib.import_module("omok-ai_b200")
     ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
     ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
     if dist:
         dist.barrier()
+    added_before = ctx.replay_info()[1]
     t0 = time.perf_counter()
     stats = ctx.selfplay_run(plies, profile=0, want_transitions=False)[0]
     sp_s = time.perf_counter() - t0
-    rows, _, episodes = ctx.replay_info()
+    rows, added, episodes = ctx.replay_info()
     if rows == 0:
         raise SystemExit("no game finished during self-play, so the replay memory is empty: raise --plies")
+    fresh = min(rows, added - added_before)         # this phase's rows: the newest, not trained on yet
+    scores = {}
+    if score:
+        scores["before"] = _score(ctx, 0, rows - fresh, fresh)
     per_rank = max(1, minibatch // world)
     sampler_seed = sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
     if gate:
@@ -214,9 +240,18 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
     losses = step.train_replay(steps, per_rank, sampler_seed)   # the whole training phase: one call, one synchronisation
     phase_s = time.perf_counter() - t1
     h2d, _ = ctx.transfer_bytes
-    times, work = sharding.reduce_measurements({"train_phase_s": phase_s, "selfplay_s": sp_s, "selfplay_gpu_ms": float(stats.gpu_ms)},
+    if score:
+        scores["after"] = _score(ctx, 0, rows - fresh, fresh)
+        if gate:
+            scores["snapshot"] = _score(ctx, 1, rows - fresh, fresh)
+    score_times = {f"score_{k}_s": s for k, (_, s) in scores.items()}
+    score_work = {f"score_{k}_{t}": float(x) * fresh for k, (m, _) in scores.items() for t, x in zip(SCORE_TERMS, m)}
+    if scores:
+        score_work["score_rows"] = fresh
+    times, work = sharding.reduce_measurements({"train_phase_s": phase_s, "selfplay_s": sp_s, "selfplay_gpu_ms": float(stats.gpu_ms),
+                                                **score_times},
                                                {"sims": int(stats.simulations), "positions": int(stats.positions),
-                                                "rows": rows, "episodes": episodes},
+                                                "rows": rows, "episodes": episodes, **score_work},
                                                device="cuda" if dist else "cpu")
     out = {"config": "AlphaZero iteration (BASELINE configs[4]), device replay memory", "n_gpus": world, "games_per_gpu": games,
            "plies": plies, "sims_per_move": count, "selfplay_sims_per_s": work["sims"] / times["selfplay_s"],
@@ -226,6 +261,12 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
            "train_steps": steps, "global_minibatch": per_rank * world, "train_step": "omk_train_replay (C ABI, fp32 CUDA kernels)",
            "train_phase_s": times["train_phase_s"], "train_step_ms": times["train_phase_s"] * 1e3 / steps,
            "first_loss": float(losses[0, 2]), "last_loss": float(losses[-1, 2]), "h2d_bytes_total": h2d}
+    if scores:  # means over every rank's rows; the wall time of the slowest rank's call
+        n_scored = work["score_rows"]
+        out["score_rows"] = n_scored
+        for k in scores:
+            out[f"score_{k}"] = {t: work[f"score_{k}_{t}"] / n_scored if n_scored else float("nan") for t in SCORE_TERMS}
+            out[f"score_{k}_s"] = times[f"score_{k}_s"]
     if evaluate:
         out.update(_evaluate(ctx, evaluate, 2 * games, count, batch, seed))
     if gate:
@@ -254,7 +295,10 @@ if __name__ == "__main__":
                     help="after training, play EPISODES games against the naive player on the device (omk_eval_naive)")
     ap.add_argument("--gate", type=int, default=0, metavar="GAMES",
                     help="after training, play GAMES games of the trained network against its pre-training snapshot (omk_match)")
+    ap.add_argument("--score", action="store_true",
+                    help="with --device-replay: the loss terms of the network on this phase's new replay rows before and after "
+                         "training (and of the snapshot with --gate), one omk_replay_score call each")
     a = ap.parse_args()
     run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
         device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate,
-        gate=a.gate)
+        gate=a.gate, score=a.score)
