@@ -108,9 +108,9 @@ OMK_API int32_t omk_net_eval_images(omk_ctx *ctx, const float *images, int32_t n
  * Replaces AgentModel::train (alpha-zero/src/agent_model.rs:136-168) and the training half of AgentModel::new's graph
  * (:26-103; network.rs:249-253): loss = mean((z - v)^2) + mean(softmax_cross_entropy_with_logits(logits, pi)),
  * tensorflow AdadeltaOptimizer with learning rate 0.01 (:24), rho 0.95, epsilon 1e-8 (the crate's defaults; the two
- * accumulators live in the context and, as in the reference, are never saved), one minimize step, then a SECOND forward
- * that reports the losses.  images[n*243] = encode_nn_input's tensor, pi[n*81] = encode_nn_targets' policy target,
- * z[n] = its value target (alpha-zero/src/encoder.rs:10-68); out_losses[3] = {p_loss, v_loss, loss} after the update.
+ * accumulators live in the context; the reference never saves them, omk_train_get_optimizer reads them out), one
+ * minimize step, then a SECOND forward that reports the losses.  images[n*243] = encode_nn_input's tensor,
+ * pi[n*81] = encode_nn_targets' policy target, z[n] = its value target (alpha-zero/src/encoder.rs:10-68); out_losses[3] = {p_loss, v_loss, loss} after the update.
  * The updated weights serve every later evaluation (omk_net_eval, the searches, the self-play driver and its cached
  * root prior): the tensor-core operand images are rebuilt by the first entry point that evaluates the network after
  * the step, not by each of an iteration's 600 steps.  fp32 CUDA kernels; correctness path, not the self-play hot path. */
@@ -125,6 +125,14 @@ OMK_API int32_t omk_train_apply(omk_ctx *ctx, float *out_losses);
 /* host copy of the last gradient, per tensor in checkpoint order (tests); zero the Adadelta accumulators */
 OMK_API int32_t omk_train_get_grads(omk_ctx *ctx, float *const *tensors, const int64_t *lens);
 OMK_API int32_t omk_train_reset_optimizer(omk_ctx *ctx);
+/* The Adadelta accumulators, per tensor in checkpoint order (lens as omk_net_get_params).  A context that has not
+ * stepped reports zeros, which is the state its first step starts from.  With omk_net_get_params and the replay rows they
+ * are what a run has to save to resume exactly (DESIGN.md 2).                                                          */
+OMK_API int32_t omk_train_get_optimizer(omk_ctx *ctx, float *const *accum, float *const *accum_update, const int64_t *lens);
+/* Replace them (allocating the optimizer state if it does not exist yet); the next step reads them.  Every entry must be
+ * finite and >= 0 (OMK_ERR_INVALID otherwise, and nothing changes).                                                    */
+OMK_API int32_t omk_train_set_optimizer(omk_ctx *ctx, const float *const *accum, const float *const *accum_update,
+                                        const int64_t *lens);
 /* Optional NCCL communicator for the gradient all-reduce (one rank per context / GPU; NVLink 5 / NVSwitch on a B200
  * box).  libnccl.so.2 is loaded with dlopen on first use (env OMK_NCCL_LIB overrides the name): rank 0 calls
  * omk_train_comm_unique_id and distributes the 128 bytes, every rank calls omk_train_comm_init; from then on
@@ -295,6 +303,15 @@ OMK_API int32_t omk_replay_info(omk_ctx *ctx, int64_t *out_len, int64_t *out_row
 /* rows[n] = logical indices (OMK_ERR_INVALID outside [0, len)); boards[n*81], turns[n], policy[n*81], z[n] (any may be NULL) */
 OMK_API int32_t omk_replay_get(omk_ctx *ctx, const int64_t *rows, int32_t n, uint8_t *out_boards, uint8_t *out_turns,
                        float *out_policy, float *out_z);
+/* Append n rows (in order, oldest first) at the newest end of the replay memory, e.g. rows omk_replay_get read out of an
+ * earlier run.  Beyond the capacity the oldest rows are dropped, as after an episode; if n > capacity, only the call's last
+ * `capacity` rows are kept.  rows_added grows by n and the episode count by `episodes` (>= 0); so after omk_replay_reset
+ * and one append, rows_added counts from the restore and equals len.  Rows use omk_replay_get's layout, z stored bit for
+ * bit (-0.0 stays -0.0).  Validation is all or nothing: cells in {0,1,2}, turn in {0,1}, policy and z finite; otherwise
+ * OMK_ERR_INVALID and the memory is unchanged.  OMK_ERR_STATE if there is no replay memory.  Allowed while a self-play
+ * driver is active: its next commits land after the appended rows.  Host-to-device copies only, no kernel.            */
+OMK_API int32_t omk_replay_append(omk_ctx *ctx, const uint8_t *boards, const uint8_t *turns, const float *policy,
+                                  const float *z, int32_t n, int64_t episodes);
 /* `steps` gradient steps, each omk_train_step's sequence (forward, loss, backward, all-reduce of an attached communicator,
  * Adadelta, reporting forward) on a minibatch of m = min(n, len) rows drawn from the replay memory and encoded as
  * encode_nn_input(board, turn) in Player mode.  Step s draws its rows with Floyd's sample without replacement on the

@@ -109,6 +109,8 @@ def load_library():
     L.omk_train_apply.argtypes = [vp, vp]
     L.omk_train_get_grads.argtypes = [vp, P(vp), P(i64)]
     L.omk_train_reset_optimizer.argtypes = [vp]
+    L.omk_train_get_optimizer.argtypes = [vp, P(vp), P(vp), P(i64)]
+    L.omk_train_set_optimizer.argtypes = [vp, P(vp), P(vp), P(i64)]
     L.omk_train_comm_unique_id.argtypes = [vp, vp]
     L.omk_train_comm_init.argtypes = [vp, vp, i32, i32]
     L.omk_train_comm_destroy.argtypes = [vp]
@@ -143,6 +145,7 @@ def load_library():
     L.omk_replay_reset.argtypes = [vp, i64]
     L.omk_replay_info.argtypes = [vp, P(i64), P(i64), P(i64)]
     L.omk_replay_get.argtypes = [vp, vp, i32, vp, vp, vp, vp]
+    L.omk_replay_append.argtypes = [vp, vp, vp, vp, vp, i32, i64]
     L.omk_train_replay.argtypes = [vp, u64, i64, i32, i32, vp, vp]
     L.omk_replay_score.argtypes = [vp, i32, vp, i64, i32, vp, vp, vp, vp]
     L.omk_naive_move.argtypes = [vp, vp, vp, i32, u64, vp, vp, vp]
@@ -184,6 +187,7 @@ class Context:
         self.h = h
         self.capacity_envs, self.capacity_trees, self.capacity_nodes = capacity_envs, capacity_trees, capacity_nodes
         self.seed = seed
+        self.replay_capacity = 0  # rows of the device replay memory (replay_reset)
 
     def _check(self, rc: int):
         if rc != 0:
@@ -289,6 +293,30 @@ class Context:
 
     def train_reset_optimizer(self):
         self._check(self.L.omk_train_reset_optimizer(self.h))
+
+    def train_get_optimizer(self):
+        """The Adadelta accumulators (accum, accum_update): two lists of 31 arrays shaped as the tensors (zeros before the
+        first step)."""
+        accum = [np.zeros(n, dtype=np.float32) for n in NET_LENS]
+        update = [np.zeros(n, dtype=np.float32) for n in NET_LENS]
+        pa = (C.c_void_p * 31)(*[a.ctypes.data for a in accum])
+        pu = (C.c_void_p * 31)(*[a.ctypes.data for a in update])
+        lens = (C.c_int64 * 31)(*NET_LENS)
+        self._check(self.L.omk_train_get_optimizer(self.h, pa, pu, lens))
+        return [a.reshape(s) for a, s in zip(accum, NET_SHAPES)], [a.reshape(s) for a, s in zip(update, NET_SHAPES)]
+
+    def train_set_optimizer(self, accum, accum_update):
+        """Replace the Adadelta accumulators (every entry finite and >= 0); the next step reads them."""
+        a = [np.ascontiguousarray(x, dtype=np.float32).reshape(-1) for x in accum]
+        u = [np.ascontiguousarray(x, dtype=np.float32).reshape(-1) for x in accum_update]
+        if len(a) != 31 or len(u) != 31:
+            raise ValueError("need 31 tensors per accumulator")
+        pa = (C.c_void_p * 31)(*[x.ctypes.data for x in a])
+        pu = (C.c_void_p * 31)(*[x.ctypes.data for x in u])
+        lens = (C.c_int64 * 31)(*[x.size for x in a])
+        if [x.size for x in u] != list(lens):
+            raise ValueError("accum and accum_update differ in shape")
+        self._check(self.L.omk_train_set_optimizer(self.h, pa, pu, lens))
 
     def train_comm_unique_id(self) -> bytes:
         buf = np.zeros(128, dtype=np.uint8)
@@ -484,6 +512,7 @@ class Context:
         """Empty the device replay memory and size it to `capacity` rows (0 frees it).  Create it before
         `selfplay_begin`: the driver feeds the replay memory that exists when it starts."""
         self._check(self.L.omk_replay_reset(self.h, int(capacity)))
+        self.replay_capacity = int(capacity)
 
     def replay_info(self):
         """(rows held, rows added since the last reset, episodes added since the last reset)."""
@@ -501,6 +530,16 @@ class Context:
         z = np.zeros(n, dtype=np.float32)
         self._check(self.L.omk_replay_get(self.h, _ptr(rows), n, _ptr(boards), _ptr(turns), _ptr(policy), _ptr(z)))
         return boards, turns, policy, z
+
+    def replay_append(self, boards, turns, policy, z, episodes: int = 0):
+        """Append rows in replay_get's layout (oldest first) at the newest end of the device replay memory; the oldest rows
+        drop beyond the capacity.  rows_added grows by the row count and the episode count by `episodes`."""
+        boards = np.ascontiguousarray(boards, dtype=np.uint8).reshape(-1, CELLS)
+        n = boards.shape[0]
+        turns = np.ascontiguousarray(turns, dtype=np.uint8).reshape(n)
+        policy = np.ascontiguousarray(policy, dtype=np.float32).reshape(n, CELLS)
+        z = np.ascontiguousarray(z, dtype=np.float32).reshape(n)
+        self._check(self.L.omk_replay_append(self.h, _ptr(boards), _ptr(turns), _ptr(policy), _ptr(z), n, int(episodes)))
 
     def train_replay(self, seed: int, first_step: int, steps: int, n: int, want_rows: bool = False):
         """`steps` trainer steps on minibatches of min(n, len) rows sampled from the device replay memory (step s on

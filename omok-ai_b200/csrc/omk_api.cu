@@ -565,6 +565,63 @@ extern "C" int32_t omk_train_reset_optimizer(omk_ctx *c) {
     return OMK_OK;
 }
 
+// the Adadelta slots as 31 host tensors per slot <-> the flat device arrays (tensor i at the sum of kLens[0 .. i))
+static int32_t check_slot_tensors(const void *const *accum, const void *const *accum_update, const int64_t *lens) {
+    if (!accum || !accum_update || !lens) return fail(OMK_ERR_INVALID, "bad arguments");
+    for (int i = 0; i < kNetTensors; ++i)
+        if (!accum[i] || !accum_update[i] || lens[i] != kLens[i])
+            return fail(OMK_ERR_INVALID, "tensor " + std::to_string(i) + ": expected " + std::to_string(kLens[i]) + " elements");
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_train_get_optimizer(omk_ctx *c, float *const *accum, float *const *accum_update, const int64_t *lens) {
+    CK(cudaSetDevice(c->device));
+    int32_t rc = check_slot_tensors((const void *const *)accum, (const void *const *)accum_update, lens);
+    if (rc) return rc;
+    float *da = nullptr, *du = nullptr;
+    if (const char *e = train_optimizer_slots(c, false, &da, &du)) return fail(OMK_ERR_CUDA, std::string("omk_train_get_optimizer: ") + e);
+    long long off = 0;
+    for (int i = 0; i < kNetTensors; ++i) {
+        const size_t bytes = sizeof(float) * (size_t)kLens[i];
+        if (da) {
+            CK(copy_d2h(c, accum[i], da + off, bytes, c->stream));
+            CK(copy_d2h(c, accum_update[i], du + off, bytes, c->stream));
+        } else {  // no step yet: the zeros the first step starts from
+            memset(accum[i], 0, bytes);
+            memset(accum_update[i], 0, bytes);
+        }
+        off += kLens[i];
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    return OMK_OK;
+}
+
+extern "C" int32_t omk_train_set_optimizer(omk_ctx *c, const float *const *accum, const float *const *accum_update,
+                                           const int64_t *lens) {
+    CK(cudaSetDevice(c->device));
+    int32_t rc = check_slot_tensors((const void *const *)accum, (const void *const *)accum_update, lens);
+    if (rc) return rc;
+    // all or nothing: every entry is checked before the first byte is copied
+    for (int i = 0; i < kNetTensors; ++i)
+        for (const float *src : {accum[i], accum_update[i]})
+            for (long long j = 0; j < kLens[i]; ++j)
+                if (!std::isfinite(src[j]) || src[j] < 0.0f)
+                    return fail(OMK_ERR_INVALID, "tensor " + std::to_string(i) + " entry " + std::to_string(j) + ": " +
+                                                     std::to_string(src[j]) + " (Adadelta accumulators are finite and >= 0)");
+    float *da = nullptr, *du = nullptr;
+    if (const char *e = train_optimizer_slots(c, true, &da, &du)) return fail(OMK_ERR_CUDA, std::string("omk_train_set_optimizer: ") + e);
+    long long off = 0;
+    for (int i = 0; i < kNetTensors; ++i) {
+        const size_t bytes = sizeof(float) * (size_t)kLens[i];
+        CK(copy_h2d(c, da + off, accum[i], bytes, c->stream));
+        CK(copy_h2d(c, du + off, accum_update[i], bytes, c->stream));
+        off += kLens[i];
+    }
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    return OMK_OK;
+}
+
 extern "C" int32_t omk_train_comm_unique_id(omk_ctx *c, uint8_t *out_id) {
     if (!out_id) return fail(OMK_ERR_INVALID, "out_id is NULL");
     if (const char *e = train_comm_unique_id(c, out_id)) return fail(OMK_ERR_STATE, std::string("NCCL: ") + e);
@@ -1399,6 +1456,59 @@ extern "C" int32_t omk_replay_get(omk_ctx *c, const int64_t *rows, int32_t n, ui
     if (out_z) CK(copy_d2h(c, out_z, d_pz + nn * kCells, sizeof(float) * nn, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     CK(cudaGetLastError());
+    return OMK_OK;
+}
+
+// Host rows at the newest end of the ring: validated whole first (input from outside the program), then copied straight
+// into the ring's arrays, at most two segments per array.  The device counters advance with the host copies: the driver's
+// next commit reads them to place its episodes after these rows.
+extern "C" int32_t omk_replay_append(omk_ctx *c, const uint8_t *boards, const uint8_t *turns, const float *policy, const float *z,
+                                     int32_t n, int64_t episodes) {
+    CK(cudaSetDevice(c->device));
+    if (n < 0 || episodes < 0) return fail(OMK_ERR_INVALID, "need n >= 0 and episodes >= 0");
+    if (n > 0 && (!boards || !turns || !policy || !z)) return fail(OMK_ERR_INVALID, "boards, turns, policy and z are required");
+    Replay &r = c->rp;
+    if (r.ring.cap == 0) return fail(OMK_ERR_STATE, "no replay memory (omk_replay_reset)");
+    const size_t nn = (size_t)n;
+    auto bad_row = [&](size_t row, const std::string &what) {
+        return fail(OMK_ERR_INVALID, "row " + std::to_string(row) + ": " + what + "; nothing was appended");
+    };
+    for (size_t e = 0; e < nn * kCells; ++e)
+        if (boards[e] > 2) return bad_row(e / kCells, "cell value " + std::to_string(boards[e]) + " outside {0, 1, 2}");
+    for (size_t i = 0; i < nn; ++i)
+        if (turns[i] > 1) return bad_row(i, "turn " + std::to_string(turns[i]) + " outside {0, 1}");
+    for (size_t e = 0; e < nn * kCells; ++e)
+        if (!std::isfinite(policy[e])) return bad_row(e / kCells, "non-finite policy entry");
+    for (size_t i = 0; i < nn; ++i)
+        if (!std::isfinite(z[i])) return bad_row(i, "non-finite z");
+    if (r.stream) CK(cudaStreamSynchronize(r.stream));  // behind the last commit
+    ReplayCounters ctr{};
+    CK(copy_d2h(c, &ctr, r.counters, sizeof ctr, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    // only the call's last `cap` rows survive it; they go to absolute rows added + skip .., i.e. ring slots phys0 .. (mod cap)
+    const long long cap = r.ring.cap, skip = n > cap ? n - cap : 0, m = n - skip;
+    const long long phys0 = (ctr.added + skip) % cap, seg0 = m < cap - phys0 ? m : cap - phys0;
+    auto put = [&](long long src, long long dst, long long rows) -> int32_t {
+        if (rows <= 0) return OMK_OK;
+        const size_t k = (size_t)rows;
+        CK(copy_h2d(c, r.ring.boards + (size_t)dst * kCells, boards + (size_t)src * kCells, k * kCells, c->stream));
+        CK(copy_h2d(c, r.ring.turns + (size_t)dst, turns + (size_t)src, k, c->stream));
+        CK(copy_h2d(c, r.ring.pi + (size_t)dst * kCells, policy + (size_t)src * kCells, sizeof(float) * k * kCells, c->stream));
+        CK(copy_h2d(c, r.ring.z + (size_t)dst, z + (size_t)src, sizeof(float) * k, c->stream));
+        return OMK_OK;
+    };
+    int32_t rc = put(skip, phys0, seg0);
+    if (rc == OMK_OK) rc = put(skip + seg0, 0, m - seg0);
+    if (rc) return rc;
+    ctr.added += n;
+    ctr.len = ctr.len + n < cap ? ctr.len + n : cap;
+    ctr.episodes += episodes;
+    CK(copy_h2d(c, r.counters, &ctr, sizeof ctr, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    CK(cudaGetLastError());
+    r.added = ctr.added;
+    r.len = ctr.len;
+    r.episodes = ctr.episodes;
     return OMK_OK;
 }
 

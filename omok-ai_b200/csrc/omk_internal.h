@@ -399,6 +399,9 @@ void launch_loss_rows(omk_ctx *c, const float *logits, int lstride, const float 
 void launch_score_reduce(omk_ctx *c, const float *row_loss, const uint8_t *top1, long long n, float *p_out, float *v_out,
                          double *block_sums, double *means4);
 void train_reset_optimizer(omk_ctx *c);
+// the Adadelta slots, flat [5 643 250] in checkpoint order (omk_train_get_optimizer / omk_train_set_optimizer); both nullptr
+// while the optimizer state does not exist, unless `create`: then it is allocated as before a first step (zeroed slots)
+const char *train_optimizer_slots(omk_ctx *c, bool create, float **accum, float **accum_update);
 const char *train_comm_unique_id(omk_ctx *c, uint8_t *out128);
 const char *train_comm_init(omk_ctx *c, const uint8_t *id128, int nranks, int rank);
 const char *train_comm_destroy(omk_ctx *c);

@@ -761,6 +761,19 @@ void train_reset_optimizer(omk_ctx *c) {
     }
     t->steps = 0;
 }
+const char *train_optimizer_slots(omk_ctx *c, bool create, float **accum, float **accum_update) {
+    *accum = *accum_update = nullptr;
+    if (!c->train_state && !create) return nullptr;
+    TrainState *t = train_state(c);
+    if (!t->grads && create) {
+        if (!train_ensure(c, t, 0)) return "optimizer state allocation failed";
+        // no gradient yet: omk_train_get_grads reads zeros rather than uninitialised memory
+        if (cudaMemsetAsync(t->grads, 0, t->grads.bytes(), c->stream) != cudaSuccess) return "optimizer state initialisation failed";
+    }
+    *accum = t->accum;
+    *accum_update = t->accum_update;
+    return nullptr;
+}
 
 // ---- NCCL through dlopen ----
 static const char *nccl_load(TrainState *t) {

@@ -75,6 +75,8 @@ extern "C" {
     pub fn omk_train_apply(ctx: *mut omk_ctx, out_losses: *mut f32) -> i32;
     pub fn omk_train_get_grads(ctx: *mut omk_ctx, tensors: *const *mut f32, lens: *const i64) -> i32;
     pub fn omk_train_reset_optimizer(ctx: *mut omk_ctx) -> i32;
+    pub fn omk_train_get_optimizer(ctx: *mut omk_ctx, accum: *const *mut f32, accum_update: *const *mut f32, lens: *const i64) -> i32;
+    pub fn omk_train_set_optimizer(ctx: *mut omk_ctx, accum: *const *const f32, accum_update: *const *const f32, lens: *const i64) -> i32;
     pub fn omk_train_comm_unique_id(ctx: *mut omk_ctx, out_id: *mut u8) -> i32;
     pub fn omk_train_comm_init(ctx: *mut omk_ctx, id: *const u8, nranks: i32, rank: i32) -> i32;
     pub fn omk_train_comm_destroy(ctx: *mut omk_ctx) -> i32;
@@ -115,6 +117,7 @@ extern "C" {
     pub fn omk_replay_reset(ctx: *mut omk_ctx, capacity: i64) -> i32;
     pub fn omk_replay_info(ctx: *mut omk_ctx, out_len: *mut i64, out_rows_added: *mut i64, out_episodes: *mut i64) -> i32;
     pub fn omk_replay_get(ctx: *mut omk_ctx, rows: *const i64, n: i32, out_boards: *mut u8, out_turns: *mut u8, out_policy: *mut f32, out_z: *mut f32) -> i32;
+    pub fn omk_replay_append(ctx: *mut omk_ctx, boards: *const u8, turns: *const u8, policy: *const f32, z: *const f32, n: i32, episodes: i64) -> i32;
     pub fn omk_train_replay(ctx: *mut omk_ctx, seed: u64, first_step: i64, steps: i32, n: i32, out_losses: *mut f32, out_rows: *mut i64) -> i32;
     pub fn omk_replay_score(ctx: *mut omk_ctx, slot: i32, rows: *const i64, first: i64, n: i32, out_means: *mut c_void, out_row_p_loss: *mut f32, out_row_v_loss: *mut f32, out_row_top1: *mut u8) -> i32;
     // evaluation against the naive player (src/trainer.rs:487-603)

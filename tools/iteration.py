@@ -21,7 +21,13 @@ With --device-replay --score the rows this phase's self-play committed, which no
 set: the network's loss terms on them (policy cross-entropy, value MSE, their sum, and top-1 agreement of the policy with
 the visit distribution) are measured by ONE omk_replay_score call before the training phase and one after it, and with
 --gate also for the snapshot; no game is played.  Under torchrun every rank scores its own memory and the means are
-combined weighted by rows."""
+combined weighted by rows.
+With --device-replay --state PATH the run is resumable across processes: if PATH exists, the weights, the Adadelta
+accumulators and the replay memory are loaded from it (run_state.load) instead of a random initialisation, the context gets
+the saved seed and the trainer's sampler streams continue at the saved step; after the training phase (and the evaluation
+and the gating match, if they run) the state is saved to PATH again.  Running the command K times continues one run over K
+processes.  Under torchrun every rank keeps its own file, PATH.rank{r}, and a file written with another world size is
+refused.  It reports state_load_s and state_save_s."""
 from __future__ import annotations
 
 import argparse
@@ -41,8 +47,9 @@ N_PARAMS = 5_643_250
 
 
 def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
-        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0, score=False):
+        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0, score=False, state=None):
     omk = importlib.import_module("omok-ai_b200")
+    run_state = importlib.import_module("omok-ai_b200.run_state")
     trainer = importlib.import_module("omok-ai_b200.trainer")
     sharding = importlib.import_module("omok-ai_b200.sharding")
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
@@ -59,11 +66,26 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         raise ValueError("--score reads the device replay memory: it needs --device-replay")
     if gate and gate < 2:
         raise ValueError("--gate GAMES needs at least 2 games: one opened by each side")
+    if state and not device_replay:
+        raise ValueError("--state saves the device replay memory: it needs --device-replay")
+    state_path = (f"{state}.rank{rank}" if world > 1 else state) if state else None
+    resume = None
+    if state_path and os.path.exists(state_path):
+        resume = run_state.read_meta(state_path)
+        if resume["world"] != world:
+            raise ValueError(f"{state_path} was written by a run of {resume['world']} ranks, this one has {world}")
     my_games = games_per_gpu
     ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games + evaluate + 4 * (gate // 2),
                       capacity_nodes=4096,
-                      seed=sharding.rank_seed(seed, rank))
-    ctx.net_init_random(seed)                       # identical weights on every rank
+                      seed=resume["seed"] if resume else sharding.rank_seed(seed, rank))
+    load_s = None
+    if resume:                                      # weights, accumulators and replay memory of the last iteration
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        run_state.load(ctx, state_path, world=world, rank=rank)
+        load_s = time.perf_counter() - t0
+    else:
+        ctx.net_init_random(seed)                   # identical weights on every rank
     if torch_step:
         step = trainer.TrainStep(ctx.net_get_params(), device=f"cuda:{local}")
     else:
@@ -75,10 +97,13 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
             dist.broadcast(t, src=0)
             uid = bytes(t.cpu().numpy().tobytes())
         step = trainer.AbiTrainStep(ctx, world=world, rank=rank, unique_id=uid)
+        if resume:
+            step.steps = resume["step"]             # the sampler streams continue where the saved run stopped
     if device_replay:
-        ctx.replay_reset(replay_capacity)           # before selfplay_begin: the driver feeds the replay that exists then
+        if not resume:
+            ctx.replay_reset(replay_capacity)       # before selfplay_begin: the driver feeds the replay that exists then
         return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
-                                  seed, quiet, replay_capacity, evaluate, gate, score)
+                                  seed, quiet, evaluate, gate, score, state_path, resume, load_s)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -210,9 +235,11 @@ def _score(ctx, slot, first, n):
     return means, time.perf_counter() - t0
 
 
-def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet, capacity,
-                       evaluate=0, gate=0, score=False):
+def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet,
+                       evaluate=0, gate=0, score=False, state_path=None, resume=None, load_s=None):
     omk = importlib.import_module("omok-ai_b200")
+    run_state = importlib.import_module("omok-ai_b200.run_state")
+    rows_at_start = ctx.replay_info()[0]
     ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
     ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
     if dist:
@@ -229,7 +256,7 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
     if score:
         scores["before"] = _score(ctx, 0, rows - fresh, fresh)
     per_rank = max(1, minibatch // world)
-    sampler_seed = sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
+    sampler_seed = resume["sampler_seed"] if resume else sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
     if gate:
         ctx.opponent_from_net()                     # the snapshot the trained network has to beat
     step.train_replay(2, per_rank, sampler_seed)   # warm-up: training workspace, split-K scratch
@@ -257,7 +284,7 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
            "plies": plies, "sims_per_move": count, "selfplay_sims_per_s": work["sims"] / times["selfplay_s"],
            "selfplay_positions_per_s": work["positions"] / times["selfplay_s"], "selfplay_wall_s": times["selfplay_s"],
            "selfplay_gpu_ms": times["selfplay_gpu_ms"], "transitions_streamed_to_host": False,
-           "replay_capacity_per_gpu": capacity, "replay_rows": work["rows"], "replay_episodes": work["episodes"],
+           "replay_capacity_per_gpu": ctx.replay_capacity, "replay_rows": work["rows"], "replay_episodes": work["episodes"],
            "train_steps": steps, "global_minibatch": per_rank * world, "train_step": "omk_train_replay (C ABI, fp32 CUDA kernels)",
            "train_phase_s": times["train_phase_s"], "train_step_ms": times["train_phase_s"] * 1e3 / steps,
            "first_loss": float(losses[0, 2]), "last_loss": float(losses[-1, 2]), "h2d_bytes_total": h2d}
@@ -271,6 +298,16 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
         out.update(_evaluate(ctx, evaluate, 2 * games, count, batch, seed))
     if gate:
         out.update(_gate(ctx, gate, 2 * games + evaluate))
+    if state_path:
+        iteration = resume["iteration"] + 1 if resume else 1
+        t0 = time.perf_counter()
+        run_state.save(ctx, state_path, seed=ctx.seed, sampler_seed=sampler_seed, step=step.steps, iteration=iteration, world=world,
+                       rank=rank)
+        save_s = time.perf_counter() - t0
+        st, sw = sharding.reduce_measurements({"state_load_s": load_s or 0.0, "state_save_s": save_s}, {"rows_at_start": rows_at_start},
+                                              device="cuda" if dist else "cpu")
+        out.update({"iteration": iteration, "replay_rows_at_start": sw["rows_at_start"],
+                    "state_load_s": st["state_load_s"] if resume else None, "state_save_s": st["state_save_s"]})
     if rank == 0 and not quiet:
         print(json.dumps(out), flush=True)
     ctx.close()
@@ -298,7 +335,10 @@ if __name__ == "__main__":
     ap.add_argument("--score", action="store_true",
                     help="with --device-replay: the loss terms of the network on this phase's new replay rows before and after "
                          "training (and of the snapshot with --gate), one omk_replay_score call each")
+    ap.add_argument("--state", metavar="PATH",
+                    help="with --device-replay: resume from PATH if it exists (weights, Adadelta accumulators, replay memory) and "
+                         "save there after the iteration (PATH.rank{r} per rank under torchrun)")
     a = ap.parse_args()
     run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
         device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate,
-        gate=a.gate, score=a.score)
+        gate=a.gate, score=a.score, state=a.state)
