@@ -282,6 +282,22 @@ OMK_API int32_t omk_selfplay_begin(omk_ctx *ctx, const omk_selfplay_config *cfg)
  * be NULL) in (ply, game) order: boards[plies*n*81], policy[plies*n*81], status[plies*n] */
 OMK_API int32_t omk_selfplay_run(omk_ctx *ctx, int32_t plies, int32_t profile, uint8_t *out_boards, float *out_policy,
                          int8_t *out_status, int32_t *out_actions, omk_selfplay_stats *stats);
+/* The model slot (0 .. 15, see omk_model_load_params; default 0, the network) whose weights the self-play driver evaluates
+ * with: omk_selfplay_begin's root evaluation of all 2n trees, the search rounds of both lanes, the ensure_action_exists
+ * evaluation of the other colour's trees and the cached empty-board prior that restarted games install.  A context setting
+ * like omk_search_set_virtual_loss: it survives omk_selfplay_begin, and it may change while a driver is active, taking
+ * effect at the driver's next evaluation.  A driver on slot s with weights W produces exactly the transitions, replay
+ * rows, statistics and random streams of a driver on slot 0 with weights W.
+ * The cached restart prior follows slot s only: it is re-evaluated when slot s changes (omk_model_load_params,
+ * omk_model_from_net, omk_opponent_load_params / omk_opponent_from_net for s = 1; omk_net_load_params, omk_net_init_random
+ * and the re-pack after training for s = 0) and, inside this call, when it switches an active driver to another slot (if
+ * that evaluation fails, the call returns its error and the driver stays on its old slot).  A
+ * change to any other slot -- training the network while s != 0 included -- leaves the driver's games untouched; with
+ * s != 0 omk_selfplay_run does not re-pack a trained network, whatever evaluates slot 0 next does.
+ * OMK_ERR_INVALID: slot outside 0 .. 15.  OMK_ERR_STATE: an active driver with OMK_EVAL_NET and an unloaded slot (nothing
+ * changes).  omk_selfplay_begin and omk_selfplay_run refuse an unloaded selected slot with OMK_ERR_STATE (e.g. after a
+ * load that failed halfway); OMK_EVAL_HASH never reads the slot.                                                         */
+OMK_API int32_t omk_selfplay_set_model(omk_ctx *ctx, int32_t slot);
 
 /* ---------------------------------------------------------------- replay memory
  * The trainer's replay memory (src/trainer.rs:27,206-352) kept on the device and fed by the self-play driver, so that
@@ -364,8 +380,9 @@ OMK_API int32_t omk_eval_naive(omk_ctx *ctx, int32_t episodes, int32_t first_tre
                                int8_t *out_status, int64_t *out_stats, float *out_gpu_ms);
 
 /* ---------------------------------------------------------------- the opponent network and the arena
- * The opponent network: a second set of weights in the context, read only by omk_opponent_eval and omk_match.  Training,
- * self-play, the searches and omk_net_* never read or change it; loading it changes nothing they produce.             */
+ * The opponent network: a second set of weights in the context (model slot 1), read by omk_opponent_eval, omk_match and
+ * a self-play driver set to slot 1 (omk_selfplay_set_model).  Training, the searches and omk_net_* never read or change
+ * it; loading it changes nothing they produce, nor what a driver on another slot produces.                             */
 OMK_API int32_t omk_opponent_load_params(omk_ctx *ctx, const float *const *tensors, const int64_t *lens); /* as omk_net_load_params */
 /* device-to-device copy of the network's current fp32 weights (e.g. before a training phase), images rebuilt from them;
  * OMK_ERR_STATE if no network is loaded */
@@ -388,12 +405,15 @@ OMK_API int32_t omk_match(omk_ctx *ctx, int32_t pairs, int32_t first_tree, int32
 
 /* ---------------------------------------------------------------- model slots and the tournament
  * A context holds 16 weight sets ("model slots").  Slot 0 is the network, slot 1 the opponent (omk_opponent_* are the calls
- * below with slot 1); slots 2 .. 15 are further weight sets, read only by omk_model_eval and omk_tournament.  A slot's device
- * buffers (about 45 MB) are allocated on its first load.  Slot 0 is OMK_ERR_INVALID in omk_model_load_params and
- * omk_model_from_net: omk_net_load_params and the trainer own it. */
+ * below with slot 1); slots 2 .. 15 are further weight sets, read only by omk_model_eval, omk_tournament and a self-play
+ * driver set to them (omk_selfplay_set_model).  A slot's device buffers (about 45 MB) are allocated on its first load.
+ * Slot 0 is OMK_ERR_INVALID in omk_model_load_params and omk_model_from_net: omk_net_load_params and the trainer own it. */
 OMK_API int32_t omk_model_load_params(omk_ctx *ctx, int32_t slot, const float *const *tensors, const int64_t *lens); /* as omk_net_load_params */
 /* device-to-device copy of the network's current fp32 weights (a snapshot); OMK_ERR_STATE if no network is loaded */
 OMK_API int32_t omk_model_from_net(omk_ctx *ctx, int32_t slot);
+/* device-to-host copy of slot `slot`'s (0 .. 15) 31 fp32 tensors in checkpoint order, lens as omk_net_load_params; slot 0 is
+ * omk_net_get_params.  OMK_ERR_INVALID: slot out of range or a bad length; OMK_ERR_STATE: the slot is not loaded. */
+OMK_API int32_t omk_model_get_params(omk_ctx *ctx, int32_t slot, float *const *tensors, const int64_t *lens);
 OMK_API int32_t omk_model_eval(omk_ctx *ctx, int32_t slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
                                float *out_p, float *out_v); /* omk_net_eval with slot `slot`'s weights; slot 0 == omk_net_eval */
 /* A round-robin of omk_match over n_models (2 .. 16) distinct slots[]: P = n(n-1)/2 pairings (i, j), i < j, in lexicographic

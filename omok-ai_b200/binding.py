@@ -142,6 +142,7 @@ def load_library():
     L.omk_pool_tree_info.argtypes = [vp, i32, vp, vp]
     L.omk_selfplay_begin.argtypes = [vp, P(SelfPlayConfig)]
     L.omk_selfplay_run.argtypes = [vp, i32, i32, vp, vp, vp, vp, P(SelfPlayStats)]
+    L.omk_selfplay_set_model.argtypes = [vp, i32]
     L.omk_replay_reset.argtypes = [vp, i64]
     L.omk_replay_info.argtypes = [vp, P(i64), P(i64), P(i64)]
     L.omk_replay_get.argtypes = [vp, vp, i32, vp, vp, vp, vp]
@@ -156,6 +157,7 @@ def load_library():
     L.omk_match.argtypes = [vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
     L.omk_model_load_params.argtypes = [vp, i32, P(vp), P(i64)]
     L.omk_model_from_net.argtypes = [vp, i32]
+    L.omk_model_get_params.argtypes = [vp, i32, P(vp), P(i64)]
     L.omk_model_eval.argtypes = [vp, i32, vp, vp, i32, i32, vp, vp]
     L.omk_tournament.argtypes = [vp, i32, vp, i32, i32, i32, i32, f32, f32, i32, vp, vp, vp, vp, P(f32)]
     L.omk_tournament_naive.argtypes = [vp, i32, vp, i32, i32, i32, i32, f32, f32, i32, u64, vp, vp, vp, vp, P(f32)]
@@ -507,6 +509,11 @@ class Context:
                                             _ptr(actions), C.byref(stats)))
         return stats, boards, policy, status, actions
 
+    def selfplay_set_model(self, slot: int):
+        """The model slot (0 .. 15, default 0 = the network) the self-play driver evaluates with; it survives selfplay_begin
+        and takes effect at an active driver's next evaluation (the restarted games' cached prior is re-evaluated here)."""
+        self._check(self.L.omk_selfplay_set_model(self.h, slot))
+
     # ---- replay memory on the device ----
     def replay_reset(self, capacity: int):
         """Empty the device replay memory and size it to `capacity` rows (0 frees it).  Create it before
@@ -603,7 +610,8 @@ class Context:
 
     # ---- the opponent network and the arena ----
     def opponent_load_params(self, params):
-        """A second set of weights, read only by opponent_eval and match (training, self-play and the searches never see it)."""
+        """A second set of weights (model slot 1), read by opponent_eval, match and a self-play driver set to slot 1
+        (selfplay_set_model); training and the searches never see it."""
         arrs = [np.ascontiguousarray(p, dtype=np.float32).reshape(-1) for p in params]
         ptrs = (C.c_void_p * 31)(*[a.ctypes.data for a in arrs])
         lens = (C.c_int64 * 31)(*[a.size for a in arrs])
@@ -643,7 +651,8 @@ class Context:
 
     # ---- model slots and the tournament ----
     def model_load_params(self, slot: int, params):
-        """Weights into model slot `slot` (1 .. 15; 1 is the opponent), read only by model_eval, match (slot 1) and tournament."""
+        """Weights into model slot `slot` (1 .. 15; 1 is the opponent), read only by model_eval, match (slot 1), tournament and a
+        self-play driver set to the slot (selfplay_set_model)."""
         arrs = [np.ascontiguousarray(p, dtype=np.float32).reshape(-1) for p in params]
         ptrs = (C.c_void_p * 31)(*[a.ctypes.data for a in arrs])
         lens = (C.c_int64 * 31)(*[a.size for a in arrs])
@@ -652,6 +661,14 @@ class Context:
     def model_from_net(self, slot: int):
         """Model slot `slot` becomes a device-side copy of the network's current weights (a snapshot)."""
         self._check(self.L.omk_model_from_net(self.h, slot))
+
+    def model_get_params(self, slot: int):
+        """Model slot `slot`'s 31 fp32 tensors (0 .. 15; slot 0 == net_get_params), shaped as net_get_params."""
+        arrs = [np.zeros(n, dtype=np.float32) for n in NET_LENS]
+        ptrs = (C.c_void_p * 31)(*[a.ctypes.data for a in arrs])
+        lens = (C.c_int64 * 31)(*NET_LENS)
+        self._check(self.L.omk_model_get_params(self.h, slot, ptrs, lens))
+        return [a.reshape(s) for a, s in zip(arrs, NET_SHAPES)]
 
     def model_eval(self, slot: int, boards, turns, mode: int = 0, want_v: bool = True):
         """net_eval with model slot `slot`'s weights (slot 0 is the network)."""

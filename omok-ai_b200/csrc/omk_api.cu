@@ -267,12 +267,16 @@ static int32_t ensure_packed(omk_ctx *c) {
     return rc;
 }
 
-static int32_t check_evaluator(omk_ctx *c, int evaluator) {
+static std::string slot_name(int slot) {
+    return slot == 0 ? "network" : (slot == 1 ? "opponent" : "model slot " + std::to_string(slot));
+}
+// slot: the model the caller's network evaluations read; only slot 0 (the network) can have stale images to re-pack
+static int32_t check_evaluator(omk_ctx *c, int evaluator, int slot = 0) {
     if (evaluator != OMK_EVAL_NET && evaluator != OMK_EVAL_HASH) return fail(OMK_ERR_INVALID, "unknown evaluator");
     if (evaluator == OMK_EVAL_HASH && c->virtual_loss)
         return fail(OMK_ERR_STATE, "virtual loss is a non-reference search mode: it is refused with the parity evaluator (OMK_EVAL_HASH)");
-    if (evaluator == OMK_EVAL_NET && !c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
-    if (evaluator == OMK_EVAL_NET) return ensure_packed(c);
+    if (evaluator == OMK_EVAL_NET && !c->slot(slot).loaded) return fail(OMK_ERR_STATE, slot_name(slot) + " weights not loaded");
+    if (evaluator == OMK_EVAL_NET && slot == 0) return ensure_packed(c);
     return OMK_OK;
 }
 
@@ -394,7 +398,7 @@ extern "C" int32_t omk_ctx_transfer_bytes(omk_ctx *c, int64_t *out_h2d, int64_t 
 }
 
 // ------------------------------------------------------------------ network
-static int32_t sp_refresh_root_policy(omk_ctx *c);  // self-play driver: re-evaluate the cached empty-board prior
+static int32_t sp_refresh_root_policy(omk_ctx *c, int slot);  // self-play driver: re-evaluate the cached empty-board prior
 
 extern "C" int32_t omk_net_load_params(omk_ctx *c, const float *const *tensors, const int64_t *lens) {
     CK(cudaSetDevice(c->device));
@@ -409,17 +413,10 @@ extern "C" int32_t omk_net_load_params(omk_ctx *c, const float *const *tensors, 
     if (!tower16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split tower weight preparation failed");
     CK(cudaStreamSynchronize(c->stream));
     c->net.loaded = true;
-    return sp_refresh_root_policy(c);
+    return sp_refresh_root_policy(c, 0);
 }
 extern "C" int32_t omk_net_get_params(omk_ctx *c, float *const *tensors, const int64_t *lens) {
-    CK(cudaSetDevice(c->device));
-    if (!c->net.loaded) return fail(OMK_ERR_STATE, "network weights not loaded");
-    for (int i = 0; i < kNetTensors; ++i)
-        if (!tensors[i] || lens[i] != kLens[i]) return fail(OMK_ERR_INVALID, "bad tensor length");
-    for (int i = 0; i < kNetTensors; ++i)
-        CK(copy_d2h(c, tensors[i], c->net.t[i], sizeof(float) * (size_t)kLens[i], c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    return OMK_OK;
+    return omk_model_get_params(c, 0, tensors, lens);
 }
 extern "C" int32_t omk_net_init_random(omk_ctx *c, uint64_t seed) {
     CK(cudaSetDevice(c->device));
@@ -431,7 +428,7 @@ extern "C" int32_t omk_net_init_random(omk_ctx *c, uint64_t seed) {
     CK(cudaStreamSynchronize(c->stream));
     CK(cudaGetLastError());
     c->net.loaded = true;
-    return sp_refresh_root_policy(c);
+    return sp_refresh_root_policy(c, 0);
 }
 
 // slot: the model whose weights evaluate (omk_model_eval); only the network's (slot 0) are changed by training steps
@@ -452,9 +449,6 @@ static int32_t net_eval_common(omk_ctx *c, int n, const float *images_dev, float
     return check_device_error(c);  // OMK_ERR_NUMERIC when the network produced a non-finite output
 }
 
-static std::string slot_name(int slot) {
-    return slot == 0 ? "network" : (slot == 1 ? "opponent" : "model slot " + std::to_string(slot));
-}
 static int32_t eval_boards(omk_ctx *c, int slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,
                            float *out_p, float *out_v) {
     CK(cudaSetDevice(c->device));
@@ -499,7 +493,7 @@ static int32_t weights_changed(omk_ctx *c) {
     if (!fc16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split fc weight preparation failed");
     if (!tower16_prepare_weights(c)) return fail(OMK_ERR_CUDA, "fp16-split tower weight preparation failed");
     CK(cudaStreamSynchronize(c->stream));
-    return sp_refresh_root_policy(c);
+    return sp_refresh_root_policy(c, 0);
 }
 
 static int32_t train_backward_impl(omk_ctx *c, const float *images, const float *pi, const float *z, int32_t n,
@@ -1096,16 +1090,18 @@ static SpLayout sp_layout(uint8_t *base, int n) {
     return L;
 }
 // Restarted games install a cached raw prior of the empty board instead of evaluating it again (Agent::new, agent.rs:16-25,
-// evaluates with the CURRENT weights).  The cache therefore follows every weight change: omk_net_load_params and
-// omk_net_init_random call this while a self-play driver is active (trainer step -> sync weights -> next self-play phase).
-static int32_t sp_refresh_root_policy(omk_ctx *c) {
-    if (!c->sp_active || c->sp_cfg.evaluator != OMK_EVAL_NET) return OMK_OK;
+// evaluates with the CURRENT weights).  The cache therefore follows every change of the weights the driver reads: every call
+// that changes model slot `slot` calls this, and it re-evaluates only when `slot` is the driver's (omk_selfplay_set_model),
+// e.g. trainer step -> sync weights -> next self-play phase with the driver on the network.
+static int32_t sp_refresh_root_policy(omk_ctx *c, int slot) {
+    if (!c->sp_active || c->sp_cfg.evaluator != OMK_EVAL_NET || slot != c->sp_model) return OMK_OK;
     int32_t rc = ensure_workspace(c, 1);
     if (rc) return rc;
     const SpLayout L = sp_layout(c->sp_buf, c->sp_cfg.n_games);
     const uint32_t one = 1;
     CK(cudaMemsetAsync(c->ws.nn_in, 0, sizeof(NNIn), c->stream));  // empty board, Black to move, EnvTurnMode::Player (== k_new_games' request)
     CK(copy_h2d(c, c->ws.n_req, &one, sizeof one, c->stream));
+    ModelScope scope(c, slot);
     if (!net_forward(c, nullptr, 1)) return fail(OMK_ERR_CUDA, "re-evaluating the empty board after a weight change failed");
     CK(cudaMemcpyAsync(L.root_policy, c->ws.P, sizeof(float) * kCells, cudaMemcpyDeviceToDevice, c->stream));
     launch_reset_requests(c);
@@ -1117,7 +1113,7 @@ extern "C" int32_t omk_selfplay_begin(omk_ctx *c, const omk_selfplay_config *cfg
     if (!cfg) return fail(OMK_ERR_INVALID, "cfg is NULL");
     if (cfg->n_games < 1 || 2 * cfg->n_games > c->cap_trees) return fail(OMK_ERR_INVALID, "need capacity_trees >= 2*n_games");
     if (cfg->batch_size < 1 || cfg->batch_size > kMaxBatchPerTree || cfg->count < 1) return fail(OMK_ERR_INVALID, "bad count/batch_size");
-    int32_t rc = check_evaluator(c, cfg->evaluator);
+    int32_t rc = check_evaluator(c, cfg->evaluator, c->sp_model);
     if (rc) return rc;
     const int n = cfg->n_games;
     const int rows = n * cfg->batch_size > 2 * n ? n * cfg->batch_size : 2 * n;
@@ -1185,7 +1181,10 @@ extern "C" int32_t omk_selfplay_begin(omk_ctx *c, const omk_selfplay_config *cfg
     // evaluating the empty board is deterministic, so reusing it is bit-identical to evaluating it again
     launch_reset_requests(c);
     launch_new_games(c, nullptr, 2 * n, nullptr, nullptr, nullptr);
-    RUN_EVAL(c, cfg->evaluator, 2 * n);
+    {
+        ModelScope model(c, c->sp_model);
+        RUN_EVAL(c, cfg->evaluator, 2 * n);
+    }
     launch_apply(c, nullptr, 2 * n, kApplyNewGame);
     CK(cudaMemcpyAsync(M.root_policy, c->tree_nodes + kOffPolicy, sizeof(float) * kCells, cudaMemcpyDeviceToDevice, c->stream));
     c->sp_active = true;
@@ -1197,10 +1196,14 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     CK(cudaSetDevice(c->device));
     if (!c->sp_active) return fail(OMK_ERR_STATE, "omk_selfplay_begin has not been called");
     if (plies < 0) return fail(OMK_ERR_INVALID, "plies < 0");
-    if (c->sp_cfg.evaluator == OMK_EVAL_NET) {  // weights updated by the trainer since the last evaluation: operand images + the cached root prior
-        int32_t rc_p = ensure_packed(c);
-        if (rc_p) return rc_p;
+    if (c->sp_cfg.evaluator == OMK_EVAL_NET) {
+        if (!c->slot(c->sp_model).loaded) return fail(OMK_ERR_STATE, slot_name(c->sp_model) + " weights not loaded (the self-play driver's model)");
+        if (c->sp_model == 0) {  // weights updated by the trainer since the last evaluation: operand images + the cached root prior
+            int32_t rc_p = ensure_packed(c);
+            if (rc_p) return rc_p;
+        }
     }
+    ModelScope model(c, c->sp_model);  // every evaluation of both lanes below
     const omk_selfplay_config &cfg = c->sp_cfg;
     const int n = cfg.n_games;
     const int rounds = (cfg.count + cfg.batch_size - 1) / cfg.batch_size;
@@ -1380,6 +1383,23 @@ extern "C" int32_t omk_selfplay_run(omk_ctx *c, int32_t plies, int32_t profile, 
     }
     c->prof_spans.clear();
     c->prof_level = 0;
+    return rc;
+}
+
+extern "C" int32_t omk_selfplay_set_model(omk_ctx *c, int32_t slot) {
+    CK(cudaSetDevice(c->device));
+    if (slot < 0 || slot >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
+    const bool net_driver = c->sp_active && c->sp_cfg.evaluator == OMK_EVAL_NET;
+    if (net_driver && !c->slot(slot).loaded)
+        return fail(OMK_ERR_STATE, slot_name(slot) + " weights not loaded: the active self-play driver keeps its model");
+    const int old = c->sp_model;
+    if (slot == old) return OMK_OK;
+    c->sp_model = slot;
+    if (!net_driver) return OMK_OK;
+    // the restarted games' cached prior follows the switch; a network changed by training is re-packed first (which
+    // refreshes the prior itself).  If that fails, the driver keeps its old slot, whose prior the cache still holds.
+    const int32_t rc = slot == 0 && c->net_pack_dirty ? ensure_packed(c) : sp_refresh_root_policy(c, slot);
+    if (rc != OMK_OK) c->sp_model = old;
     return rc;
 }
 
@@ -1779,7 +1799,21 @@ extern "C" int32_t omk_model_load_params(omk_ctx *c, int32_t slot, const float *
     m.loaded = false;  // until the images below are built
     for (int i = 0; i < kNetTensors; ++i)
         CK(copy_h2d(c, m.t[i], tensors[i], sizeof(float) * (size_t)kLens[i], c->stream));
-    return model_prepare(c, slot);
+    rc = model_prepare(c, slot);
+    return rc ? rc : sp_refresh_root_policy(c, slot);
+}
+
+extern "C" int32_t omk_model_get_params(omk_ctx *c, int32_t slot, float *const *tensors, const int64_t *lens) {
+    CK(cudaSetDevice(c->device));
+    if (slot < 0 || slot >= kModelSlots) return fail(OMK_ERR_INVALID, "model slot out of range [0, " + std::to_string(kModelSlots - 1) + "]");
+    const NetWeights &m = c->slot(slot);
+    if (!m.loaded) return fail(OMK_ERR_STATE, slot_name(slot) + " weights not loaded");
+    for (int i = 0; i < kNetTensors; ++i)
+        if (!tensors[i] || lens[i] != kLens[i]) return fail(OMK_ERR_INVALID, "bad tensor length");
+    for (int i = 0; i < kNetTensors; ++i)
+        CK(copy_d2h(c, tensors[i], m.t[i], sizeof(float) * (size_t)kLens[i], c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return OMK_OK;
 }
 
 extern "C" int32_t omk_model_from_net(omk_ctx *c, int32_t slot) {
@@ -1793,7 +1827,8 @@ extern "C" int32_t omk_model_from_net(omk_ctx *c, int32_t slot) {
     m.loaded = false;
     for (int i = 0; i < kNetTensors; ++i)
         CK(cudaMemcpyAsync(m.t[i], c->net.t[i], sizeof(float) * (size_t)kLens[i], cudaMemcpyDeviceToDevice, c->stream));
-    return model_prepare(c, slot);
+    rc = model_prepare(c, slot);
+    return rc ? rc : sp_refresh_root_policy(c, slot);
 }
 
 extern "C" int32_t omk_model_eval(omk_ctx *c, int32_t slot, const uint8_t *boards, const uint8_t *turns, int32_t n, int32_t mode,

@@ -252,6 +252,7 @@ struct omk_ctx {
     // self-play driver state
     omk_selfplay_config sp_cfg{};
     bool sp_active = false;
+    int sp_model = 0;                 // the model slot the driver evaluates with (omk_selfplay_set_model); survives omk_selfplay_begin
     omk::Buf<int32_t> sp_ply;         // [n_games] device ply counters
     omk::Buf<uint8_t> sp_buf;         // per-game scratch (ids, actions, modes, status, cached root policy)
     // Transition ring of the self-play driver (BASELINE config 4: positions streamed to the host replay buffer): kSpRing

@@ -7,6 +7,11 @@ game.  To resume, recreate the context with the saved `seed`, call `load`, and c
 saved `step` (`AbiTrainStep.steps = step`).  A run that is resumed then produces the replay rows, losses, weights and
 accumulators of a run that was never stopped but restarted its driver at the same boundary, bit for bit (DESIGN.md 2).
 
+A gated run (tools/iteration.py --gated) also keeps its best network, the weights of a model slot other than the network,
+as `best_00 .. best_30`; a file without them is a run that has none.  `read_meta` and `load` report a best network as the
+metadata key `best` (True), present only when the file holds one, so that a file without one yields exactly the metadata
+it always did: test it with `meta.get("best", False)`.
+
 The reference's checkpoint (model_io.py) still holds the weights only.
 """
 from __future__ import annotations
@@ -30,8 +35,10 @@ def _key(kind: str, i: int) -> str:
     return f"{kind}_{i:02d}"
 
 
-def save(ctx, path, *, seed: int, sampler_seed: int, step: int, iteration: int, world: int, rank: int) -> None:
-    """Write the state of `ctx` with the run's metadata to `path` (the file is replaced only once it is complete)."""
+def save(ctx, path, *, seed: int, sampler_seed: int, step: int, iteration: int, world: int, rank: int,
+         best_slot: int | None = None) -> None:
+    """Write the state of `ctx` with the run's metadata to `path` (the file is replaced only once it is complete).  With
+    `best_slot`, that model slot's weights are saved too, as the run's best network."""
     meta = dict(seed=seed, sampler_seed=sampler_seed, step=step, iteration=iteration, world=world, rank=rank)
     for k, v in meta.items():
         if not 0 <= int(v) < 2**64:
@@ -41,6 +48,8 @@ def save(ctx, path, *, seed: int, sampler_seed: int, step: int, iteration: int, 
     accum, accum_update = ctx.train_get_optimizer()
     for i, (p, a, u) in enumerate(zip(ctx.net_get_params(), accum, accum_update)):
         arrays[_key("param", i)], arrays[_key("accum", i)], arrays[_key("accum_update", i)] = p, a, u
+    if best_slot is not None:
+        arrays.update({_key("best", i): p for i, p in enumerate(ctx.model_get_params(best_slot))})
     n, _, episodes = ctx.replay_info()
     boards = np.empty((n, CELLS), np.uint8)
     turns = np.empty(n, np.uint8)
@@ -70,7 +79,8 @@ def _expect(f, key: str, shape, dtype) -> np.ndarray:
 
 
 def read_meta(path) -> dict:
-    """The metadata of a run state file ({seed, sampler_seed, step, iteration, world, rank}), after its version check."""
+    """The metadata of a run state file ({seed, sampler_seed, step, iteration, world, rank}, and best = True if it holds a
+    best network), after its version check."""
     with np.load(path, allow_pickle=False) as f:
         return _meta(f)
 
@@ -79,13 +89,21 @@ def _meta(f) -> dict:
     version = int(_expect(f, "version", (), np.int64))
     if version != FORMAT_VERSION:
         raise RunStateError(f"run state format {version}; this version reads format {FORMAT_VERSION}")
-    return {k: int(_expect(f, k, (), np.uint64)) for k in META}
+    meta = {k: int(_expect(f, k, (), np.uint64)) for k in META}
+    if _has_best(f):
+        meta["best"] = True
+    return meta
 
 
-def load(ctx, path, *, world: int | None = None, rank: int | None = None) -> dict:
-    """Restore the state in `path` into `ctx`: net_load_params, train_set_optimizer, replay_reset(capacity), replay_append.
-    Every array is checked before the context is touched.  With `world` / `rank` given, a file written by another world size
-    or rank is refused.  Returns the metadata."""
+def _has_best(f) -> bool:
+    return any(k.startswith("best_") for k in f.files)
+
+
+def load(ctx, path, *, world: int | None = None, rank: int | None = None, best_slot: int | None = None) -> dict:
+    """Restore the state in `path` into `ctx`: net_load_params, the best network with model_load_params(best_slot) if the
+    file holds one and `best_slot` is given, train_set_optimizer, replay_reset(capacity), replay_append.  Every array is
+    checked before the context is touched: a best network must be complete.  With `world` / `rank` given, a file written by
+    another world size or rank is refused.  Returns the metadata, with best = True if the file holds a best network."""
     with np.load(path, allow_pickle=False) as f:
         meta = _meta(f)
         for k, want in (("world", world), ("rank", rank)):
@@ -93,6 +111,7 @@ def load(ctx, path, *, world: int | None = None, rank: int | None = None) -> dic
                 raise RunStateError(f"run state written with {k} {meta[k]}, this run has {k} {want}")
         params, accum, accum_update = ([_expect(f, _key(kind, i), s, np.float32) for i, s in enumerate(NET_SHAPES)]
                                        for kind in ("param", "accum", "accum_update"))
+        best = [_expect(f, _key("best", i), s, np.float32) for i, s in enumerate(NET_SHAPES)] if _has_best(f) else None
         capacity = int(_expect(f, "replay_capacity", (), np.int64))
         episodes = int(_expect(f, "replay_episodes", (), np.int64))
         z = f["replay_z"] if "replay_z" in f.files else None
@@ -104,6 +123,8 @@ def load(ctx, path, *, world: int | None = None, rank: int | None = None) -> dic
         policy = _expect(f, "replay_policy", (n, CELLS), np.float32)
         z = _expect(f, "replay_z", (n,), np.float32)
     ctx.net_load_params(params)
+    if best is not None and best_slot is not None:
+        ctx.model_load_params(best_slot, best)
     ctx.train_set_optimizer(accum, accum_update)
     ctx.replay_reset(capacity)
     if n or episodes:

@@ -20,6 +20,17 @@ def rank_seed(base_seed: int, rank: int) -> int:
     return (base_seed + 0x9E3779B97F4A7C15 * (rank + 1)) & 0xFFFFFFFFFFFFFFFF
 
 
+def iteration_seed(seed: int, iteration: int) -> int:
+    """The context seed of iteration `iteration` of a run whose previous iteration's context had `seed` (splitmix64's
+    finaliser of seed ^ iteration * K: for a given iteration, distinct seeds stay distinct, so the ranks keep distinct
+    streams)."""
+    m = 0xFFFFFFFFFFFFFFFF
+    z = (seed ^ (0xD1B54A32D192ED03 * iteration)) & m
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & m
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & m
+    return z ^ (z >> 31)
+
+
 def reduce_measurements(times: dict[str, float], work: dict[str, int], device: str = "cpu"):
     """max-over-ranks of every time, sum-over-ranks of every work counter (an int counter stays an int, a float one -- e.g. a
     mean weighted by its rows -- a float).  No-op without a process group."""

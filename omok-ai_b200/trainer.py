@@ -287,3 +287,18 @@ class AbiTrainStep:
     def sync_to(self, ctx) -> None:
         if ctx is not self.ctx:
             ctx.net_load_params(self.numpy_params())
+
+
+# ---------------------------------------------------------------------------------------------- gating (AlphaGo Zero)
+def gate_decision(results, threshold: float = 0.55) -> tuple[float, bool]:
+    """The gating match's verdict: `results` holds one (candidate wins, best wins, draws) triple per rank (or one triple
+    already summed over the ranks).  score = (candidate wins + draws / 2) / games over all of them; the candidate replaces
+    the best network when score >= threshold (AlphaGo Zero: 0.55).  Returns (score, promote)."""
+    wins = losses = draws = 0
+    for w, l, d in results:
+        wins, losses, draws = wins + int(w), losses + int(l), draws + int(d)
+    games = wins + losses + draws
+    if games < 1:
+        raise ValueError("the gating match played no game")
+    score = (wins + 0.5 * draws) / games
+    return score, bool(score >= threshold)

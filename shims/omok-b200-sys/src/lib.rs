@@ -113,6 +113,7 @@ extern "C" {
     // device-resident self-play driver (src/trainer.rs:86-204)
     pub fn omk_selfplay_begin(ctx: *mut omk_ctx, cfg: *const omk_selfplay_config) -> i32;
     pub fn omk_selfplay_run(ctx: *mut omk_ctx, plies: i32, profile: i32, out_boards: *mut u8, out_policy: *mut f32, out_status: *mut i8, out_actions: *mut i32, stats: *mut omk_selfplay_stats) -> i32;
+    pub fn omk_selfplay_set_model(ctx: *mut omk_ctx, slot: i32) -> i32;
     // device replay memory (src/trainer.rs:27,206-352) and the training phase on it
     pub fn omk_replay_reset(ctx: *mut omk_ctx, capacity: i64) -> i32;
     pub fn omk_replay_info(ctx: *mut omk_ctx, out_len: *mut i64, out_rows_added: *mut i64, out_episodes: *mut i64) -> i32;
@@ -131,6 +132,7 @@ extern "C" {
     // model slots and the tournament (a round-robin of the arena)
     pub fn omk_model_load_params(ctx: *mut omk_ctx, slot: i32, tensors: *const *const f32, lens: *const i64) -> i32;
     pub fn omk_model_from_net(ctx: *mut omk_ctx, slot: i32) -> i32;
+    pub fn omk_model_get_params(ctx: *mut omk_ctx, slot: i32, tensors: *const *mut f32, lens: *const i64) -> i32;
     pub fn omk_model_eval(ctx: *mut omk_ctx, slot: i32, boards: *const u8, turns: *const u8, n: i32, mode: i32, out_p: *mut f32, out_v: *mut f32) -> i32;
     pub fn omk_tournament(ctx: *mut omk_ctx, n_models: i32, slots: *const i32, pairs: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;
     pub fn omk_tournament_naive(ctx: *mut omk_ctx, n_models: i32, slots: *const i32, pairs: i32, first_tree: i32, count: i32, batch_size: i32, epsilon: f32, alpha: f32, evaluator: i32, seed: u64, out_result: *mut i32, out_moves: *mut i8, out_status: *mut i8, out_stats: *mut i64, out_gpu_ms: *mut f32) -> i32;

@@ -27,7 +27,17 @@ accumulators and the replay memory are loaded from it (run_state.load) instead o
 the saved seed and the trainer's sampler streams continue at the saved step; after the training phase (and the evaluation
 and the gating match, if they run) the state is saved to PATH again.  Running the command K times continues one run over K
 processes.  Under torchrun every rank keeps its own file, PATH.rank{r}, and a file written with another world size is
-refused.  It reports state_load_s and state_save_s."""
+refused.  It reports state_load_s and state_save_s.
+With --device-replay --gate GAMES --gated the run acts on the gating answer, as AlphaGo Zero does: the context's opponent
+(model slot 1) holds the BEST network, self-play reads it (omk_selfplay_set_model(1)) and the network (slot 0) is the
+candidate the trainer keeps changing.  A fresh run starts with best = the initial network; with --state the best is saved
+and resumed with the rest, and a state file without one is refused.  No snapshot is taken before training: the gating match
+is the candidate against the best, and if the candidate's score (wins + draws / 2) / games over all ranks reaches
+--promote-at (default 0.55) every rank copies it into slot 1, so the next self-play phase plays the new best.  A resumed
+gated run does not reuse the saved context seed: it derives the next one from it and the iteration
+(sharding.iteration_seed), because a kept best network with the same random streams would replay the previous process's
+games and append them to the replay memory again.  It reports gate_score and promoted, the gating match's wins as
+gate_trained_wins / gate_best_wins, and --score labels slot 1's terms "best"."""
 from __future__ import annotations
 
 import argparse
@@ -47,7 +57,7 @@ N_PARAMS = 5_643_250
 
 
 def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=128, seed=0, quiet=False, gather=False, torch_step=False,
-        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0, score=False, state=None):
+        device_replay=False, replay_capacity=600_000, evaluate=0, gate=0, score=False, state=None, gated=False, promote_at=0.55):
     omk = importlib.import_module("omok-ai_b200")
     run_state = importlib.import_module("omok-ai_b200.run_state")
     trainer = importlib.import_module("omok-ai_b200.trainer")
@@ -68,24 +78,32 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         raise ValueError("--gate GAMES needs at least 2 games: one opened by each side")
     if state and not device_replay:
         raise ValueError("--state saves the device replay memory: it needs --device-replay")
+    if gated and not (device_replay and gate):
+        raise ValueError("--gated acts on the gating match of the device-replay run: it needs --device-replay and --gate GAMES")
     state_path = (f"{state}.rank{rank}" if world > 1 else state) if state else None
     resume = None
     if state_path and os.path.exists(state_path):
         resume = run_state.read_meta(state_path)
         if resume["world"] != world:
             raise ValueError(f"{state_path} was written by a run of {resume['world']} ranks, this one has {world}")
+        if gated and not resume.get("best"):
+            raise ValueError(f"{state_path} holds no best network: it was not written by a --gated run")
     my_games = games_per_gpu
+    ctx_seed = resume["seed"] if resume else sharding.rank_seed(seed, rank)
+    if resume and gated:                            # fresh self-play streams: the best network may be the one that played last time
+        ctx_seed = sharding.iteration_seed(ctx_seed, resume["iteration"] + 1)
     ctx = omk.Context(device=local, capacity_envs=4, capacity_trees=2 * my_games + evaluate + 4 * (gate // 2),
-                      capacity_nodes=4096,
-                      seed=resume["seed"] if resume else sharding.rank_seed(seed, rank))
+                      capacity_nodes=4096, seed=ctx_seed)
     load_s = None
     if resume:                                      # weights, accumulators and replay memory of the last iteration
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        run_state.load(ctx, state_path, world=world, rank=rank)
+        run_state.load(ctx, state_path, world=world, rank=rank, best_slot=1 if gated else None)
         load_s = time.perf_counter() - t0
     else:
         ctx.net_init_random(seed)                   # identical weights on every rank
+        if gated:
+            ctx.opponent_from_net()                 # the best network so far: the initial one
     if torch_step:
         step = trainer.TrainStep(ctx.net_get_params(), device=f"cuda:{local}")
     else:
@@ -103,7 +121,7 @@ def run(games_per_gpu=1024, plies=12, count=800, batch=16, steps=20, minibatch=1
         if not resume:
             ctx.replay_reset(replay_capacity)       # before selfplay_begin: the driver feeds the replay that exists then
         return _run_device_replay(ctx, step, sharding, dist, rank, world, games_per_gpu, plies, count, batch, steps, minibatch,
-                                  seed, quiet, evaluate, gate, score, state_path, resume, load_s)
+                                  seed, quiet, evaluate, gate, score, state_path, resume, load_s, gated, promote_at)
     mem = trainer.ReplayMemory(capacity=600_000, seed=seed + rank)
 
     # ---- self-play phase: per-GPU game pools, transitions streamed to the host (pinned ring inside the library) ----
@@ -209,15 +227,15 @@ def _evaluate(ctx, episodes, first_tree, count, batch, seed):
             "eval_draws": draw, "eval_moves": stats["moves"], "eval_host_syncs": stats["host_syncs"], "eval_gpu_ms": stats["gpu_ms"]}
 
 
-def _gate(ctx, games, first_tree):
-    """The gating match: the trained network against the snapshot taken before training, one omk_match call at the
-    benchmark's constants."""
+def _gate(ctx, games, first_tree, opponent="snapshot"):
+    """The gating match: the trained network against the opponent (the snapshot taken before training, or the best network
+    of a gated run), one omk_match call at the benchmark's constants."""
     omk = importlib.import_module("omok-ai_b200")
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     (net, snap, draw), _, _, stats = ctx.match(games // 2, first_tree=first_tree, count=800, batch_size=8, epsilon=0.0, alpha=1.0,
                                                evaluator=omk.EVAL_NET)
-    return {"gate_games": 2 * (games // 2), "gate_phase_s": time.perf_counter() - t0, "gate_trained_wins": net, "gate_snapshot_wins": snap,
+    return {"gate_games": 2 * (games // 2), "gate_phase_s": time.perf_counter() - t0, "gate_trained_wins": net, f"gate_{opponent}_wins": snap,
             "gate_draws": draw, "gate_moves": stats["moves"], "gate_host_syncs": stats["host_syncs"], "gate_gpu_ms": stats["gpu_ms"]}
 
 
@@ -236,10 +254,13 @@ def _score(ctx, slot, first, n):
 
 
 def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, count, batch, steps, minibatch, seed, quiet,
-                       evaluate=0, gate=0, score=False, state_path=None, resume=None, load_s=None):
+                       evaluate=0, gate=0, score=False, state_path=None, resume=None, load_s=None, gated=False, promote_at=0.55):
     omk = importlib.import_module("omok-ai_b200")
     run_state = importlib.import_module("omok-ai_b200.run_state")
+    trainer = importlib.import_module("omok-ai_b200.trainer")
     rows_at_start = ctx.replay_info()[0]
+    if gated:
+        ctx.selfplay_set_model(1)                   # the best network (slot 1) generates the self-play data
     ctx.selfplay_begin(games, count, batch, 0.25, 0.03, 1.0, 30, omk.EVAL_NET)
     ctx.selfplay_run(2, profile=0, want_transitions=False)        # warm-up: allocations, lane set-up
     if dist:
@@ -257,7 +278,7 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
         scores["before"] = _score(ctx, 0, rows - fresh, fresh)
     per_rank = max(1, minibatch // world)
     sampler_seed = resume["sampler_seed"] if resume else sharding.rank_seed(seed, rank)   # every rank samples its own replay memory
-    if gate:
+    if gate and not gated:
         ctx.opponent_from_net()                     # the snapshot the trained network has to beat
     step.train_replay(2, per_rank, sampler_seed)   # warm-up: training workspace, split-K scratch
     torch.cuda.synchronize()
@@ -270,7 +291,7 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
     if score:
         scores["after"] = _score(ctx, 0, rows - fresh, fresh)
         if gate:
-            scores["snapshot"] = _score(ctx, 1, rows - fresh, fresh)
+            scores["best" if gated else "snapshot"] = _score(ctx, 1, rows - fresh, fresh)
     score_times = {f"score_{k}_s": s for k, (_, s) in scores.items()}
     score_work = {f"score_{k}_{t}": float(x) * fresh for k, (m, _) in scores.items() for t, x in zip(SCORE_TERMS, m)}
     if scores:
@@ -297,12 +318,22 @@ def _run_device_replay(ctx, step, sharding, dist, rank, world, games, plies, cou
     if evaluate:
         out.update(_evaluate(ctx, evaluate, 2 * games, count, batch, seed))
     if gate:
-        out.update(_gate(ctx, gate, 2 * games + evaluate))
+        g = _gate(ctx, gate, 2 * games + evaluate, "best" if gated else "snapshot")
+        out.update(g)
+        if gated:  # every rank decides on the same sums, so the best stays identical across ranks
+            _, summed = sharding.reduce_measurements({"gate_phase_s": g["gate_phase_s"]},
+                                                     {k: g[k] for k in ("gate_trained_wins", "gate_best_wins", "gate_draws")},
+                                                     device="cuda" if dist else "cpu")
+            gate_score, promoted = trainer.gate_decision(
+                [(summed["gate_trained_wins"], summed["gate_best_wins"], summed["gate_draws"])], promote_at)
+            if promoted:
+                ctx.opponent_from_net()             # the candidate becomes the best; the driver's restart prior follows
+            out.update({"gate_score": gate_score, "promote_at": promote_at, "promoted": promoted})
     if state_path:
         iteration = resume["iteration"] + 1 if resume else 1
         t0 = time.perf_counter()
         run_state.save(ctx, state_path, seed=ctx.seed, sampler_seed=sampler_seed, step=step.steps, iteration=iteration, world=world,
-                       rank=rank)
+                       rank=rank, best_slot=1 if gated else None)
         save_s = time.perf_counter() - t0
         st, sw = sharding.reduce_measurements({"state_load_s": load_s or 0.0, "state_save_s": save_s}, {"rows_at_start": rows_at_start},
                                               device="cuda" if dist else "cpu")
@@ -338,7 +369,12 @@ if __name__ == "__main__":
     ap.add_argument("--state", metavar="PATH",
                     help="with --device-replay: resume from PATH if it exists (weights, Adadelta accumulators, replay memory) and "
                          "save there after the iteration (PATH.rank{r} per rank under torchrun)")
+    ap.add_argument("--gated", action="store_true",
+                    help="with --device-replay --gate GAMES: the best network (slot 1) plays self-play and is replaced by the "
+                         "trained one when its gating score reaches --promote-at")
+    ap.add_argument("--promote-at", type=float, default=0.55, metavar="X",
+                    help="with --gated: the candidate's score (wins + draws / 2) / games that promotes it (AlphaGo Zero: 0.55)")
     a = ap.parse_args()
     run(games_per_gpu=a.games_per_gpu, plies=a.plies, count=a.count, steps=a.steps, minibatch=a.minibatch, gather=a.gather, torch_step=a.torch_step,
         device_replay=a.device_replay, replay_capacity=a.replay_capacity, evaluate=a.evaluate,
-        gate=a.gate, score=a.score, state=a.state)
+        gate=a.gate, score=a.score, state=a.state, gated=a.gated, promote_at=a.promote_at)
